@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- panoramas/s of the render hot path on N B200s (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch B] [--dump-outputs DIR]
 
 Workload (N=1 and per rank for N>1): BASELINE.json configs[1] ("C2") -- synthetic SRTM1 tiles N32..N35 x
 W119..W116, viewer (34+1/7200, -117+1/7200), render_radius_m = 150 km (R = 5858 cells, 137 M vertices, 274 M
@@ -48,6 +48,29 @@ TILES_DIR = os.environ.get("HZ_BENCH_TILES", "/tmp/hz_tiles_c2")
 
 def algorithmic_bytes(R, W, H):
     return 2 * (2 * R) ** 2 + 7 * W * H          # SURVEY.md 8(d)
+
+
+DUMP_SAMPLE = 1 << 19           # pixels drawn from the whole step for the *_sample arrays of --dump-outputs
+
+
+def dump_outputs(directory, d_img, d_rng):
+    """--dump-outputs: what one batch call handed back (d_img (B, H, W, 3) uint8 B,G,R, d_rng (B, H, W) float32), as
+    .npy files that two builds can be compared by, 47 MB for the C2 workload:
+      image.npy (H, W, 3), ranges.npy (H, W)            the step's first panorama in full, float32
+      sample_index.npy (N,)                             flat indices into (B, H, W), seed 0, sorted, float64
+      image_sample.npy (N, 3), ranges_sample.npy (N,)   those pixels of every panorama of the step, float32"""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    B, H, W = d_rng.shape
+    n = B * H * W
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_SAMPLE, n), replace=False))
+    d_idx = torch.from_numpy(idx).to(d_rng.device)
+    out = {"image": d_img[0].float(), "ranges": d_rng[0],
+           "sample_index": torch.from_numpy(idx.astype(np.float64)),
+           "image_sample": d_img.view(n, 3)[d_idx].float(), "ranges_sample": d_rng.view(n)[d_idx]}
+    for name, t in out.items():
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
 
 
 def measured_peak_gbs():
@@ -341,6 +364,8 @@ def run_b200(args):
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     ms_total_max = max_over_ranks(ms_total)
     value = world * K * B / (ms_total_max / 1e3)
+    if args.dump_outputs and rank == 0:         # before the C5 grid below renders into the same buffers
+        dump_outputs(args.dump_outputs, d_img, d_rng)
 
     # ---- C5: distinct viewpoints of the 64x64 grid, this rank's disjoint block, in calls of B ----
     grid = [(la, lo, C2["az0"], C2["az1"]) for la, lo in c5_grid(world, rank)]
@@ -840,8 +865,13 @@ def main():
     ap.add_argument("--batch", type=int, default=256, help="panoramas per step (one call of the batch entry point)")
     ap.add_argument("--grid-views", type=int, default=0, help="viewpoints of the C5 grid per GPU (0 = its whole block)")
     ap.add_argument("--no-c4", action="store_true", help="skip the 36000x4000 wedge panorama (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's image and ranges (the first panorama in full and "
+                         "a seeded sample of all of them) as DIR/<name>.npy; rank 0 only")
     ap.add_argument("--llvmpipe-child", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.llvmpipe_child:
         return llvmpipe_child(args)
     if args.warmup < 3 and args.impl == "b200":
