@@ -119,6 +119,8 @@ def _declare(lib):
         "horizonator_host_free": (None, [vp]),
         "horizonator_profile_enable": (b, [ctx, b]),
         "horizonator_profile_read": (b, [ctx, P(f * 6), P(i)]),
+        "horizonator_viewshed_device": (b, [ctx, i, P(view_t), f, vp, vp, vp]),
+        "horizonator_viewshed": (b, [ctx, i, P(view_t), f, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         try:
@@ -148,6 +150,7 @@ EXPORTED_SYMBOLS = (
     "horizonator_render_wedge_peers", "horizonator_peer_barrier", "horizonator_reload_tunables",
     "horizonator_render_wedge_host", "horizonator_host_register", "horizonator_host_unregister",
     "horizonator_debug_device_math", "horizonator_set_lod",
+    "horizonator_viewshed_device", "horizonator_viewshed",
 )
 
 if not os.path.exists(LIBRARY_PATH):
@@ -437,6 +440,38 @@ class horizonator:
         if not lib.horizonator_horizon_profile_device(C.byref(self._ctx), d_ranges, int(n), d_rows, d_range,
                                                       stream or None):
             raise RuntimeError("horizonator_horizon_profile_device() failed")
+
+    # viewsheds (horizonator-batch.h: which vertices of the loaded square each view sees)
+    @property
+    def size(self):
+        """N = 2R: the loaded square is N x N vertices."""
+        return 2 * self._ctx.dems.radius_cells
+
+    @staticmethod
+    def _eyes(views):
+        """views: (lat, lon), or (lat, lon, az_deg0, az_deg1[, viewer_z]) as render_batch takes them (the azimuth
+        window is ignored: a viewshed covers the full circle)."""
+        return horizonator._views([tuple(v) + (0., 0.) if len(v) == 2 else v for v in views])
+
+    def viewshed(self, views, target_height=0., counts=False):
+        """Host arrays: masks (n, N, N) bool, [j north][i east], True where the view sees the vertex (a point
+        target_height metres above it); with counts=True also (N, N) uint32, how many of the views see each vertex."""
+        n, N = len(views), self.size
+        w32 = (N + 31) // 32
+        words = np.empty((n, N, w32), np.uint32)
+        cnt = np.zeros((N, N), np.uint32) if counts else None
+        if not lib.horizonator_viewshed(C.byref(self._ctx), n, self._eyes(views), float(target_height),
+                                        words.ctypes.data, cnt.ctypes.data if counts else None):
+            raise RuntimeError("horizonator_viewshed() failed")
+        bits = np.unpackbits(words.view(np.uint8), axis=-1, bitorder="little")[..., :N].astype(bool)
+        return (bits, cnt) if counts else bits
+
+    def viewshed_device(self, views, d_masks=0, d_counts=0, target_height=0., stream=0):
+        """Device-pointer variant: d_masks (n, N, (N+31)//32) uint32 words, overwritten; d_counts (N, N) uint32,
+        added to.  Integer device addresses, either may be 0 (not both); stream as render_batch_device."""
+        if not lib.horizonator_viewshed_device(C.byref(self._ctx), len(views), self._eyes(views), float(target_height),
+                                               d_masks or None, d_counts or None, stream or None):
+            raise RuntimeError("horizonator_viewshed_device() failed")
 
 
 class _PinnedBlock:

@@ -191,6 +191,14 @@ struct Slot
     bool collect_stats = false;      // culling counters (horizonator_render_counters); off: the kernels skip them
     std::vector<cudaEvent_t> prof_events;
     size_t prof_used = 0;
+
+    // viewsheds, allocated by the first viewshed call that needs them: the masks of one chunk of views for calls that
+    // want only counts or want the masks in host memory, and the counts of the host-memory call.  A call's stream
+    // waits for `vs_done` of the call before it, which may have been queued on another stream and use the same scratch.
+    uint32_t* d_vs_masks = nullptr;
+    int       vs_mask_views = 0;
+    uint32_t* d_vs_counts = nullptr;
+    cudaEvent_t vs_done = nullptr;
 };
 
 std::mutex          g_table_mutex;
@@ -432,6 +440,8 @@ void destroy_slot(Slot* s)
     for(int i = 0; i < 4; i++) for(int j = 0; j < 4; j++) cudaFree((void*)s->tiles.tile[i][j]);
     for(cudaEvent_t e : s->prof_events) cudaEventDestroy(e);
     cudaFree(s->d_mm_block); cudaFree(s->d_mm_tile);
+    if(s->vs_done) { cudaEventSynchronize(s->vs_done); cudaEventDestroy(s->vs_done); }
+    cudaFree(s->d_vs_masks); cudaFree(s->d_vs_counts);
     if(s->stream) cudaStreamDestroy(s->stream);
     delete s;
 }
@@ -1485,6 +1495,126 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         CUDA_TRY(cudaEventRecord(s->sets[g]->done, s->sets[g]->stream));
         CUDA_TRY(cudaStreamWaitEvent(st, s->sets[g]->done, 0));
     }
+    return true;
+}
+
+// ---- viewsheds (horizonator-batch.h) -------------------------------------------------------------------------------
+//
+// The views go in chunks of up to HZ_VS_MAX_VIEWS, each one k_viewshed launch (gridDim.y = view) into its masks --
+// the caller's, or the scratch when the masks are not wanted in device memory -- then k_viewshed_count into the
+// counts and/or a copy of the masks to host memory, all on `st`.
+static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
+                            float target_height, uint32_t* d_masks, uint32_t* d_counts, uint32_t* h_masks,
+                            cudaStream_t st)
+{
+    const int N = s->N, w32 = (N + 31) / 32;
+    const size_t mwords = (size_t)N * w32;
+    std::vector<HzViewshedEye> eyes((size_t)n);
+    for(int k = 0; k < n; k++)
+    {
+        ViewState vs;
+        float z = views[k].viewer_z;
+        if(!compute_move(ctx, &z, views[k].lat, views[k].lon, vs)) return false;
+        if(!(vs.viewer_cell_i >= 0.f && vs.viewer_cell_i < (float)(N - 1) &&
+             vs.viewer_cell_j >= 0.f && vs.viewer_cell_j < (float)(N - 1)))
+        {
+            MSG("viewshed: the eye of view %d (cell %g, %g) is not inside the loaded square [0, %d)", k,
+                (double)vs.viewer_cell_i, (double)vs.viewer_cell_j, N - 1);
+            return false;
+        }
+        eyes[k] = HzViewshedEye{ vs.viewer_cell_i, vs.viewer_cell_j, vs.viewer_z, vs.cos_viewer_lat };
+    }
+    if(n == 0) return true;
+
+    const int chunk = n < HZ_VS_MAX_VIEWS ? n : HZ_VS_MAX_VIEWS;
+    if(s->vs_done == nullptr) CUDA_TRY(cudaEventCreateWithFlags(&s->vs_done, cudaEventDisableTiming));
+    else CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done, 0));
+    if(d_masks == nullptr && s->vs_mask_views < chunk)
+    {
+        CUDA_TRY(cudaEventSynchronize(s->vs_done));
+        cudaFree(s->d_vs_masks);
+        s->d_vs_masks = nullptr; s->vs_mask_views = 0;
+        if(cudaMalloc(&s->d_vs_masks, (size_t)chunk * mwords * sizeof(uint32_t)) != cudaSuccess)
+        {
+            cudaGetLastError();
+            MSG("Could not allocate the viewshed masks of %d views (%zu MB)", chunk, (size_t)chunk * mwords * 4 >> 20);
+            return false;
+        }
+        s->vs_mask_views = chunk;
+    }
+
+    HzViewshed p{};
+    p.mosaic = s->d_mosaic; p.N = N; p.pitch = s->pitch; p.w32 = w32;
+    p.deg_per_cell = 1.0f / (float)s->cpd;                                // lib:577
+    p.curvature = s->curvature;
+    p.target_height = target_height;
+    for(int k0 = 0; k0 < n; k0 += chunk)
+    {
+        const int m = n - k0 < chunk ? n - k0 : chunk;
+        p.masks = d_masks ? d_masks + (size_t)k0 * mwords : s->d_vs_masks;
+        for(int k = 0; k < m; k++) p.eye[k] = eyes[(size_t)(k0 + k)];
+        CUDA_TRY(cudaMemsetAsync(p.masks, 0, (size_t)m * mwords * sizeof(uint32_t), st));
+        CUDA_TRY(hz_launch_viewshed(p, m, st));
+        if(d_counts) CUDA_TRY(hz_launch_viewshed_count(p.masks, m, N, w32, d_counts, st));
+        if(h_masks)
+            CUDA_TRY(cudaMemcpyAsync(h_masks + (size_t)k0 * mwords, p.masks, (size_t)m * mwords * sizeof(uint32_t),
+                                     cudaMemcpyDeviceToHost, st));
+    }
+    CUDA_TRY(cudaEventRecord(s->vs_done, st));
+    return true;
+}
+
+bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                 float target_height_m, void* d_masks, void* d_counts, void* stream)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
+    if(d_masks == nullptr && d_counts == nullptr)
+    {
+        MSG("horizonator_viewshed_device: neither masks nor counts asked for");
+        return false;
+    }
+    DeviceGuard g(s->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if(!viewshed_common(ctx, s, n, views, target_height_m, (uint32_t*)d_masks, (uint32_t*)d_counts, nullptr, st))
+        return false;
+    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
+    return true;
+}
+
+bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                          float target_height_m, uint32_t* masks, uint32_t* counts)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
+    if(masks == nullptr && counts == nullptr)
+    {
+        MSG("horizonator_viewshed: neither masks nor counts asked for");
+        return false;
+    }
+    DeviceGuard g(s->device);
+    const size_t cells = (size_t)s->N * s->N;
+    if(counts && n > 0 && s->d_vs_counts == nullptr)
+    {
+        if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done));
+        if(cudaMalloc(&s->d_vs_counts, cells * sizeof(uint32_t)) != cudaSuccess)
+        {
+            cudaGetLastError();
+            MSG("Could not allocate the viewshed counts (%zu MB)", cells * 4 >> 20);
+            return false;
+        }
+    }
+    // the counts' upload waits for whatever an earlier call still does with the same buffer
+    if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(s->stream, s->vs_done, 0));
+    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts, counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream));
+    if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts : nullptr, masks, s->stream))
+    {
+        cudaStreamSynchronize(s->stream);
+        cudaGetLastError();
+        return false;
+    }
+    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts, cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
     return true;
 }
 

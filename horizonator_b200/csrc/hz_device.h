@@ -187,5 +187,22 @@ cudaError_t hz_launch_big    (const HzView& v, const HzView* d_v, int nviews, cu
 cudaError_t hz_launch_resolve(const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);
 bool        hz_resolve_is_vectorisable(const HzView& v);
 cudaError_t hz_launch_horizon(const float* ranges, int n, int W, int H, int* rows, float* range, cudaStream_t stream);
+// ---- viewsheds (horizonator_viewshed*: the definition is in include/horizonator-batch.h) ------
+constexpr int HZ_VS_MAX_VIEWS = 64;     // views per k_viewshed launch (gridDim.y); their eyes travel in the parameters
+struct HzViewshedEye { float vci, vcj, vz, cos_lat; };     // compute_move()'s eye, float as there
+struct HzViewshed
+{
+    const int16_t* mosaic;       // [N + HZ_MESH_PAD][pitch]
+    int   N, pitch;
+    int   w32;                   // words per mask row, (N + 31) / 32
+    float deg_per_cell, curvature, target_height;
+    uint32_t* masks;             // view y's mask at masks + y * N * w32, zeroed before the launch
+    HzViewshedEye eye[HZ_VS_MAX_VIEWS];
+};
+cudaError_t hz_launch_viewshed(const HzViewshed& p, int nviews, cudaStream_t stream);
+// counts[j * N + i] += the number of the nviews masks (N * w32 words apart) with cell (i, j) set
+cudaError_t hz_launch_viewshed_count(const uint32_t* masks, int nviews, int N, int w32, uint32_t* counts,
+                                     cudaStream_t stream);
+
 cudaError_t hz_launch_math_probe(int n, const float* e, const float* nn, const float* h, const float* d2, float* az, float* el,
                                  cudaStream_t stream);

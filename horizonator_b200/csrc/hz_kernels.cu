@@ -18,6 +18,8 @@
 //   k_peer_barrier (multi-GPU)  barrier between the ranks of a wedge-sharded panorama through peer memory
 //   k_resolve4 / k_resolve1 (render)  keys -> BGR8 image + float range image, top row first   lib:936-1048
 //   k_horizon  (extra)   range image -> per-column topmost terrain row and its range
+//   k_viewshed, k_viewshed_count (viewsheds)  R2 ray casting over the DEM square, one thread per ray -> bit masks;
+//                        masks -> per-vertex counts of the views that see it
 //
 // The mesh is never materialised: triangle t of the reference's index buffer is (cell = t>>1, half = t&1)
 // and its vertices are read straight from the int16 mosaic.
@@ -1943,6 +1945,183 @@ cudaError_t hz_launch_horizon(const float* ranges, int n, int W, int H, int* row
     const long long total = (long long)n * W;
     if(total <= 0) return cudaSuccess;
     k_horizon<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(ranges, n, W, H, rows, range);
+    return cudaGetLastError();
+}
+
+// ================================================================================================
+// k_viewshed: R2 ray casting (include/horizonator-batch.h states the definition; oracle/viewshed_oracle.c restates it
+// operation for operation, and the masks must agree bit for bit).  Every operation of a ray is written as an
+// explicitly rounded intrinsic, so that neither -fmad nor the optimiser can contract or reorder it.
+// ================================================================================================
+
+// metres from the eye along one axis at cell coordinate x (vertex.glsl:128-130 with x in place of the vertex index, as
+// k_prepare's axis tables): scale = cos_viewer_lat east, 1 north
+__device__ __forceinline__ float hz_vs_metres(float x, float v, float dpc, float scale)
+{
+    return __fmul_rn(__fdiv_rn(__fmul_rn(__fmul_rn(__fmul_rn(__fsub_rn(x, v), dpc), HZ_REARTH_F), HZ_PI_F), 180.f), scale);
+}
+
+// A lane collects the bits of one mask word while its ray stays inside that word (a column-stepping ray crosses a new
+// word every 32 steps or when its row changes) and hands them on when it leaves it; lanes handing on the same word
+// merge their bits first (a row-stepping warp's 32 rays usually land in one or two words), so one atomicOr per word.
+// Warp-collective: every lane of the warp calls it at the same step.
+__device__ __forceinline__ void hz_vs_collect(uint32_t*& pend, uint32_t& pbits, uint32_t* word, uint32_t bit, bool last,
+                                              unsigned int lane)
+{
+    const bool change = word != nullptr && word != pend;
+    const bool flush = pbits != 0u && (change || last);
+    const unsigned int fm = __ballot_sync(0xffffffffu, flush);
+    if(flush)
+    {
+        const unsigned int peers = __match_any_sync(fm, (unsigned long long)pend);
+        const unsigned int v = __reduce_or_sync(peers, pbits);
+        if(lane == (unsigned int)(__ffs(peers) - 1)) atomicOr(pend, v);
+    }
+    if(change) { pend = word; pbits = bit; }
+    else pbits = last ? 0u : (pbits | bit);
+}
+
+#define HZ_VS_WARPS  4     /* warps per CTA */
+#define HZ_VS_UNROLL 4     /* steps whose heights are loaded before the first of them is evaluated */
+
+// One thread per ray, gridDim.y = view.  The 4N-4 rays go to warps side by side: bottom row, top row, left column,
+// right column (without the corners), each side padded to whole warps, so that a warp holds 32 adjacent rays.  A
+// warp's rays run for a common number of steps (each lane's own count masks the rest): a side's rays that step
+// along the same axis all end on the same column or row, and the collective hand-on of mask bits needs every lane.
+__global__ void __launch_bounds__(HZ_VS_WARPS * 32)
+k_viewshed(const __grid_constant__ HzViewshed p)
+{
+    const int N = p.N;
+    const HzViewshedEye E = p.eye[blockIdx.y];
+    uint32_t* const mask = p.masks + (size_t)blockIdx.y * N * p.w32;
+    if(blockIdx.x == 0 && threadIdx.x < 4)
+    {
+        // the four vertices around the eye
+        const int i = (int)floorf(E.vci) + (int)(threadIdx.x & 1), j = (int)floorf(E.vcj) + (int)(threadIdx.x >> 1);
+        atomicOr(mask + (size_t)j * p.w32 + (i >> 5), 1u << (i & 31));
+    }
+
+    const unsigned int lane = threadIdx.x & 31;
+    int w = (int)(blockIdx.x * HZ_VS_WARPS + (threadIdx.x >> 5));
+    const int wrow = (N + 31) >> 5, wcol = (N - 2 + 31) >> 5;
+    int ti, tj;
+    bool valid;
+    if(w < 2 * wrow)
+    {
+        const int k = (w % wrow) * 32 + (int)lane;
+        valid = k < N; ti = k; tj = w < wrow ? 0 : N - 1;
+    }
+    else
+    {
+        w -= 2 * wrow;
+        if(w >= 2 * wcol) return;                             // whole warps only
+        const int k = (w % wcol) * 32 + (int)lane;
+        valid = k < N - 2; ti = w < wcol ? 0 : N - 1; tj = k + 1;
+    }
+
+    // "a" is the axis the ray steps along, "b" the other one
+    const float di = __fsub_rn((float)ti, E.vci), dj = __fsub_rn((float)tj, E.vcj);
+    const bool xmaj = fabsf(di) >= fabsf(dj);
+    const float va = xmaj ? E.vci : E.vcj, vb = xmaj ? E.vcj : E.vci;
+    const float da = xmaj ? di : dj, db = xmaj ? dj : di;
+    const float sa = xmaj ? E.cos_lat : 1.0f, sb = xmaj ? 1.0f : E.cos_lat;
+    const int ta = xmaj ? ti : tj;
+    const float slope = da != 0.f ? __fdiv_rn(db, da) : 0.f;
+    const int step = da > 0.f ? 1 : -1;
+    const int a0 = da > 0.f ? (int)floorf(va) + 1 : (int)ceilf(va) - 1;
+    const int nsteps = (valid && da != 0.f) ? abs(ta - a0) + 1 : 0;
+    const int maxsteps = (int)__reduce_max_sync(0xffffffffu, (unsigned int)nsteps);
+
+    // height at (a, b): mosaic[b][a] on a column-stepping ray (its warp reads 32 rows of one column per step; a
+    // transposed copy of the mosaic for these rays measured 3 % slower, DESIGN.md section 9), mosaic[a][b] on a
+    // row-stepping one
+    const int16_t* const base = p.mosaic;
+    const size_t stride_a = xmaj ? 1 : (size_t)p.pitch, stride_b = xmaj ? (size_t)p.pitch : 1;
+    const float vz = E.vz, curv = p.curvature, th = p.target_height, dpc = p.deg_per_cell;
+
+    float smax = __int_as_float(0xff800000);                  // -inf
+    uint32_t* pend = nullptr;
+    uint32_t pbits = 0;
+    for(int k0 = 0; k0 < maxsteps; k0 += HZ_VS_UNROLL)
+    {
+        // the addresses of the next steps do not depend on the running maximum: their loads go out first
+        float zlo[HZ_VS_UNROLL], zhi[HZ_VS_UNROLL];
+        #pragma unroll
+        for(int u = 0; u < HZ_VS_UNROLL; u++)
+        {
+            zlo[u] = zhi[u] = 0.f;
+            if(k0 + u < nsteps)
+            {
+                const int a = a0 + (k0 + u) * step;
+                const float b = __fadd_rn(vb, __fmul_rn(__fsub_rn((float)a, va), slope));
+                const int b0 = min(max((int)floorf(b), 0), N - 2);
+                const int16_t* q = base + (size_t)a * stride_a + (size_t)b0 * stride_b;
+                zlo[u] = (float)__ldg(q);
+                zhi[u] = (float)__ldg(q + stride_b);
+            }
+        }
+        #pragma unroll
+        for(int u = 0; u < HZ_VS_UNROLL; u++)
+        {
+            uint32_t* word = nullptr;
+            uint32_t bit = 0;
+            if(k0 + u < nsteps)
+            {
+                const int a = a0 + (k0 + u) * step;
+                const float b = __fadd_rn(vb, __fmul_rn(__fsub_rn((float)a, va), slope));
+                const int b0 = min(max((int)floorf(b), 0), N - 2);
+                const int r = min(max(__float2int_rn(b), 0), N - 1);
+                // the surface at (a, b): linear along the grid edge between b0 and b0 + 1
+                const float t = __fsub_rn(b, (float)b0);
+                const float z = __fadd_rn(zlo[u], __fmul_rn(__fsub_rn(zhi[u], zlo[u]), t));
+                const float ma = hz_vs_metres((float)a, va, dpc, sa), mb = hz_vs_metres(b, vb, dpc, sb);
+                const float d2 = __fadd_rn(__fmul_rn(ma, ma), __fmul_rn(mb, mb));
+                const float s = __fdiv_rn(__fsub_rn(__fsub_rn(z, vz), __fmul_rn(curv, d2)), __fsqrt_rn(d2));
+                // the vertex (a, rint(b)) against the steps before this one
+                const float zr = r == b0 ? zlo[u] : zhi[u];
+                const float mr = hz_vs_metres((float)r, vb, dpc, sb);
+                const float d2r = __fadd_rn(__fmul_rn(ma, ma), __fmul_rn(mr, mr));
+                const float q = __fdiv_rn(__fadd_rn(__fsub_rn(__fsub_rn(zr, vz), __fmul_rn(curv, d2r)), th), __fsqrt_rn(d2r));
+                if(q >= smax)
+                {
+                    const int i = xmaj ? a : r, j = xmaj ? r : a;
+                    word = mask + (size_t)j * p.w32 + (i >> 5);
+                    bit = 1u << (i & 31);
+                }
+                smax = fmaxf(smax, s);
+            }
+            hz_vs_collect(pend, pbits, word, bit, false, lane);
+        }
+    }
+    hz_vs_collect(pend, pbits, nullptr, 0u, true, lane);
+}
+
+cudaError_t hz_launch_viewshed(const HzViewshed& p, int nviews, cudaStream_t stream)
+{
+    if(nviews <= 0) return cudaSuccess;
+    const int warps = 2 * ((p.N + 31) / 32) + 2 * ((p.N - 2 + 31) / 32);
+    k_viewshed<<<dim3((unsigned)((warps + HZ_VS_WARPS - 1) / HZ_VS_WARPS), (unsigned)nviews), HZ_VS_WARPS * 32, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+// counts[j][i] += the views' bits of cell (i, j): one thread per cell, the 32 threads of a word share its loads
+__global__ void __launch_bounds__(256)
+k_viewshed_count(const uint32_t* __restrict__ masks, int nviews, int N, int w32, uint32_t* __restrict__ counts)
+{
+    const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x), j = (int)blockIdx.y;
+    if(i >= N) return;
+    const size_t per_view = (size_t)N * w32;
+    const uint32_t* m = masks + (size_t)j * w32 + (i >> 5);
+    unsigned int c = 0;
+    for(int v = 0; v < nviews; v++) c += (__ldg(m + (size_t)v * per_view) >> (i & 31)) & 1u;
+    if(c) counts[(size_t)j * N + i] += c;
+}
+
+cudaError_t hz_launch_viewshed_count(const uint32_t* masks, int nviews, int N, int w32, uint32_t* counts,
+                                     cudaStream_t stream)
+{
+    if(nviews <= 0) return cudaSuccess;
+    k_viewshed_count<<<dim3((unsigned)((N + 255) / 256), (unsigned)N), 256, 0, stream>>>(masks, nviews, N, w32, counts);
     return cudaGetLastError();
 }
 

@@ -6,7 +6,8 @@ collective on the data path of a render:
 
 * viewpoint batch -- every viewpoint is an independent render against the same read-only DEM square, which each
   rank loads for itself.  Viewpoints are block-partitioned; outputs stay sharded on the rank that made them.
-  Only reduced products (horizon profiles, a few bytes per image column) are gathered.
+  Only reduced products (horizon profiles, a few bytes per image column) are gathered.  Viewsheds partition the same
+  way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).
 * azimuth wedges  -- one giant panorama: rank g renders columns [edges[g], edges[g+1]), bit-identical to the same
   columns of an unsharded render.  PeerPanorama fuses the exchange into the renderer: each rank's resolve kernel
   stores its wedge straight into every rank's full panorama over NVLink (peer memory), a barrier is the only
@@ -285,6 +286,33 @@ class HostPanorama:
                     os.unlink(self.path)
                 except OSError:
                     pass
+
+
+def reduce_counts(counts, group=None, root=None):
+    """Sums every rank's (N, N) viewshed counts: on every rank with root=None (all_reduce), else only on rank `root`
+    (reduce; the other ranks' tensors then hold partial sums).  In place; returns `counts`."""
+    world, _ = _world(group)
+    if world > 1:
+        if root is None:
+            dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=group)
+        else:
+            dist.reduce(counts, dst=root, op=dist.ReduceOp.SUM, group=group)
+    return counts
+
+
+def viewshed_counts_sharded(h, views, group=None, root=None, target_height=0.):
+    """BASELINE configs[4] as a viewshed: block-partitions `views` over the ranks, adds this rank's viewsheds into
+    counts on its own GPU (horizonator_viewshed_device) and sums the ranks' counts with one collective (see
+    reduce_counts).  Returns the (N, N) int32 CUDA tensor: for every vertex of the loaded square, how many of the views
+    see it.  All ranks must hold contexts of the same DEM square."""
+    world, rank = _world(group)
+    lo, hi = block_partition(len(views), world, rank)
+    N = h.size
+    counts = torch.zeros((N, N), dtype=torch.int32, device=torch.device("cuda", torch.cuda.current_device()))
+    if hi > lo:
+        h.viewshed_device(views[lo:hi], d_counts=counts.data_ptr(), target_height=target_height,
+                          stream=torch.cuda.current_stream().cuda_stream)
+    return reduce_counts(counts, group, root)
 
 
 def render_batch_sharded(h, views, group=None, gather_profiles=True):

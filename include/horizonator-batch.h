@@ -159,6 +159,45 @@ bool horizonator_horizon_profile_device(const horizonator_context_t* ctx,
                                         void* d_rows, void* d_range,
                                         void* stream);
 
+/* Viewsheds: which vertices of the loaded DEM square each of n views sees, and for every vertex from how many of them.
+ *
+ * Definition (R2, the ray-casting viewshed of Franklin & Ray; the GPU kernel and the test oracle agree bit for bit):
+ *   - Domain: the N x N vertices (i, j) of the loaded square (N = 2R), indexed like horizonator_download_mosaic()
+ *     (row j north, column i east).  The point tested is the vertex's terrain height plus target_height_m.
+ *   - Eye: as horizonator_move() computes it from lat, lon and viewer_z (< 0: the highest of the 4 surrounding
+ *     samples + 1 m), in float.  az_deg0 / az_deg1 are ignored: a viewshed covers the full circle.  The eye's cell
+ *     coordinates must lie in [0, N-1); otherwise the call fails (the render calls accept such eyes).
+ *   - Metres: east and north offsets by the renderer's axis-table formulas (vertex.glsl:128-130) evaluated at the
+ *     (possibly fractional) cell coordinate; the apparent height of a point at horizontal distance^2 d2 with terrain
+ *     height z is z - viewer_z - curvature * d2, so horizonator_set_earth_curvature() applies (off by default).
+ *   - Rays: one per boundary vertex of the square, 4N - 4.  A ray with |di| >= |dj| (di, dj: target minus eye, in
+ *     cells) steps over the integer columns i strictly beyond the eye up to the target's; at column i,
+ *     y = eye_j + (i - eye_i) * (dj / di), the surface is the linear interpolation between rows floor(y) and
+ *     floor(y) + 1 of column i (a grid edge, hence exact on the mesh's triangles; the rows clamped to [0, N-2] and
+ *     [1, N-1]), and its horizon slope is s = apparent height / horizontal distance.  The vertex that step decides is
+ *     (i, rint(y)) (clamped to [0, N-1]): visible iff (its apparent height + target_height_m) / its own horizontal
+ *     distance >= the largest s of the ray's EARLIER steps (-inf at the first step).  Rays with |dj| > |di| step
+ *     over rows the same way, axes swapped.
+ *   - A vertex is visible iff some ray finds it visible; the four vertices around the eye are visible.
+ *   - fp32, every operation rounded once in the order written in hz_kernels.cu (k_viewshed) and
+ *     oracle/viewshed_oracle.c (vs_oracle_r2).
+ * R2 is an approximation of line of sight: on seeded synthetic terrain it disagrees with the exact line of sight on
+ * the same triangulation on about 1 % of the vertices (DESIGN.md, viewsheds).
+ *
+ * masks: n x N x W32 uint32 (W32 = (N + 31) / 32; cell i of row j = bit (i & 31) of word [j][i >> 5], unused bits
+ *        0), overwritten;
+ * counts: N x N uint32, += the number of the n views that see each cell (the caller zeroes it; several calls and
+ *        several ranks can add into one buffer);
+ * either may be NULL, not both.  n = 0 does nothing.  Both DEVICE pointers here, stream as for the batch render.
+ * Sizes at N = 11716 (150 km of SRTM1): one mask 17.2 MB, the counts 549 MB.  A call that wants only counts uses a
+ * scratch of up to 64 masks, allocated on first use; the views go in chunks of up to 64 per kernel launch. */
+bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                 float target_height_m, void* d_masks, void* d_counts, void* stream);
+
+/* Same, into HOST memory, synchronous. */
+bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                          float target_height_m, uint32_t* masks, uint32_t* counts);
+
 /* Per-kernel device times.  While enabled, every render records CUDA events around each of
  * its kernels on the stream it runs on.  horizonator_profile_read() waits for them and reports
  * the MEAN duration in milliseconds per render of: out_ms[0] k_prepare (clear + axis tables),
