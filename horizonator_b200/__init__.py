@@ -110,7 +110,6 @@ def _declare(lib):
         "horizonator_peer_free": (b, [ctx, vp]),
         "horizonator_render_wedge_peers": (b, [ctx, i, i, i, P(vp), P(vp), vp]),
         "horizonator_peer_barrier": (b, [ctx, i, i, P(vp), C.c_uint, vp]),
-        "horizonator_reload_tunables": (b, [ctx]),
         "horizonator_debug_device_math": (b, [i, vp, vp, vp, vp, vp, vp]),
         "horizonator_render_wedge_host": (b, [ctx, i, i, vp, vp]),
         "horizonator_host_register": (b, [vp, C.c_size_t]),
@@ -147,7 +146,7 @@ EXPORTED_SYMBOLS = (
     "horizonator_host_alloc", "horizonator_host_free",
     "horizonator_render_counters", "horizonator_horizon_profile_device", "horizonator_set_earth_curvature", "horizonator_set_seam_wrap",
     "horizonator_peer_alloc", "horizonator_peer_open", "horizonator_peer_close", "horizonator_peer_free",
-    "horizonator_render_wedge_peers", "horizonator_peer_barrier", "horizonator_reload_tunables",
+    "horizonator_render_wedge_peers", "horizonator_peer_barrier",
     "horizonator_render_wedge_host", "horizonator_host_register", "horizonator_host_unregister",
     "horizonator_debug_device_math", "horizonator_set_lod",
     "horizonator_viewshed_device", "horizonator_viewshed",
@@ -392,16 +391,6 @@ class horizonator:
                                                 image.ctypes.data if image is not None else None,
                                                 ranges.ctypes.data if ranges is not None else None):
             raise RuntimeError("horizonator_render_offscreen() failed")
-
-    def reload_tunables(self, **env):
-        """Sets the given HORIZONATOR_* environment variables (None = unset) and makes the context read them again."""
-        for k, v in env.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = str(v)
-        if not lib.horizonator_reload_tunables(C.byref(self._ctx)):
-            raise RuntimeError("horizonator_reload_tunables() failed")
 
     def profile(self, on=True):
         """Record CUDA events around every kernel of every render from now on (see profile_read)."""

@@ -16,7 +16,6 @@
 #include <cstdlib>
 #include <cstring>
 #include <atomic>
-#include <chrono>
 #include <condition_variable>
 #include <mutex>
 #include <thread>
@@ -46,6 +45,37 @@ constexpr int   MAX_BANDS       = HZ_MAX_BANDS;
 // [5+4b] block_count, [6+4b] tri_count, [7+4b] big_count of band b, then the stats
 constexpr int   STATS_AT        = 4 + 4 * MAX_BANDS;
 constexpr int   N_COUNTERS      = STATS_AT + HZ_STAT_COUNT;
+
+// ---- the render chain's configuration.  Each value won its sweep (profiles/); a new sweep edits a constant and
+// compares a second build of the library (build_library(extra_flags, name) + HORIZONATOR_LIBRARY).
+
+constexpr int NEAR_RINGS = 2;                   // rings of tiles around the eye's tile drawn first, without culling tests
+// largest bounding box (pixels) a triangle's own thread rasterises always / where enough lanes of its warp have one
+// (zoomed-in views only: fill_view); larger ones go to k_big
+constexpr int SMALL_MAX_PIX = 16, MID_MAX_PIX = 64;
+// most views of a batch rendered by one chain of launches, view sets in flight at once (render_batch_common), and
+// executable instances of each captured chain (capture_graph)
+constexpr int VIEWS_PER_SET = 64, N_SETS_MAX = 4, GRAPH_INSTANCES = 2;
+
+// Rings (in tiles around the eye's tile) at which the bands end; the last band runs to the edge of the mesh.
+struct Bands { int n; int end[MAX_BANDS]; };
+
+// A lone view is latency-bound; the views of a batch want throughput.
+// - bands: more bands = more of the mesh culled by what nearer bands drew, but four more kernels each.  A lone view
+//   gets two bands.  The views of a batch share their launches -- up to 64 views per chain, so a launch costs next to
+//   nothing per view -- and get ten, each reaching about 1.5 times as far as the one before (measured on 256 distinct
+//   viewpoints, profiles/r02s_sweep.jsonl: 13.4k panoramas/s with five bands and 16 views per chain, 15.6k with ten
+//   and 64; the benchmark viewpoint repeated 30.3k -> 33.0k).  The image is the same either way.
+// - occl_tile_max_pix, occl_block_max_pix: largest screen box one thread checks against the visibility buffer.  In a
+//   lone view a long walk by one thread holds its kernel up; the views of a batch hide that behind each other and
+//   gain from the extra culling.
+// - grid_percent: see hz_grid() in hz_kernels.cu.
+// - mid_level: blocks of live tiles tested in two levels (k_blocks_mid: fewer tests, one more in a row).
+struct ChainConfig { Bands bands; int occl_tile_max_pix, occl_block_max_pix, grid_percent; bool mid_level; };
+constexpr ChainConfig LONE  = { { 2, { 48, 1 << 20 } },                                64,  32, 100, false };
+constexpr ChainConfig BATCH = { { 10, { 5, 8, 12, 18, 27, 40, 60, 90, 135, 1 << 20 } }, 128, 128, 200, true };
+// (with the opt-in level of detail every render has HZ_MAX_LOD more bands: enqueue_views)
+static_assert(LONE.bands.n + HZ_MAX_LOD <= HZ_MAX_BANDS && BATCH.bands.n + HZ_MAX_LOD <= HZ_MAX_BANDS, "too many bands");
 
 // what the reference keeps in GL uniforms
 struct ViewState
@@ -88,11 +118,11 @@ struct Scratch
 
 // Up to `cap` views that are rendered TOGETHER: one chain of kernel launches whose grids have a view dimension
 // (gridDim.y), each view with its own scratch.  The context's own view is a set of one; the batch calls use sets of
-// up to Slot::views_per_set, each with its own stream, so that the tail of one set's kernels overlaps another's.
+// up to VIEWS_PER_SET, each with its own stream, so that the tail of one set's kernels overlaps another's.
 struct ViewSet
 {
     int  cap = 0;
-    bool batch = false;                // band structure and grid scale of batched views
+    bool batch = false;                // the chain configuration of batched views (config_of)
     cudaStream_t stream = nullptr;     // batch sets only
     cudaEvent_t  done = nullptr;       // batch sets only
     std::vector<Scratch> sc;           // grows on demand up to cap (ensure_views)
@@ -130,22 +160,6 @@ struct Slot
     HzTiles  tiles{};
     short2 *d_mm_block = nullptr, *d_mm_tile = nullptr;   // culling pyramid
     int nb = 0, nt = 0;
-    int near_rings = 2;
-    // largest screen box one thread checks against the visibility buffer: a lone view is latency-bound and a long walk
-    // by one thread holds its kernel up; the views of a batch hide that behind each other and gain from the extra culling
-    int occl_tile_max_pix = 64, occl_block_max_pix = 32, occl_tile_max_pix_batch = 128, occl_block_max_pix_batch = 128;
-    int small_max_pix = 16, mid_max_pix = 64;
-    int grid_percent_single = 100, grid_percent_batch = 200;   // see hz_grid() in hz_kernels.cu
-    // Rings (in tiles around the eye's tile) at which the bands end; the last band runs to the edge of the mesh.
-    // More bands = more of the mesh culled by what nearer bands drew, but four more kernels each.  A lone view is
-    // latency-bound and gets two bands.  The views of a batch share their launches -- up to 64 views per chain, so a
-    // launch costs next to nothing per view -- and get ten, each reaching about 1.5 times as far as the one before
-    // (measured on 256 distinct viewpoints, profiles/r02s_sweep.jsonl: 13.4k panoramas/s with five bands and 16 views
-    // per chain, 15.6k with ten and 64; the benchmark viewpoint repeated 30.3k -> 33.0k).  The image is the same either way.
-    struct Bands { int n; int end[MAX_BANDS]; };
-    Bands bands_single = { 2, { 48, 1 << 20 } };
-    Bands bands_batch  = { 10, { 5, 8, 12, 18, 27, 40, 60, 90, 135, 1 << 20 } };
-    int views_per_set = 64, n_sets_max = 4, graph_instances = 2;
 
     // target
     int W = 0, H = 0;
@@ -182,12 +196,6 @@ struct Slot
     float lod_pixels = 0.f;          // opt-in (horizonator_set_lod); 0 = every band meshed at full density like the reference
     bool  seam_wrap = false;         // opt-in (horizonator_set_seam_wrap); false = seam triangles dropped like the reference
     float curvature = 0.f;           // opt-in (horizonator_set_earth_curvature); 0 = flat earth like the reference
-    bool use_graphs = true;
-    // blocks of live tiles tested in two levels (k_blocks_mid: fewer tests, one more in a row): the views of a batch
-    int mid_level_single = 0, mid_level_batch = 1;
-    // near pass's k_big beside the bands (launch_chain).  Measured on one box against the chain in line: lone C2 view
-    // 111 -> 108 us, 10-degree zoom 0.38 -> 0.35 ms, 5-degree 0.28 -> 0.25 ms, eye 12 km +1 %, batches +0.5 %
-    int fork_single = 1, fork_batch = 1;
     bool collect_stats = false;      // culling counters (horizonator_render_counters); off: the kernels skip them
     std::vector<cudaEvent_t> prof_events;
     size_t prof_used = 0;
@@ -403,14 +411,14 @@ int ensure_views(Slot& s, ViewSet& vs, int n)
     return (int)vs.sc.size() < n ? (int)vs.sc.size() : n;
 }
 
-// the batch sets: up to n_sets_max, created on demand
+// the batch sets: up to N_SETS_MAX, created on demand
 ViewSet* batch_set(Slot& s, int k)
 {
     if(s.fork_ev == nullptr && cudaEventCreateWithFlags(&s.fork_ev, cudaEventDisableTiming) != cudaSuccess) return nullptr;
     while((int)s.sets.size() <= k)
     {
         ViewSet* g = new ViewSet;
-        bool ok = alloc_set(*g, s.views_per_set, true);
+        bool ok = alloc_set(*g, VIEWS_PER_SET, true);
         if(ok && s.target_pixels > 0)
             ok = cudaMallocHost(&g->h_tanel, (size_t)PARAM_RING * g->cap * s.H * sizeof(float)) == cudaSuccess;
         if(!ok)
@@ -483,15 +491,15 @@ const float* tanel_row(Slot& s, float az_deg0, float az_deg1)
     return r.row.data();
 }
 
-const Slot::Bands& bands_of(const Slot& s, const ViewSet& set)
+const ChainConfig& config_of(const ViewSet& set)
 {
-    return set.batch ? s.bands_batch : s.bands_single;
+    return set.batch ? BATCH : LONE;
 }
 
 // bands of a render chain: the configured ones, plus two more where the opt-in level of detail changes (fill: enqueue_views)
 int n_bands_of(const Slot& s, const ViewSet& set)
 {
-    return bands_of(s, set).n + (s.lod_pixels > 0.f ? HZ_MAX_LOD : 0);
+    return config_of(set).bands.n + (s.lod_pixels > 0.f ? HZ_MAX_LOD : 0);
 }
 
 // Zoomed-in views (small angle per pixel) show triangles many pixels large even far from the eye: each band then draws
@@ -516,8 +524,10 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
     if(ev) CUDA_TRY(cudaEventRecord(ev[2], st));
     // The near pass's large triangles: in line, or (fork) beside the bands on the set's side stream.  The bands' culling
     // then sees less of the foreground in the visibility buffer -- it only ever removes work, the image is the same --
-    // and the chain is a kernel shorter.
-    const bool fork = ev == nullptr && (set.batch ? s.fork_batch : s.fork_single);
+    // and the chain is a kernel shorter.  Measured on one box against the chain in line: lone C2 view 111 -> 108 us,
+    // 10-degree zoom 0.38 -> 0.35 ms, 5-degree 0.28 -> 0.25 ms, eye 12 km +1 %, batches +0.5 %.  A profiled chain
+    // (ev) runs it in line, so that the events time each kernel.
+    const bool fork = ev == nullptr;
     if(fork && set.side == nullptr)
     {
         CUDA_TRY(cudaEventCreateWithFlags(&set.ev_fork, cudaEventDisableTiming));
@@ -568,7 +578,7 @@ ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bo
         ok = launch_chain(s, set, hv, m, big_per_band, true, true, cs, nullptr, &launches);
         if(cudaStreamEndCapture(cs, &g) != cudaSuccess) ok = false;
     }
-    for(int k = 0; ok && k < s.graph_instances; k++)
+    for(int k = 0; ok && k < GRAPH_INSTANCES; k++)
     {
         cudaGraphExec_t e = nullptr;
         if(cudaGraphInstantiate(&e, g, 0) != cudaSuccess) ok = false; else exec.push_back(e);
@@ -634,16 +644,17 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
     v.tile_queue = sc.d_tile_queue; v.block_queue = sc.d_block_queue;
     v.tri_queue = sc.d_tri_queue; v.tri_capacity = s.tri_capacity;
     v.bigtri = sc.d_bigtri; v.bigtri_count = sc.d_counters + 3; v.bigtri_capacity = s.bigtri_capacity;
-    v.occl_tile_max_pix  = set.batch ? s.occl_tile_max_pix_batch  : s.occl_tile_max_pix;
-    v.occl_block_max_pix = set.batch ? s.occl_block_max_pix_batch : s.occl_block_max_pix;
+    const ChainConfig& cfg = config_of(set);
+    v.occl_tile_max_pix  = cfg.occl_tile_max_pix;
+    v.occl_block_max_pix = cfg.occl_block_max_pix;
     // (middle-sized triangles are drawn by their own threads only in zoomed-in views, where whole warps have them; in a
     // wide view they sit right around the eye, and walking them in k_raster holds that kernel up for nothing)
     // (... and in such views the threads walk boxes twice as large themselves: measured 5 % faster)
     const bool zoomed = big_after_every_band(s, vs);
-    v.small_max_pix = zoomed ? 2 * s.small_max_pix : s.small_max_pix; v.mid_max_pix = zoomed ? s.mid_max_pix : 0;
-    v.grid_percent = set.batch ? s.grid_percent_batch : s.grid_percent_single;
+    v.small_max_pix = zoomed ? 2 * SMALL_MAX_PIX : SMALL_MAX_PIX; v.mid_max_pix = zoomed ? MID_MAX_PIX : 0;
+    v.grid_percent = cfg.grid_percent;
     v.lod_capable = s.lod_pixels > 0.f;
-    v.mid_level = set.batch ? s.mid_level_batch : s.mid_level_single;
+    v.mid_level = cfg.mid_level;
     v.big_capacity = s.big_capacity;
 
     // the eye's tile, and how many rings of tiles around it form the foreground pass
@@ -651,7 +662,7 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
         const int ti = (int)floorf(vs.viewer_cell_i / (float)HZ_TILE_CELLS), tj = (int)floorf(vs.viewer_cell_j / (float)HZ_TILE_CELLS);
         v.eye_ti = ti < 0 ? 0 : (ti >= s.nt ? s.nt - 1 : ti);
         v.eye_tj = tj < 0 ? 0 : (tj >= s.nt ? s.nt - 1 : tj);
-        v.near_rings = s.near_rings;
+        v.near_rings = NEAR_RINGS;
     }
 
     // for the depth bound of hz_rect_test: the diagonal of one cell on the ground
@@ -672,27 +683,9 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
 
 // Enqueues one render of columns [x0,x1) of m views (m <= what ensure_views() gave) on stream st: view k uses scratch
 // set.sc[k] and writes to outs[k] (device memory).  All views of one call must have the same kinds of output.
-// HORIZONATOR_TRACE_HOST=1: where the host time of enqueue_views() goes, printed when the context is destroyed
-struct HostTrace
-{
-    bool on = getenv("HORIZONATOR_TRACE_HOST") != nullptr;
-    double wait_ring = 0, fill = 0, copy = 0, launch = 0;
-    long calls = 0, views = 0;
-    static double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-    ~HostTrace()
-    {
-        if(on && calls)
-            fprintf(stderr, "horizonator host trace: %ld enqueues, %ld views; per enqueue: ring wait %.1f us, fill %.1f us, "
-                    "parameter copy %.1f us, launch %.1f us\n", calls, views, wait_ring / calls * 1e6, fill / calls * 1e6,
-                    copy / calls * 1e6, launch / calls * 1e6);
-    }
-};
-HostTrace g_trace;
-
 bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st)
 {
     if(s.W <= 0 || s.H <= 0 || m < 1 || m > (int)set.sc.size()) return false;
-    const double t_begin = g_trace.on ? HostTrace::now() : 0;
     const bool want_image = outs[0].image[0] != nullptr, want_ranges = outs[0].ranges[0] != nullptr;
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
     if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy, 0));
@@ -702,9 +695,8 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     const int slot = set.ring_next;
     set.ring_next = (set.ring_next + 1) % PARAM_RING;
     CUDA_TRY(cudaEventSynchronize(set.ring_ev[slot]));            // the copies that last used this slot are done
-    const double t_ring = g_trace.on ? HostTrace::now() : 0;
     HzView* hv = set.h_views + (size_t)slot * set.cap * HZ_V_COUNT;
-    const Slot::Bands& bands = bands_of(s, set);
+    const Bands& bands = config_of(set).bands;
     bool big_per_band = false, vectorisable = true;
     for(int k = 0; k < m; k++) big_per_band = big_per_band || big_after_every_band(s, vs[k]);
     for(int k = 0; k < m; k++)
@@ -745,7 +737,7 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
                 n_ends++;
             }
         }
-        int lo = s.near_rings + 1;
+        int lo = NEAR_RINGS + 1;
         for(int b = 0; b < n_ends; b++)
         {
             HzView& vb = hk[HZ_V_BAND0 + b];
@@ -770,24 +762,12 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
             sc.tanel_key.valid = true; sc.tanel_key.daz = vs[k].az_deg1 - vs[k].az_deg0; sc.tanel_key.W = s.W; sc.tanel_key.H = s.H;
         }
     }
-    const double t_fill = g_trace.on ? HostTrace::now() : 0;
     CUDA_TRY(cudaMemcpyAsync(set.d_views, hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaEventRecord(set.ring_ev[slot], st));
-    const double t_copy = g_trace.on ? HostTrace::now() : 0;
-    struct TraceEnd
-    {
-        double a, b, c, d; int m;
-        ~TraceEnd()
-        {
-            if(!g_trace.on) return;
-            g_trace.wait_ring += b - a; g_trace.fill += c - b; g_trace.copy += d - c; g_trace.launch += HostTrace::now() - d;
-            g_trace.calls++; g_trace.views += m;
-        }
-    } trace_end{ t_begin, t_ring, t_fill, t_copy, m };
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
     const bool is_main = (&set == &s.main);
-    const bool standard = !s.profiling && s.use_graphs && x0 == 0 && x1 == s.W && (want_image || want_ranges) &&
+    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (want_image || want_ranges) &&
                           outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && vectorisable;
     if(standard && !set.graph_failed)
     {
@@ -830,48 +810,6 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
 bool enqueue_render(Slot& s, const ViewState& vs, int x0, int x1, const OutSpec& out, cudaStream_t st)
 {
     return enqueue_views(s, s.main, 1, &vs, x0, x1, &out, st);
-}
-
-// The tunables of the render chain, from the environment (defaults in Slot).  Read at init; horizonator_reload_tunables()
-// reads them again.
-void read_tunables(Slot& s)
-{
-    if(const char* env = getenv("HORIZONATOR_NEAR_RINGS")) s.near_rings = atoi(env) < 0 ? 0 : atoi(env);
-    // (the plain variable sets both; ..._BATCH the value for the views of a batch only)
-    if(const char* env = getenv("HORIZONATOR_OCCL_TILE_PIX"))  s.occl_tile_max_pix  = s.occl_tile_max_pix_batch  = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_OCCL_BLOCK_PIX")) s.occl_block_max_pix = s.occl_block_max_pix_batch = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_OCCL_TILE_PIX_BATCH"))  s.occl_tile_max_pix_batch  = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_OCCL_BLOCK_PIX_BATCH")) s.occl_block_max_pix_batch = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_SMALL_PIX"))      s.small_max_pix = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_MID_PIX"))        s.mid_max_pix = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_GRID_SCALE"))       s.grid_percent_single = atoi(env);
-    if(const char* env = getenv("HORIZONATOR_GRID_SCALE_BATCH")) s.grid_percent_batch  = atoi(env);
-    // HORIZONATOR_BANDS / HORIZONATOR_BANDS_BATCH: comma-separated rings at which the bands end (lone views / views
-    // of a batch; the first also sets the second unless that is given); the last band always runs to the edge
-    auto parse_bands = [](const char* env, Slot::Bands& out) {
-        int n = 0;
-        for(const char* p = env; *p && n < MAX_BANDS - HZ_MAX_LOD - 1; )
-        {
-            const int r = atoi(p);
-            if(r > 0) out.end[n++] = r;
-            while(*p && *p != ',') p++;
-            if(*p == ',') p++;
-        }
-        out.end[n++] = 1 << 20;
-        out.n = n;
-    };
-    if(const char* env = getenv("HORIZONATOR_BANDS")) { parse_bands(env, s.bands_single); s.bands_batch = s.bands_single; }
-    if(const char* env = getenv("HORIZONATOR_BANDS_BATCH")) parse_bands(env, s.bands_batch);
-    if(const char* env = getenv("HORIZONATOR_GRAPHS")) s.use_graphs = atoi(env) != 0;
-    if(const char* env = getenv("HORIZONATOR_MID_LEVEL"))       s.mid_level_single = s.mid_level_batch = atoi(env) != 0;
-    if(const char* env = getenv("HORIZONATOR_MID_LEVEL_BATCH")) s.mid_level_batch = atoi(env) != 0;
-    if(const char* env = getenv("HORIZONATOR_FORK"))       s.fork_single = s.fork_batch = atoi(env) != 0;
-    if(const char* env = getenv("HORIZONATOR_FORK_BATCH")) s.fork_batch = atoi(env) != 0;
-    if(const char* env = getenv("HORIZONATOR_GRAPH_INSTANCES")) s.graph_instances = atoi(env) < 1 ? 1 : (atoi(env) > 16 ? 16 : atoi(env));
-    // HORIZONATOR_LANES: most views of a batch rendered by one chain of launches; HORIZONATOR_SETS: how many such
-    // sets may be in flight (each on its own stream)
-    if(const char* env = getenv("HORIZONATOR_LANES")) s.views_per_set = atoi(env) < 1 ? 1 : (atoi(env) > 64 ? 64 : atoi(env));
-    if(const char* env = getenv("HORIZONATOR_SETS"))  s.n_sets_max = atoi(env) < 1 ? 1 : (atoi(env) > 8 ? 8 : atoi(env));
 }
 
 // lib:765-789, float as written there.  The four samples come from the host mmaps (dem.h).
@@ -943,7 +881,6 @@ private:
         if(started_) return;
         started_ = true;
         int n = 3;
-        if(const char* env = getenv("HORIZONATOR_COPY_THREADS")) n = atoi(env) - 1;
         const int hw = (int)std::thread::hardware_concurrency();
         if(hw > 0 && n > hw - 1) n = hw - 1;
         for(int k = 0; k < n; k++) workers_.emplace_back([this] { loop(); });
@@ -1017,13 +954,12 @@ bool copy_results_to_host(Slot& s, char* image, float* ranges, const uint8_t* d_
     Out outs[2] = { { image, (const char*)d_image, px * 3 }, { (char*)ranges, (const char*)d_ranges, px * sizeof(float) } };
     std::vector<HostCopyPool::Part> parts;
     size_t staged = 0;
-    static const bool pipeline = [] { const char* e = getenv("HORIZONATOR_COPY_THREADS"); return e == nullptr || atoi(e) > 0; }();
     for(const Out& o : outs)
     {
         if(o.dst == nullptr) continue;
         // Page-locked destinations (cudaHostAlloc / cudaHostRegister / horizonator_host_alloc) are written by DMA at
         // PCIe speed
-        if(!pipeline || staged + o.bytes > STAGE_MAX_BYTES || !is_pageable(o.dst))
+        if(staged + o.bytes > STAGE_MAX_BYTES || !is_pageable(o.dst))
         {
             CUDA_TRY(cudaMemcpyAsync(o.dst, o.src, o.bytes, cudaMemcpyDeviceToHost, st));
             continue;
@@ -1168,7 +1104,6 @@ bool horizonator_init(horizonator_context_t* ctx,
                 "cudaMemset(mosaic)")) break;
         s->nb = (s->N - 1 + HZ_BLOCK_CELLS - 1) / HZ_BLOCK_CELLS;
         s->nt = (s->N - 1 + HZ_TILE_CELLS - 1) / HZ_TILE_CELLS;
-        read_tunables(*s);
         if(fail(cudaMalloc(&s->d_mm_block, (size_t)s->nb * s->nb * sizeof(short2)), "cudaMalloc(pyramid)")) break;
         if(fail(cudaMalloc(&s->d_mm_tile, (size_t)s->nt * s->nt * sizeof(short2)), "cudaMalloc(pyramid)")) break;
         if(!alloc_set(s->main, 1, false) || ensure_views(*s, s->main, 1) != 1) break;
@@ -1405,9 +1340,9 @@ bool horizonator_unproject(float* lat, float* lon, int x, int y,
 
 // ---- additive API (include/horizonator-batch.h) -----------------------------------------------------------
 
-// Common part of the two batch calls.  The views are cut into chunks of up to views_per_set; a chunk is rendered by
+// Common part of the two batch calls.  The views are cut into chunks of up to VIEWS_PER_SET; a chunk is rendered by
 // ONE chain of kernel launches whose grids have a view dimension (one parameter copy and one CUDA-graph launch per
-// chunk, whatever its size), on the stream of one of up to n_sets_max view sets, so that the tails of one chunk's
+// chunk, whatever its size), on the stream of one of up to N_SETS_MAX view sets, so that the tails of one chunk's
 // kernels overlap another chunk's.  The sets start after everything already queued on `st`, and `st` continues after
 // all of them.  to_host: outputs go through the views' device staging buffers and device->host copies on the set's
 // stream, which overlap the other sets' kernels.
@@ -1424,15 +1359,15 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     }
     if(n == 0) return true;
 
-    // chunk size: the views spread evenly over the sets, at most views_per_set each, at most what fits in memory
+    // chunk size: the views spread evenly over the sets, at most VIEWS_PER_SET each, at most what fits in memory
     int n_sets = 0, chunk = 0;
     if(n > 1)
     {
         // (no fewer than 8 to a chunk where there are that many: a launch pays off with views to share it)
-        n_sets = s->n_sets_max;
+        n_sets = N_SETS_MAX;
         chunk = (n + n_sets - 1) / n_sets;
         if(chunk < 8) chunk = n < 8 ? n : 8;
-        if(chunk > s->views_per_set) chunk = s->views_per_set;
+        if(chunk > VIEWS_PER_SET) chunk = VIEWS_PER_SET;
         n_sets = (n + chunk - 1) / chunk < n_sets ? (n + chunk - 1) / chunk : n_sets;
         for(int g = 0; g < n_sets; g++)
         {
@@ -1869,32 +1804,6 @@ bool horizonator_debug_device_math(int n, const float* e, const float* north, co
     if(!ok) MSG("CUDA error in horizonator_debug_device_math: %s", cudaGetErrorString(cudaGetLastError()));
     cudaFree(d);
     return ok;
-}
-
-bool horizonator_reload_tunables(const horizonator_context_t* ctx)
-{
-    Slot* s = slot_of(ctx);
-    if(s == nullptr) return false;
-    DeviceGuard g(s->device);
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    for(ViewSet* v : s->sets) CUDA_TRY(cudaStreamSynchronize(v->stream));
-    if(s->main.busy_recorded) CUDA_TRY(cudaEventSynchronize(s->main.busy));
-    for(ViewSet* v : s->sets) if(v->busy_recorded) CUDA_TRY(cudaEventSynchronize(v->busy));
-    // the captured chains and the batch sets embody the old values
-    drop_graphs(s->main);
-    for(ViewSet* v : s->sets) { free_set(*v); delete v; }
-    s->sets.clear();
-    {
-        const Slot d;       // the defaults
-        s->near_rings = d.near_rings; s->occl_tile_max_pix = d.occl_tile_max_pix; s->occl_block_max_pix = d.occl_block_max_pix;
-        s->occl_tile_max_pix_batch = d.occl_tile_max_pix_batch; s->occl_block_max_pix_batch = d.occl_block_max_pix_batch;
-        s->small_max_pix = d.small_max_pix; s->mid_max_pix = d.mid_max_pix; s->grid_percent_single = d.grid_percent_single;
-        s->grid_percent_batch = d.grid_percent_batch; s->bands_single = d.bands_single; s->bands_batch = d.bands_batch;
-        s->use_graphs = d.use_graphs; s->views_per_set = d.views_per_set; s->n_sets_max = d.n_sets_max;
-        s->graph_instances = d.graph_instances; s->mid_level_single = d.mid_level_single; s->mid_level_batch = d.mid_level_batch; s->fork_single = d.fork_single; s->fork_batch = d.fork_batch;
-    }
-    read_tunables(*s);
-    return true;
 }
 
 void* horizonator_host_alloc(size_t bytes)

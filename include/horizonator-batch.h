@@ -124,11 +124,6 @@ bool horizonator_set_seam_wrap(const horizonator_context_t* ctx, bool on);
  * faster.  Applies to all later renders of the context. */
 bool horizonator_set_lod(const horizonator_context_t* ctx, float max_cell_pixels);
 
-/* Reads the HORIZONATOR_* tuning variables (INTEGRATION.md) again -- they are otherwise read once, by
- * horizonator_init() -- after waiting for everything the context has in flight.  Variables that are not set
- * go back to their defaults.  For parameter sweeps inside one process; the images do not depend on them. */
-bool horizonator_reload_tunables(const horizonator_context_t* ctx);
-
 /* Test hook: the renderer's own fp32 angle functions (csrc/hz_math.cuh) evaluated on the current CUDA device for n
  * argument sets in host arrays: az[k] = atan2(e[k], north[k]) (vertex.glsl:136), el[k] = atan(h[k] / sqrt(d2[k]))
  * (vertex.glsl:153).  tests/test_device_math.py measures their error in ulp against double precision. */

@@ -347,21 +347,15 @@ def test_reference_python_binding_on_this_library(hz, tiles_c1):
 
 # ------------------------------------------------------------------------------------------ rarely taken paths
 
-@pytest.mark.parametrize("env", [
-    {"HORIZONATOR_TRI_CAPACITY": "1000"},                                 # triangle list overflows: drawn in the mesh kernel
-    {"HORIZONATOR_BIG_CAPACITY": "50"},                                   # sub-box queue overflows
-    {"HORIZONATOR_BIGTRI_CAPACITY": "7"},                                 # record pool overflows
-    {"HORIZONATOR_BANDS": "4,9,20", "HORIZONATOR_NEAR_RINGS": "0"},       # other band structures
-    {"HORIZONATOR_BANDS": "100000", "HORIZONATOR_NEAR_RINGS": "5", "HORIZONATOR_SMALL_PIX": "1"},
-    {"HORIZONATOR_GRAPHS": "0", "HORIZONATOR_OCCL_TILE_PIX": "0", "HORIZONATOR_OCCL_BLOCK_PIX": "0"},
-    {"HORIZONATOR_MID_LEVEL": "1", "HORIZONATOR_FORK": "0"},             # two-level block test for lone views too; k_big in line
-    {"HORIZONATOR_MID_LEVEL_BATCH": "0", "HORIZONATOR_FORK_BATCH": "0", "HORIZONATOR_BANDS_BATCH": "10,24,56,120",
-     "HORIZONATOR_OCCL_TILE_PIX_BATCH": "256", "HORIZONATOR_OCCL_BLOCK_PIX_BATCH": "64"},    # the batch defaults the round started with
-], ids=["tri_overflow", "big_overflow", "record_overflow", "bands3", "one_band", "no_graph_no_occlusion", "mid_level_no_fork",
-        "old_batch_defaults"])
-def test_overflow_paths_and_tunables_do_not_change_the_image(hz, tiles_c1, env, monkeypatch):
-    """Queue overflows fall back to a slow in-kernel path, and the band/occlusion tunables only move work around:
-    the image must be the one the default configuration produces, bit for bit."""
+@pytest.mark.parametrize("env,profiled", [
+    ({"HORIZONATOR_TRI_CAPACITY": "1000"}, False),                        # triangle list overflows: drawn in the mesh kernel
+    ({"HORIZONATOR_BIG_CAPACITY": "50"}, False),                          # sub-box queue overflows
+    ({"HORIZONATOR_BIGTRI_CAPACITY": "7"}, False),                        # record pool overflows
+    ({}, True),                                                           # the eager chain, k_big of the near pass in line
+], ids=["tri_overflow", "big_overflow", "record_overflow", "profiled"])
+def test_overflow_paths_and_profiling_do_not_change_the_image(hz, tiles_c1, env, profiled, monkeypatch):
+    """Queue overflows fall back to a slow in-kernel path, and a profiled render launches the kernels one by one
+    instead of replaying a captured graph: the image must be the one the default configuration produces, bit for bit."""
     W, H, R = 1000, 160, 420
     h0 = hz.horizonator(C1_LAT, C1_LON, W, H, dir_dems=tiles_c1, render_radius_cells=R)
     want = h0.render(-180.05, 179.95, zfar=100000.)
@@ -369,11 +363,15 @@ def test_overflow_paths_and_tunables_do_not_change_the_image(hz, tiles_c1, env, 
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     h1 = hz.horizonator(C1_LAT, C1_LON, W, H, dir_dems=tiles_c1, render_radius_cells=R)
+    if profiled:
+        h1.profile(True)
     got = h1.render(-180.05, 179.95, zfar=100000.)
     assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
     views = [(C1_LAT + 0.02 * k, C1_LON - 0.01 * k, -180.05, 179.95) for k in range(3)]
     h1.set_zextents(100., 100000.)
     bi, br = h1.render_batch(views)
+    if profiled:
+        assert h1.profile_read()["renders"] == 2        # the single render and the batch's one chunk
     for k, (la, lo, a0, a1) in enumerate(views):
         for key in env:
             monkeypatch.delenv(key)
@@ -397,8 +395,11 @@ def test_batch_with_more_windows_than_table_slots(hz, tiles_c1):
         assert np.array_equal(bi[k], wi) and np.array_equal(br[k], wr), k
 
 
-@pytest.mark.parametrize("lanes,sets", [(16, 2), (5, 3), (64, 1), (1, 1)])
-def test_ragged_mixed_batch_equals_single_renders(hz, tiles_c1, lanes, sets):
+# chunks of up to 64 views on up to 4 view sets (render_batch_common): 1 view is rendered on the context's own scratch;
+# 5 views are one chunk; 37 are chunks of 10/10/10/7 on four sets, the last one ragged; 257 are four chunks of 64, then
+# set 0 again, while in flight, for 1 view
+@pytest.mark.parametrize("n", [1, 5, 37, 257])
+def test_ragged_mixed_batch_equals_single_renders(hz, tiles_c1, n):
     """A batch is rendered in chunks by launches with a view dimension: more views than one chunk holds, a ragged last
     chunk, wide and zoomed-in windows (different chain shapes) and explicit eye heights in one call -- every view must
     equal its single render bit for bit, whatever the chunking."""
@@ -406,10 +407,9 @@ def test_ragged_mixed_batch_equals_single_renders(hz, tiles_c1, lanes, sets):
     W, H, R = 480, 96, 180
     h = hz.horizonator(C1_LAT, C1_LON, W, H, dir_dems=tiles_c1, render_radius_cells=R)
     h.set_zextents(100., 60000.)
-    h.reload_tunables(HORIZONATOR_LANES=lanes, HORIZONATOR_SETS=sets)
     rs = np.random.RandomState(5)
     views = []
-    for k in range(37):
+    for k in range(n):
         la, lo = C1_LAT + rs.uniform(-0.05, 0.05), C1_LON + rs.uniform(-0.05, 0.05)
         c = rs.uniform(-180, 180)
         half = (180.0, 45.0, 6.0)[k % 3]
@@ -437,7 +437,6 @@ def test_ragged_mixed_batch_equals_single_renders(hz, tiles_c1, lanes, sets):
             wi = hz.pinned_array((H, W, 3), np.uint8); wr = hz.pinned_array((H, W), np.float32)
             h.render_into(wi, wr)
             assert np.array_equal(bi[k], wi) and np.array_equal(br[k], wr), (rep, k)
-    h.reload_tunables(HORIZONATOR_LANES=None, HORIZONATOR_SETS=None)
     # image only / ranges only
     h.render_batch_device(views[:7], di.data_ptr(), 0, torch.cuda.current_stream().cuda_stream)
     torch.cuda.synchronize()

@@ -1,11 +1,11 @@
-"""Sweep of the batch tunables on the C2 workload, in one process (horizonator_reload_tunables):
+"""Batch throughput of the library it loads on the C2 workload:
 
-    python tools/batch_sweep.py [--out gpurun_out/sweep.jsonl] [--reps 5] CONFIG ...
+    python tools/batch_sweep.py [--out sweep.jsonl] [--reps 5] [--batches 16,64]
 
-CONFIG = comma-separated KEY=VALUE with the HORIZONATOR_ prefix dropped, e.g. "LANES=16,SETS=2,GRID_SCALE_BATCH=200"
-(empty string = defaults).  Per config and batch size (16 and 64): device-resident panoramas/s for the benchmark
-viewpoint repeated (what bench.py's `value` is) and for distinct viewpoints of the 8x8 grid over the central degree
-(C5 flavour), with the host time spent enqueueing per panorama.
+Per batch size: device-resident panoramas/s for the benchmark viewpoint repeated (what bench.py's `value` is) and for
+distinct viewpoints of the 8x8 grid over the central degree (C5 flavour), with the host time spent enqueueing per
+panorama.  To compare a compile-time variant, build it under another name (build.py: build_library(extra_flags,
+name=...)) and run this once per library with HORIZONATOR_LIBRARY=<path>.
 """
 import argparse
 import json
@@ -20,8 +20,6 @@ import horizonator_b200 as hz  # noqa: E402
 from tools import synth  # noqa: E402
 
 C2_LAT, C2_LON = 34.0 + 1.0 / 7200.0, -117.0 + 1.0 / 7200.0
-KEYS = ("LANES", "SETS", "GRID_SCALE_BATCH", "GRID_SCALE", "BANDS", "BANDS_BATCH", "NEAR_RINGS", "OCCL_TILE_PIX",
-        "OCCL_BLOCK_PIX", "OCCL_TILE_PIX_BATCH", "OCCL_BLOCK_PIX_BATCH", "SMALL_PIX", "MID_PIX", "GRAPHS", "GRAPH_INSTANCES", "MID_LEVEL", "MID_LEVEL_BATCH", "FORK", "FORK_BATCH")
 
 
 def grid_views(g=8):
@@ -67,7 +65,6 @@ def main():
     ap.add_argument("--grid", action="store_true", help="with --once: the distinct viewpoints of the 8x8 grid (C5 flavour) "
                     "instead of the benchmark viewpoint repeated")
     ap.add_argument("--grid-size", type=int, default=8, help="distinct viewpoints: a g x g grid over the central degree")
-    ap.add_argument("configs", nargs="*", default=[""])
     a = ap.parse_args()
     tiles = synth.config2_tiles(os.environ.get("HZ_BENCH_TILES", "/tmp/hz_tiles_c2"))
     h = hz.horizonator(C2_LAT, C2_LON, 3600, 600, SRTM1=True, dir_dems=tiles, render_radius_m=150000.)
@@ -84,24 +81,17 @@ def main():
             torch.cuda.synchronize()
         return
     grid = grid_views(a.grid_size)
-    out = open(a.out, "a") if a.out else None
-    for cfg in a.configs:
-        env = {"HORIZONATOR_" + k: None for k in KEYS}
-        for kv in filter(None, cfg.split(",")):
-            k, v = kv.split("=")
-            env["HORIZONATOR_" + k] = v.replace(":", ",")
-        h.reload_tunables(**env)
-        row = {"config": cfg}
-        for B in (int(b) for b in a.batches.split(",")):
-            same, enq_same = timed(h, [(C2_LAT, C2_LON, -180.05, 179.95)] * max(B, 64), B, d_img, d_rng, a.reps)
-            dist, enq_dist = timed(h, grid, B, d_img, d_rng, a.reps)
-            row["B%d" % B] = {"same_view_pano_s": round(same), "host_us_per_pano": round(enq_same, 2),
-                              "grid_pano_s": round(dist), "grid_host_us_per_pano": round(enq_dist, 2)}
-        line = json.dumps(row)
-        print(line, flush=True)
-        if out:
+    row = {"library": hz.LIBRARY_PATH}
+    for B in (int(b) for b in a.batches.split(",")):
+        same, enq_same = timed(h, [(C2_LAT, C2_LON, -180.05, 179.95)] * max(B, 64), B, d_img, d_rng, a.reps)
+        dist, enq_dist = timed(h, grid, B, d_img, d_rng, a.reps)
+        row["B%d" % B] = {"same_view_pano_s": round(same), "host_us_per_pano": round(enq_same, 2),
+                          "grid_pano_s": round(dist), "grid_host_us_per_pano": round(enq_dist, 2)}
+    line = json.dumps(row)
+    print(line, flush=True)
+    if a.out:
+        with open(a.out, "a") as out:
             out.write(line + "\n")
-            out.flush()
 
 
 if __name__ == "__main__":

@@ -18,5 +18,5 @@ python tools/launch_table.py gpurun_out/${T}_launch_grid256.csv --last 184 --vie
 # (the report itself is ~70 MB, more than gpurun copies back: it stays in /tmp, its summary comes home)
 ncu --set full --clock-control none --import-source on -k regex:"k_mesh|k_blocks|k_raster|k_tiles|k_big|k_resolve4|k_near|k_prepare" -s 368 -c 46 -o /tmp/${T}_batch_chain python tools/batch_sweep.py --once 256 > gpurun_out/${T}_ncu_full.log 2>&1
 python tools/ncu_summary.py /tmp/${T}_batch_chain.ncu-rep > gpurun_out/${T}_batch_chain_ncu_summary.txt 2>&1
-HORIZONATOR_TRACE_HOST=1 python tools/batch_sweep.py --reps 4 --batches 16,64,256 --grid-size 16 --out gpurun_out/${T}_sweep.jsonl "" 2>&1 | tail -2 | tee gpurun_out/${T}_host_trace.txt
+python tools/batch_sweep.py --reps 4 --batches 16,64,256 --grid-size 16
 ls -la gpurun_out | tail -20

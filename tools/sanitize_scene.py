@@ -1,13 +1,9 @@
 """One mid-size scene through every kernel and host path, for compute-sanitizer: single renders (wide and zoomed-in:
-near pass, bands, large triangles, middle-sized triangles), a batch of 11 views in chunks with a view dimension on
-three view sets, pageable and page-locked destinations, a wedge into a host panorama, the horizon profile."""
+near pass, bands, large triangles, middle-sized triangles), a batch of 11 views in chunks of 8 and 3 with a view
+dimension on two view sets, pageable and page-locked destinations, a wedge into a host panorama, the horizon profile."""
 import os, sys, tempfile
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
-os.environ.setdefault("HORIZONATOR_BANDS", "6")
-os.environ.setdefault("HORIZONATOR_BANDS_BATCH", "5,9")
-os.environ.setdefault("HORIZONATOR_LANES", "4")
-os.environ.setdefault("HORIZONATOR_SETS", "3")
 import horizonator_b200 as hz
 from tools import synth
 d = synth.config1_tiles(os.path.join(tempfile.gettempdir(), "hz_smoke_tiles"))
