@@ -17,8 +17,11 @@
 #include <cstring>
 #include <atomic>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <thread>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 namespace {
@@ -41,10 +44,68 @@ constexpr float PI_F            = 3.14159265358979f;       // vertex.glsl:31
 //   set-up records of those triangles:                         max(2^18, pixels/16); beyond that k_big repeats the set-up
 constexpr int   PROF_EVENTS     = 7;            // 6 stages per render
 constexpr int   MAX_BANDS       = HZ_MAX_BANDS;
-// [0] big_count near, [1] spare, [2] tri_count near, [3] big-triangle records, [4+4b] tile_count,
-// [5+4b] block_count, [6+4b] tri_count, [7+4b] big_count of band b, then the stats
-constexpr int   STATS_AT        = 4 + 4 * MAX_BANDS;
-constexpr int   N_COUNTERS      = STATS_AT + HZ_STAT_COUNT;
+
+// The counters of a render (a scratch's d_counters).  k_prepare zeroes all N_COUNTERS words; the kernels get
+// pointers to the single words.
+struct BandCounters { uint32_t tile, block, tri, big; };   // live tiles, live blocks, listed triangles, big-triangle entries
+struct Counters
+{
+    uint32_t near_big;                 // entries of the near pass's big-triangle queue
+    uint32_t near_tri;                 // triangles of the near pass's list
+    uint32_t bigtri;                   // big-triangle records (one pool for all passes)
+    BandCounters band[MAX_BANDS];
+    uint32_t stats[HZ_STAT_COUNT];     // horizonator_render_counters
+};
+constexpr int   N_COUNTERS      = sizeof(Counters) / sizeof(uint32_t);
+
+// ---- owning handles of CUDA resources: a handle releases what it holds when its owner goes or when another handle
+// is assigned to it.  The make_*() helpers return an empty handle on failure (cudaGetLastError() says why).
+struct DeviceFree    { void operator()(void* p) const { cudaFree(p); } };
+struct HostFree      { void operator()(void* p) const { cudaFreeHost(p); } };
+struct StreamFree    { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventFree     { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct GraphExecFree { void operator()(cudaGraphExec_t e) const { cudaGraphExecDestroy(e); } };
+struct GraphFree     { void operator()(cudaGraph_t g) const { cudaGraphDestroy(g); } };
+
+template<class T> using DevPtr  = std::unique_ptr<T, DeviceFree>;     // device memory
+template<class T> using HostPtr = std::unique_ptr<T, HostFree>;       // page-locked host memory
+using StreamHandle    = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamFree>;
+using EventHandle     = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventFree>;
+using GraphExecHandle = std::unique_ptr<std::remove_pointer_t<cudaGraphExec_t>, GraphExecFree>;
+using GraphHandle     = std::unique_ptr<std::remove_pointer_t<cudaGraph_t>, GraphFree>;
+
+template<class T> DevPtr<T> make_device(size_t n)
+{
+    void* p = nullptr;
+    return DevPtr<T>(cudaMalloc(&p, n * sizeof(T)) == cudaSuccess ? (T*)p : nullptr);
+}
+
+template<class T> HostPtr<T> make_host(size_t n)
+{
+    void* p = nullptr;
+    return HostPtr<T>(cudaMallocHost(&p, n * sizeof(T)) == cudaSuccess ? (T*)p : nullptr);
+}
+
+StreamHandle make_stream()
+{
+    cudaStream_t s = nullptr;
+    return StreamHandle(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) == cudaSuccess ? s : nullptr);
+}
+
+// (events that time kernels: flags = cudaEventDefault)
+EventHandle make_event(unsigned int flags = cudaEventDisableTiming)
+{
+    cudaEvent_t e = nullptr;
+    return EventHandle(cudaEventCreateWithFlags(&e, flags) == cudaSuccess ? e : nullptr);
+}
+
+// true if a make_*() helper left h empty, after reporting the error as CUDA_TRY does
+template<class H> bool empty_handle(const H& h, const char* what)
+{
+    if(h) return false;
+    MSG("CUDA error: %s failed: %s", what, cudaGetErrorString(cudaGetLastError()));
+    return true;
+}
 
 // ---- the render chain's configuration.  Each value won its sweep (profiles/); a new sweep edits a constant and
 // compares a second build of the library (build_library(extra_flags, name) + HORIZONATOR_LIBRARY).
@@ -94,21 +155,21 @@ struct TanelKey
     bool is(float daz_, int W_, int H_) const { return valid && W == W_ && H == H_ && memcmp(&daz, &daz_, sizeof(float)) == 0; }
 };
 
-// everything one view in flight writes besides its outputs
+// everything one view in flight writes besides its outputs (the device buffers: scratch_buffers)
 struct Scratch
 {
-    unsigned long long* d_vis = nullptr;
-    float *d_e = nullptr, *d_n = nullptr;
-    uint32_t *d_tile_queue = nullptr, *d_block_queue = nullptr, *d_tri_queue = nullptr;
-    uint2*    d_big_queue = nullptr;   // [2][BIG_CAPACITY]: near pass, bands
-    uint4*    d_bigtri = nullptr;      // [BIGTRI_CAPACITY][6]
-    uint32_t* d_counters  = nullptr;   // [N_COUNTERS]
-    uint8_t*  d_image  = nullptr;      // batch sets only: staging of one view's outputs for the host-pointer batch call
-    float*    d_ranges = nullptr;
+    DevPtr<unsigned long long> d_vis;
+    DevPtr<float>    d_e, d_n;
+    DevPtr<uint32_t> d_tile_queue, d_block_queue, d_tri_queue;
+    DevPtr<uint2>    d_big_queue;      // [2][BIG_CAPACITY]: near pass, bands
+    DevPtr<uint4>    d_bigtri;         // [BIGTRI_CAPACITY][6]
+    DevPtr<Counters> d_counters;
+    DevPtr<uint8_t>  d_image;          // batch sets only: staging of one view's outputs for the host-pointer batch call
+    DevPtr<float>    d_ranges;
     // tan(elevation) per row of the window this scratch last rendered (lib:1007-1012; computed on the host like the
     // reference's read-back does, uploaded on the stream of the render that needs it -- so nothing else can be
     // reading the row when it is replaced)
-    float*    d_tanel = nullptr;       // [H]
+    DevPtr<float>    d_tanel;          // [H]
     TanelKey  tanel_key;
     // renders made with this visibility buffer since it was allocated: the epoch of the keys counts down from 7 with it,
     // and the buffer is cleared only when that wraps (hz_device.h, the visibility key)
@@ -123,28 +184,28 @@ struct ViewSet
 {
     int  cap = 0;
     bool batch = false;                // the chain configuration of batched views (config_of)
-    cudaStream_t stream = nullptr;     // batch sets only
-    cudaEvent_t  done = nullptr;       // batch sets only
+    StreamHandle stream;               // batch sets only
+    EventHandle  done;                 // batch sets only
     std::vector<Scratch> sc;           // grows on demand up to cap (ensure_views)
 
     // parameters of the renders in flight: the kernels read d_views; the host fills a slot of the pinned ring and
     // copies it over (the ring lets several renders be queued without waiting)
-    HzView* d_views = nullptr;         // [cap][HZ_V_COUNT]
-    HzView* h_views = nullptr;         // pinned [PARAM_RING][cap][HZ_V_COUNT]
-    float*  h_tanel = nullptr;         // pinned [PARAM_RING][cap][H] (alloc_target)
-    cudaEvent_t ring_ev[PARAM_RING] = {};
+    DevPtr<HzView>  d_views;           // [cap][HZ_V_COUNT]
+    HostPtr<HzView> h_views;           // pinned [PARAM_RING][cap][HZ_V_COUNT]
+    HostPtr<float>  h_tanel;           // pinned [PARAM_RING][cap][H] (alloc_set_target)
+    EventHandle ring_ev[PARAM_RING];
     int ring_next = 0;
-    cudaEvent_t  busy = nullptr;       // recorded after the last render that used this set
+    EventHandle  busy;                 // recorded after the last render that used this set
     // the large triangles of the near pass (k_big) are drawn beside the first bands, on a stream of their own
     // (launch_chain): fork after the near pass's k_raster, join before the resolve
-    cudaStream_t side = nullptr;
-    cudaEvent_t  ev_fork = nullptr, ev_join = nullptr;
+    StreamHandle side;
+    EventHandle  ev_fork, ev_join;
     cudaStream_t last_stream = nullptr;
     bool busy_recorded = false;
     // the standard chain, captured on first use per (number of views, shape)
     // (several executable instances each, used in turn: an instance that is still in flight makes the next launch of
     // the SAME instance wait on the host)
-    struct Graph { int m; bool big_per_band; std::vector<cudaGraphExec_t> exec; size_t next; int launches; };
+    struct Graph { int m; bool big_per_band; std::vector<GraphExecHandle> exec; size_t next; int launches; };
     std::vector<Graph> graphs;
     bool graph_failed = false;
 };
@@ -152,26 +213,27 @@ struct ViewSet
 struct Slot
 {
     int device = 0;
-    cudaStream_t stream = nullptr;
+    StreamHandle stream;
 
     // terrain
     int N = 0, pitch = 0, cpd = 0;
-    int16_t* d_mosaic = nullptr;
-    HzTiles  tiles{};
-    short2 *d_mm_block = nullptr, *d_mm_tile = nullptr;   // culling pyramid
+    DevPtr<int16_t> d_mosaic;
+    HzTiles tiles{};
+    DevPtr<uint8_t> d_tiles[4][4];     // what tiles.tile points to
+    DevPtr<short2> d_mm_block, d_mm_tile;    // culling pyramid
     int nb = 0, nt = 0;
 
     // target
     int W = 0, H = 0;
-    uint8_t* d_image  = nullptr;
-    float*   d_ranges = nullptr;
+    DevPtr<uint8_t> d_image;
+    DevPtr<float>   d_ranges;
     size_t   target_pixels = 0;      // capacity of the buffers above
     uint32_t tri_capacity = 0, big_capacity = 0, bigtri_capacity = 0;
 
     // page-locked staging for results that go to pageable host memory (copy_to_pageable): made on first use
-    char*  h_stage = nullptr;
+    HostPtr<char> h_stage;
     size_t h_stage_bytes = 0;
-    std::vector<cudaEvent_t> stage_ev;
+    std::vector<EventHandle> stage_ev;
 
     // host-side cache of tan(elevation) row tables (tanf() per row is not free; callers re-render the same few windows)
     struct TanelRow { TanelKey key; std::vector<float> row; };
@@ -181,8 +243,8 @@ struct Slot
     // `main` serves the single-view entry points (and keeps the last visibility buffer for horizonator_pick);
     // `sets` are made on demand by the batch entry points.
     ViewSet main;
-    std::vector<ViewSet*> sets;
-    cudaEvent_t fork_ev = nullptr;
+    std::vector<std::unique_ptr<ViewSet>> sets;
+    EventHandle fork_ev;
 
     ViewState view;
     float znear = HORIZONATOR_ZNEAR_DEFAULT, zfar = HORIZONATOR_ZFAR_DEFAULT;
@@ -197,18 +259,20 @@ struct Slot
     bool  seam_wrap = false;         // opt-in (horizonator_set_seam_wrap); false = seam triangles dropped like the reference
     float curvature = 0.f;           // opt-in (horizonator_set_earth_curvature); 0 = flat earth like the reference
     bool collect_stats = false;      // culling counters (horizonator_render_counters); off: the kernels skip them
-    std::vector<cudaEvent_t> prof_events;
+    std::vector<EventHandle> prof_events;
     size_t prof_used = 0;
 
     // viewsheds, allocated by the first viewshed call that needs them: the masks of one chunk of views for calls that
     // want only counts or want the masks in host memory, and the counts of the host-memory call.  A call's stream
     // waits for `vs_done` of the call before it, which may have been queued on another stream and use the same scratch.
-    uint32_t* d_vs_masks = nullptr;
-    int       vs_mask_views = 0;
-    uint32_t* d_vs_counts = nullptr;
-    cudaEvent_t vs_done = nullptr;
+    DevPtr<uint32_t> d_vs_masks;
+    int              vs_mask_views = 0;
+    DevPtr<uint32_t> d_vs_counts;
+    EventHandle      vs_done;
 };
 
+// raw pointers: a slot is deleted by horizonator_deinit(), never by a destructor at exit, when the CUDA runtime may
+// already be gone
 std::mutex          g_table_mutex;
 std::vector<Slot*>  g_table;         // handle = index + 1
 
@@ -232,73 +296,71 @@ struct DeviceGuard
     ~DeviceGuard() { if(prev >= 0) cudaSetDevice(prev); }
 };
 
-void drop_graphs(ViewSet& vs)
+// The device buffers of a scratch, as (member, number of elements): those sized by the terrain unless `image_only`,
+// then, if the slot has a target, those sized by the image (staging: the outputs of a batch set's view).
+// alloc_scratch() allocates them from this list, and ensure_views() budgets with its sum.
+template<class F> void scratch_buffers(const Slot& s, bool staging, bool image_only, F&& f)
 {
-    for(ViewSet::Graph& g : vs.graphs) for(cudaGraphExec_t e : g.exec) cudaGraphExecDestroy(e);
-    vs.graphs.clear();
-    vs.graph_failed = false;
-}
-
-// the part of a scratch whose size depends on the image
-void free_scratch_target(Scratch& c)
-{
-    cudaFree(c.d_vis); cudaFree(c.d_image); cudaFree(c.d_ranges);
-    cudaFree(c.d_tri_queue); cudaFree(c.d_big_queue); cudaFree(c.d_bigtri); cudaFree(c.d_tanel);
-    c.d_vis = nullptr; c.d_image = nullptr; c.d_ranges = nullptr;
-    c.d_tri_queue = nullptr; c.d_big_queue = nullptr; c.d_bigtri = nullptr; c.d_tanel = nullptr;
-    c.tanel_key = TanelKey{};
-    c.renders = 0;
-}
-
-bool alloc_scratch_target(const Slot& s, Scratch& c, bool staging)
-{
+    if(!image_only)
+    {
+        f(&Scratch::d_e, (size_t)s.N + HZ_MESH_PAD);
+        f(&Scratch::d_n, (size_t)s.N + HZ_MESH_PAD);
+        f(&Scratch::d_tile_queue, (size_t)s.nt * s.nt);
+        f(&Scratch::d_block_queue, (size_t)s.nb * s.nb);
+        f(&Scratch::d_counters, (size_t)1);
+    }
     const size_t px = s.target_pixels;
-    CUDA_TRY(cudaMalloc(&c.d_vis, px * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMalloc(&c.d_tri_queue, (size_t)s.tri_capacity * sizeof(uint32_t)));
-    CUDA_TRY(cudaMalloc(&c.d_big_queue, 2 * (size_t)s.big_capacity * sizeof(uint2)));
-    CUDA_TRY(cudaMalloc(&c.d_bigtri, (size_t)s.bigtri_capacity * 6 * sizeof(uint4)));
-    CUDA_TRY(cudaMalloc(&c.d_tanel, (size_t)s.H * sizeof(float)));
+    if(px == 0) return;
+    f(&Scratch::d_vis, px);
+    f(&Scratch::d_tri_queue, (size_t)s.tri_capacity);
+    f(&Scratch::d_big_queue, 2 * (size_t)s.big_capacity);
+    f(&Scratch::d_bigtri, 6 * (size_t)s.bigtri_capacity);
+    f(&Scratch::d_tanel, (size_t)s.H);
     if(staging)
     {
-        CUDA_TRY(cudaMalloc(&c.d_image, px * 3));
-        CUDA_TRY(cudaMalloc(&c.d_ranges, px * sizeof(float)));
+        f(&Scratch::d_image, 3 * px);
+        f(&Scratch::d_ranges, px);
     }
+}
+
+// Allocates the buffers scratch_buffers() lists and moves them into c once all of them are there (assigning a handle
+// releases the buffer it held).  A new visibility buffer starts a new count of renders: its first render clears it.
+bool alloc_scratch(const Slot& s, Scratch& c, bool staging, bool image_only)
+{
+    Scratch fresh;
+    bool ok = true;
+    scratch_buffers(s, staging, image_only, [&](auto m, size_t n) {
+        using T = typename std::remove_reference_t<decltype(fresh.*m)>::element_type;
+        if(ok) ok = (fresh.*m = make_device<T>(n)) != nullptr;
+    });
+    if(!ok) return false;
+    scratch_buffers(s, staging, image_only, [&](auto m, size_t) { c.*m = std::move(fresh.*m); });
+    c.tanel_key = TanelKey{};
+    c.renders = 0;
     return true;
 }
 
-void free_set_target(ViewSet& vs)
-{
-    drop_graphs(vs);
-    for(Scratch& c : vs.sc) free_scratch_target(c);
-    cudaFreeHost(vs.h_tanel); vs.h_tanel = nullptr;
-}
-
+// (Re)allocates what of a set depends on the image, one scratch at a time so that a whole set's old and new buffers are
+// never in memory together.  The captured chains hold the addresses of the old buffers, so they go first.
 bool alloc_set_target(const Slot& s, ViewSet& vs)
 {
-    CUDA_TRY(cudaMallocHost(&vs.h_tanel, (size_t)PARAM_RING * vs.cap * s.H * sizeof(float)));
-    for(Scratch& c : vs.sc) if(!alloc_scratch_target(s, c, vs.batch)) return false;
+    vs.graphs.clear();
+    vs.graph_failed = false;
+    if(s.target_pixels == 0) return true;
+    HostPtr<float> h_tanel = make_host<float>((size_t)PARAM_RING * vs.cap * s.H);
+    if(!h_tanel) return false;
+    for(Scratch& c : vs.sc) if(!alloc_scratch(s, c, vs.batch, true)) return false;
+    vs.h_tanel = std::move(h_tanel);
     return true;
-}
-
-void free_target(Slot& s)
-{
-    free_set_target(s.main);
-    for(ViewSet* g : s.sets) free_set_target(*g);
-    cudaFree(s.d_image);  s.d_image = nullptr;
-    cudaFree(s.d_ranges); s.d_ranges = nullptr;
-    cudaFreeHost(s.h_stage); s.h_stage = nullptr; s.h_stage_bytes = 0;
-    for(cudaEvent_t e : s.stage_ev) cudaEventDestroy(e);
-    s.stage_ev.clear();
-    s.target_pixels = 0;
-    s.tanel_cache.clear();
 }
 
 // A failure part way leaves the context without a target (W = H = 0): later renders return false instead of
 // running kernels on buffers that are not there.
 bool alloc_target(Slot& s, int W, int H)
 {
-    free_target(s);
-    s.W = 0; s.H = 0; s.have_render = false;
+    s.W = 0; s.H = 0; s.target_pixels = 0; s.have_render = false;
+    s.h_stage = nullptr; s.h_stage_bytes = 0;      // sized for the old target; copy_results_to_host makes a new one
+    s.tanel_cache.clear();
     const size_t px = (size_t)W * (size_t)H;
     auto cap = [px](size_t floor_, size_t div) {
         const size_t c = px / div > floor_ ? px / div : floor_;
@@ -309,80 +371,37 @@ bool alloc_target(Slot& s, int W, int H)
     if(const char* env = getenv("HORIZONATOR_TRI_CAPACITY"))    s.tri_capacity    = (uint32_t)(atoi(env) > 1 ? atoi(env) : 1);
     if(const char* env = getenv("HORIZONATOR_BIG_CAPACITY"))    s.big_capacity    = (uint32_t)(atoi(env) > 1 ? atoi(env) : 1);
     if(const char* env = getenv("HORIZONATOR_BIGTRI_CAPACITY")) s.bigtri_capacity = (uint32_t)(atoi(env) > 1 ? atoi(env) : 1);
-    s.target_pixels = px; s.W = W; s.H = H;       // alloc_*_target() size their buffers from these
-    bool ok = alloc_set_target(s, s.main);
-    for(ViewSet* g : s.sets) ok = ok && alloc_set_target(s, *g);
-    ok = ok && cudaMalloc(&s.d_image, px * 3) == cudaSuccess && cudaMalloc(&s.d_ranges, px * sizeof(float)) == cudaSuccess;
+    s.target_pixels = px; s.W = W; s.H = H;       // scratch_buffers() sizes the buffers from these
+    DevPtr<uint8_t> image = make_device<uint8_t>(px * 3);
+    DevPtr<float> ranges = make_device<float>(px);
+    bool ok = image && ranges && alloc_set_target(s, s.main);
+    for(const auto& g : s.sets) ok = ok && alloc_set_target(s, *g);
     if(!ok)
     {
         MSG("Could not allocate the %d x %d render target", W, H);
         cudaGetLastError();
-        free_target(s);
-        s.W = 0; s.H = 0;
+        s.W = 0; s.H = 0; s.target_pixels = 0;
         return false;
     }
+    s.d_image = std::move(image);
+    s.d_ranges = std::move(ranges);
     return true;
-}
-
-void free_scratch(Scratch& c)
-{
-    free_scratch_target(c);
-    cudaFree(c.d_e); cudaFree(c.d_n);
-    cudaFree(c.d_tile_queue); cudaFree(c.d_block_queue);
-    cudaFree(c.d_counters);
-    c = Scratch{};
-}
-
-// everything but the image-sized part (alloc_scratch_target)
-bool alloc_scratch(const Slot& s, Scratch& c)
-{
-    CUDA_TRY(cudaMalloc(&c.d_e, (size_t)(s.N + HZ_MESH_PAD) * sizeof(float)));
-    CUDA_TRY(cudaMalloc(&c.d_n, (size_t)(s.N + HZ_MESH_PAD) * sizeof(float)));
-    CUDA_TRY(cudaMalloc(&c.d_tile_queue, (size_t)s.nt * s.nt * sizeof(uint32_t)));
-    CUDA_TRY(cudaMalloc(&c.d_block_queue, (size_t)s.nb * s.nb * sizeof(uint32_t)));
-    CUDA_TRY(cudaMalloc(&c.d_counters, N_COUNTERS * sizeof(uint32_t)));
-    return true;
-}
-
-void free_set(ViewSet& vs)
-{
-    free_set_target(vs);
-    for(Scratch& c : vs.sc) free_scratch(c);
-    vs.sc.clear();
-    cudaFree(vs.d_views); cudaFreeHost(vs.h_views);
-    for(cudaEvent_t e : vs.ring_ev) if(e) cudaEventDestroy(e);
-    if(vs.busy) cudaEventDestroy(vs.busy);
-    if(vs.ev_fork) cudaEventDestroy(vs.ev_fork);
-    if(vs.ev_join) cudaEventDestroy(vs.ev_join);
-    if(vs.side) cudaStreamDestroy(vs.side);
-    if(vs.done) cudaEventDestroy(vs.done);
-    if(vs.stream) cudaStreamDestroy(vs.stream);
-    vs = ViewSet{};
 }
 
 // the set's own resources; its scratches come with ensure_views()
-bool alloc_set(ViewSet& vs, int cap, bool batch)
+bool alloc_set(ViewSet& out, int cap, bool batch)
 {
+    ViewSet vs;
     vs.cap = cap; vs.batch = batch;
-    CUDA_TRY(cudaMalloc(&vs.d_views, (size_t)cap * HZ_V_COUNT * sizeof(HzView)));
-    CUDA_TRY(cudaMallocHost(&vs.h_views, (size_t)PARAM_RING * cap * HZ_V_COUNT * sizeof(HzView)));
-    for(cudaEvent_t& e : vs.ring_ev) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventCreateWithFlags(&vs.busy, cudaEventDisableTiming));
-    if(batch)
-    {
-        CUDA_TRY(cudaStreamCreateWithFlags(&vs.stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&vs.done, cudaEventDisableTiming));
-    }
+    vs.d_views = make_device<HzView>((size_t)cap * HZ_V_COUNT);
+    vs.h_views = make_host<HzView>((size_t)PARAM_RING * cap * HZ_V_COUNT);
+    bool ok = vs.d_views && vs.h_views;
+    for(EventHandle& e : vs.ring_ev) ok = ok && (e = make_event());
+    ok = ok && (vs.busy = make_event()) && (vs.side = make_stream()) && (vs.ev_fork = make_event()) && (vs.ev_join = make_event());
+    if(batch) ok = ok && (vs.stream = make_stream()) && (vs.done = make_event());
+    if(!ok) return false;
+    out = std::move(vs);
     return true;
-}
-
-// bytes of device memory one scratch takes (what ensure_views() budgets with)
-size_t scratch_bytes(const Slot& s)
-{
-    const size_t px = s.target_pixels;
-    return px * (sizeof(unsigned long long) + 3 + sizeof(float)) +
-           ((size_t)s.tri_capacity + (size_t)s.nt * s.nt + (size_t)s.nb * s.nb + 2 * (size_t)s.N) * sizeof(uint32_t) +
-           2 * (size_t)s.big_capacity * sizeof(uint2) + (size_t)s.bigtri_capacity * 6 * sizeof(uint4);
 }
 
 // Makes sure the set has scratch for up to n views (n <= cap) and returns how many it has to use.  Batch sets only
@@ -393,20 +412,20 @@ int ensure_views(Slot& s, ViewSet& vs, int n)
     if(n > vs.cap) n = vs.cap;
     while((int)vs.sc.size() < n)
     {
+        Scratch c;
         if(vs.batch)
         {
-            size_t free_b = 0, total_b = 0;
-            if(cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || scratch_bytes(s) > free_b / 2) break;
+            size_t bytes = 0, free_b = 0, total_b = 0;
+            scratch_buffers(s, true, false, [&](auto m, size_t len) { bytes += len * sizeof(*(c.*m)); });
+            if(cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || bytes > free_b / 2) break;
         }
-        Scratch c;
-        if(!alloc_scratch(s, c) || (s.target_pixels > 0 && !alloc_scratch_target(s, c, vs.batch)))
+        if(!alloc_scratch(s, c, vs.batch, false))
         {
             MSG("Could not allocate the scratch of view %d of a set", (int)vs.sc.size());
             cudaGetLastError();
-            free_scratch(c);
             break;
         }
-        vs.sc.push_back(c);
+        vs.sc.push_back(std::move(c));
     }
     return (int)vs.sc.size() < n ? (int)vs.sc.size() : n;
 }
@@ -414,43 +433,29 @@ int ensure_views(Slot& s, ViewSet& vs, int n)
 // the batch sets: up to N_SETS_MAX, created on demand
 ViewSet* batch_set(Slot& s, int k)
 {
-    if(s.fork_ev == nullptr && cudaEventCreateWithFlags(&s.fork_ev, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+    if(!s.fork_ev && !(s.fork_ev = make_event())) return nullptr;
     while((int)s.sets.size() <= k)
     {
-        ViewSet* g = new ViewSet;
-        bool ok = alloc_set(*g, VIEWS_PER_SET, true);
-        if(ok && s.target_pixels > 0)
-            ok = cudaMallocHost(&g->h_tanel, (size_t)PARAM_RING * g->cap * s.H * sizeof(float)) == cudaSuccess;
-        if(!ok)
+        auto g = std::make_unique<ViewSet>();
+        if(!alloc_set(*g, VIEWS_PER_SET, true) || !alloc_set_target(s, *g))
         {
             MSG("Could not allocate view set %d", (int)s.sets.size());
             cudaGetLastError();
-            free_set(*g);
-            delete g;
             return nullptr;
         }
-        s.sets.push_back(g);
+        s.sets.push_back(std::move(g));
     }
-    return s.sets[k];
+    return s.sets[k].get();
 }
 
+// waits for the slot's work, then releases it (its handles)
 void destroy_slot(Slot* s)
 {
     if(s == nullptr) return;
     DeviceGuard g(s->device);
-    if(s->stream) cudaStreamSynchronize(s->stream);
-    for(ViewSet* v : s->sets) if(v->stream) cudaStreamSynchronize(v->stream);
-    free_target(*s);
-    free_set(s->main);
-    for(ViewSet* v : s->sets) { free_set(*v); delete v; }
-    if(s->fork_ev) cudaEventDestroy(s->fork_ev);
-    cudaFree(s->d_mosaic);
-    for(int i = 0; i < 4; i++) for(int j = 0; j < 4; j++) cudaFree((void*)s->tiles.tile[i][j]);
-    for(cudaEvent_t e : s->prof_events) cudaEventDestroy(e);
-    cudaFree(s->d_mm_block); cudaFree(s->d_mm_tile);
-    if(s->vs_done) { cudaEventSynchronize(s->vs_done); cudaEventDestroy(s->vs_done); }
-    cudaFree(s->d_vs_masks); cudaFree(s->d_vs_counts);
-    if(s->stream) cudaStreamDestroy(s->stream);
+    if(s->stream) cudaStreamSynchronize(s->stream.get());
+    for(const auto& v : s->sets) cudaStreamSynchronize(v->stream.get());
+    if(s->vs_done) cudaEventSynchronize(s->vs_done.get());
     delete s;
 }
 
@@ -512,37 +517,31 @@ bool big_after_every_band(const Slot& s, const ViewState& vs)
 
 // the kernels of one render of m views, in order, reading their parameters from set.d_views; hv = the host copy of those
 bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool worst_case, bool resolve,
-                  cudaStream_t st, cudaEvent_t* ev, int* launches)
+                  cudaStream_t st, const EventHandle* ev, int* launches)
 {
-    const HzView* dv = set.d_views;
+    const HzView* dv = set.d_views.get();
     int n = 0;
-    if(ev) CUDA_TRY(cudaEventRecord(ev[0], st));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[0].get(), st));
     CUDA_TRY(hz_launch_prepare(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++;
-    if(ev) CUDA_TRY(cudaEventRecord(ev[1], st));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[1].get(), st));
     CUDA_TRY(hz_launch_near(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++;
     CUDA_TRY(hz_launch_raster(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++;
-    if(ev) CUDA_TRY(cudaEventRecord(ev[2], st));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[2].get(), st));
     // The near pass's large triangles: in line, or (fork) beside the bands on the set's side stream.  The bands' culling
     // then sees less of the foreground in the visibility buffer -- it only ever removes work, the image is the same --
     // and the chain is a kernel shorter.  Measured on one box against the chain in line: lone C2 view 111 -> 108 us,
     // 10-degree zoom 0.38 -> 0.35 ms, 5-degree 0.28 -> 0.25 ms, eye 12 km +1 %, batches +0.5 %.  A profiled chain
     // (ev) runs it in line, so that the events time each kernel.
     const bool fork = ev == nullptr;
-    if(fork && set.side == nullptr)
-    {
-        CUDA_TRY(cudaEventCreateWithFlags(&set.ev_fork, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&set.ev_join, cudaEventDisableTiming));
-        CUDA_TRY(cudaStreamCreateWithFlags(&set.side, cudaStreamNonBlocking));
-    }
     if(fork)
     {
-        CUDA_TRY(cudaEventRecord(set.ev_fork, st));
-        CUDA_TRY(cudaStreamWaitEvent(set.side, set.ev_fork, 0));
-        CUDA_TRY(hz_launch_big(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, set.side)); n++;
-        CUDA_TRY(cudaEventRecord(set.ev_join, set.side));
+        CUDA_TRY(cudaEventRecord(set.ev_fork.get(), st));
+        CUDA_TRY(cudaStreamWaitEvent(set.side.get(), set.ev_fork.get(), 0));
+        CUDA_TRY(hz_launch_big(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, set.side.get())); n++;
+        CUDA_TRY(cudaEventRecord(set.ev_join.get(), set.side.get()));
     }
     else { CUDA_TRY(hz_launch_big(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
-    if(ev) CUDA_TRY(cudaEventRecord(ev[3], st));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[3].get(), st));
     const int n_bands = n_bands_of(s, set);
     for(int b = 0; b < n_bands; b++)
     {
@@ -550,14 +549,14 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
         int k = 0;
         CUDA_TRY(hz_launch_band(hv[HZ_V_BAND0 + b], dv + HZ_V_BAND0 + b, m, worst_case, st, &k));
         n += k;
-        if(last && ev) CUDA_TRY(cudaEventRecord(ev[4], st));
+        if(last && ev) CUDA_TRY(cudaEventRecord(ev[4].get(), st));
         // all bands share one queue and counter unless every band has its own k_big (see fill_views)
         if(last || (big_per_band && k > 0)) { CUDA_TRY(hz_launch_big(hv[HZ_V_BAND0 + b], dv + HZ_V_BAND0 + b, m, st)); n++; }
     }
-    if(ev) CUDA_TRY(cudaEventRecord(ev[5], st));
-    if(fork) CUDA_TRY(cudaStreamWaitEvent(st, set.ev_join, 0));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[5].get(), st));
+    if(fork) CUDA_TRY(cudaStreamWaitEvent(st, set.ev_join.get(), 0));
     if(resolve) { CUDA_TRY(hz_launch_resolve(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
-    if(ev) CUDA_TRY(cudaEventRecord(ev[6], st));
+    if(ev) CUDA_TRY(cudaEventRecord(ev[6].get(), st));
     *launches = n;
     return true;
 }
@@ -567,32 +566,30 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
 // launches cost more host time than the GPU needs for the render.
 ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band)
 {
-    cudaStream_t cs = nullptr;
-    if(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-    cudaGraph_t g = nullptr;
-    std::vector<cudaGraphExec_t> exec;
-    bool ok = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
+    const StreamHandle cs = make_stream();
+    if(!cs) { cudaGetLastError(); return nullptr; }
+    cudaGraph_t captured = nullptr;
+    bool ok = cudaStreamBeginCapture(cs.get(), cudaStreamCaptureModeThreadLocal) == cudaSuccess;
     int launches = 0;
     if(ok)
     {
-        ok = launch_chain(s, set, hv, m, big_per_band, true, true, cs, nullptr, &launches);
-        if(cudaStreamEndCapture(cs, &g) != cudaSuccess) ok = false;
+        ok = launch_chain(s, set, hv, m, big_per_band, true, true, cs.get(), nullptr, &launches);
+        if(cudaStreamEndCapture(cs.get(), &captured) != cudaSuccess) ok = false;
     }
+    const GraphHandle g(captured);
+    std::vector<GraphExecHandle> exec;
     for(int k = 0; ok && k < GRAPH_INSTANCES; k++)
     {
         cudaGraphExec_t e = nullptr;
-        if(cudaGraphInstantiate(&e, g, 0) != cudaSuccess) ok = false; else exec.push_back(e);
+        if(cudaGraphInstantiate(&e, g.get(), 0) != cudaSuccess) ok = false; else exec.emplace_back(e);
     }
-    if(!ok) for(cudaGraphExec_t e : exec) cudaGraphExecDestroy(e);
-    if(g) cudaGraphDestroy(g);
-    cudaStreamDestroy(cs);
     if(!ok)
     {
         cudaGetLastError();
         MSG("CUDA graph capture of the render chain failed; launching the kernels one by one instead");
         return nullptr;
     }
-    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, exec, 0, launches });
+    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, std::move(exec), 0, launches });
     return &set.graphs.back();
 }
 
@@ -619,10 +616,10 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
                HzView& v)
 {
     v = HzView{};
-    v.mosaic = s.d_mosaic; v.N = s.N; v.pitch = s.pitch;
-    v.e_tab = sc.d_e; v.n_tab = sc.d_n;
-    v.mm_block = s.d_mm_block; v.nb = s.nb;
-    v.mm_tile  = s.d_mm_tile;  v.nt = s.nt;
+    v.mosaic = s.d_mosaic.get(); v.N = s.N; v.pitch = s.pitch;
+    v.e_tab = sc.d_e.get(); v.n_tab = sc.d_n.get();
+    v.mm_block = s.d_mm_block.get(); v.nb = s.nb;
+    v.mm_tile  = s.d_mm_tile.get();  v.nt = s.nt;
     v.viewer_cell_i = vs.viewer_cell_i; v.viewer_cell_j = vs.viewer_cell_j; v.viewer_z = vs.viewer_z;
     v.deg_per_cell = 1.0f / (float)s.cpd;                                // lib:577
     v.cos_viewer_lat = vs.cos_viewer_lat;
@@ -639,11 +636,11 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
 
     v.znear = s.znear; v.zfar = s.zfar; v.znear_color = s.znear_color; v.zfar_color = s.zfar_color;
     v.W = s.W; v.H = s.H; v.x0 = x0; v.x1 = x1;
-    v.vis = sc.d_vis;
-    v.stats      = s.collect_stats ? sc.d_counters + STATS_AT : nullptr;
-    v.tile_queue = sc.d_tile_queue; v.block_queue = sc.d_block_queue;
-    v.tri_queue = sc.d_tri_queue; v.tri_capacity = s.tri_capacity;
-    v.bigtri = sc.d_bigtri; v.bigtri_count = sc.d_counters + 3; v.bigtri_capacity = s.bigtri_capacity;
+    v.vis = sc.d_vis.get();
+    v.stats      = s.collect_stats ? sc.d_counters->stats : nullptr;
+    v.tile_queue = sc.d_tile_queue.get(); v.block_queue = sc.d_block_queue.get();
+    v.tri_queue = sc.d_tri_queue.get(); v.tri_capacity = s.tri_capacity;
+    v.bigtri = sc.d_bigtri.get(); v.bigtri_count = &sc.d_counters->bigtri; v.bigtri_capacity = s.bigtri_capacity;
     const ChainConfig& cfg = config_of(set);
     v.occl_tile_max_pix  = cfg.occl_tile_max_pix;
     v.occl_block_max_pix = cfg.occl_block_max_pix;
@@ -675,8 +672,8 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
         v.inv_zrange = (s.zfar > s.znear) ? 1.0f / (s.zfar - s.znear) : 0.0f;   // 0: no far/occlusion culling
     }
 
-    v.counters = sc.d_counters; v.ncounters = N_COUNTERS;
-    v.tanel = sc.d_tanel;
+    v.counters = reinterpret_cast<uint32_t*>(sc.d_counters.get()); v.ncounters = N_COUNTERS;
+    v.tanel = sc.d_tanel.get();
     v.n_out = out.n; v.out_stride = out.stride > 0 ? out.stride : x1 - x0; v.out_x0 = out.x_off;
     for(int d = 0; d < out.n; d++) { v.out_image[d] = out.image[d]; v.out_ranges[d] = out.ranges[d]; }
 }
@@ -688,14 +685,14 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     if(s.W <= 0 || s.H <= 0 || m < 1 || m > (int)set.sc.size()) return false;
     const bool want_image = outs[0].image[0] != nullptr, want_ranges = outs[0].ranges[0] != nullptr;
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
-    if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy, 0));
+    if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy.get(), 0));
 
-    // ---- the parameter block: per view, variants for the near pass, the far queue and each band, into a slot of the
-    // pinned ring, then one small copy to the device
+    // ---- the parameter block: per view, variants for the near pass and each band, into a slot of the pinned ring,
+    // then one small copy to the device
     const int slot = set.ring_next;
     set.ring_next = (set.ring_next + 1) % PARAM_RING;
-    CUDA_TRY(cudaEventSynchronize(set.ring_ev[slot]));            // the copies that last used this slot are done
-    HzView* hv = set.h_views + (size_t)slot * set.cap * HZ_V_COUNT;
+    CUDA_TRY(cudaEventSynchronize(set.ring_ev[slot].get()));            // the copies that last used this slot are done
+    HzView* hv = set.h_views.get() + (size_t)slot * set.cap * HZ_V_COUNT;
     const Bands& bands = config_of(set).bands;
     bool big_per_band = false, vectorisable = true;
     for(int k = 0; k < m; k++) big_per_band = big_per_band || big_after_every_band(s, vs[k]);
@@ -711,12 +708,10 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         sc.renders++;
         vectorisable = vectorisable && hz_resolve_is_vectorisable(hk[0]);
         for(int j = 1; j < HZ_V_COUNT; j++) hk[j] = hk[0];
-        hk[HZ_V_NEAR].tri_count = sc.d_counters + 2;
-        hk[HZ_V_NEAR].big_queue = sc.d_big_queue;                 hk[HZ_V_NEAR].big_count = sc.d_counters + 0;
-        for(int j = HZ_V_FAR; j < HZ_V_COUNT; j++)
-        {
-            hk[j].big_queue = sc.d_big_queue + s.big_capacity;      hk[j].big_count = sc.d_counters + 1;
-        }
+        Counters* const cnt = sc.d_counters.get();
+        hk[HZ_V_NEAR].tri_count = &cnt->near_tri;
+        hk[HZ_V_NEAR].big_queue = sc.d_big_queue.get();           hk[HZ_V_NEAR].big_count = &cnt->near_big;
+        for(int j = HZ_V_BAND0; j < HZ_V_COUNT; j++) hk[j].big_queue = sc.d_big_queue.get() + s.big_capacity;
         // The bands: the configured ring limits -- plus, with the opt-in level of detail, the two rings from which on a
         // cell of 2x2 / 4x4 DEM cells, seen from that ring's nearest edge, is at most lod_pixels pixels across: the level
         // is then the same throughout a band, and the image does not depend on how the bands were configured.
@@ -742,11 +737,11 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         {
             HzView& vb = hk[HZ_V_BAND0 + b];
             vb.ring_lo = lo; vb.ring_hi = ends[b] > lo ? ends[b] : lo;
-            vb.tile_count = sc.d_counters + 4 + 4 * b; vb.block_count = sc.d_counters + 5 + 4 * b;
-            vb.tri_count  = sc.d_counters + 6 + 4 * b;
+            vb.tile_count = &cnt->band[b].tile; vb.block_count = &cnt->band[b].block;
+            vb.tri_count  = &cnt->band[b].tri;
             // one k_big per band: each band counts its own entries from 0 (the queue memory is reused, the bands run
             // one after the other); one k_big at the end: all bands append to the same count
-            vb.big_count  = sc.d_counters + 7 + (big_per_band ? 4 * b : 0);
+            vb.big_count  = &cnt->band[big_per_band ? b : 0].big;
             int lod = 0;
             while(lod < HZ_MAX_LOD && vb.ring_lo >= lod_from[lod + 1]) lod++;
             vb.lod = lod;
@@ -756,14 +751,14 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         // the row table of this view's window, unless the scratch still holds it from its previous render
         if(want_ranges && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
         {
-            float* h_row = set.h_tanel + ((size_t)slot * set.cap + k) * s.H;
+            float* h_row = set.h_tanel.get() + ((size_t)slot * set.cap + k) * s.H;
             memcpy(h_row, tanel_row(s, vs[k].az_deg0, vs[k].az_deg1), (size_t)s.H * sizeof(float));
-            CUDA_TRY(cudaMemcpyAsync(sc.d_tanel, h_row, (size_t)s.H * sizeof(float), cudaMemcpyHostToDevice, st));
+            CUDA_TRY(cudaMemcpyAsync(sc.d_tanel.get(), h_row, (size_t)s.H * sizeof(float), cudaMemcpyHostToDevice, st));
             sc.tanel_key.valid = true; sc.tanel_key.daz = vs[k].az_deg1 - vs[k].az_deg0; sc.tanel_key.W = s.W; sc.tanel_key.H = s.H;
         }
     }
-    CUDA_TRY(cudaMemcpyAsync(set.d_views, hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaEventRecord(set.ring_ev[slot], st));
+    CUDA_TRY(cudaMemcpyAsync(set.d_views.get(), hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaEventRecord(set.ring_ev[slot].get(), st));
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
     const bool is_main = (&set == &s.main);
@@ -776,23 +771,23 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         if(g == nullptr && (g = capture_graph(s, set, hv, m, big_per_band)) == nullptr) set.graph_failed = true;
         if(g != nullptr)
         {
-            CUDA_TRY(cudaGraphLaunch(g->exec[g->next], st));
+            CUDA_TRY(cudaGraphLaunch(g->exec[g->next].get(), st));
             g->next = (g->next + 1) % g->exec.size();
-            CUDA_TRY(cudaEventRecord(set.busy, st)); set.last_stream = st; set.busy_recorded = true;
+            CUDA_TRY(cudaEventRecord(set.busy.get(), st)); set.last_stream = st; set.busy_recorded = true;
             s.launches_last = g->launches;
             if(is_main) s.have_render = true;
             return true;
         }
     }
 
-    cudaEvent_t* ev = nullptr;
+    const EventHandle* ev = nullptr;
     if(s.profiling)
     {
         while(s.prof_events.size() < s.prof_used + PROF_EVENTS)
         {
-            cudaEvent_t e;
-            CUDA_TRY(cudaEventCreate(&e));
-            s.prof_events.push_back(e);
+            EventHandle e = make_event(cudaEventDefault);
+            if(empty_handle(e, "cudaEventCreate")) return false;
+            s.prof_events.push_back(std::move(e));
         }
         ev = &s.prof_events[s.prof_used];
         s.prof_used += PROF_EVENTS;
@@ -800,7 +795,7 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     int launches = 0;
     // grids sized for this view's eye tile only when there is just one view
     if(!launch_chain(s, set, hv, m, big_per_band, m > 1, want_image || want_ranges, st, ev, &launches)) return false;
-    CUDA_TRY(cudaEventRecord(set.busy, st)); set.last_stream = st; set.busy_recorded = true;
+    CUDA_TRY(cudaEventRecord(set.busy.get(), st)); set.last_stream = st; set.busy_recorded = true;
     s.launches_last = launches;
     if(is_main) s.have_render = (x0 == 0 && x1 == s.W);
     return true;
@@ -964,12 +959,12 @@ bool copy_results_to_host(Slot& s, char* image, float* ranges, const uint8_t* d_
             CUDA_TRY(cudaMemcpyAsync(o.dst, o.src, o.bytes, cudaMemcpyDeviceToHost, st));
             continue;
         }
-        if(s.h_stage == nullptr)
+        if(!s.h_stage)
         {
             const size_t want = px * 7 < STAGE_MAX_BYTES ? px * 7 : STAGE_MAX_BYTES;
-            if(cudaMallocHost(&s.h_stage, want) != cudaSuccess)
+            if(!(s.h_stage = make_host<char>(want)))
             {
-                cudaGetLastError(); s.h_stage = nullptr;
+                cudaGetLastError();
                 CUDA_TRY(cudaMemcpyAsync(o.dst, o.src, o.bytes, cudaMemcpyDeviceToHost, st));
                 continue;
             }
@@ -991,13 +986,13 @@ bool copy_results_to_host(Slot& s, char* image, float* ranges, const uint8_t* d_
             n = left < want ? left : want;
             if(parts.size() >= s.stage_ev.size())
             {
-                cudaEvent_t e;
-                CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                s.stage_ev.push_back(e);
+                EventHandle e = make_event();
+                if(empty_handle(e, "cudaEventCreate")) return false;
+                s.stage_ev.push_back(std::move(e));
             }
-            CUDA_TRY(cudaMemcpyAsync(s.h_stage + staged + off, o.src + off, n, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaEventRecord(s.stage_ev[parts.size()], st));
-            parts.push_back({ o.dst + off, s.h_stage + staged + off, n, s.stage_ev[parts.size()] });
+            CUDA_TRY(cudaMemcpyAsync(s.h_stage.get() + staged + off, o.src + off, n, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaEventRecord(s.stage_ev[parts.size()].get(), st));
+            parts.push_back({ o.dst + off, s.h_stage.get() + staged + off, n, s.stage_ev[parts.size()].get() });
         }
         staged += o.bytes;
     }
@@ -1074,7 +1069,8 @@ bool horizonator_init(horizonator_context_t* ctx,
             if(e != cudaSuccess) MSG("CUDA error: %s: %s", what, cudaGetErrorString(e));
             return e != cudaSuccess;
         };
-        if(fail(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking), "cudaStreamCreate")) break;
+        if(empty_handle(s->stream = make_stream(), "cudaStreamCreate")) break;
+        cudaStream_t const st = s->stream.get();
 
         const horizonator_dem_context_t* d = &ctx->dems;
         s->cpd = d->cells_per_deg;
@@ -1090,32 +1086,34 @@ bool horizonator_init(horizonator_context_t* ctx,
             for(int j = 0; j < d->Ndems_ij[1] && !bad; j++)
             {
                 if(d->dems[i][j] == nullptr) continue;
-                uint8_t* p = nullptr;
-                bad = fail(cudaMalloc(&p, d->mmap_sizes[i][j] + 16), "cudaMalloc(tile)") ||
-                      fail(cudaMemcpyAsync(p, d->dems[i][j], d->mmap_sizes[i][j], cudaMemcpyHostToDevice, s->stream),
+                DevPtr<uint8_t>& p = s->d_tiles[i][j];
+                bad = empty_handle(p = make_device<uint8_t>(d->mmap_sizes[i][j] + 16), "cudaMalloc(tile)") ||
+                      fail(cudaMemcpyAsync(p.get(), d->dems[i][j], d->mmap_sizes[i][j], cudaMemcpyHostToDevice, st),
                            "cudaMemcpy(tile)");
-                s->tiles.tile[i][j] = p;
+                s->tiles.tile[i][j] = p.get();
             }
         if(bad) break;
 
         // (HZ_MESH_PAD zero rows after the last: see hz_device.h)
-        if(fail(cudaMalloc(&s->d_mosaic, (size_t)(s->N + HZ_MESH_PAD) * s->pitch * sizeof(int16_t)), "cudaMalloc(mosaic)")) break;
-        if(fail(cudaMemsetAsync(s->d_mosaic + (size_t)s->N * s->pitch, 0, (size_t)HZ_MESH_PAD * s->pitch * sizeof(int16_t), s->stream),
+        if(empty_handle(s->d_mosaic = make_device<int16_t>((size_t)(s->N + HZ_MESH_PAD) * s->pitch), "cudaMalloc(mosaic)")) break;
+        int16_t* const mosaic = s->d_mosaic.get();
+        if(fail(cudaMemsetAsync(mosaic + (size_t)s->N * s->pitch, 0, (size_t)HZ_MESH_PAD * s->pitch * sizeof(int16_t), st),
                 "cudaMemset(mosaic)")) break;
         s->nb = (s->N - 1 + HZ_BLOCK_CELLS - 1) / HZ_BLOCK_CELLS;
         s->nt = (s->N - 1 + HZ_TILE_CELLS - 1) / HZ_TILE_CELLS;
-        if(fail(cudaMalloc(&s->d_mm_block, (size_t)s->nb * s->nb * sizeof(short2)), "cudaMalloc(pyramid)")) break;
-        if(fail(cudaMalloc(&s->d_mm_tile, (size_t)s->nt * s->nt * sizeof(short2)), "cudaMalloc(pyramid)")) break;
-        if(!alloc_set(s->main, 1, false) || ensure_views(*s, s->main, 1) != 1) break;
-        if(fail(hz_launch_mosaic(s->tiles, s->d_mosaic, s->N, s->pitch, s->stream), "k_mosaic")) break;
-        if(fail(hz_launch_pyramid(s->d_mosaic, s->N, s->pitch, s->d_mm_block, s->nb, s->d_mm_tile, s->nt, s->stream),
+        if(empty_handle(s->d_mm_block = make_device<short2>((size_t)s->nb * s->nb), "cudaMalloc(pyramid)")) break;
+        if(empty_handle(s->d_mm_tile = make_device<short2>((size_t)s->nt * s->nt), "cudaMalloc(pyramid)")) break;
+        if(!alloc_set(s->main, 1, false)) { MSG("Could not allocate the context's view set"); break; }
+        if(ensure_views(*s, s->main, 1) != 1) break;
+        if(fail(hz_launch_mosaic(s->tiles, mosaic, s->N, s->pitch, st), "k_mosaic")) break;
+        if(fail(hz_launch_pyramid(mosaic, s->N, s->pitch, s->d_mm_block.get(), s->nb, s->d_mm_tile.get(), s->nt, st),
                 "k_minmax")) break;
 
         // without an offscreen size the reference opens a 1024x1024 window (lib:142)
         const int W = offscreen_width > 0 ? offscreen_width : 1024;
         const int H = offscreen_width > 0 ? offscreen_height : 1024;
         if(!alloc_target(*s, W, H)) break;
-        if(fail(cudaStreamSynchronize(s->stream), "DEM upload/decode")) break;
+        if(fail(cudaStreamSynchronize(st), "DEM upload/decode")) break;
         ok = true;
     } while(0);
 
@@ -1189,7 +1187,7 @@ bool horizonator_resized(const horizonator_context_t* ctx, int width, int height
     }
     if(width <= 0 || height <= 0) return false;
     DeviceGuard g(s->device);
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
     return alloc_target(*s, width, height);
 }
 
@@ -1229,8 +1227,8 @@ bool horizonator_redraw(const horizonator_context_t* ctx)
     Slot* s = slot_of(ctx);
     if(s == nullptr) return false;
     DeviceGuard g(s->device);
-    if(!enqueue_render(*s, s->view, 0, s->W, single_out(s->d_image, s->d_ranges), s->stream)) return false;
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if(!enqueue_render(*s, s->view, 0, s->W, single_out(s->d_image.get(), s->d_ranges.get()), s->stream.get())) return false;
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
     return true;
 }
 
@@ -1246,8 +1244,8 @@ bool horizonator_render_offscreen(const horizonator_context_t* ctx, char* image,
     DeviceGuard g(s->device);
     const size_t px = (size_t)s->W * s->H;
     if(!enqueue_render(*s, s->view, 0, s->W,
-                       single_out(image ? s->d_image : nullptr, ranges ? s->d_ranges : nullptr), s->stream)) return false;
-    return copy_results_to_host(*s, image, ranges, s->d_image, s->d_ranges, px, s->stream);
+                       single_out(image ? s->d_image.get() : nullptr, ranges ? s->d_ranges.get() : nullptr), s->stream.get())) return false;
+    return copy_results_to_host(*s, image, ranges, s->d_image.get(), s->d_ranges.get(), px, s->stream.get());
 }
 
 bool horizonator_pick(const horizonator_context_t* ctx, float* lat, float* lon, int x, int y)
@@ -1257,8 +1255,8 @@ bool horizonator_pick(const horizonator_context_t* ctx, float* lat, float* lon, 
     if(x < 0 || y < 0 || x >= s->W || y >= s->H) return false;
     DeviceGuard g(s->device);
     unsigned long long key = 0;
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    CUDA_TRY(cudaMemcpy(&key, s->main.sc[0].d_vis + (size_t)(s->H - 1 - y) * s->W + x, sizeof(key), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+    CUDA_TRY(cudaMemcpy(&key, s->main.sc[0].d_vis.get() + (size_t)(s->H - 1 - y) * s->W + x, sizeof(key), cudaMemcpyDeviceToHost));
     const float depth = (float)((double)hz_key_q(key, s->main.sc[0].last_epoch) * (1.0 / 16777215.0));
     if(depth >= 1.0f) return false;                                     // lib:1272
     // lib:1282-1295: the depth is treated as horizontal distance
@@ -1387,8 +1385,8 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         // one view, or no memory for a set: one at a time on the context's own scratch
         for(int k = 0; k < n; k++)
         {
-            uint8_t* di = images ? (to_host ? s->d_image  : images + (size_t)k * px * 3) : nullptr;
-            float*   dr = ranges ? (to_host ? s->d_ranges : ranges + (size_t)k * px)     : nullptr;
+            uint8_t* di = images ? (to_host ? s->d_image.get()  : images + (size_t)k * px * 3) : nullptr;
+            float*   dr = ranges ? (to_host ? s->d_ranges.get() : ranges + (size_t)k * px)     : nullptr;
             if(!enqueue_render(*s, vs[k], 0, s->W, single_out(di, dr), st)) return false;
             if(to_host)
             {
@@ -1400,8 +1398,8 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         return true;
     }
 
-    CUDA_TRY(cudaEventRecord(s->fork_ev, st));
-    for(int g = 0; g < n_sets; g++) CUDA_TRY(cudaStreamWaitEvent(s->sets[g]->stream, s->fork_ev, 0));
+    CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
+    for(int g = 0; g < n_sets; g++) CUDA_TRY(cudaStreamWaitEvent(s->sets[g]->stream.get(), s->fork_ev.get(), 0));
     bool ok = true;
     std::vector<OutSpec> outs((size_t)chunk);
     for(int k0 = 0, c = 0; k0 < n && ok; k0 += chunk, c++)
@@ -1409,26 +1407,26 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         ViewSet& set = *s->sets[c % n_sets];
         const int m = n - k0 < chunk ? n - k0 : chunk;
         for(int k = 0; k < m; k++)
-            outs[k] = single_out(images ? (to_host ? set.sc[k].d_image  : images + (size_t)(k0 + k) * px * 3) : nullptr,
-                                 ranges ? (to_host ? set.sc[k].d_ranges : ranges + (size_t)(k0 + k) * px)     : nullptr);
-        ok = enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), set.stream);
+            outs[k] = single_out(images ? (to_host ? set.sc[k].d_image.get()  : images + (size_t)(k0 + k) * px * 3) : nullptr,
+                                 ranges ? (to_host ? set.sc[k].d_ranges.get() : ranges + (size_t)(k0 + k) * px)     : nullptr);
+        ok = enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), set.stream.get());
         for(int k = 0; k < m && ok && to_host; k++)
         {
-            if(images) ok = ok && copy_to_host(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image, px * 3, set.stream);
-            if(ranges) ok = ok && copy_to_host(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges, px * sizeof(float), set.stream);
+            if(images) ok = ok && copy_to_host(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3, set.stream.get());
+            if(ranges) ok = ok && copy_to_host(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges.get(), px * sizeof(float), set.stream.get());
         }
     }
     if(!ok)
     {
         // whatever was queued may still be writing into the caller's buffers: let it finish before reporting failure
-        for(int g = 0; g < n_sets; g++) cudaStreamSynchronize(s->sets[g]->stream);
+        for(int g = 0; g < n_sets; g++) cudaStreamSynchronize(s->sets[g]->stream.get());
         cudaGetLastError();
         return false;
     }
     for(int g = 0; g < n_sets; g++)
     {
-        CUDA_TRY(cudaEventRecord(s->sets[g]->done, s->sets[g]->stream));
-        CUDA_TRY(cudaStreamWaitEvent(st, s->sets[g]->done, 0));
+        CUDA_TRY(cudaEventRecord(s->sets[g]->done.get(), s->sets[g]->stream.get()));
+        CUDA_TRY(cudaStreamWaitEvent(st, s->sets[g]->done.get(), 0));
     }
     return true;
 }
@@ -1462,14 +1460,13 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
     if(n == 0) return true;
 
     const int chunk = n < HZ_VS_MAX_VIEWS ? n : HZ_VS_MAX_VIEWS;
-    if(s->vs_done == nullptr) CUDA_TRY(cudaEventCreateWithFlags(&s->vs_done, cudaEventDisableTiming));
-    else CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done, 0));
+    if(!s->vs_done) { if(empty_handle(s->vs_done = make_event(), "cudaEventCreate")) return false; }
+    else CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
     if(d_masks == nullptr && s->vs_mask_views < chunk)
     {
-        CUDA_TRY(cudaEventSynchronize(s->vs_done));
-        cudaFree(s->d_vs_masks);
-        s->d_vs_masks = nullptr; s->vs_mask_views = 0;
-        if(cudaMalloc(&s->d_vs_masks, (size_t)chunk * mwords * sizeof(uint32_t)) != cudaSuccess)
+        CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
+        s->d_vs_masks = nullptr; s->vs_mask_views = 0;          // the smaller masks go before the larger ones come
+        if(!(s->d_vs_masks = make_device<uint32_t>((size_t)chunk * mwords)))
         {
             cudaGetLastError();
             MSG("Could not allocate the viewshed masks of %d views (%zu MB)", chunk, (size_t)chunk * mwords * 4 >> 20);
@@ -1479,14 +1476,14 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
     }
 
     HzViewshed p{};
-    p.mosaic = s->d_mosaic; p.N = N; p.pitch = s->pitch; p.w32 = w32;
+    p.mosaic = s->d_mosaic.get(); p.N = N; p.pitch = s->pitch; p.w32 = w32;
     p.deg_per_cell = 1.0f / (float)s->cpd;                                // lib:577
     p.curvature = s->curvature;
     p.target_height = target_height;
     for(int k0 = 0; k0 < n; k0 += chunk)
     {
         const int m = n - k0 < chunk ? n - k0 : chunk;
-        p.masks = d_masks ? d_masks + (size_t)k0 * mwords : s->d_vs_masks;
+        p.masks = d_masks ? d_masks + (size_t)k0 * mwords : s->d_vs_masks.get();
         for(int k = 0; k < m; k++) p.eye[k] = eyes[(size_t)(k0 + k)];
         CUDA_TRY(cudaMemsetAsync(p.masks, 0, (size_t)m * mwords * sizeof(uint32_t), st));
         CUDA_TRY(hz_launch_viewshed(p, m, st));
@@ -1495,7 +1492,7 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
             CUDA_TRY(cudaMemcpyAsync(h_masks + (size_t)k0 * mwords, p.masks, (size_t)m * mwords * sizeof(uint32_t),
                                      cudaMemcpyDeviceToHost, st));
     }
-    CUDA_TRY(cudaEventRecord(s->vs_done, st));
+    CUDA_TRY(cudaEventRecord(s->vs_done.get(), st));
     return true;
 }
 
@@ -1510,7 +1507,7 @@ bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const 
         return false;
     }
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     if(!viewshed_common(ctx, s, n, views, target_height_m, (uint32_t*)d_masks, (uint32_t*)d_counts, nullptr, st))
         return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
@@ -1529,10 +1526,10 @@ bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizon
     }
     DeviceGuard g(s->device);
     const size_t cells = (size_t)s->N * s->N;
-    if(counts && n > 0 && s->d_vs_counts == nullptr)
+    if(counts && n > 0 && !s->d_vs_counts)
     {
-        if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done));
-        if(cudaMalloc(&s->d_vs_counts, cells * sizeof(uint32_t)) != cudaSuccess)
+        if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
+        if(!(s->d_vs_counts = make_device<uint32_t>(cells)))
         {
             cudaGetLastError();
             MSG("Could not allocate the viewshed counts (%zu MB)", cells * 4 >> 20);
@@ -1540,16 +1537,16 @@ bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizon
         }
     }
     // the counts' upload waits for whatever an earlier call still does with the same buffer
-    if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(s->stream, s->vs_done, 0));
-    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts, counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream));
-    if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts : nullptr, masks, s->stream))
+    if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(s->stream.get(), s->vs_done.get(), 0));
+    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts.get(), counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream.get()));
+    if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts.get() : nullptr, masks, s->stream.get()))
     {
-        cudaStreamSynchronize(s->stream);
+        cudaStreamSynchronize(s->stream.get());
         cudaGetLastError();
         return false;
     }
-    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts, cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream));
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts.get(), cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream.get()));
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
     return true;
 }
 
@@ -1559,7 +1556,7 @@ bool horizonator_render_batch_device(const horizonator_context_t* ctx, int n, co
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     if(!render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st)) return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1571,8 +1568,8 @@ bool horizonator_render_batch(const horizonator_context_t* ctx, int n, const hor
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
     DeviceGuard g(s->device);
-    if(!render_batch_common(ctx, s, n, views, (uint8_t*)images, ranges, true, s->stream)) return false;
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if(!render_batch_common(ctx, s, n, views, (uint8_t*)images, ranges, true, s->stream.get())) return false;
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
     return true;
 }
 
@@ -1587,7 +1584,7 @@ bool horizonator_render_wedge_device(const horizonator_context_t* ctx, int x0, i
         return false;
     }
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     if(!enqueue_render(*s, s->view, x0, x1, single_out((uint8_t*)d_image, (float*)d_ranges), st)) return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1604,13 +1601,13 @@ bool horizonator_render_wedge_host(const horizonator_context_t* ctx, int x0, int
     }
     if(image == nullptr && ranges == nullptr) return true;
     DeviceGuard g(s->device);
-    cudaStream_t st = s->stream;
+    cudaStream_t st = s->stream.get();
     // the context's own output buffers serve as the slab [H][x1-x0]; from there straight into the caller's columns
     const size_t w = (size_t)(x1 - x0);
-    if(!enqueue_render(*s, s->view, x0, x1, single_out(image ? s->d_image : nullptr, ranges ? s->d_ranges : nullptr), st)) return false;
-    if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, s->d_image, w * 3, w * 3, (size_t)s->H,
+    if(!enqueue_render(*s, s->view, x0, x1, single_out(image ? s->d_image.get() : nullptr, ranges ? s->d_ranges.get() : nullptr), st)) return false;
+    if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, s->d_image.get(), w * 3, w * 3, (size_t)s->H,
                                           cudaMemcpyDeviceToHost, st));
-    if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), s->d_ranges, w * sizeof(float),
+    if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), s->d_ranges.get(), w * sizeof(float),
                                           w * sizeof(float), (size_t)s->H, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1644,18 +1641,17 @@ bool horizonator_peer_alloc(const horizonator_context_t* ctx, size_t bytes, void
     if(s == nullptr || d_ptr == nullptr || handle == nullptr || bytes == 0) return false;
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     DeviceGuard g(s->device);
-    void* p = nullptr;
-    CUDA_TRY(cudaMalloc(&p, bytes));
+    DevPtr<uint8_t> p = make_device<uint8_t>(bytes);
+    if(empty_handle(p, "cudaMalloc")) return false;
     cudaIpcMemHandle_t h;
-    const cudaError_t e = cudaIpcGetMemHandle(&h, p);
+    const cudaError_t e = cudaIpcGetMemHandle(&h, p.get());
     if(e != cudaSuccess)
     {
         MSG("cudaIpcGetMemHandle failed: %s", cudaGetErrorString(e));
-        cudaFree(p);
         return false;
     }
     memcpy(handle, &h, 64);
-    *d_ptr = p;
+    *d_ptr = p.release();          // the caller's: horizonator_peer_free
     return true;
 }
 
@@ -1716,7 +1712,7 @@ bool horizonator_render_wedge_peers(const horizonator_context_t* ctx, int x0, in
         }
     }
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     if(!enqueue_render(*s, s->view, x0, x1, out, st)) return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1735,7 +1731,7 @@ bool horizonator_peer_barrier(const horizonator_context_t* ctx, int n_ranks, int
         f.arrive[r] = (uint32_t*)d_flags[r];
     }
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     CUDA_TRY(hz_launch_peer_barrier(f, epoch, st));
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1762,12 +1758,13 @@ bool horizonator_set_lod(const horizonator_context_t* ctx, float max_cell_pixels
     {
         // the captured chains launch a different instantiation of k_blocks: wait for what is in flight, drop them
         DeviceGuard g(s->device);
-        CUDA_TRY(cudaStreamSynchronize(s->stream));
-        for(ViewSet* v : s->sets) CUDA_TRY(cudaStreamSynchronize(v->stream));
-        if(s->main.busy_recorded) CUDA_TRY(cudaEventSynchronize(s->main.busy));
-        for(ViewSet* v : s->sets) if(v->busy_recorded) CUDA_TRY(cudaEventSynchronize(v->busy));
-        drop_graphs(s->main);
-        for(ViewSet* v : s->sets) drop_graphs(*v);
+        CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+        for(const auto& v : s->sets) CUDA_TRY(cudaStreamSynchronize(v->stream.get()));
+        if(s->main.busy_recorded) CUDA_TRY(cudaEventSynchronize(s->main.busy.get()));
+        for(const auto& v : s->sets) if(v->busy_recorded) CUDA_TRY(cudaEventSynchronize(v->busy.get()));
+        s->main.graphs.clear();
+        s->main.graph_failed = false;
+        for(const auto& v : s->sets) { v->graphs.clear(); v->graph_failed = false; }
     }
     s->lod_pixels = max_cell_pixels;
     return true;
@@ -1791,9 +1788,10 @@ bool horizonator_debug_device_math(int n, const float* e, const float* north, co
 {
     if(n < 0 || (n > 0 && (!e || !north || !h || !d2 || !az || !el))) return false;
     if(n == 0) return true;
-    float* d = nullptr;
+    const DevPtr<float> buf = make_device<float>(6 * (size_t)n);
+    if(empty_handle(buf, "cudaMalloc")) return false;
+    float* const d = buf.get();
     const size_t bytes = (size_t)n * sizeof(float);
-    CUDA_TRY(cudaMalloc(&d, 6 * bytes));
     bool ok = cudaMemcpy(d, e, bytes, cudaMemcpyHostToDevice) == cudaSuccess &&
               cudaMemcpy(d + n, north, bytes, cudaMemcpyHostToDevice) == cudaSuccess &&
               cudaMemcpy(d + 2 * (size_t)n, h, bytes, cudaMemcpyHostToDevice) == cudaSuccess &&
@@ -1802,7 +1800,6 @@ bool horizonator_debug_device_math(int n, const float* e, const float* north, co
               cudaMemcpy(az, d + 4 * (size_t)n, bytes, cudaMemcpyDeviceToHost) == cudaSuccess &&
               cudaMemcpy(el, d + 5 * (size_t)n, bytes, cudaMemcpyDeviceToHost) == cudaSuccess;
     if(!ok) MSG("CUDA error in horizonator_debug_device_math: %s", cudaGetErrorString(cudaGetLastError()));
-    cudaFree(d);
     return ok;
 }
 
@@ -1828,8 +1825,8 @@ bool horizonator_download_mosaic(const horizonator_context_t* ctx, int16_t* mosa
     Slot* s = slot_of(ctx);
     if(s == nullptr || mosaic == nullptr) return false;
     DeviceGuard g(s->device);
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    CUDA_TRY(cudaMemcpy2D(mosaic, (size_t)s->N * sizeof(int16_t), s->d_mosaic, (size_t)s->pitch * sizeof(int16_t),
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+    CUDA_TRY(cudaMemcpy2D(mosaic, (size_t)s->N * sizeof(int16_t), s->d_mosaic.get(), (size_t)s->pitch * sizeof(int16_t),
                           (size_t)s->N * sizeof(int16_t), s->N, cudaMemcpyDeviceToHost));
     return true;
 }
@@ -1839,17 +1836,15 @@ bool horizonator_time_mosaic(const horizonator_context_t* ctx, int reps, float* 
     Slot* s = slot_of(ctx);
     if(s == nullptr || reps <= 0 || ms_per_run == nullptr) return false;
     DeviceGuard g(s->device);
-    cudaEvent_t a, b;
-    CUDA_TRY(cudaEventCreate(&a));
-    CUDA_TRY(cudaEventCreate(&b));
-    CUDA_TRY(hz_launch_mosaic(s->tiles, s->d_mosaic, s->N, s->pitch, s->stream));      // warm-up
-    CUDA_TRY(cudaEventRecord(a, s->stream));
-    for(int k = 0; k < reps; k++) CUDA_TRY(hz_launch_mosaic(s->tiles, s->d_mosaic, s->N, s->pitch, s->stream));
-    CUDA_TRY(cudaEventRecord(b, s->stream));
-    CUDA_TRY(cudaEventSynchronize(b));
+    const EventHandle a = make_event(cudaEventDefault), b = make_event(cudaEventDefault);
+    if(empty_handle(a, "cudaEventCreate") || empty_handle(b, "cudaEventCreate")) return false;
+    CUDA_TRY(hz_launch_mosaic(s->tiles, s->d_mosaic.get(), s->N, s->pitch, s->stream.get()));      // warm-up
+    CUDA_TRY(cudaEventRecord(a.get(), s->stream.get()));
+    for(int k = 0; k < reps; k++) CUDA_TRY(hz_launch_mosaic(s->tiles, s->d_mosaic.get(), s->N, s->pitch, s->stream.get()));
+    CUDA_TRY(cudaEventRecord(b.get(), s->stream.get()));
+    CUDA_TRY(cudaEventSynchronize(b.get()));
     float ms = 0;
-    CUDA_TRY(cudaEventElapsedTime(&ms, a, b));
-    cudaEventDestroy(a); cudaEventDestroy(b);
+    CUDA_TRY(cudaEventElapsedTime(&ms, a.get(), b.get()));
     *ms_per_run = ms / (float)reps;
     return true;
 }
@@ -1872,12 +1867,12 @@ bool horizonator_profile_read(const horizonator_context_t* ctx, float out_ms[6],
     const size_t n = s->prof_used / PROF_EVENTS;
     for(size_t r = 0; r < n; r++)
     {
-        cudaEvent_t* ev = &s->prof_events[PROF_EVENTS * r];
-        CUDA_TRY(cudaEventSynchronize(ev[PROF_EVENTS - 1]));
+        const EventHandle* ev = &s->prof_events[PROF_EVENTS * r];
+        CUDA_TRY(cudaEventSynchronize(ev[PROF_EVENTS - 1].get()));
         for(int k = 0; k < PROF_EVENTS - 1; k++)
         {
             float ms = 0;
-            CUDA_TRY(cudaEventElapsedTime(&ms, ev[k], ev[k + 1]));
+            CUDA_TRY(cudaEventElapsedTime(&ms, ev[k].get(), ev[k + 1].get()));
             sum[k] += ms;
         }
     }
@@ -1892,14 +1887,14 @@ bool horizonator_last_render_stats(const horizonator_context_t* ctx, unsigned in
     Slot* s = slot_of(ctx);
     if(s == nullptr) return false;
     DeviceGuard g(s->device);
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    unsigned int counters[N_COUNTERS] = {};
-    CUDA_TRY(cudaMemcpy(counters, s->main.sc[0].d_counters, sizeof(counters), cudaMemcpyDeviceToHost));
-    out[0] = counters[0];
-    for(int b = 0; b < MAX_BANDS; b++) out[0] += counters[7 + 4 * b];
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+    Counters c{};
+    CUDA_TRY(cudaMemcpy(&c, s->main.sc[0].d_counters.get(), sizeof(c), cudaMemcpyDeviceToHost));
+    out[0] = c.near_big;
+    for(const BandCounters& b : c.band) out[0] += b.big;
     out[1] = 2 * s->big_capacity; out[2] = s->launches_last; out[3] = (unsigned)s->device;
-    out[4] = counters[2];
-    for(int b = 0; b < MAX_BANDS; b++) out[4] += counters[6 + 4 * b];     // triangle lists of the near pass and the bands
+    out[4] = c.near_tri;
+    for(const BandCounters& b : c.band) out[4] += b.tri;         // triangle lists of the near pass and the bands
     return true;
 }
 
@@ -1908,8 +1903,8 @@ bool horizonator_render_counters(const horizonator_context_t* ctx, unsigned int 
     Slot* s = slot_of(ctx);
     if(s == nullptr || out == nullptr) return false;
     DeviceGuard g(s->device);
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    CUDA_TRY(cudaMemcpy(out, s->main.sc[0].d_counters + STATS_AT, HZ_STAT_COUNT * sizeof(unsigned int), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+    CUDA_TRY(cudaMemcpy(out, s->main.sc[0].d_counters->stats, HZ_STAT_COUNT * sizeof(unsigned int), cudaMemcpyDeviceToHost));
     return true;
 }
 
@@ -1919,7 +1914,7 @@ bool horizonator_horizon_profile_device(const horizonator_context_t* ctx, const 
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || d_ranges == nullptr || d_rows == nullptr || d_range == nullptr) return false;
     DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     CUDA_TRY(hz_launch_horizon((const float*)d_ranges, n, s->W, s->H, (int*)d_rows, (float*)d_range, st));
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;

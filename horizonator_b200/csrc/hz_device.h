@@ -160,7 +160,7 @@ struct alignas(16) HzView      // (16-byte units: the kernels fetch their copy w
 // A render's parameters live in device memory as a small array of HzView variants that differ only in the
 // queue/counter/band fields: the kernels take a pointer to their variant, so that the same captured CUDA graph can
 // be replayed for every view after one small host->device copy.
-enum { HZ_V_NEAR = 0, HZ_V_FAR = 1, HZ_V_BAND0 = 2 };
+enum { HZ_V_NEAR = 0, HZ_V_BAND0 = 1 };
 constexpr int HZ_MAX_BANDS = 14;
 constexpr int HZ_V_COUNT   = HZ_V_BAND0 + HZ_MAX_BANDS;
 
