@@ -1160,32 +1160,54 @@ __device__ __forceinline__ bool hz_box_occluded_thread(const HzView& P, const Hz
     return true;
 }
 
-// Appends `value` of every thread with `on` to queue[*count...] with ONE global atomic per CTA: thousands of warps
-// bumping the same counter serialise in one L2 slice, which is what these short kernels would otherwise wait on.
-// Every thread of the CTA must call it (it synchronises the CTA), with `on` false where there is nothing to add.
-struct HzCtaAppend
+enum { HZ_RECT_OCCLUDED = 4 };
+
+__device__ __forceinline__ int
+hz_rect_cull(const HzView& P, int c_lo, int c_hi, int r_lo, int r_hi, float zmin, float zmax, int max_pix)
 {
-    unsigned int count, base;
-    unsigned int buf[256];
+    HzBox B;
+    const int r = hz_rect_test(P, c_lo, c_hi, r_lo, r_hi, zmin, zmax, B);
+    return (r == HZ_RECT_BOXED && hz_box_occluded_thread(P, B, max_pix)) ? (int)HZ_RECT_OCCLUDED : r;
+}
+
+// counts the outcome of a rectangle's test; true if the rectangle lives on
+__device__ __forceinline__ bool hz_rect_tally(int r, unsigned int& n_far, unsigned int& n_window, unsigned int& n_occl)
+{
+    n_far += r == HZ_RECT_DEAD_FAR; n_window += r == HZ_RECT_DEAD_WINDOW; n_occl += r == HZ_RECT_OCCLUDED;
+    return r == HZ_RECT_ALIVE || r == HZ_RECT_BOXED;
+}
+
+// What lives on goes to the band's queue through a stage per warp in shared memory, written out with one global atomic
+// whenever it holds 32 or more, and at the end: a few per cent of the rectangles live on, so that is few atomics (thousands
+// of warps bumping the same counter serialise in one L2 slice), and no warp waits for another.
+struct HzCullWarp                  // a culling warp's shared memory
+{
+    unsigned int stage[64];        // queue entries not written out yet (< 32 pending + at most 32 new)
+    unsigned int mids[32];         // (k_blocks_mid) the mids that live on
 };
 
+// writes stage[0..n) to queue[*count ...] with one atomic; all lanes call (n the same in all of them)
 __device__ __forceinline__ void
-hz_cta_append(HzCtaAppend& A, bool on, unsigned int value, unsigned int* queue, unsigned int* count)
+hz_stage_write(unsigned int* stage, unsigned int& n, unsigned int* queue, unsigned int* count, unsigned int lane)
 {
-    const int lane = threadIdx.x & 31;
-    if(threadIdx.x == 0) A.count = 0;
-    __syncthreads();
+    __syncwarp();
+    unsigned int base = 0;
+    if(lane == 0) base = atomicAdd(count, n);
+    base = __shfl_sync(0xffffffffu, base, 0);
+    for(unsigned int k = lane; k < n; k += 32u) queue[base + k] = stage[k];
+    __syncwarp();
+    n = 0;
+}
+
+// stages `value` of the lanes with `on`; all lanes call
+__device__ __forceinline__ void
+hz_stage_push(unsigned int* stage, unsigned int& n, bool on, unsigned int value, unsigned int* queue, unsigned int* count,
+              unsigned int lane)
+{
     const unsigned int ballot = __ballot_sync(0xffffffffu, on);
-    unsigned int wbase = 0;
-    if(lane == 0 && ballot) wbase = atomicAdd(&A.count, (unsigned int)__popc(ballot));
-    wbase = __shfl_sync(0xffffffffu, wbase, 0);
-    if(on) A.buf[wbase + __popc(ballot & ((1u << lane) - 1u))] = value;
-    __syncthreads();
-    const unsigned int n = A.count;
-    if(n == 0) return;                                   // the same for the whole CTA
-    if(threadIdx.x == 0) A.base = atomicAdd(count, n);
-    __syncthreads();
-    if(threadIdx.x < n) queue[A.base + threadIdx.x] = A.buf[threadIdx.x];
+    if(on) stage[n + __popc(ballot & ((1u << lane) - 1u))] = value;
+    n += (unsigned int)__popc(ballot);
+    if(n >= 32u) hz_stage_write(stage, n, queue, count, lane);
 }
 
 // diagnostics: per-CTA sums in shared memory, then one global atomic per counter and CTA (only when P.stats is set)
@@ -1200,48 +1222,75 @@ __device__ __forceinline__ void hz_cta_stats4(unsigned int* s4, unsigned int* gl
     if(threadIdx.x < 4 && s4[threadIdx.x]) atomicAdd(global4 + threadIdx.x, s4[threadIdx.x]);
 }
 
+// The tiles of a band: Chebyshev distance [lo, hi) from the eye's tile (ex, ey), 1 <= lo < hi, clipped to the mesh --
+// the square [ox0, ox1] x [oy0, oy1] without the hole [hx0, hx1] x [hy0, hy1] around the eye's tile.  Numbered row by
+// row: the rows below the hole, then the rows beside it (left piece, then right piece), then the rows above it.
+struct HzRing
+{
+    int ox0, ox1, oy0, oy1, hx0, hx1, hy0, hy1;
+    __host__ __device__ HzRing(int ex, int ey, int nt, int lo, int hi)
+        : ox0(max(ex - (hi - 1), 0)), ox1(min(ex + (hi - 1), nt - 1)), oy0(max(ey - (hi - 1), 0)), oy1(min(ey + (hi - 1), nt - 1)),
+          hx0(max(ex - (lo - 1), 0)), hx1(min(ex + (lo - 1), nt - 1)), hy0(max(ey - (lo - 1), 0)), hy1(min(ey + (lo - 1), nt - 1)) {}
+    __host__ __device__ unsigned int width()  const { return (unsigned int)(ox1 - ox0 + 1); }
+    __host__ __device__ unsigned int below()  const { return (unsigned int)(hy0 - oy0) * width(); }
+    __host__ __device__ unsigned int side()   const { return (unsigned int)((hx0 - ox0) + (ox1 - hx1)); }   // per row beside the hole
+    __host__ __device__ unsigned int beside() const { return side() * (unsigned int)(hy1 - hy0 + 1); }
+    __host__ __device__ unsigned int count()  const { return below() + beside() + (unsigned int)(oy1 - hy1) * width(); }
+    __device__ void tile(unsigned int k, int& ti, int& tj) const
+    {
+        if(k < below()) { const unsigned int row = k / width(); ti = ox0 + (int)(k - row * width()); tj = oy0 + (int)row; return; }
+        k -= below();
+        if(k < beside())
+        {
+            const unsigned int row = k / side();
+            const int c = (int)(k - row * side()), left = hx0 - ox0;
+            ti = c < left ? ox0 + c : hx1 + 1 + (c - left); tj = hy0 + (int)row;
+            return;
+        }
+        k -= beside();
+        const unsigned int row = k / width();
+        ti = ox0 + (int)(k - row * width()); tj = hy1 + 1 + (int)row;
+    }
+};
+
+// The culling kernels' loops are grid-strided with warp-uniform trips (every lane of a warp calls the stage), one
+// rectangle per lane and trip, and no CTA barrier inside them.
 __global__ void __launch_bounds__(256, 3)
 k_tiles(const HzView* __restrict__ V)
 {
     HZ_KERNEL_PROLOGUE(V, P);
-    __shared__ HzCtaAppend s_app;
+    __shared__ HzCullWarp s_warp[8];
     __shared__ unsigned int s_stats[4];
+    const unsigned int lane = threadIdx.x & 31u;
+    HzCullWarp& S = s_warp[threadIdx.x >> 5];
     const int nt = P.nt, N = P.N;
     const int rmax = max(max(P.eye_ti, nt - 1 - P.eye_ti), max(P.eye_tj, nt - 1 - P.eye_tj));
     const int ring_hi = min(P.ring_hi, rmax + 1), ring_lo = P.ring_lo;
     if(ring_lo >= ring_hi) return;
-    // the band = the tiles of Chebyshev distance [ring_lo, ring_hi) from the eye's tile: the threads walk the part of
-    // its bounding square that lies inside the mesh, row by row, and skip the hole in the middle
-    const int tx0 = max(P.eye_ti - (ring_hi - 1), 0), tx1 = min(P.eye_ti + (ring_hi - 1), nt - 1);
-    const int ty0 = max(P.eye_tj - (ring_hi - 1), 0), ty1 = min(P.eye_tj + (ring_hi - 1), nt - 1);
-    const unsigned int bw = (unsigned int)(tx1 - tx0 + 1), last = bw * (unsigned int)(ty1 - ty0 + 1);
+    // thread = tile of the band's ring, clipped to the mesh
+    const HzRing ring(P.eye_ti, P.eye_tj, nt, ring_lo, ring_hi);
+    const unsigned int last = ring.count();
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0;
-    for(unsigned int k0 = blockIdx.x * blockDim.x; k0 < last; k0 += nth)      // the same trip count CTA-wide
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    for(unsigned int k0 = blockIdx.x * blockDim.x + threadIdx.x - lane; k0 < last; k0 += nth)
     {
-        const unsigned int k = k0 + threadIdx.x;
+        const unsigned int k = k0 + lane;
+        const bool mine = k < last;
+        int ti = 0, tj = 0;
         bool on = false;
-        unsigned int id = 0;
-        if(k < last)
+        if(mine)
         {
-            const unsigned int row = k / bw;
-            const int ti = tx0 + (int)(k - row * bw), tj = ty0 + (int)row;
-            if(max(abs(ti - P.eye_ti), abs(tj - P.eye_tj)) >= ring_lo)
-            {
-                n_all++;
-                const int tc0 = ti * HZ_TILE_CELLS, tr0 = tj * HZ_TILE_CELLS;
-                const short2 mt = __ldg(P.mm_tile + (size_t)tj * nt + ti);
-                HzBox B;
-                const int r = hz_rect_test(P, tc0, min(tc0 + HZ_TILE_CELLS, N - 1), tr0, min(tr0 + HZ_TILE_CELLS, N - 1),
-                                           (float)mt.x, (float)mt.y, B);
-                if(r == HZ_RECT_DEAD_FAR)         n_far++;
-                else if(r == HZ_RECT_DEAD_WINDOW) n_window++;
-                else if(r == HZ_RECT_BOXED && hz_box_occluded_thread(P, B, P.occl_tile_max_pix)) n_occl++;
-                else { on = true; id = ((unsigned int)tj << 16) | (unsigned int)ti; }
-            }
+            ring.tile(k, ti, tj);
+            const short2 mt = __ldg(P.mm_tile + (size_t)tj * nt + ti);
+            const int tc0 = ti * HZ_TILE_CELLS, tr0 = tj * HZ_TILE_CELLS;
+            const int r = hz_rect_cull(P, tc0, min(tc0 + HZ_TILE_CELLS, N - 1), tr0, min(tr0 + HZ_TILE_CELLS, N - 1),
+                                       (float)mt.x, (float)mt.y, P.occl_tile_max_pix);
+            n_all++;
+            on = hz_rect_tally(r, n_far, n_window, n_occl);
         }
-        hz_cta_append(s_app, on, id, P.tile_queue, P.tile_count);
+        hz_stage_push(S.stage, staged, on, ((unsigned int)tj << 16) | (unsigned int)ti, P.tile_queue, P.tile_count, lane);
     }
+    if(staged) hz_stage_write(S.stage, staged, P.tile_queue, P.tile_count, lane);
     if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_TILES, n_all, n_far, n_window, n_occl);
 }
 
@@ -1252,24 +1301,26 @@ __global__ void __launch_bounds__(256, 3)
 k_blocks(const HzView* __restrict__ V)
 {
     HZ_KERNEL_PROLOGUE(V, P);
-    __shared__ HzCtaAppend s_app;
+    __shared__ HzCullWarp s_warp[8];
     __shared__ unsigned int s_stats[4];
+    const unsigned int lane = threadIdx.x & 31u;
+    HzCullWarp& S = s_warp[threadIdx.x >> 5];
     const int nb = P.nb, N = P.N;
     // blocks of (4 << lod) cells: (8 >> lod)^2 of them per tile
     const int lod = LOD ? P.lod : 0, sh = 3 - lod, side = 1 << sh, cells = HZ_BLOCK_CELLS << lod;
     const unsigned int total = *P.tile_count << (2 * sh);
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0;
-    for(unsigned int t0 = blockIdx.x * blockDim.x; t0 < total; t0 += nth)     // (the same trip count CTA-wide)
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    for(unsigned int t0 = blockIdx.x * blockDim.x + threadIdx.x - lane; t0 < total; t0 += nth)
     {
-        const unsigned int t = t0 + threadIdx.x;
+        const unsigned int t = t0 + lane;
         bool on = false;
-        unsigned int id = 0;
+        int bj = 0, bi = 0;
         if(t < total)
         {
             const unsigned int tile = P.tile_queue[t >> (2 * sh)];
             const int tj = (int)(tile >> 16), ti = (int)(tile & 0xFFFFu);
-            const int bj = tj * side + (int)((t >> sh) & (unsigned int)(side - 1)), bi = ti * side + (int)(t & (unsigned int)(side - 1));
+            bj = tj * side + (int)((t >> sh) & (unsigned int)(side - 1)); bi = ti * side + (int)(t & (unsigned int)(side - 1));
             if((bj << lod) < nb && (bi << lod) < nb)
             {
                 short2 mm = __ldg(P.mm_block + (size_t)(bj << lod) * nb + (bi << lod));
@@ -1285,19 +1336,16 @@ k_blocks(const HzView* __restrict__ V)
                         }
                     mm = make_short2((short)lo, (short)hi);
                 }
-                HzBox B;
                 const int c0 = bi * cells, r0 = bj * cells;
-                const int r = hz_rect_test(P, c0, min(c0 + cells, N - 1), r0, min(r0 + cells, N - 1),
-                                           (float)mm.x, (float)mm.y, B);
+                const int r = hz_rect_cull(P, c0, min(c0 + cells, N - 1), r0, min(r0 + cells, N - 1), (float)mm.x, (float)mm.y,
+                                           P.occl_block_max_pix);
                 n_all++;
-                if(r == HZ_RECT_DEAD_FAR)         n_far++;
-                else if(r == HZ_RECT_DEAD_WINDOW) n_window++;
-                else if(r == HZ_RECT_BOXED && hz_box_occluded_thread(P, B, P.occl_block_max_pix)) n_occl++;
-                else { on = true; id = ((unsigned int)bj << 16) | (unsigned int)bi; }
+                on = hz_rect_tally(r, n_far, n_window, n_occl);
             }
         }
-        hz_cta_append(s_app, on, id, P.block_queue, P.block_count);
+        hz_stage_push(S.stage, staged, on, ((unsigned int)bj << 16) | (unsigned int)bi, P.block_queue, P.block_count, lane);
     }
+    if(staged) hz_stage_write(S.stage, staged, P.block_queue, P.block_count, lane);
     if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
 }
 
@@ -1306,86 +1354,61 @@ k_blocks(const HzView* __restrict__ V)
 // Most of a live tile is dead at the block level (seen at a grazing angle a stretch of terrain is a fraction of a pixel
 // high and holds no pixel centre; what does is mostly hidden), and a rectangle test costs a few hundred instructions.
 // The MID variant therefore tests the 16 "mids" of every live tile first -- squares of 2x2 blocks = 8x8 cells, (min, max)
-// taken from the four blocks' entries of the pyramid -- one per thread, collects the survivors in shared memory, and then
-// tests their four blocks each, densely again (thread = (surviving mid, block), 256 at a time): about half the rectangle
-// tests per live tile, in full warps.  It is what the views of a batch use (throughput); a lone view is latency-bound
-// and keeps the one-level kernel, whose threads have one test each behind them instead of two.
-enum { HZ_RECT_OCCLUDED = 4 };
-
-__device__ __forceinline__ int
-hz_rect_cull(const HzView& P, int c_lo, int c_hi, int r_lo, int r_hi, float zmin, float zmax, int max_pix)
-{
-    HzBox B;
-    const int r = hz_rect_test(P, c_lo, c_hi, r_lo, r_hi, zmin, zmax, B);
-    return (r == HZ_RECT_BOXED && hz_box_occluded_thread(P, B, max_pix)) ? (int)HZ_RECT_OCCLUDED : r;
-}
-
-// appends `value` of the threads with `on` to list[*n ...] in shared memory; every thread of the CTA calls, *n was zeroed
-// (and the CTA synchronised) before, and the caller synchronises before it reads the list
-__device__ __forceinline__ void hz_smem_append(bool on, unsigned int value, unsigned int* list, unsigned int* n)
-{
-    const unsigned int lane = threadIdx.x & 31u;
-    const unsigned int ballot = __ballot_sync(0xffffffffu, on);
-    unsigned int base = 0;
-    if(lane == 0 && ballot) base = atomicAdd(n, (unsigned int)__popc(ballot));
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if(on) list[base + __popc(ballot & ((1u << lane) - 1u))] = value;
-}
-
+// taken from the four blocks' entries of the pyramid -- and then the four blocks of each mid that lives on: about half
+// the rectangle tests per live tile, in full warps.  A warp takes the 32 mids of two live tiles per trip, one per lane,
+// compacts the survivors in its shared memory and tests their blocks 32 at a time.  It is what the views of a batch use
+// (throughput); a lone view is latency-bound and keeps the one-level kernel, whose threads have one test each behind
+// them instead of two.
 __global__ void __launch_bounds__(256, 3)
 k_blocks_mid(const HzView* __restrict__ V)
 {
     HZ_KERNEL_PROLOGUE(V, P);
-    __shared__ HzCtaAppend s_app;
-    __shared__ unsigned int s_mids[256], s_nmids;
+    __shared__ HzCullWarp s_warp[8];
     __shared__ unsigned int s_stats[4];
+    const unsigned int lane = threadIdx.x & 31u;
+    HzCullWarp& S = s_warp[threadIdx.x >> 5];
     const int nb = P.nb, N = P.N;
     const int mid_pix = P.occl_tile_max_pix, block_pix = P.occl_block_max_pix;
     const unsigned int total = *P.tile_count * 16u;
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0;
-    for(unsigned int t0 = blockIdx.x * blockDim.x; t0 < total; t0 += nth)     // (the same trip counts CTA-wide, here and below)
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    for(unsigned int t0 = blockIdx.x * blockDim.x + threadIdx.x - lane; t0 < total; t0 += nth)
     {
-        __syncthreads();
-        if(threadIdx.x == 0) s_nmids = 0;
-        __syncthreads();
+        const unsigned int t = t0 + lane;
+        bool live = false;
+        int mj = 0, mi = 0;
+        if(t < total)
         {
-            const unsigned int t = t0 + threadIdx.x;
-            bool on = false;
-            unsigned int id = 0;
-            if(t < total)
+            const unsigned int tile = P.tile_queue[t >> 4];
+            mj = (int)(tile >> 16) * 4 + (int)((t >> 2) & 3u); mi = (int)(tile & 0xFFFFu) * 4 + (int)(t & 3u);
+            const int bj = 2 * mj, bi = 2 * mi;
+            if(bj < nb && bi < nb)
             {
-                const unsigned int tile = P.tile_queue[t >> 4];
-                const int mj = (int)(tile >> 16) * 4 + (int)((t >> 2) & 3u), mi = (int)(tile & 0xFFFFu) * 4 + (int)(t & 3u);
-                const int bj = 2 * mj, bi = 2 * mi;
-                if(bj < nb && bi < nb)
-                {
-                    const short2* mm = P.mm_block + (size_t)bj * nb + bi;
-                    const bool right = bi + 1 < nb, up = bj + 1 < nb;
-                    const short2 a = __ldg(mm), b = right ? __ldg(mm + 1) : a, c = up ? __ldg(mm + nb) : a,
-                                 d = (right && up) ? __ldg(mm + nb + 1) : a;
-                    const int lo = min(min((int)a.x, (int)b.x), min((int)c.x, (int)d.x));
-                    const int hi = max(max((int)a.y, (int)b.y), max((int)c.y, (int)d.y));
-                    const int c0 = bi * HZ_BLOCK_CELLS, r0 = bj * HZ_BLOCK_CELLS;
-                    const int r = hz_rect_cull(P, c0, min(c0 + 2 * HZ_BLOCK_CELLS, N - 1), r0, min(r0 + 2 * HZ_BLOCK_CELLS, N - 1),
-                                               (float)lo, (float)hi, mid_pix);
-                    on = r == HZ_RECT_ALIVE || r == HZ_RECT_BOXED;
-                    id = ((unsigned int)mj << 16) | (unsigned int)mi;
-                }
+                const short2* mm = P.mm_block + (size_t)bj * nb + bi;
+                const bool right = bi + 1 < nb, up = bj + 1 < nb;
+                const short2 a = __ldg(mm), b = right ? __ldg(mm + 1) : a, c = up ? __ldg(mm + nb) : a,
+                             d = (right && up) ? __ldg(mm + nb + 1) : a;
+                const int lo = min(min((int)a.x, (int)b.x), min((int)c.x, (int)d.x));
+                const int hi = max(max((int)a.y, (int)b.y), max((int)c.y, (int)d.y));
+                const int c0 = bi * HZ_BLOCK_CELLS, r0 = bj * HZ_BLOCK_CELLS;
+                const int r = hz_rect_cull(P, c0, min(c0 + 2 * HZ_BLOCK_CELLS, N - 1), r0, min(r0 + 2 * HZ_BLOCK_CELLS, N - 1),
+                                           (float)lo, (float)hi, mid_pix);
+                live = r == HZ_RECT_ALIVE || r == HZ_RECT_BOXED;
             }
-            hz_smem_append(on, id, s_mids, &s_nmids);
         }
-        __syncthreads();
-        const unsigned int items = s_nmids * 4u;
-        for(unsigned int jb = 0; jb < items; jb += 256u)
+        const unsigned int ballot = __ballot_sync(0xffffffffu, live);
+        if(live) S.mids[__popc(ballot & ((1u << lane) - 1u))] = ((unsigned int)mj << 16) | (unsigned int)mi;
+        __syncwarp();
+        const unsigned int items = (unsigned int)__popc(ballot) * 4u;
+        for(unsigned int jb = 0; jb < items; jb += 32u)
         {
-            const unsigned int item = jb + threadIdx.x;
+            const unsigned int item = jb + lane;
             bool on = false;
-            unsigned int id = 0;
+            int bj = 0, bi = 0;
             if(item < items)
             {
-                const unsigned int mid = s_mids[item >> 2];
-                const int bj = (int)(mid >> 16) * 2 + (int)((item >> 1) & 1u), bi = (int)(mid & 0xFFFFu) * 2 + (int)(item & 1u);
+                const unsigned int mid = S.mids[item >> 2];
+                bj = (int)(mid >> 16) * 2 + (int)((item >> 1) & 1u); bi = (int)(mid & 0xFFFFu) * 2 + (int)(item & 1u);
                 if(bj < nb && bi < nb)
                 {
                     const short2 mm = __ldg(P.mm_block + (size_t)bj * nb + bi);
@@ -1393,14 +1416,14 @@ k_blocks_mid(const HzView* __restrict__ V)
                     const int r = hz_rect_cull(P, c0, min(c0 + HZ_BLOCK_CELLS, N - 1), r0, min(r0 + HZ_BLOCK_CELLS, N - 1),
                                                (float)mm.x, (float)mm.y, block_pix);
                     n_all++;
-                    n_far += (r == HZ_RECT_DEAD_FAR); n_window += (r == HZ_RECT_DEAD_WINDOW); n_occl += (r == HZ_RECT_OCCLUDED);
-                    on = r == HZ_RECT_ALIVE || r == HZ_RECT_BOXED;
-                    id = ((unsigned int)bj << 16) | (unsigned int)bi;
+                    on = hz_rect_tally(r, n_far, n_window, n_occl);
                 }
             }
-            hz_cta_append(s_app, on, id, P.block_queue, P.block_count);
+            hz_stage_push(S.stage, staged, on, ((unsigned int)bj << 16) | (unsigned int)bi, P.block_queue, P.block_count, lane);
         }
+        __syncwarp();                                   // (the next trip writes S.mids again)
     }
+    if(staged) hz_stage_write(S.stage, staged, P.block_queue, P.block_count, lane);
     if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
 }
 
@@ -1620,8 +1643,14 @@ cudaError_t hz_launch_band(const HzView& v, const HzView* d_v, int nviews, bool 
     const bool any_band = worst_case && v.lod_capable;
     const int ring_hi = any_band ? v.nt : min(v.ring_hi, rmax + 1);
     if(!any_band && v.ring_lo >= ring_hi) return cudaSuccess;
-    // (the threads walk the band's bounding square, clipped to the mesh)
-    const long long side = min(2 * ring_hi - 1, v.nt), ntiles = side * side;
+    // (thread = tile of the band's ring: this view's, or for any eye at most the unclipped ring and at most the mesh)
+    long long ntiles;
+    if(worst_case)
+    {
+        const long long side = min(2 * ring_hi - 1, v.nt), hole = any_band ? 0 : 2 * v.ring_lo - 1;
+        ntiles = min(side * side, (2LL * ring_hi - 1) * (2 * ring_hi - 1) - hole * hole);
+    }
+    else ntiles = HzRing(v.eye_ti, v.eye_tj, v.nt, v.ring_lo, ring_hi).count();
     long long ctas = (ntiles + 255) / 256;
     if(ctas > (long long)hz_grid(v, 8, nviews)) ctas = hz_grid(v, 8, nviews);
     const unsigned int ny = (unsigned int)nviews;
