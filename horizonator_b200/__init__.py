@@ -72,6 +72,20 @@ class view_t(C.Structure):
     ]
 
 
+class poi_t(C.Structure):
+    """include/horizonator-batch.h: horizonator_poi_t (24 bytes)."""
+    _fields_ = [("lat", C.c_double), ("lon", C.c_double), ("ele", C.c_double)]
+
+
+class label_t(C.Structure):
+    """include/horizonator-batch.h: horizonator_label_t (16 bytes)."""
+    _fields_ = [("x", C.c_float), ("y", C.c_float), ("range_m", C.c_float), ("range_rendered_m", C.c_float)]
+
+
+#: numpy dtype of label_t: what annotate() returns
+LABEL_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("range_m", np.float32), ("range_rendered_m", np.float32)])
+
+
 def _declare(lib):
     P = C.POINTER
     ctx = P(context_t)
@@ -120,6 +134,8 @@ def _declare(lib):
         "horizonator_profile_read": (b, [ctx, P(f * 6), P(i)]),
         "horizonator_viewshed_device": (b, [ctx, i, P(view_t), f, vp, vp, vp]),
         "horizonator_viewshed": (b, [ctx, i, P(view_t), f, vp, vp]),
+        "horizonator_annotate_batch_device": (b, [ctx, i, P(view_t), i, vp, vp, vp, vp, vp]),
+        "horizonator_annotate_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         try:
@@ -150,6 +166,7 @@ EXPORTED_SYMBOLS = (
     "horizonator_render_wedge_host", "horizonator_host_register", "horizonator_host_unregister",
     "horizonator_debug_device_math", "horizonator_set_lod",
     "horizonator_viewshed_device", "horizonator_viewshed",
+    "horizonator_annotate_batch_device", "horizonator_annotate_batch",
 )
 
 if not os.path.exists(LIBRARY_PATH):
@@ -461,6 +478,42 @@ class horizonator:
         if not lib.horizonator_viewshed_device(C.byref(self._ctx), len(views), self._eyes(views), float(target_height),
                                                d_masks or None, d_counts or None, stream or None):
             raise RuntimeError("horizonator_viewshed_device() failed")
+
+
+    # labels of points of interest (horizonator_annotate_batch*: which POIs each view sees, and where)
+    @staticmethod
+    def pois_array(pois):
+        """A sequence of (lat, lon, ele) or an (m, 3) array -> (m, 3) C-contiguous float64 (horizonator_poi_t[m])."""
+        return np.ascontiguousarray(np.asarray(pois, dtype=np.float64).reshape(-1, 3))
+
+    def annotate(self, views, pois):
+        """views as render_batch takes them; pois: (lat, lon, ele) each, ele in metres.  Returns an (n, m) structured
+        array (LABEL_DTYPE): x, y (marker pixel; all fields -1 where the POI is outside the window), range_m, and
+        range_rendered_m (> 0 exactly when the view sees the POI).  Only the labels leave the GPU."""
+        p = self.pois_array(pois)
+        n, m = len(views), p.shape[0]
+        out = _pool.array((n, m, 4), np.float32)
+        if not lib.horizonator_annotate_batch(C.byref(self._ctx), n, self._views(views), m, p.ctypes.data if m else None,
+                                              out.ctypes.data if out.size else None):
+            raise RuntimeError("horizonator_annotate_batch() failed")
+        return out.view(LABEL_DTYPE).reshape(n, m)
+
+    def annotate_device(self, views, d_pois, d_labels, d_images=0, d_ranges=0, stream=0, m=None):
+        """Device-memory variant.  d_pois: an (m, 3) float64 CUDA tensor, or an integer device address with `m` given;
+        d_labels: an (n, m, 4) float32 CUDA tensor (a view as LABEL_DTYPE is the same memory) or an integer address;
+        d_images / d_ranges as render_batch_device (0 = not written); stream as render_batch_device."""
+        if hasattr(d_pois, "data_ptr"):
+            if m is None:
+                m = d_pois.shape[0]
+            d_pois = d_pois.data_ptr()
+        if m is None:
+            raise ValueError("annotate_device: m is needed when d_pois is an address")
+        if hasattr(d_labels, "data_ptr"):
+            d_labels = d_labels.data_ptr()
+        if not lib.horizonator_annotate_batch_device(C.byref(self._ctx), len(views), self._views(views), int(m),
+                                                     d_pois or None, d_labels or None, d_images or None, d_ranges or None,
+                                                     stream or None):
+            raise RuntimeError("horizonator_annotate_batch_device() failed")
 
 
 class _PinnedBlock:

@@ -45,7 +45,7 @@ def build_library(force=False, extra_flags=(), verbose=False, name="libhorizonat
     os.makedirs(LIB, exist_ok=True)
     out = os.path.join(LIB, name)
     srcs = [os.path.join(CSRC, f) for f in ("hz_kernels.cu", "hz_api.cpp", "hz_dem.cpp")]
-    deps = srcs + [os.path.join(CSRC, f) for f in ("hz_device.h", "hz_math.cuh")] + \
+    deps = srcs + [os.path.join(CSRC, f) for f in ("hz_device.h", "hz_math.cuh", "hz_project.h")] + \
         [os.path.join(ROOT, "include", f) for f in ("horizonator.h", "horizonator-batch.h", "dem.h", "util.h")] + \
         [os.path.abspath(__file__)]
     if force or _newer(out, deps):

@@ -10,6 +10,7 @@
 #include "horizonator-batch.h"
 #include "util.h"
 #include "hz_device.h"
+#include "hz_project.h"
 
 #include <cmath>
 #include <cstddef>
@@ -205,9 +206,17 @@ struct ViewSet
     // the standard chain, captured on first use per (number of views, shape)
     // (several executable instances each, used in turn: an instance that is still in flight makes the next launch of
     // the SAME instance wait on the host)
-    struct Graph { int m; bool big_per_band; std::vector<GraphExecHandle> exec; size_t next; int launches; };
+    // (variants: with k_resolve or without it -- labels only -- and with k_annotate after the chain or without it)
+    struct Graph { int m; bool big_per_band, resolve, annotate; std::vector<GraphExecHandle> exec; size_t next; int launches; };
     std::vector<Graph> graphs;
     bool graph_failed = false;
+    // labels of points of interest (horizonator_annotate_batch*), made on first use: k_annotate's per-chunk block (a
+    // pinned ring beside h_views, copied with them to one device address, so that a captured chain replays for any
+    // POIs), and for the host-memory call the labels of one chunk, copied to the caller on the set's stream
+    DevPtr<HzAnnotate>  d_annot;
+    HostPtr<HzAnnotate> h_annot;       // pinned [PARAM_RING]
+    DevPtr<float4>      d_labels;
+    size_t labels_cap = 0;             // labels d_labels holds
 };
 
 struct Slot
@@ -269,6 +278,10 @@ struct Slot
     int              vs_mask_views = 0;
     DevPtr<uint32_t> d_vs_counts;
     EventHandle      vs_done;
+
+    // labels (horizonator_annotate_batch): the POIs of the host-memory call, uploaded per call, made on first use
+    DevPtr<double>   d_pois;             // [pois_cap][3]
+    size_t           pois_cap = 0;
 };
 
 // raw pointers: a slot is deleted by horizonator_deinit(), never by a destructor at exit, when the CUDA runtime may
@@ -517,7 +530,7 @@ bool big_after_every_band(const Slot& s, const ViewState& vs)
 
 // the kernels of one render of m views, in order, reading their parameters from set.d_views; hv = the host copy of those
 bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool worst_case, bool resolve,
-                  cudaStream_t st, const EventHandle* ev, int* launches)
+                  bool annotate, cudaStream_t st, const EventHandle* ev, int* launches)
 {
     const HzView* dv = set.d_views.get();
     int n = 0;
@@ -557,6 +570,9 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
     if(fork) CUDA_TRY(cudaStreamWaitEvent(st, set.ev_join.get(), 0));
     if(resolve) { CUDA_TRY(hz_launch_resolve(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
     if(ev) CUDA_TRY(cudaEventRecord(ev[6].get(), st));
+    // the labels: after the join (the near pass's large triangles are in the visibility buffers), before the set's next
+    // chunk reuses those buffers (the same stream)
+    if(annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.d_annot.get(), m, st)); n++; }
     *launches = n;
     return true;
 }
@@ -564,7 +580,7 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
 // Captures the standard chain (full width, vectorised resolve, grids sized for any eye position) for m views of the
 // set; every later standard render of m views is one cudaGraphLaunch after the parameter copy.  A dozen separate
 // launches cost more host time than the GPU needs for the render.
-ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band)
+ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool resolve, bool annotate)
 {
     const StreamHandle cs = make_stream();
     if(!cs) { cudaGetLastError(); return nullptr; }
@@ -573,7 +589,7 @@ ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bo
     int launches = 0;
     if(ok)
     {
-        ok = launch_chain(s, set, hv, m, big_per_band, true, true, cs.get(), nullptr, &launches);
+        ok = launch_chain(s, set, hv, m, big_per_band, true, resolve, annotate, cs.get(), nullptr, &launches);
         if(cudaStreamEndCapture(cs.get(), &captured) != cudaSuccess) ok = false;
     }
     const GraphHandle g(captured);
@@ -589,7 +605,7 @@ ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bo
         MSG("CUDA graph capture of the render chain failed; launching the kernels one by one instead");
         return nullptr;
     }
-    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, std::move(exec), 0, launches });
+    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, resolve, annotate, std::move(exec), 0, launches });
     return &set.graphs.back();
 }
 
@@ -678,12 +694,33 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
     for(int d = 0; d < out.n; d++) { v.out_image[d] = out.image[d]; v.out_ranges[d] = out.ranges[d]; }
 }
 
+// The labels of a chunk's views (k_annotate): the POIs (device), how many, where the label of the chunk's first view and
+// POI 0 goes (device; view k's follow m labels further per view), and the per-view inputs of the projection.
+struct AnnotSpec
+{
+    const double* pois;
+    int m;
+    float4* labels;
+    const HzAnnotView* views;
+};
+static_assert(sizeof(((HzAnnotate*)nullptr)->view) / sizeof(HzAnnotView) >= VIEWS_PER_SET, "HzAnnotate: a view set's views");
+
 // Enqueues one render of columns [x0,x1) of m views (m <= what ensure_views() gave) on stream st: view k uses scratch
-// set.sc[k] and writes to outs[k] (device memory).  All views of one call must have the same kinds of output.
-bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st)
+// set.sc[k] and writes to outs[k] (device memory), and, with `ann`, the labels of the POIs for each view after the
+// render.  All views of one call must have the same kinds of output.
+bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st,
+                   const AnnotSpec* ann = nullptr)
 {
     if(s.W <= 0 || s.H <= 0 || m < 1 || m > (int)set.sc.size()) return false;
     const bool want_image = outs[0].image[0] != nullptr, want_ranges = outs[0].ranges[0] != nullptr;
+    const bool resolve = want_image || want_ranges, annotate = ann != nullptr;
+    if(annotate && !set.d_annot)
+    {
+        DevPtr<HzAnnotate> d = make_device<HzAnnotate>(1);
+        HostPtr<HzAnnotate> h = make_host<HzAnnotate>(PARAM_RING);
+        if(empty_handle(d, "cudaMalloc(annotate)") || empty_handle(h, "cudaMallocHost(annotate)")) return false;
+        set.d_annot = std::move(d); set.h_annot = std::move(h);
+    }
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
     if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy.get(), 0));
 
@@ -748,8 +785,9 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
             vb.cell_diag2 = hk[0].cell_diag2 * (float)((1 << lod) * (1 << lod));
             lo = vb.ring_hi;
         }
-        // the row table of this view's window, unless the scratch still holds it from its previous render
-        if(want_ranges && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
+        // the row table of this view's window, unless the scratch still holds it from its previous render (the ranges and
+        // the labels' rendered ranges need it)
+        if((want_ranges || annotate) && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
         {
             float* h_row = set.h_tanel.get() + ((size_t)slot * set.cap + k) * s.H;
             memcpy(h_row, tanel_row(s, vs[k].az_deg0, vs[k].az_deg1), (size_t)s.H * sizeof(float));
@@ -758,17 +796,26 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         }
     }
     CUDA_TRY(cudaMemcpyAsync(set.d_views.get(), hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
+    if(annotate)
+    {
+        HzAnnotate* ha = set.h_annot.get() + slot;
+        ha->pois = ann->pois; ha->labels = ann->labels; ha->m = ann->m; ha->pad = 0;
+        for(int k = 0; k < m; k++) ha->view[k] = ann->views[k];
+        CUDA_TRY(cudaMemcpyAsync(set.d_annot.get(), ha, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView),
+                                 cudaMemcpyHostToDevice, st));
+    }
     CUDA_TRY(cudaEventRecord(set.ring_ev[slot].get(), st));
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
     const bool is_main = (&set == &s.main);
-    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (want_image || want_ranges) &&
-                          outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && vectorisable;
+    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (resolve || annotate) &&
+                          outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && (vectorisable || !resolve);
     if(standard && !set.graph_failed)
     {
         ViewSet::Graph* g = nullptr;
-        for(ViewSet::Graph& c : set.graphs) if(c.m == m && c.big_per_band == big_per_band) g = &c;
-        if(g == nullptr && (g = capture_graph(s, set, hv, m, big_per_band)) == nullptr) set.graph_failed = true;
+        for(ViewSet::Graph& c : set.graphs)
+            if(c.m == m && c.big_per_band == big_per_band && c.resolve == resolve && c.annotate == annotate) g = &c;
+        if(g == nullptr && (g = capture_graph(s, set, hv, m, big_per_band, resolve, annotate)) == nullptr) set.graph_failed = true;
         if(g != nullptr)
         {
             CUDA_TRY(cudaGraphLaunch(g->exec[g->next].get(), st));
@@ -794,7 +841,7 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     }
     int launches = 0;
     // grids sized for this view's eye tile only when there is just one view
-    if(!launch_chain(s, set, hv, m, big_per_band, m > 1, want_image || want_ranges, st, ev, &launches)) return false;
+    if(!launch_chain(s, set, hv, m, big_per_band, m > 1, resolve, annotate, st, ev, &launches)) return false;
     CUDA_TRY(cudaEventRecord(set.busy.get(), st)); set.last_stream = st; set.busy_recorded = true;
     s.launches_last = launches;
     if(is_main) s.have_render = (x0 == 0 && x1 == s.W);
@@ -802,9 +849,10 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
 }
 
 // one view on the context's own scratch
-bool enqueue_render(Slot& s, const ViewState& vs, int x0, int x1, const OutSpec& out, cudaStream_t st)
+bool enqueue_render(Slot& s, const ViewState& vs, int x0, int x1, const OutSpec& out, cudaStream_t st,
+                    const AnnotSpec* ann = nullptr)
 {
-    return enqueue_views(s, s.main, 1, &vs, x0, x1, &out, st);
+    return enqueue_views(s, s.main, 1, &vs, x0, x1, &out, st, ann);
 }
 
 // lib:765-789, float as written there.  The four samples come from the host mmaps (dem.h).
@@ -1266,26 +1314,12 @@ bool horizonator_pick(const horizonator_context_t* ctx, float* lat, float* lon, 
                                  s->view.az_deg0, s->view.az_deg1, s->W, s->H);
 }
 
-// ---- pure host geometry (lib:1053-1213): double precision, no device involved ----------------------------
-
-static double unwrap_near_rad_d(double x, double near)
-{
-    const double d = (x - near) / (2. * M_PI);
-    return (d - round(d)) * 2. * M_PI + near;
-}
+// ---- host geometry (lib:1053-1213): double precision; the projection is hz_project.h, which k_annotate shares -------
 
 bool horizonator_x_from_az(double* x, double* az_ndc_per_rad,
                            double az_rad, double az_rad0, double az_rad1, int width)
 {
-    az_rad1 = unwrap_near_rad_d(az_rad1 - az_rad0, M_PI) + az_rad0;
-    const double center = (az_rad0 + az_rad1) / 2.;
-    az_rad = unwrap_near_rad_d(az_rad, center);
-    const double per_rad = 2.0 / (az_rad1 - az_rad0);
-    const double az_ndc  = (az_rad - center) * per_rad;
-    if(!(-1. <= az_ndc && az_ndc <= 1.)) return false;
-    if(az_ndc_per_rad != nullptr) *az_ndc_per_rad = per_rad;
-    *x = (az_ndc + 1.) / 2. * width - 0.5;                               // NDC [-1,1] -> pixel (-0.5, W-0.5)
-    return true;
+    return hz_x_from_az(x, az_ndc_per_rad, az_rad, az_rad0, az_rad1, width);     // (hz_project.h: k_annotate shares it)
 }
 
 bool horizonator_project(double* x, double* y, double* range,
@@ -1293,23 +1327,8 @@ bool horizonator_project(double* x, double* y, double* range,
                          double lat, double lon, double ele,
                          double az_rad0, double az_rad1, int width, int height)
 {
-    const float Rearth = 6371000.0;
-    const double dlat = (lat - lat_viewer) * M_PI / 180;
-    const double dlon = (lon - lon_viewer) * M_PI / 180;
-    const double east  = dlon * Rearth * cos_lat_viewer;
-    const double north = dlat * Rearth;
-    const double d2 = east * east + north * north;
-
-    double per_rad;
-    if(!horizonator_x_from_az(x, &per_rad, atan2(east, north), az_rad0, az_rad1, width)) return false;
-
-    const double h = ele - ele_viewer;
-    *range = sqrt(d2 + h * h);
-    const double aspect = (double)width / (double)height;
-    const double el_ndc = atan2(h, sqrt(d2)) * aspect * per_rad;
-    if(!(-1. <= el_ndc && el_ndc <= 1.)) return false;
-    *y = (-el_ndc + 1.) / 2. * height - 0.5;
-    return true;
+    return hz_project(x, y, range, lat_viewer, cos_lat_viewer, lon_viewer, ele_viewer, lat, lon, ele,
+                      az_rad0, az_rad1, width, height);
 }
 
 bool horizonator_unproject(float* lat, float* lon, int x, int y,
@@ -1344,8 +1363,29 @@ bool horizonator_unproject(float* lat, float* lon, int x, int y,
 // kernels overlap another chunk's.  The sets start after everything already queued on `st`, and `st` continues after
 // all of them.  to_host: outputs go through the views' device staging buffers and device->host copies on the set's
 // stream, which overlap the other sets' kernels.
+// ann: the labels of m POIs for every view as well (horizonator_annotate_batch*), by k_annotate after each chunk's chain;
+// into device memory, or (to_host) through the set's label scratch and a copy on its stream.
+struct AnnotReq
+{
+    const double* d_pois;
+    int m;
+    float4* labels;              // [n][m]: device memory, or host memory when to_host
+};
+
+// makes sure a set's label scratch holds `count` labels (host-memory call only; those are synchronous, so nothing queued
+// still uses the old buffer once the set's stream is idle)
+static bool ensure_labels(ViewSet& set, cudaStream_t st, size_t count)
+{
+    if(set.labels_cap >= count) return true;
+    CUDA_TRY(cudaStreamSynchronize(st));
+    set.d_labels = nullptr; set.labels_cap = 0;
+    if(empty_handle(set.d_labels = make_device<float4>(count), "cudaMalloc(labels)")) return false;
+    set.labels_cap = count;
+    return true;
+}
+
 static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
-                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st)
+                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const AnnotReq* ann = nullptr)
 {
     const size_t px = (size_t)s->W * s->H;
     std::vector<ViewState> vs((size_t)n);
@@ -1356,6 +1396,15 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         vs[k].az_deg0 = views[k].az_deg0; vs[k].az_deg1 = views[k].az_deg1;
     }
     if(n == 0) return true;
+    // the projection's inputs per view, as write_labels() of the command-line tool forms them (horizonator-batch.h)
+    std::vector<HzAnnotView> av(ann ? (size_t)n : 0);
+    for(size_t k = 0; k < av.size(); k++)
+    {
+        const double lat = (double)views[k].lat;
+        av[k] = HzAnnotView{ lat, (double)views[k].lon, cos(lat * M_PI / 180.), (double)vs[k].viewer_z,
+                             (double)views[k].az_deg0 * M_PI / 180., (double)views[k].az_deg1 * M_PI / 180. };
+    }
+    const size_t m_poi = ann ? (size_t)ann->m : 0;
 
     // chunk size: the views spread evenly over the sets, at most VIEWS_PER_SET each, at most what fits in memory
     int n_sets = 0, chunk = 0;
@@ -1383,21 +1432,27 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     if(n_sets == 0)
     {
         // one view, or no memory for a set: one at a time on the context's own scratch
+        if(ann && to_host && !ensure_labels(s->main, st, m_poi)) return false;
         for(int k = 0; k < n; k++)
         {
             uint8_t* di = images ? (to_host ? s->d_image.get()  : images + (size_t)k * px * 3) : nullptr;
             float*   dr = ranges ? (to_host ? s->d_ranges.get() : ranges + (size_t)k * px)     : nullptr;
-            if(!enqueue_render(*s, vs[k], 0, s->W, single_out(di, dr), st)) return false;
+            AnnotSpec a{};
+            if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? s->main.d_labels.get() : ann->labels + (size_t)k * m_poi, &av[k] };
+            if(!enqueue_render(*s, vs[k], 0, s->W, single_out(di, dr), st, ann ? &a : nullptr)) return false;
             if(to_host)
             {
                 if(images && !copy_to_host(images + (size_t)k * px * 3, di, px * 3, st)) return false;
                 if(ranges && !copy_to_host(ranges + (size_t)k * px, dr, px * sizeof(float), st)) return false;
+                if(ann && !copy_to_host(ann->labels + (size_t)k * m_poi, a.labels, m_poi * sizeof(float4), st)) return false;
             }
         }
         s->have_render = false;     // the visibility buffer no longer matches the context's own view
         return true;
     }
 
+    for(int g = 0; g < n_sets && ann && to_host; g++)
+        if(!ensure_labels(*s->sets[g], s->sets[g]->stream.get(), (size_t)chunk * m_poi)) return false;
     CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
     for(int g = 0; g < n_sets; g++) CUDA_TRY(cudaStreamWaitEvent(s->sets[g]->stream.get(), s->fork_ev.get(), 0));
     bool ok = true;
@@ -1409,12 +1464,16 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         for(int k = 0; k < m; k++)
             outs[k] = single_out(images ? (to_host ? set.sc[k].d_image.get()  : images + (size_t)(k0 + k) * px * 3) : nullptr,
                                  ranges ? (to_host ? set.sc[k].d_ranges.get() : ranges + (size_t)(k0 + k) * px)     : nullptr);
-        ok = enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), set.stream.get());
+        AnnotSpec a{};
+        if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? set.d_labels.get() : ann->labels + (size_t)k0 * m_poi, &av[k0] };
+        ok = enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), set.stream.get(), ann ? &a : nullptr);
         for(int k = 0; k < m && ok && to_host; k++)
         {
             if(images) ok = ok && copy_to_host(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3, set.stream.get());
             if(ranges) ok = ok && copy_to_host(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges.get(), px * sizeof(float), set.stream.get());
         }
+        if(ok && ann && to_host)
+            ok = copy_to_host(ann->labels + (size_t)k0 * m_poi, a.labels, (size_t)m * m_poi * sizeof(float4), set.stream.get());
     }
     if(!ok)
     {
@@ -1570,6 +1629,65 @@ bool horizonator_render_batch(const horizonator_context_t* ctx, int n, const hor
     DeviceGuard g(s->device);
     if(!render_batch_common(ctx, s, n, views, (uint8_t*)images, ranges, true, s->stream.get())) return false;
     CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
+    return true;
+}
+
+// ---- labels of points of interest (horizonator-batch.h) ----------------------------------------------------------
+
+// the argument rules of both annotate calls; false: nothing may be done
+static bool annotate_args_ok(const char* fn, int n, const horizonator_view_t* views, int m, const void* pois, const void* labels)
+{
+    if(n < 0 || m < 0) { MSG("%s: negative count (n = %d, m = %d)", fn, n, m); return false; }
+    if(n == 0 || m == 0) return true;
+    if(views == nullptr || pois == nullptr || labels == nullptr) { MSG("%s: views, POIs and labels are required", fn); return false; }
+    return true;
+}
+
+bool horizonator_annotate_batch_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                       int m, const horizonator_poi_t* d_pois, horizonator_label_t* d_labels,
+                                       void* d_images, void* d_ranges, void* stream)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !annotate_args_ok("horizonator_annotate_batch_device", n, views, m, d_pois, d_labels)) return false;
+    if(n == 0 || m == 0) return true;
+    if(((uintptr_t)d_pois & 7) != 0 || ((uintptr_t)d_labels & 15) != 0)
+    {
+        MSG("horizonator_annotate_batch_device: d_pois must be 8-byte and d_labels 16-byte aligned");
+        return false;
+    }
+    DeviceGuard g(s->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
+    const AnnotReq ann{ (const double*)d_pois, m, (float4*)d_labels };
+    if(!render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &ann)) return false;
+    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
+    return true;
+}
+
+bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                int m, const horizonator_poi_t* pois, horizonator_label_t* labels)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !annotate_args_ok("horizonator_annotate_batch", n, views, m, pois, labels)) return false;
+    if(n == 0 || m == 0) return true;
+    DeviceGuard g(s->device);
+    cudaStream_t st = s->stream.get();
+    // the POIs go up once per call into the context's scratch (the call is synchronous: no earlier one still reads it)
+    if(s->pois_cap < (size_t)m)
+    {
+        CUDA_TRY(cudaStreamSynchronize(st));
+        s->d_pois = nullptr; s->pois_cap = 0;
+        if(empty_handle(s->d_pois = make_device<double>(3 * (size_t)m), "cudaMalloc(POIs)")) return false;
+        s->pois_cap = (size_t)m;
+    }
+    CUDA_TRY(cudaMemcpyAsync(s->d_pois.get(), pois, (size_t)m * sizeof(horizonator_poi_t), cudaMemcpyHostToDevice, st));
+    const AnnotReq ann{ s->d_pois.get(), m, (float4*)labels };
+    if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &ann))
+    {
+        cudaStreamSynchronize(st);
+        cudaGetLastError();
+        return false;
+    }
+    CUDA_TRY(cudaStreamSynchronize(st));
     return true;
 }
 

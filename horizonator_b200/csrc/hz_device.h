@@ -187,6 +187,22 @@ cudaError_t hz_launch_big    (const HzView& v, const HzView* d_v, int nviews, cu
 cudaError_t hz_launch_resolve(const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);
 bool        hz_resolve_is_vectorisable(const HzView& v);
 cudaError_t hz_launch_horizon(const float* ranges, int n, int W, int H, int* rows, float* range, cudaStream_t stream);
+// ---- labels of points of interest (horizonator_annotate_batch*: the rule is in include/horizonator-batch.h) -----
+// What k_annotate needs of a view beyond its HzView (whose size the 128-bit prologue fixes), computed on the host as
+// write_labels() of the command-line tool does: the eye in double, cos(lat) of the eye, the azimuths in radians.
+struct HzAnnotView { double lat, lon, cos_lat, ele, az_rad0, az_rad1; };
+// The per-chunk block, copied to the device with the HzView variants (one fixed address per view set, so a captured
+// chain replays for any POI set).  The label of the chunk's view k and POI i is labels[k * m + i].
+struct HzAnnotate
+{
+    const double* pois;          // [m][3] lat, lon, ele (horizonator_poi_t)
+    float4*       labels;        // x, y, range_m, range_rendered_m (horizonator_label_t)
+    int           m;
+    int           pad;
+    HzAnnotView   view[64];      // [nviews] (VIEWS_PER_SET)
+};
+// after the render chain of a chunk (its visibility buffers and tan(elevation) rows), on the same stream
+cudaError_t hz_launch_annotate(const HzView& v, const HzView* d_v, const HzAnnotate* d_a, int nviews, cudaStream_t stream);
 // ---- viewsheds (horizonator_viewshed*: the definition is in include/horizonator-batch.h) ------
 constexpr int HZ_VS_MAX_VIEWS = 64;     // views per k_viewshed launch (gridDim.y); their eyes travel in the parameters
 struct HzViewshedEye { float vci, vcj, vz, cos_lat; };     // compute_move()'s eye, float as there

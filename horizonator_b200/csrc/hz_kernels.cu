@@ -18,6 +18,8 @@
 //   k_peer_barrier (multi-GPU)  barrier between the ranks of a wedge-sharded panorama through peer memory
 //   k_resolve4 / k_resolve1 (render)  keys -> BGR8 image + float range image, top row first   lib:936-1048
 //   k_horizon  (extra)   range image -> per-column topmost terrain row and its range
+//   k_annotate (labels)  points of interest -> marker position and the matched rendered range, read from the
+//                        visibility buffers of the views just rendered                     annotator.c:280-348
 //   k_viewshed, k_viewshed_count (viewsheds)  R2 ray casting over the DEM square, one thread per ray -> bit masks;
 //                        masks -> per-vertex counts of the views that see it
 //
@@ -27,7 +29,9 @@
 // Compiled with -fmad=false: plain a*b+c is two IEEE roundings (see hz_math.cuh).
 #include "hz_device.h"
 #include "hz_math.cuh"
+#include "hz_project.h"
 
+#include <cfloat>
 #include <cstdint>
 #include <cstdlib>
 
@@ -1975,6 +1979,77 @@ cudaError_t hz_launch_horizon(const float* ranges, int n, int W, int H, int* row
     if(total <= 0) return cudaSuccess;
     k_horizon<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(ranges, n, W, H, rows, range);
     return cudaGetLastError();
+}
+
+// ================================================================================================
+// k_annotate: labels of points of interest (include/horizonator-batch.h states the rule: the command-line tool's
+// write_labels(), annotator.c:280-348), read straight from the visibility buffers of the chunk just rendered
+// ================================================================================================
+
+#define HZ_ANNOT_CTAS   16          /* CTAs per view: a fixed grid, so that one captured chain serves any number of POIs */
+#define HZ_MARKER_DIST_MIN   500.0  /* annotator.c:19-23 */
+#define HZ_MARKER_DIST_MAX   100000.0
+#define HZ_MARKER_RANGE_FUZZ 500.0
+#define HZ_MARKER_PIXEL_FUZZ 6
+
+// One thread per (view, POI), gridDim.y = view of the chunk, the POIs strided over the view's CTAs.  The projection is
+// hz_project() in double (the host's horizonator_project(), same source); the <= 12 rendered ranges of the vertical
+// search are the keys of GL row H-1-r, column col, converted by hz_range_of_q() exactly as k_resolve converts them, so
+// that a label equals one computed from the range image of the same render.  Register budget: 4 CTAs of 256 threads per
+// SM, 64 registers (ptxas -v: no spills).
+__global__ void __launch_bounds__(HZ_CTA_THREADS, 4)
+k_annotate(const HzView* __restrict__ V, const HzAnnotate* __restrict__ A)
+{
+    HZ_KERNEL_PROLOGUE(V, P);
+    const HzAnnotView& v = A->view[blockIdx.y];
+    const double lat = v.lat, lon = v.lon, cos_lat = v.cos_lat, ele = v.ele, az0 = v.az_rad0, az1 = v.az_rad1;
+    const int W = P.W, H = P.H, m = A->m;
+    const unsigned int ep = P.epoch;
+    const float znear = P.znear, zfar = P.zfar;
+    const unsigned long long* const vis = P.vis;
+    const float* const tanel = P.tanel;
+    const double* const pois = A->pois;
+    float4* const labels = A->labels + (size_t)blockIdx.y * (size_t)m;
+
+    for(int i = blockIdx.x * HZ_CTA_THREADS + threadIdx.x; i < m; i += gridDim.x * HZ_CTA_THREADS)
+    {
+        float4 out = make_float4(-1.0f, -1.0f, -1.0f, -1.0f);
+        double x, y, range;
+        if(hz_project(&x, &y, &range, lat, cos_lat, lon, ele, pois[3 * i], pois[3 * i + 1], pois[3 * i + 2], az0, az1, W, H))
+        {
+            out.x = (float)x; out.y = (float)y; out.z = (float)range;
+            const long col = lround(x);
+            if(range >= HZ_MARKER_DIST_MIN && range <= HZ_MARKER_DIST_MAX && col >= 0 && col < W)
+            {
+                int best = 0;
+                double best_err = DBL_MAX;
+                float best_have = -1.0f;
+                const long ry = lround(y);
+                for(int d = -HZ_MARKER_PIXEL_FUZZ; d < HZ_MARKER_PIXEL_FUZZ; d++)
+                {
+                    if(y + (double)d < 0) continue;
+                    if(y + (double)d >= H) break;
+                    const long r = ry + d;
+                    if(r < 0 || r >= H) continue;
+                    const int gl = H - 1 - (int)r;                   // image row r (top first) = GL row H-1-r
+                    const unsigned int q = hz_key_q(vis[(size_t)gl * (size_t)W + (size_t)col], ep);
+                    const float have = hz_range_of_q(q, __ldg(tanel + gl), znear, zfar);
+                    if(have <= 0.0f) continue;
+                    const double err = fabs(range - (double)have);
+                    if(err < best_err) { best_err = err; best = d; best_have = have; }
+                    else break;                                 // ranges only get nearer further down
+                }
+                if(best_err < HZ_MARKER_RANGE_FUZZ) { out.y = (float)(y + (double)best); out.w = best_have; }
+            }
+        }
+        labels[i] = out;
+    }
+}
+
+cudaError_t hz_launch_annotate(const HzView& v, const HzView* d_v, const HzAnnotate* d_a, int nviews, cudaStream_t stream)
+{
+    (void)v;
+    return hz_launch(k_annotate, dim3(HZ_ANNOT_CTAS, (unsigned)nviews), dim3(HZ_CTA_THREADS), stream, d_v, d_a);
 }
 
 // ================================================================================================

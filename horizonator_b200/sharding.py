@@ -7,7 +7,8 @@ collective on the data path of a render:
 * viewpoint batch -- every viewpoint is an independent render against the same read-only DEM square, which each
   rank loads for itself.  Viewpoints are block-partitioned; outputs stay sharded on the rank that made them.
   Only reduced products (horizon profiles, a few bytes per image column) are gathered.  Viewsheds partition the same
-  way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).
+  way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).  Labels of
+  points of interest too: 16 bytes per (view, POI) are gathered (annotate_sharded).
 * azimuth wedges  -- one giant panorama: rank g renders columns [edges[g], edges[g+1]), bit-identical to the same
   columns of an unsharded render.  PeerPanorama fuses the exchange into the renderer: each rank's resolve kernel
   stores its wedge straight into every rank's full panorama over NVLink (peer memory), a barrier is the only
@@ -332,3 +333,19 @@ def render_batch_sharded(h, views, group=None, gather_profiles=True):
         rows, r = horizon_profile(rng)
         profiles = (gather_blocks(rows, len(views), group), gather_blocks(r, len(views), group))
     return img, rng, (lo, hi), profiles
+
+
+def annotate_sharded(h, views, pois, group=None):
+    """Labels of points of interest for a viewpoint batch over the ranks: `views` block-partitioned, this rank's share
+    labelled on its own GPU without writing any panorama (horizonator_annotate_batch_device), and the labels gathered.
+    pois: (lat, lon, ele) each, or an (m, 3) array.  Returns the (n, m, 4) float32 CUDA tensor of all views' labels
+    (x, y, range_m, range_rendered_m; see horizonator-batch.h) on every rank.  All ranks must hold contexts of the same
+    DEM square and size."""
+    world, rank = _world(group)
+    lo, hi = block_partition(len(views), world, rank)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    p = torch.as_tensor(h.pois_array(pois), device=dev)
+    labels = torch.empty((hi - lo, p.shape[0], 4), dtype=torch.float32, device=dev)
+    if hi > lo and p.shape[0] > 0:
+        h.annotate_device(views[lo:hi], p, labels, stream=torch.cuda.current_stream().cuda_stream)
+    return gather_blocks(labels, len(views), group)

@@ -193,6 +193,57 @@ bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const 
 bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
                           float target_height_m, uint32_t* masks, uint32_t* counts);
 
+/* Labels of points of interest (POIs): for each of n views and each of m POIs, whether the view sees the POI and where
+ * its marker goes -- the rule of the reference's annotator (annotator.c:280-348), which the command-line tool's
+ * --labels output follows (cli/horizonator-standalone.c, write_labels()), evaluated on the GPU for whole batches.
+ *
+ * Rule, per (view, POI):
+ *   - Projection: horizonator_project() in double with lat_viewer = (double)view.lat, lon_viewer = (double)view.lon,
+ *     cos_lat_viewer = cos(lat_viewer * pi / 180) (computed on the host per view), ele_viewer = the eye height as
+ *     horizonator_move() computes it (automatic when viewer_z < 0), az_rad0/1 = (double)az_deg0/1 * pi / 180, and the
+ *     context's W and H.  The GPU evaluates the same source operator for operator (no fused multiply-adds); only
+ *     atan2() may differ from the host's in the last bit.
+ *   - Gates: 500 m <= range <= 100 km, and lround(x) in [0, W).
+ *   - Vertical search, at column col = lround(x): for d = -6 .. 5 in turn: skip d while y + d < 0, stop once
+ *     y + d >= H; row r = lround(y) + d, skipped outside [0, H); skip rows whose rendered range is <= 0 (sky); the
+ *     error is |range - rendered range|: keep the first d with the smallest error so far and stop as soon as an error
+ *     is not smaller than the best.  The POI is visible iff the best error is below 500 m.
+ *   - The rendered ranges are the render's own, bit-identical to what the range image of the same render holds
+ *     (they are read from the visibility buffer and converted exactly as the range image is).
+ * Output, horizonator_label_t, each double rounded to float once:
+ *   - horizonator_project() fails (outside the window): all four fields -1;
+ *   - otherwise x and range_m are set; y is the projected y plus the search offset when visible, the projected y
+ *     otherwise; range_rendered_m is the matched rendered range when visible, -1 otherwise: visible <=> > 0.
+ * Known limits:
+ *   - A window of exactly 360 degrees (az_deg1 - az_deg0 == 360 in double, e.g. -180 .. 180) places no POI: the
+ *     reference's horizonator_project() unwraps its width to 0 and fails for every point, so every label is -1.
+ *     A window a fraction of a degree narrower works.
+ *   - The projection is the reference's flat-earth one.  With horizonator_set_earth_curvature() on, distant terrain is
+ *     drawn lower than horizonator_project() puts the POIs on it, so a POI far enough away sits above the terrain as
+ *     drawn and the +-6-row search can miss it.  The labels do not correct for that.
+ *   - The labels take n * m * 16 bytes.  For the host-memory call, from roughly 50 k POIs per view copying them, not
+ *     rendering, is what limits the rate (an estimate from the measured device->host copy rate, not a measurement).
+ */
+typedef struct { double lat, lon, ele; } horizonator_poi_t;                     /* 24 bytes; ele in metres */
+typedef struct { float x, y, range_m, range_rendered_m; } horizonator_label_t;  /* 16 bytes */
+
+/* Renders the n views exactly as horizonator_render_batch_device() does (same chunks, the context's z extents, size
+ * and opt-in modes) and writes d_labels[k * m + i] for view k and POI i.  views: host memory; d_pois (8-byte aligned)
+ * and d_labels (16-byte aligned): DEVICE memory.  d_images / d_ranges as in horizonator_render_batch_device(), either
+ * or both may be NULL: with both NULL no panorama is written at all, only the labels.  Stream as for the batch render.
+ * n == 0 or m == 0: nothing is done, true.  n < 0, m < 0, or NULL views / POIs / labels otherwise: false, nothing is
+ * written. */
+bool horizonator_annotate_batch_device(const horizonator_context_t* ctx,
+                                       int n, const horizonator_view_t* views,
+                                       int m, const horizonator_poi_t* d_pois,
+                                       horizonator_label_t* d_labels,
+                                       void* d_images, void* d_ranges, void* stream);
+
+/* Same with pois and labels in HOST memory, synchronous; no panorama is written, and only the n * m labels cross the
+ * bus (into page-locked memory by DMA; see horizonator_host_alloc()). */
+bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                int m, const horizonator_poi_t* pois, horizonator_label_t* labels);
+
 /* Per-kernel device times.  While enabled, every render records CUDA events around each of
  * its kernels on the stream it runs on.  horizonator_profile_read() waits for them and reports
  * the MEAN duration in milliseconds per render of: out_ms[0] k_prepare (clear + axis tables),
