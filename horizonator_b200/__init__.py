@@ -432,7 +432,7 @@ class horizonator:
 
     COUNTER_NAMES = ("tiles", "tiles_far", "tiles_window", "tiles_occluded",
                      "blocks", "blocks_far", "blocks_window", "blocks_occluded",
-                     "blocks_meshed", "triangles", "big_entries")
+                     "blocks_meshed", "triangles", "big_entries", "occluded_by_grid", "span_blocks")
 
     def render_counters(self):
         """Culling counters of the most recent render (horizonator_render_counters)."""

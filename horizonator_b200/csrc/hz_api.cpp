@@ -160,6 +160,8 @@ struct TanelKey
 struct Scratch
 {
     DevPtr<unsigned long long> d_vis;
+    DevPtr<uint32_t> d_hiz;            // span grid over d_vis (hz_device.h): one word per 8 keys of a row
+    DevPtr<uint8_t>  d_hiz_flags;      // ... and one byte per 8x8 block of keys
     DevPtr<float>    d_e, d_n;
     DevPtr<uint32_t> d_tile_queue, d_block_queue, d_tri_queue;
     DevPtr<uint2>    d_big_queue;      // [2][BIG_CAPACITY]: near pass, bands
@@ -325,6 +327,8 @@ template<class F> void scratch_buffers(const Slot& s, bool staging, bool image_o
     const size_t px = s.target_pixels;
     if(px == 0) return;
     f(&Scratch::d_vis, px);
+    f(&Scratch::d_hiz, (size_t)s.H * hz_spans((unsigned int)s.W));
+    f(&Scratch::d_hiz_flags, ((size_t)hz_spans((unsigned int)s.H) * hz_spans((unsigned int)s.W) + 3) & ~(size_t)3);   // (k_prepare zeroes words)
     f(&Scratch::d_tri_queue, (size_t)s.tri_capacity);
     f(&Scratch::d_big_queue, 2 * (size_t)s.big_capacity);
     f(&Scratch::d_bigtri, 6 * (size_t)s.bigtri_capacity);
@@ -652,7 +656,7 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
 
     v.znear = s.znear; v.zfar = s.zfar; v.znear_color = s.znear_color; v.zfar_color = s.zfar_color;
     v.W = s.W; v.H = s.H; v.x0 = x0; v.x1 = x1;
-    v.vis = sc.d_vis.get();
+    v.vis = sc.d_vis.get(); v.hiz = sc.d_hiz.get(); v.hiz_flags = sc.d_hiz_flags.get();
     v.stats      = s.collect_stats ? sc.d_counters->stats : nullptr;
     v.tile_queue = sc.d_tile_queue.get(); v.block_queue = sc.d_block_queue.get();
     v.tri_queue = sc.d_tri_queue.get(); v.tri_capacity = s.tri_capacity;

@@ -33,6 +33,19 @@ static __host__ __device__ inline unsigned int hz_key_q(unsigned long long key, 
     return (top >> 24) == ep ? (top & HZ_Q_MAX) : HZ_Q_MAX;
 }
 
+// ---- span grid -------------------------------------------------------------------------------
+// A span is 8 consecutive keys of one row of the visibility buffer.  Its word in HzView::hiz is never below the current
+// upper word (key >> 32) of any of its keys.  That holds without fences: during a render keys only decrease (the
+// min()), and a word left from an earlier render (or the all-ones of a clear) carries an earlier epoch, so it is
+// larger than any key of this render.  An occlusion test may therefore take "every span word below the bound" for
+// "every key below the bound"; where a span word is not, it reads the keys.
+// The flags of an 8x8 block of keys: TOUCHED = a key of it was written this render (k_prepare zeroes the flags every
+// render), DIRTY = written since k_depth_grid last recomputed its spans.
+#define HZ_SPAN_KEYS    8
+#define HZ_FLAG_TOUCHED 2u
+#define HZ_FLAG_DIRTY   1u
+static __host__ __device__ inline unsigned int hz_spans(unsigned int n) { return (n + HZ_SPAN_KEYS - 1) / HZ_SPAN_KEYS; }
+
 // ---- tiles as uploaded (raw file bytes) ------------------------------------------------------
 struct HzTiles
 {
@@ -70,6 +83,8 @@ enum HzStat
     HZ_STAT_BLOCKS_MESHED,      // blocks whose 32 triangles were projected and tested exactly
     HZ_STAT_TRIANGLES,          // triangles that passed the exact integer tests and went to set-up
     HZ_STAT_BIG_ENTRIES,        // (triangle, sub-box) pairs queued for k_big
+    HZ_STAT_OCCLUDED_BY_GRID,   // tiles and blocks found occluded from the span grid alone (part of the two above)
+    HZ_STAT_SPAN_BLOCKS,        // 8x8 blocks of keys whose spans k_depth_grid recomputed
     HZ_STAT_COUNT = 16
 };
 
@@ -107,6 +122,10 @@ struct alignas(16) HzView      // (16-byte units: the kernels fetch their copy w
     unsigned long long* vis;     // [H][x1-x0], GL row order (row 0 = bottom)
     unsigned int epoch;          // of this render's keys (see the visibility key)
     unsigned int clear_keys;     // k_prepare clears this many keys (the whole allocation when the epoch wrapped, else 0)
+    // The span grid over vis (see "span grid" below): hiz[y][s] bounds the upper words of keys [8s, 8s+8) of row y from
+    // above; hiz_flags[y/8][x/8], one byte per 8x8 block of keys, HZ_FLAG_TOUCHED | HZ_FLAG_DIRTY
+    uint32_t* hiz;               // [H][hz_spans(x1-x0)]
+    uint8_t*  hiz_flags;         // [hz_spans(H)][hz_spans(x1-x0)]
 
     // The mesh is walked outwards from the eye.  Tiles within `near_rings` (Chebyshev distance in tiles) of the
     // eye's tile go first and completely (k_near + k_big), then bands of rings [ring_lo, ring_hi), each through
@@ -179,7 +198,7 @@ cudaError_t hz_launch_peer_barrier(const HzPeerFlags& f, unsigned int epoch, cud
 cudaError_t hz_launch_mosaic (const HzTiles& t, int16_t* mosaic, int N, int pitch, cudaStream_t stream);
 cudaError_t hz_launch_pyramid(const int16_t* mosaic, int N, int pitch, short2* mm_block, int nb,
                               short2* mm_tile, int nt, cudaStream_t stream);
-cudaError_t hz_launch_prepare(const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);  // clear keys, axis tables, counters
+cudaError_t hz_launch_prepare(const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);  // clear keys, flags, axis tables, counters
 cudaError_t hz_launch_near   (const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);  // foreground tiles -> triangle list
 cudaError_t hz_launch_raster (const HzView& v, const HzView* d_v, int nviews, cudaStream_t stream);  // set-up + rasterise a triangle list
 cudaError_t hz_launch_band   (const HzView& v, const HzView* d_v, int nviews, bool worst_case, cudaStream_t stream, int* launches);

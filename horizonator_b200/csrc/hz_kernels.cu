@@ -4,6 +4,8 @@
 //                                                                              (2R)^2 times at horizonator-lib.c:435-439
 //   k_minmax_* (init)    (min,max) height per 4x4-cell block and per 32x32-cell tile: the culling pyramid
 //   k_prepare  (render)  clear visibility keys, per-column/row metre tables    glClear, lib:896; vertex.glsl:128-130
+//   k_depth_grid (render) before each band's culling: recomputes the span grid's words of the 8x8 blocks of keys
+//                        drawn into since the last time (hz_device.h, span grid)
 //   k_near     (render)  the tiles around the eye: mesh generation, projection,  lib:496-508 (index pattern), vertex.glsl,
 //                        exact integer cull -> list of triangles                  GL cull/clip
 //   k_tiles, k_blocks / k_blocks_mid, k_mesh (render)
@@ -213,6 +215,15 @@ k_prepare(const HzView* __restrict__ V)
         }
         for(; k < npairs; k += nth) v2[k] = clear2;
         if(tid == 0 && (nkeys & 1)) P.vis[nkeys - 1] = HZ_KEY_CLEAR;
+        // ... and with it the span grid, all of it: a later render of another width lays its spans out differently
+        // (in every other render the words left from earlier ones carry earlier epochs, see the span grid)
+        const unsigned int nspans = (unsigned int)P.H * hz_spans((unsigned int)P.W);
+        for(unsigned int s = tid; s < nspans; s += nth) P.hiz[s] = 0xFFFFFFFFu;
+    }
+    // nothing of this render drawn yet: every block's flags 0 (one byte per 8x8 block, four per store)
+    {
+        const unsigned int nflags = hz_spans((unsigned int)P.H) * hz_spans((unsigned int)(P.x1 - P.x0));
+        for(unsigned int f = tid; f < (nflags + 3u) / 4u; f += nth) ((uint32_t*)P.hiz_flags)[f] = 0u;
     }
 
     // vertex.glsl:128-130, operator by operator:
@@ -436,6 +447,21 @@ __device__ __forceinline__ void hz_red_min(unsigned long long* p, unsigned long 
     asm volatile("red.relaxed.gpu.global.min.u64 [%0], %1;" :: "l"(__cvta_generic_to_global(p)), "l"(key) : "memory");
 }
 
+// A block's flags (span grid) are stored with relaxed byte stores: k_depth_grid may be reading and resetting them while
+// the near pass's k_big, which runs beside the first bands, marks them.  A mark lost that way leaves the block's spans
+// higher than they need be, never lower.
+__device__ __forceinline__ void hz_store_flag(uint8_t* f, unsigned int v)
+{
+    asm volatile("st.relaxed.gpu.global.u8 [%0], %1;" :: "l"(__cvta_generic_to_global(f)), "r"(v) : "memory");
+}
+
+// marks the key's 8x8 block touched and dirty
+__device__ __forceinline__ void hz_mark_block(const HzView& P, int px, int py)
+{
+    hz_store_flag(P.hiz_flags + (size_t)((unsigned int)py / HZ_SPAN_KEYS) * hz_spans((unsigned int)(P.x1 - P.x0)) +
+                  (unsigned int)(px - P.x0) / HZ_SPAN_KEYS, HZ_FLAG_TOUCHED | HZ_FLAG_DIRTY);
+}
+
 // depth test + colour write for one covered pixel centre
 __device__ __forceinline__ void hz_fragment(const HzView& P, const HzTri& T, int px, int py)
 {
@@ -452,6 +478,7 @@ __device__ __forceinline__ void hz_fragment(const HzView& P, const HzTri& T, int
     const unsigned long long key = ((unsigned long long)((P.epoch << 24) | q) << HZ_KEY_Q_SHIFT) |
                                    ((unsigned long long)(T.id & HZ_ID_CELL_MASK) << 8) | r8;
     hz_red_min(&P.vis[(size_t)py * (size_t)(P.x1 - P.x0) + (size_t)(px - P.x0)], key);
+    hz_mark_block(P, px, py);
 }
 
 // Edge functions E_k(P) = dx_k*(Py - Y_k) - dy_k*(Px - X_k) on the snapped positions (F3); an edge owns its
@@ -1112,8 +1139,9 @@ cudaError_t hz_launch_near(const HzView& v, const HzView* d_v, int nviews, cudaS
 // ================================================================================================
 //
 // The rest of the mesh is walked in a few bands of growing Chebyshev distance (in tiles) around the eye's tile.
-// Per band four kernels run back to back, each with one unit of work per thread or warp so that no warp ever
+// Per band five kernels run back to back, each with one unit of work per thread or warp so that no warp ever
 // carries a long serial chain:
+//   k_depth_grid  the span grid of the blocks drawn into since its last run (what the bands' culling reads first)
 //   k_tiles   thread = tile (32x32 cells): conservative test of the whole tile        -> queue of live tiles
 //   k_blocks  thread = block (4x4 cells) of a live tile: the same test on the block   -> queue of live blocks
 //   k_mesh    warp   = live block: projection, exact integer cull (lane = triangle)   -> list of triangles
@@ -1121,63 +1149,88 @@ cudaError_t hz_launch_near(const HzView& v, const HzView* d_v, int nviews, cudaS
 // Everything a band draws is in the visibility buffer before the next band is tested against it, and within a
 // band whatever has already been drawn helps too.
 
-// The box is walked along its longer side, HZ_OCCL_FETCH keys per round (so that the L2 round trips overlap: a lone view
-// waits for every one of them); only the upper half of a key is fetched -- epoch and depth sit in its top 27 bits --
-// and the walk ends at the first round that shows something not nearer.  (The first version walked the box as one run
-// of pixels: the wrap to the next row, tested per pixel, cost as much as the fetch and the comparison together.)
-#ifndef HZ_OCCL_FETCH
-#define HZ_OCCL_FETCH 8            /* (16 and 32 measured no better, lone or batched) */
-#endif
-__device__ __forceinline__ bool hz_box_occluded_thread(const HzView& P, const HzBox& B, int max_pix)
+// The box is tested against the span grid first (hz_device.h): the span words that overlap it are walked along the
+// box's longer side (in spans), HZ_SPAN_KEYS = 8 words per round, so that the L2 round trips overlap -- a lone view waits
+// for every one of them.  A word below the bound stands for its 8 keys.  Only where a word is not below it are the keys
+// of that span inside the box fetched, again all in one round, and the test ends at the first key that is not nearer.
+// So the answer is the one the keys alone give: every key of the box below the bound.  Only the upper half of a key
+// is fetched -- epoch and depth sit in its top 27 bits.  (The first version walked the box as one run of pixels: the
+// wrap to the next row, tested per pixel, cost as much as the fetch and the comparison together.  The next walked every
+// key of the box; most boxes walked are occluded, so most walks were full-length.)
+// (A round is as long as a span so that one round fetches a span's keys too.  The walk over keys alone measured 16 and
+// 32 loads per round no better than 8, lone or batched.)
+enum { HZ_BOX_VISIBLE = 0, HZ_BOX_OCCLUDED = 1, HZ_BOX_OCCLUDED_BY_GRID = 2 };
+__device__ __forceinline__ int hz_box_occluded_thread(const HzView& P, const HzBox& B, int max_pix)
 {
     const int w = B.px1 - B.px0 + 1, h = B.py1 - B.py0 + 1;
-    if(w * h > max_pix) return false;
-    const unsigned int Wt2 = 2u * (unsigned int)(P.x1 - P.x0);                // 32-bit words per row of keys
-    // (upper word of the first key of the box)
-    const unsigned int* line = (const unsigned int*)P.vis + ((size_t)B.py0 * Wt2 + 2u * (unsigned int)(B.px0 - P.x0) + 1u);
+    if(w * h > max_pix) return HZ_BOX_VISIBLE;
+    const unsigned int Wt = (unsigned int)(P.x1 - P.x0), Ws = hz_spans(Wt);  // keys and spans per row
+    const int c0 = B.px0 - P.x0, c1 = B.px1 - P.x0;                           // the box's columns in the buffer
+    const int s0 = c0 / HZ_SPAN_KEYS, ns = c1 / HZ_SPAN_KEYS - s0 + 1;        // ... and its spans
     const unsigned int qmin_hi = B.qmin << (HZ_KEY_Q_SHIFT - 32);             // the bound, placed like the key's upper word
-    const bool rows = w >= h;                                                 // lines = rows of the box, or its columns
-    const int n_lines = rows ? h : w, n_along = rows ? w : h;
-    const unsigned int step_line = rows ? Wt2 : 2u, step_along = rows ? 2u : Wt2;
+    const bool rows = ns >= h;                                                // lines = rows of spans, or columns of them
+    const int n_lines = rows ? h : ns, n_along = rows ? ns : h;
+    const unsigned int step_line = rows ? Ws : 1u, step_along = rows ? 1u : Ws;
+    const unsigned int* line = P.hiz + ((size_t)B.py0 * Ws + (unsigned int)s0);
+    int result = HZ_BOX_OCCLUDED_BY_GRID;
     for(int l = 0; l < n_lines; l++, line += step_line)
     {
         const unsigned int* p = line;
-        for(int a = 0; a < n_along; a += HZ_OCCL_FETCH, p += HZ_OCCL_FETCH * step_along)
+        for(int a = 0; a < n_along; a += HZ_SPAN_KEYS, p += HZ_SPAN_KEYS * step_along)
         {
-            // all fetches of the round first, none of them conditional (beyond the end of the line the last key is
+            // all fetches of the round first, none of them conditional (beyond the end of the line the last word is
             // fetched again).  Whether the loads really go out together hangs on ptxas's register heuristics: one
             // build of k_tiles came out with 40 instead of 48 registers, two or three loads in flight instead of
             // eight, and a lone panorama 12 us slower.  The culling kernels therefore say __launch_bounds__(256, 3):
-            // with a stated register budget (85) ptxas schedules for the loads, and uses 48 (tools/sass_census.py).
-            unsigned int k[HZ_OCCL_FETCH];
+            // with a stated register budget (85) ptxas schedules for the loads (tools/sass_census.py).
+            unsigned int sw[HZ_SPAN_KEYS];
             const int last = n_along - 1 - a;
             #pragma unroll
-            for(int u = 0; u < HZ_OCCL_FETCH; u++) k[u] = __ldcg(p + (unsigned int)min(u, last) * step_along);
-            unsigned int farthest = 0;
+            for(int u = 0; u < HZ_SPAN_KEYS; u++) sw[u] = __ldcg(p + (unsigned int)min(u, last) * step_along);
+            unsigned int open = 0;                                            // spans of the round not below the bound
             #pragma unroll
-            for(int u = 0; u < HZ_OCCL_FETCH; u++) farthest = max(farthest, k[u]);
-            // (the upper word holds epoch | depth | the top 5 bits of the triangle number: comparing it whole against
-            // the bound with those 5 bits clear is the same test as comparing the top 27 bits)
-            if(farthest >= qmin_hi) return false;
+            for(int u = 0; u < HZ_SPAN_KEYS; u++) open |= (unsigned int)(u <= last && sw[u] >= qmin_hi) << u;
+            while(open)
+            {
+                const int u = __ffs(open) - 1;
+                open &= open - 1u;
+                const int y = B.py0 + (rows ? l : a + u), s = s0 + (rows ? a + u : l);
+                const int k0 = max(s * HZ_SPAN_KEYS, c0), kl = min(s * HZ_SPAN_KEYS + HZ_SPAN_KEYS - 1, c1) - k0;
+                const unsigned int* kp = (const unsigned int*)P.vis + ((size_t)y * 2u * Wt + 2u * (unsigned int)k0 + 1u);
+                unsigned int k[HZ_SPAN_KEYS];
+                #pragma unroll
+                for(int v = 0; v < HZ_SPAN_KEYS; v++) k[v] = __ldcg(kp + 2u * (unsigned int)min(v, kl));
+                unsigned int farthest = 0;
+                #pragma unroll
+                for(int v = 0; v < HZ_SPAN_KEYS; v++) farthest = max(farthest, k[v]);
+                // (the upper word holds epoch | depth | the top 5 bits of the triangle number: comparing it whole
+                // against the bound with those 5 bits clear is the same test as comparing the top 27 bits)
+                if(farthest >= qmin_hi) return HZ_BOX_VISIBLE;
+                result = HZ_BOX_OCCLUDED;
+            }
         }
     }
-    return true;
+    return result;
 }
 
-enum { HZ_RECT_OCCLUDED = 4 };
+enum { HZ_RECT_OCCLUDED = 4, HZ_RECT_OCCLUDED_BY_GRID = 5 };
 
 __device__ __forceinline__ int
 hz_rect_cull(const HzView& P, int c_lo, int c_hi, int r_lo, int r_hi, float zmin, float zmax, int max_pix)
 {
     HzBox B;
     const int r = hz_rect_test(P, c_lo, c_hi, r_lo, r_hi, zmin, zmax, B);
-    return (r == HZ_RECT_BOXED && hz_box_occluded_thread(P, B, max_pix)) ? (int)HZ_RECT_OCCLUDED : r;
+    if(r != HZ_RECT_BOXED) return r;
+    const int o = hz_box_occluded_thread(P, B, max_pix);
+    return o == HZ_BOX_VISIBLE ? r : (o == HZ_BOX_OCCLUDED ? (int)HZ_RECT_OCCLUDED : (int)HZ_RECT_OCCLUDED_BY_GRID);
 }
 
 // counts the outcome of a rectangle's test; true if the rectangle lives on
-__device__ __forceinline__ bool hz_rect_tally(int r, unsigned int& n_far, unsigned int& n_window, unsigned int& n_occl)
+__device__ __forceinline__ bool hz_rect_tally(int r, unsigned int& n_far, unsigned int& n_window, unsigned int& n_occl,
+                                              unsigned int& n_grid)
 {
-    n_far += r == HZ_RECT_DEAD_FAR; n_window += r == HZ_RECT_DEAD_WINDOW; n_occl += r == HZ_RECT_OCCLUDED;
+    n_far += r == HZ_RECT_DEAD_FAR; n_window += r == HZ_RECT_DEAD_WINDOW; n_occl += r >= HZ_RECT_OCCLUDED;
+    n_grid += r == HZ_RECT_OCCLUDED_BY_GRID;
     return r == HZ_RECT_ALIVE || r == HZ_RECT_BOXED;
 }
 
@@ -1224,6 +1277,13 @@ __device__ __forceinline__ void hz_cta_stats4(unsigned int* s4, unsigned int* gl
     if((threadIdx.x & 31) == 0) { atomicAdd(s4 + 0, a); atomicAdd(s4 + 1, b); atomicAdd(s4 + 2, c); atomicAdd(s4 + 3, d); }
     __syncthreads();
     if(threadIdx.x < 4 && s4[threadIdx.x]) atomicAdd(global4 + threadIdx.x, s4[threadIdx.x]);
+}
+
+// one more counter: one global atomic per warp that has something to add; all lanes call
+__device__ __forceinline__ void hz_warp_stat(unsigned int* global, unsigned int a)
+{
+    a = hz_warp_sum(a);
+    if((threadIdx.x & 31) == 0 && a) atomicAdd(global, a);
 }
 
 // The tiles of a band: Chebyshev distance [lo, hi) from the eye's tile (ex, ey), 1 <= lo < hi, clipped to the mesh --
@@ -1275,7 +1335,7 @@ k_tiles(const HzView* __restrict__ V)
     const HzRing ring(P.eye_ti, P.eye_tj, nt, ring_lo, ring_hi);
     const unsigned int last = ring.count();
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, n_grid = 0, staged = 0;
     for(unsigned int k0 = blockIdx.x * blockDim.x + threadIdx.x - lane; k0 < last; k0 += nth)
     {
         const unsigned int k = k0 + lane;
@@ -1290,12 +1350,16 @@ k_tiles(const HzView* __restrict__ V)
             const int r = hz_rect_cull(P, tc0, min(tc0 + HZ_TILE_CELLS, N - 1), tr0, min(tr0 + HZ_TILE_CELLS, N - 1),
                                        (float)mt.x, (float)mt.y, P.occl_tile_max_pix);
             n_all++;
-            on = hz_rect_tally(r, n_far, n_window, n_occl);
+            on = hz_rect_tally(r, n_far, n_window, n_occl, n_grid);
         }
         hz_stage_push(S.stage, staged, on, ((unsigned int)tj << 16) | (unsigned int)ti, P.tile_queue, P.tile_count, lane);
     }
     if(staged) hz_stage_write(S.stage, staged, P.tile_queue, P.tile_count, lane);
-    if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_TILES, n_all, n_far, n_window, n_occl);
+    if(P.stats)
+    {
+        hz_cta_stats4(s_stats, P.stats + HZ_STAT_TILES, n_all, n_far, n_window, n_occl);
+        hz_warp_stat(P.stats + HZ_STAT_OCCLUDED_BY_GRID, n_grid);
+    }
 }
 
 // LOD = false: the reference's mesh (lod = 0 known at compile time: fewer registers, more resident warps); true: the
@@ -1314,7 +1378,7 @@ k_blocks(const HzView* __restrict__ V)
     const int lod = LOD ? P.lod : 0, sh = 3 - lod, side = 1 << sh, cells = HZ_BLOCK_CELLS << lod;
     const unsigned int total = *P.tile_count << (2 * sh);
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, n_grid = 0, staged = 0;
     for(unsigned int t0 = blockIdx.x * blockDim.x + threadIdx.x - lane; t0 < total; t0 += nth)
     {
         const unsigned int t = t0 + lane;
@@ -1344,13 +1408,17 @@ k_blocks(const HzView* __restrict__ V)
                 const int r = hz_rect_cull(P, c0, min(c0 + cells, N - 1), r0, min(r0 + cells, N - 1), (float)mm.x, (float)mm.y,
                                            P.occl_block_max_pix);
                 n_all++;
-                on = hz_rect_tally(r, n_far, n_window, n_occl);
+                on = hz_rect_tally(r, n_far, n_window, n_occl, n_grid);
             }
         }
         hz_stage_push(S.stage, staged, on, ((unsigned int)bj << 16) | (unsigned int)bi, P.block_queue, P.block_count, lane);
     }
     if(staged) hz_stage_write(S.stage, staged, P.block_queue, P.block_count, lane);
-    if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
+    if(P.stats)
+    {
+        hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
+        hz_warp_stat(P.stats + HZ_STAT_OCCLUDED_BY_GRID, n_grid);
+    }
 }
 
 // ---- k_blocks with a level in between (MID) ----------------------------------------------------------------------------
@@ -1375,7 +1443,7 @@ k_blocks_mid(const HzView* __restrict__ V)
     const int mid_pix = P.occl_tile_max_pix, block_pix = P.occl_block_max_pix;
     const unsigned int total = *P.tile_count * 16u;
     const unsigned int nth = gridDim.x * blockDim.x;
-    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, staged = 0;
+    unsigned int n_all = 0, n_far = 0, n_window = 0, n_occl = 0, n_grid = 0, staged = 0;
     for(unsigned int t0 = blockIdx.x * blockDim.x + threadIdx.x - lane; t0 < total; t0 += nth)
     {
         const unsigned int t = t0 + lane;
@@ -1420,7 +1488,7 @@ k_blocks_mid(const HzView* __restrict__ V)
                     const int r = hz_rect_cull(P, c0, min(c0 + HZ_BLOCK_CELLS, N - 1), r0, min(r0 + HZ_BLOCK_CELLS, N - 1),
                                                (float)mm.x, (float)mm.y, block_pix);
                     n_all++;
-                    on = hz_rect_tally(r, n_far, n_window, n_occl);
+                    on = hz_rect_tally(r, n_far, n_window, n_occl, n_grid);
                 }
             }
             hz_stage_push(S.stage, staged, on, ((unsigned int)bj << 16) | (unsigned int)bi, P.block_queue, P.block_count, lane);
@@ -1428,7 +1496,11 @@ k_blocks_mid(const HzView* __restrict__ V)
         __syncwarp();                                   // (the next trip writes S.mids again)
     }
     if(staged) hz_stage_write(S.stage, staged, P.block_queue, P.block_count, lane);
-    if(P.stats) hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
+    if(P.stats)
+    {
+        hz_cta_stats4(s_stats, P.stats + HZ_STAT_BLOCKS, n_all, n_far, n_window, n_occl);
+        hz_warp_stat(P.stats + HZ_STAT_OCCLUDED_BY_GRID, n_grid);
+    }
 }
 
 __global__ void __launch_bounds__(HZ_WARPS_PER_CTA * 32, HZ_MESH_CTAS)
@@ -1635,8 +1707,57 @@ cudaError_t hz_launch_raster(const HzView& v, const HzView* d_v, int nviews, cud
     return hz_launch(k_raster, dim3(hz_grid(v, 6, nviews), (unsigned)nviews), dim3(256), stream, d_v);
 }
 
+// ================================================================================================
+// k_depth_grid: the span grid (hz_device.h) of the blocks drawn into since the last run
+// ================================================================================================
+
+// A warp takes 32 blocks' flags per trip and compacts the dirty ones by ballot; then its lanes recompute them four
+// blocks at a time, lane = one row of one block: the row's 8 keys read in one round, their largest upper word written.
+// (One block at a time, with each lane reading two keys and shuffles reducing the rows, made every dirty block a chain
+// of dependent L2 round trips: a lone C2 panorama took 144 instead of 118 us, profiles/r06_depth_grid_ab.txt.)  A
+// block's flag is reset to "touched" after its keys were read; a block drawn into meanwhile (only the near pass's k_big
+// runs concurrently) may lose its dirty mark, which leaves its spans high -- an upper bound still.
+__global__ void __launch_bounds__(256)
+k_depth_grid(const HzView* __restrict__ V)
+{
+    HZ_KERNEL_PROLOGUE(V, P);
+    const unsigned int lane = threadIdx.x & 31u;
+    const unsigned int Wt = (unsigned int)(P.x1 - P.x0), H = (unsigned int)P.H, Ws = hz_spans(Wt);
+    const unsigned int nflags = hz_spans(H) * Ws;
+    const unsigned int r = lane % HZ_SPAN_KEYS;                              // this lane's row of a block
+    unsigned int n_blocks = 0;
+    for(unsigned int f0 = blockIdx.x * blockDim.x + threadIdx.x - lane; f0 < nflags; f0 += gridDim.x * blockDim.x)
+    {
+        const unsigned int f = f0 + lane;
+        const bool dirty = f < nflags && (__ldcg(P.hiz_flags + f) & HZ_FLAG_DIRTY);
+        const unsigned int todo = __ballot_sync(0xffffffffu, dirty);
+        const unsigned int n = (unsigned int)__popc(todo);
+        n_blocks += n;
+        for(unsigned int j = lane / HZ_SPAN_KEYS; j < n; j += 32u / HZ_SPAN_KEYS)
+        {
+            const unsigned int b = f0 + (unsigned int)__fns(todo, 0u, (int)j + 1);   // the j-th dirty block
+            const unsigned int by = b / Ws, bx = b - by * Ws, y = by * HZ_SPAN_KEYS + r, x = bx * HZ_SPAN_KEYS;
+            if(y >= H) continue;
+            const unsigned int last = min(Wt - x, (unsigned int)HZ_SPAN_KEYS) - 1u;
+            const unsigned int* k = (const unsigned int*)P.vis + ((size_t)y * 2u * Wt + 2u * x + 1u);
+            unsigned int w[HZ_SPAN_KEYS];
+            #pragma unroll
+            for(int u = 0; u < HZ_SPAN_KEYS; u++) w[u] = __ldcg(k + 2u * min((unsigned int)u, last));
+            unsigned int m = 0;
+            #pragma unroll
+            for(int u = 0; u < HZ_SPAN_KEYS; u++) m = max(m, w[u]);
+            // (P.hiz comes out of the shared-memory copy of the parameters: said explicitly, a global store)
+            asm volatile("st.global.u32 [%0], %1;" :: "l"(__cvta_generic_to_global(P.hiz + (size_t)y * Ws + bx)), "r"(m) : "memory");
+        }
+        __syncwarp();
+        if(dirty) hz_store_flag(P.hiz_flags + f, HZ_FLAG_TOUCHED);
+    }
+    if(P.stats) hz_warp_stat(P.stats + HZ_STAT_SPAN_BLOCKS, lane == 0 ? n_blocks : 0u);
+}
+
 // `worst_case`: size the tile kernel for any eye position (a CUDA graph is captured once per context and replayed
 // for every view); otherwise for this view's eye tile, and nothing is launched if the band is empty.
+// Each band first brings the span grid up to date with what the near pass and the bands before it drew.
 cudaError_t hz_launch_band(const HzView& v, const HzView* d_v, int nviews, bool worst_case, cudaStream_t stream, int* launches)
 {
     *launches = 0;
@@ -1660,9 +1781,13 @@ cudaError_t hz_launch_band(const HzView& v, const HzView* d_v, int nviews, bool 
     const unsigned int ny = (unsigned int)nviews;
     cudaError_t e;
     void (*blocks)(const HzView*) = v.lod_capable ? k_blocks<true> : (v.mid_level ? k_blocks_mid : k_blocks<false>);
+    // (k_depth_grid: a thread per block flag, at most the grid of the other device-counted kernels)
+    const unsigned int nflags = hz_spans((unsigned int)v.H) * hz_spans((unsigned int)(v.x1 - v.x0));
+    const unsigned int grid_ctas = min((nflags + 255u) / 256u, hz_grid(v, 4, nviews));
+    if((e = hz_launch(k_depth_grid, dim3(grid_ctas, ny), dim3(256), stream, d_v)) != cudaSuccess) return e;
     if((e = hz_launch(k_tiles, dim3((unsigned)ctas, ny), dim3(256), stream, d_v)) != cudaSuccess) return e;
     if((e = hz_launch(blocks,  dim3(hz_grid(v, 8, nviews), ny), dim3(256), stream, d_v)) != cudaSuccess) return e;
-    *launches = 4;
+    *launches = 5;
     if((e = hz_launch(k_mesh,   dim3(hz_grid(v, 4, nviews), ny), dim3(HZ_WARPS_PER_CTA * 32), stream, d_v)) != cudaSuccess) return e;
     if((e = hz_launch(k_raster, dim3(hz_grid(v, 6, nviews), ny), dim3(256), stream, d_v)) != cudaSuccess) return e;
     return cudaSuccess;
@@ -1816,14 +1941,24 @@ k_resolve4(const HzView* __restrict__ V)
     const ulonglong2* src = (const ulonglong2*)(P.vis + (size_t)y * Wt);
     const size_t dst_row = (size_t)((unsigned int)P.H - 1u - y) * (unsigned int)P.out_stride + (unsigned int)P.out_x0;   // top row first (lib:949-958, 1026-1038)
 
+    // Most of a panorama is sky.  The keys of a group are read only where its 8x8 block was drawn into this render (its
+    // touched flag, span grid): elsewhere none of them is of this render, and a cleared key stands for them.
+    const uint8_t* flags = P.hiz_flags + (size_t)(y / HZ_SPAN_KEYS) * hz_spans(Wt);
+    const ulonglong2 sky = make_ulonglong2(HZ_KEY_CLEAR, HZ_KEY_CLEAR);
     unsigned int xg = threadIdx.x + (spread ? HZ_CTA_THREADS * blockIdx.x : 0u);
-    ulonglong2 k01 = make_ulonglong2(0, 0), k23 = k01;
-    if(xg < gpr) { k01 = __ldcs(src + 2 * xg); k23 = __ldcs(src + 2 * xg + 1); }   // read once: streaming
+    ulonglong2 k01 = sky, k23 = sky;
+    if(xg < gpr && (__ldg(flags + xg / 2u) & HZ_FLAG_TOUCHED))
+    {
+        k01 = __ldcs(src + 2 * xg); k23 = __ldcs(src + 2 * xg + 1);          // read once: streaming
+    }
     while(xg < gpr)
     {
         const unsigned int xg_next = xg + stride;
-        ulonglong2 n01 = k01, n23 = k23;
-        if(xg_next < gpr) { n01 = __ldcs(src + 2 * xg_next); n23 = __ldcs(src + 2 * xg_next + 1); }
+        ulonglong2 n01 = sky, n23 = sky;
+        if(xg_next < gpr && (__ldg(flags + xg_next / 2u) & HZ_FLAG_TOUCHED))
+        {
+            n01 = __ldcs(src + 2 * xg_next); n23 = __ldcs(src + 2 * xg_next + 1);
+        }
 
         const unsigned int q0 = hz_key_q(k01.x, ep), q1 = hz_key_q(k01.y, ep), q2 = hz_key_q(k23.x, ep), q3 = hz_key_q(k23.y, ep);
         // hit: (B,G,R) = (0,0,r8) ; sky: clear colour (0,0,1) read as BGR = (255,0,0)   lib:185, 938-939

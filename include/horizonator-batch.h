@@ -265,8 +265,10 @@ bool horizonator_last_render_stats(const horizonator_context_t* ctx, unsigned in
  * is on (all zero otherwise): out[0..3] far-pass tiles looked at / dropped
  * beyond zfar / dropped without a pixel centre in their screen box / dropped as occluded,
  * out[4..7] the same for 4x4-cell blocks (both passes), out[8] blocks whose 32 triangles were
- * projected and tested exactly, out[9] triangles set up, out[10] large-triangle queue entries;
- * out[11..15] reserved (0). */
+ * projected and tested exactly, out[9] triangles set up, out[10] large-triangle queue entries,
+ * out[11] tiles and blocks found occluded from the span grid alone, without reading their keys
+ * (counted in out[3] and out[7] too), out[12] 8x8 blocks of the visibility buffer whose span
+ * grid words were recomputed; out[13..15] reserved (0). */
 bool horizonator_render_counters(const horizonator_context_t* ctx, unsigned int out[16]);
 
 #ifdef __cplusplus
