@@ -156,7 +156,7 @@ struct TanelKey
     bool is(float daz_, int W_, int H_) const { return valid && W == W_ && H == H_ && memcmp(&daz, &daz_, sizeof(float)) == 0; }
 };
 
-// everything one view in flight writes besides its outputs (the device buffers: scratch_buffers)
+// everything one view in flight writes (the device buffers: scratch_buffers)
 struct Scratch
 {
     DevPtr<unsigned long long> d_vis;
@@ -167,7 +167,7 @@ struct Scratch
     DevPtr<uint2>    d_big_queue;      // [2][BIG_CAPACITY]: near pass, bands
     DevPtr<uint4>    d_bigtri;         // [BIGTRI_CAPACITY][6]
     DevPtr<Counters> d_counters;
-    DevPtr<uint8_t>  d_image;          // batch sets only: staging of one view's outputs for the host-pointer batch call
+    DevPtr<uint8_t>  d_image;          // the view's outputs where they do not go straight to the caller's device memory
     DevPtr<float>    d_ranges;
     // tan(elevation) per row of the window this scratch last rendered (lib:1007-1012; computed on the host like the
     // reference's read-back does, uploaded on the stream of the render that needs it -- so nothing else can be
@@ -187,7 +187,7 @@ struct ViewSet
 {
     int  cap = 0;
     bool batch = false;                // the chain configuration of batched views (config_of)
-    StreamHandle stream;               // batch sets only
+    StreamHandle stream;               // batch sets only: the context's own set renders on the caller's stream
     EventHandle  done;                 // batch sets only
     std::vector<Scratch> sc;           // grows on demand up to cap (ensure_views)
 
@@ -234,11 +234,9 @@ struct Slot
     DevPtr<short2> d_mm_block, d_mm_tile;    // culling pyramid
     int nb = 0, nt = 0;
 
-    // target
+    // target (the image-sized buffers are in the views' scratch)
     int W = 0, H = 0;
-    DevPtr<uint8_t> d_image;
-    DevPtr<float>   d_ranges;
-    size_t   target_pixels = 0;      // capacity of the buffers above
+    size_t   target_pixels = 0;
     uint32_t tri_capacity = 0, big_capacity = 0, bigtri_capacity = 0;
 
     // page-locked staging for results that go to pageable host memory (copy_to_pageable): made on first use
@@ -251,8 +249,8 @@ struct Slot
     std::vector<TanelRow> tanel_cache;
     size_t tanel_cache_next = 0;
 
-    // `main` serves the single-view entry points (and keeps the last visibility buffer for horizonator_pick);
-    // `sets` are made on demand by the batch entry points.
+    // `main` serves the single-view entry points and batch calls that render one view at a time (and keeps the last
+    // visibility buffer for horizonator_pick); `sets` are made on demand by the batch entry points.
     ViewSet main;
     std::vector<std::unique_ptr<ViewSet>> sets;
     EventHandle fork_ev;
@@ -312,9 +310,9 @@ struct DeviceGuard
 };
 
 // The device buffers of a scratch, as (member, number of elements): those sized by the terrain unless `image_only`,
-// then, if the slot has a target, those sized by the image (staging: the outputs of a batch set's view).
-// alloc_scratch() allocates them from this list, and ensure_views() budgets with its sum.
-template<class F> void scratch_buffers(const Slot& s, bool staging, bool image_only, F&& f)
+// then, if the slot has a target, those sized by the image.  alloc_scratch() allocates them from this list, and
+// ensure_views() budgets with its sum.
+template<class F> void scratch_buffers(const Slot& s, bool image_only, F&& f)
 {
     if(!image_only)
     {
@@ -333,25 +331,22 @@ template<class F> void scratch_buffers(const Slot& s, bool staging, bool image_o
     f(&Scratch::d_big_queue, 2 * (size_t)s.big_capacity);
     f(&Scratch::d_bigtri, 6 * (size_t)s.bigtri_capacity);
     f(&Scratch::d_tanel, (size_t)s.H);
-    if(staging)
-    {
-        f(&Scratch::d_image, 3 * px);
-        f(&Scratch::d_ranges, px);
-    }
+    f(&Scratch::d_image, 3 * px);
+    f(&Scratch::d_ranges, px);
 }
 
 // Allocates the buffers scratch_buffers() lists and moves them into c once all of them are there (assigning a handle
 // releases the buffer it held).  A new visibility buffer starts a new count of renders: its first render clears it.
-bool alloc_scratch(const Slot& s, Scratch& c, bool staging, bool image_only)
+bool alloc_scratch(const Slot& s, Scratch& c, bool image_only)
 {
     Scratch fresh;
     bool ok = true;
-    scratch_buffers(s, staging, image_only, [&](auto m, size_t n) {
+    scratch_buffers(s, image_only, [&](auto m, size_t n) {
         using T = typename std::remove_reference_t<decltype(fresh.*m)>::element_type;
         if(ok) ok = (fresh.*m = make_device<T>(n)) != nullptr;
     });
     if(!ok) return false;
-    scratch_buffers(s, staging, image_only, [&](auto m, size_t) { c.*m = std::move(fresh.*m); });
+    scratch_buffers(s, image_only, [&](auto m, size_t) { c.*m = std::move(fresh.*m); });
     c.tanel_key = TanelKey{};
     c.renders = 0;
     return true;
@@ -366,8 +361,16 @@ bool alloc_set_target(const Slot& s, ViewSet& vs)
     if(s.target_pixels == 0) return true;
     HostPtr<float> h_tanel = make_host<float>((size_t)PARAM_RING * vs.cap * s.H);
     if(!h_tanel) return false;
-    for(Scratch& c : vs.sc) if(!alloc_scratch(s, c, vs.batch, true)) return false;
+    for(Scratch& c : vs.sc) if(!alloc_scratch(s, c, true)) return false;
     vs.h_tanel = std::move(h_tanel);
+    return true;
+}
+
+// calls f on the context's own view set, then on each batch set, until one returns false
+template<class F> bool for_each_set(Slot& s, F&& f)
+{
+    if(!f(s.main)) return false;
+    for(const auto& v : s.sets) if(!f(*v)) return false;
     return true;
 }
 
@@ -389,19 +392,13 @@ bool alloc_target(Slot& s, int W, int H)
     if(const char* env = getenv("HORIZONATOR_BIG_CAPACITY"))    s.big_capacity    = (uint32_t)(atoi(env) > 1 ? atoi(env) : 1);
     if(const char* env = getenv("HORIZONATOR_BIGTRI_CAPACITY")) s.bigtri_capacity = (uint32_t)(atoi(env) > 1 ? atoi(env) : 1);
     s.target_pixels = px; s.W = W; s.H = H;       // scratch_buffers() sizes the buffers from these
-    DevPtr<uint8_t> image = make_device<uint8_t>(px * 3);
-    DevPtr<float> ranges = make_device<float>(px);
-    bool ok = image && ranges && alloc_set_target(s, s.main);
-    for(const auto& g : s.sets) ok = ok && alloc_set_target(s, *g);
-    if(!ok)
+    if(!for_each_set(s, [&](ViewSet& vs) { return alloc_set_target(s, vs); }))
     {
         MSG("Could not allocate the %d x %d render target", W, H);
         cudaGetLastError();
         s.W = 0; s.H = 0; s.target_pixels = 0;
         return false;
     }
-    s.d_image = std::move(image);
-    s.d_ranges = std::move(ranges);
     return true;
 }
 
@@ -433,10 +430,10 @@ int ensure_views(Slot& s, ViewSet& vs, int n)
         if(vs.batch)
         {
             size_t bytes = 0, free_b = 0, total_b = 0;
-            scratch_buffers(s, true, false, [&](auto m, size_t len) { bytes += len * sizeof(*(c.*m)); });
+            scratch_buffers(s, false, [&](auto m, size_t len) { bytes += len * sizeof(*(c.*m)); });
             if(cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || bytes > free_b / 2) break;
         }
-        if(!alloc_scratch(s, c, vs.batch, false))
+        if(!alloc_scratch(s, c, false))
         {
             MSG("Could not allocate the scratch of view %d of a set", (int)vs.sc.size());
             cudaGetLastError();
@@ -852,13 +849,6 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     return true;
 }
 
-// one view on the context's own scratch
-bool enqueue_render(Slot& s, const ViewState& vs, int x0, int x1, const OutSpec& out, cudaStream_t st,
-                    const AnnotSpec* ann = nullptr)
-{
-    return enqueue_views(s, s.main, 1, &vs, x0, x1, &out, st, ann);
-}
-
 // lib:765-789, float as written there.  The four samples come from the host mmaps (dem.h).
 bool compute_move(const horizonator_context_t* ctx, float* viewer_z, float lat, float lon, ViewState& vs)
 {
@@ -1058,11 +1048,12 @@ bool copy_results_to_host(Slot& s, char* image, float* ranges, const uint8_t* d_
     return true;
 }
 
-// plain asynchronous device -> host copy (the batch call: its destinations are written while later views render)
-bool copy_to_host(void* dst, const void* src, size_t bytes, cudaStream_t st)
+// the columns [x0,x1) of a wedge: a non-empty part of the target
+bool wedge_columns_ok(const Slot& s, int x0, int x1)
 {
-    CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st));
-    return true;
+    if(x0 >= 0 && x1 <= s.W && x0 < x1) return true;
+    MSG("wedge columns [%d,%d) are not inside [0,%d)", x0, x1, s.W);
+    return false;
 }
 
 } // namespace
@@ -1279,7 +1270,9 @@ bool horizonator_redraw(const horizonator_context_t* ctx)
     Slot* s = slot_of(ctx);
     if(s == nullptr) return false;
     DeviceGuard g(s->device);
-    if(!enqueue_render(*s, s->view, 0, s->W, single_out(s->d_image.get(), s->d_ranges.get()), s->stream.get())) return false;
+    const Scratch& own = s->main.sc[0];
+    const OutSpec out = single_out(own.d_image.get(), own.d_ranges.get());
+    if(!enqueue_views(*s, s->main, 1, &s->view, 0, s->W, &out, s->stream.get())) return false;
     CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
     return true;
 }
@@ -1295,9 +1288,10 @@ bool horizonator_render_offscreen(const horizonator_context_t* ctx, char* image,
     }
     DeviceGuard g(s->device);
     const size_t px = (size_t)s->W * s->H;
-    if(!enqueue_render(*s, s->view, 0, s->W,
-                       single_out(image ? s->d_image.get() : nullptr, ranges ? s->d_ranges.get() : nullptr), s->stream.get())) return false;
-    return copy_results_to_host(*s, image, ranges, s->d_image.get(), s->d_ranges.get(), px, s->stream.get());
+    const Scratch& own = s->main.sc[0];
+    const OutSpec out = single_out(image ? own.d_image.get() : nullptr, ranges ? own.d_ranges.get() : nullptr);
+    if(!enqueue_views(*s, s->main, 1, &s->view, 0, s->W, &out, s->stream.get())) return false;
+    return copy_results_to_host(*s, image, ranges, own.d_image.get(), own.d_ranges.get(), px, s->stream.get());
 }
 
 bool horizonator_pick(const horizonator_context_t* ctx, float* lat, float* lon, int x, int y)
@@ -1361,12 +1355,12 @@ bool horizonator_unproject(float* lat, float* lon, int x, int y,
 
 // ---- additive API (include/horizonator-batch.h) -----------------------------------------------------------
 
-// Common part of the two batch calls.  The views are cut into chunks of up to VIEWS_PER_SET; a chunk is rendered by
+// Common part of the batch calls.  The views are cut into chunks of up to VIEWS_PER_SET; a chunk is rendered by
 // ONE chain of kernel launches whose grids have a view dimension (one parameter copy and one CUDA-graph launch per
-// chunk, whatever its size), on the stream of one of up to N_SETS_MAX view sets, so that the tails of one chunk's
+// chunk, whatever its size), on the stream of one of up to N_SETS_MAX batch view sets, so that the tails of one chunk's
 // kernels overlap another chunk's.  The sets start after everything already queued on `st`, and `st` continues after
-// all of them.  to_host: outputs go through the views' device staging buffers and device->host copies on the set's
-// stream, which overlap the other sets' kernels.
+// all of them.  to_host: outputs go through the views' scratch and device->host copies on the set's stream, which
+// overlap the other sets' kernels.
 // ann: the labels of m POIs for every view as well (horizonator_annotate_batch*), by k_annotate after each chunk's chain;
 // into device memory, or (to_host) through the set's label scratch and a copy on its stream.
 struct AnnotReq
@@ -1410,7 +1404,7 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     }
     const size_t m_poi = ann ? (size_t)ann->m : 0;
 
-    // chunk size: the views spread evenly over the sets, at most VIEWS_PER_SET each, at most what fits in memory
+    // chunk size: the views spread evenly over the batch sets, at most VIEWS_PER_SET each, at most what fits in memory
     int n_sets = 0, chunk = 0;
     if(n > 1)
     {
@@ -1433,64 +1427,60 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         }
     }
 
-    if(n_sets == 0)
-    {
-        // one view, or no memory for a set: one at a time on the context's own scratch
-        if(ann && to_host && !ensure_labels(s->main, st, m_poi)) return false;
-        for(int k = 0; k < n; k++)
-        {
-            uint8_t* di = images ? (to_host ? s->d_image.get()  : images + (size_t)k * px * 3) : nullptr;
-            float*   dr = ranges ? (to_host ? s->d_ranges.get() : ranges + (size_t)k * px)     : nullptr;
-            AnnotSpec a{};
-            if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? s->main.d_labels.get() : ann->labels + (size_t)k * m_poi, &av[k] };
-            if(!enqueue_render(*s, vs[k], 0, s->W, single_out(di, dr), st, ann ? &a : nullptr)) return false;
-            if(to_host)
-            {
-                if(images && !copy_to_host(images + (size_t)k * px * 3, di, px * 3, st)) return false;
-                if(ranges && !copy_to_host(ranges + (size_t)k * px, dr, px * sizeof(float), st)) return false;
-                if(ann && !copy_to_host(ann->labels + (size_t)k * m_poi, a.labels, m_poi * sizeof(float4), st)) return false;
-            }
-        }
-        s->have_render = false;     // the visibility buffer no longer matches the context's own view
-        return true;
-    }
+    // The view sets that render the chunks: the batch sets, each on its own stream, or -- one view, or no memory for a
+    // batch set -- the context's own set, one view at a time on `st`.
+    std::vector<ViewSet*> sets;
+    for(int g = 0; g < n_sets; g++) sets.push_back(s->sets[g].get());
+    const bool forked = n_sets > 0;
+    if(!forked) { sets.push_back(&s->main); chunk = 1; }
+    auto stream_of = [st](const ViewSet& set) { return set.stream ? set.stream.get() : st; };
 
-    for(int g = 0; g < n_sets && ann && to_host; g++)
-        if(!ensure_labels(*s->sets[g], s->sets[g]->stream.get(), (size_t)chunk * m_poi)) return false;
-    CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
-    for(int g = 0; g < n_sets; g++) CUDA_TRY(cudaStreamWaitEvent(s->sets[g]->stream.get(), s->fork_ev.get(), 0));
-    bool ok = true;
-    std::vector<OutSpec> outs((size_t)chunk);
-    for(int k0 = 0, c = 0; k0 < n && ok; k0 += chunk, c++)
+    for(ViewSet* set : sets)
+        if(ann && to_host && !ensure_labels(*set, stream_of(*set), (size_t)chunk * m_poi)) return false;
+    if(forked)
     {
-        ViewSet& set = *s->sets[c % n_sets];
-        const int m = n - k0 < chunk ? n - k0 : chunk;
+        CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
+        for(ViewSet* set : sets) CUDA_TRY(cudaStreamWaitEvent(set->stream.get(), s->fork_ev.get(), 0));
+    }
+    // views [k0, k0+m) on one set: the chain, then (to_host) the copies of their outputs out of the set's scratch
+    std::vector<OutSpec> outs((size_t)chunk);
+    auto enqueue_chunk = [&](ViewSet& set, int k0, int m) {
+        const cudaStream_t sst = stream_of(set);
         for(int k = 0; k < m; k++)
             outs[k] = single_out(images ? (to_host ? set.sc[k].d_image.get()  : images + (size_t)(k0 + k) * px * 3) : nullptr,
                                  ranges ? (to_host ? set.sc[k].d_ranges.get() : ranges + (size_t)(k0 + k) * px)     : nullptr);
         AnnotSpec a{};
         if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? set.d_labels.get() : ann->labels + (size_t)k0 * m_poi, &av[k0] };
-        ok = enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), set.stream.get(), ann ? &a : nullptr);
-        for(int k = 0; k < m && ok && to_host; k++)
+        if(!enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), sst, ann ? &a : nullptr)) return false;
+        for(int k = 0; k < m && to_host; k++)
         {
-            if(images) ok = ok && copy_to_host(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3, set.stream.get());
-            if(ranges) ok = ok && copy_to_host(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges.get(), px * sizeof(float), set.stream.get());
+            if(images) CUDA_TRY(cudaMemcpyAsync(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3,
+                                                cudaMemcpyDeviceToHost, sst));
+            if(ranges) CUDA_TRY(cudaMemcpyAsync(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges.get(), px * sizeof(float),
+                                                cudaMemcpyDeviceToHost, sst));
         }
-        if(ok && ann && to_host)
-            ok = copy_to_host(ann->labels + (size_t)k0 * m_poi, a.labels, (size_t)m * m_poi * sizeof(float4), set.stream.get());
-    }
+        if(ann && to_host)
+            CUDA_TRY(cudaMemcpyAsync(ann->labels + (size_t)k0 * m_poi, a.labels, (size_t)m * m_poi * sizeof(float4),
+                                     cudaMemcpyDeviceToHost, sst));
+        return true;
+    };
+    bool ok = true;
+    for(int k0 = 0, c = 0; k0 < n && ok; k0 += chunk, c++)
+        ok = enqueue_chunk(*sets[(size_t)c % sets.size()], k0, n - k0 < chunk ? n - k0 : chunk);
+    if(!forked) s->have_render = false;     // the context's visibility buffer no longer holds the context's own view
     if(!ok)
     {
         // whatever was queued may still be writing into the caller's buffers: let it finish before reporting failure
-        for(int g = 0; g < n_sets; g++) cudaStreamSynchronize(s->sets[g]->stream.get());
+        for(ViewSet* set : sets) cudaStreamSynchronize(stream_of(*set));
         cudaGetLastError();
         return false;
     }
-    for(int g = 0; g < n_sets; g++)
-    {
-        CUDA_TRY(cudaEventRecord(s->sets[g]->done.get(), s->sets[g]->stream.get()));
-        CUDA_TRY(cudaStreamWaitEvent(st, s->sets[g]->done.get(), 0));
-    }
+    if(forked)
+        for(ViewSet* set : sets)
+        {
+            CUDA_TRY(cudaEventRecord(set->done.get(), set->stream.get()));
+            CUDA_TRY(cudaStreamWaitEvent(st, set->done.get(), 0));
+        }
     return true;
 }
 
@@ -1699,15 +1689,11 @@ bool horizonator_render_wedge_device(const horizonator_context_t* ctx, int x0, i
                                      void* d_image, void* d_ranges, void* stream)
 {
     Slot* s = slot_of(ctx);
-    if(s == nullptr) return false;
-    if(x0 < 0 || x1 > s->W || x0 >= x1)
-    {
-        MSG("wedge columns [%d,%d) are not inside [0,%d)", x0, x1, s->W);
-        return false;
-    }
+    if(s == nullptr || !wedge_columns_ok(*s, x0, x1)) return false;
     DeviceGuard g(s->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    if(!enqueue_render(*s, s->view, x0, x1, single_out((uint8_t*)d_image, (float*)d_ranges), st)) return false;
+    const OutSpec out = single_out((uint8_t*)d_image, (float*)d_ranges);
+    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
 }
@@ -1715,21 +1701,18 @@ bool horizonator_render_wedge_device(const horizonator_context_t* ctx, int x0, i
 bool horizonator_render_wedge_host(const horizonator_context_t* ctx, int x0, int x1, char* image, float* ranges)
 {
     Slot* s = slot_of(ctx);
-    if(s == nullptr) return false;
-    if(x0 < 0 || x1 > s->W || x0 >= x1)
-    {
-        MSG("wedge columns [%d,%d) are not inside [0,%d)", x0, x1, s->W);
-        return false;
-    }
+    if(s == nullptr || !wedge_columns_ok(*s, x0, x1)) return false;
     if(image == nullptr && ranges == nullptr) return true;
     DeviceGuard g(s->device);
     cudaStream_t st = s->stream.get();
-    // the context's own output buffers serve as the slab [H][x1-x0]; from there straight into the caller's columns
+    // the context's own scratch serves as the slab [H][x1-x0]; from there straight into the caller's columns
     const size_t w = (size_t)(x1 - x0);
-    if(!enqueue_render(*s, s->view, x0, x1, single_out(image ? s->d_image.get() : nullptr, ranges ? s->d_ranges.get() : nullptr), st)) return false;
-    if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, s->d_image.get(), w * 3, w * 3, (size_t)s->H,
+    const Scratch& own = s->main.sc[0];
+    const OutSpec out = single_out(image ? own.d_image.get() : nullptr, ranges ? own.d_ranges.get() : nullptr);
+    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
+    if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, own.d_image.get(), w * 3, w * 3, (size_t)s->H,
                                           cudaMemcpyDeviceToHost, st));
-    if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), s->d_ranges.get(), w * sizeof(float),
+    if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), own.d_ranges.get(), w * sizeof(float),
                                           w * sizeof(float), (size_t)s->H, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return true;
@@ -1810,12 +1793,7 @@ bool horizonator_render_wedge_peers(const horizonator_context_t* ctx, int x0, in
                                     void* const* d_images, void* const* d_ranges, void* stream)
 {
     Slot* s = slot_of(ctx);
-    if(s == nullptr) return false;
-    if(x0 < 0 || x1 > s->W || x0 >= x1)
-    {
-        MSG("wedge columns [%d,%d) are not inside [0,%d)", x0, x1, s->W);
-        return false;
-    }
+    if(s == nullptr || !wedge_columns_ok(*s, x0, x1)) return false;
     if(n_peers < 1 || n_peers > HZ_MAX_OUT || (d_images == nullptr && d_ranges == nullptr))
     {
         MSG("need 1..%d destinations and at least one kind of output", HZ_MAX_OUT);
@@ -1835,7 +1813,7 @@ bool horizonator_render_wedge_peers(const horizonator_context_t* ctx, int x0, in
     }
     DeviceGuard g(s->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    if(!enqueue_render(*s, s->view, x0, x1, out, st)) return false;
+    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
 }
@@ -1881,12 +1859,14 @@ bool horizonator_set_lod(const horizonator_context_t* ctx, float max_cell_pixels
         // the captured chains launch a different instantiation of k_blocks: wait for what is in flight, drop them
         DeviceGuard g(s->device);
         CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
-        for(const auto& v : s->sets) CUDA_TRY(cudaStreamSynchronize(v->stream.get()));
-        if(s->main.busy_recorded) CUDA_TRY(cudaEventSynchronize(s->main.busy.get()));
-        for(const auto& v : s->sets) if(v->busy_recorded) CUDA_TRY(cudaEventSynchronize(v->busy.get()));
-        s->main.graphs.clear();
-        s->main.graph_failed = false;
-        for(const auto& v : s->sets) { v->graphs.clear(); v->graph_failed = false; }
+        const bool idle = for_each_set(*s, [](ViewSet& v) {
+            if(v.stream) CUDA_TRY(cudaStreamSynchronize(v.stream.get()));
+            if(v.busy_recorded) CUDA_TRY(cudaEventSynchronize(v.busy.get()));
+            v.graphs.clear();
+            v.graph_failed = false;
+            return true;
+        });
+        if(!idle) return false;
     }
     s->lod_pixels = max_cell_pixels;
     return true;
