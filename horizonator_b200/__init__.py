@@ -86,11 +86,12 @@ class label_t(C.Structure):
 LABEL_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("range_m", np.float32), ("range_rendered_m", np.float32)])
 
 
-def _declare(lib):
+def _signatures():
+    """{symbol: (restype, argtypes)} of every function include/*.h declares."""
     P = C.POINTER
     ctx = P(context_t)
     f, d, i, b, vp, cp = C.c_float, C.c_double, C.c_int, C.c_bool, C.c_void_p, C.c_char_p
-    sigs = {
+    return {
         "horizonator_init": (b, [ctx, f, f, P(f), i, i, i, f, b, b, b, cp, cp, cp, cp, b]),
         "horizonator_deinit": (None, [ctx]),
         "horizonator_resized": (b, [ctx, i, i]),
@@ -137,7 +138,10 @@ def _declare(lib):
         "horizonator_annotate_batch_device": (b, [ctx, i, P(view_t), i, vp, vp, vp, vp, vp]),
         "horizonator_annotate_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
     }
-    for name, (res, args) in sigs.items():
+
+
+def _declare(lib):
+    for name, (res, args) in _signatures().items():
         try:
             fn = getattr(lib, name)
         except AttributeError:
@@ -149,25 +153,7 @@ def _declare(lib):
 
 
 #: every symbol include/*.h declares (tests check that the library exports each of them)
-EXPORTED_SYMBOLS = (
-    "horizonator_init", "horizonator_deinit", "horizonator_resized", "horizonator_pan_zoom",
-    "horizonator_move", "horizonator_set_zextents", "horizonator_redraw", "horizonator_pick",
-    "horizonator_render_offscreen", "horizonator_x_from_az", "horizonator_project",
-    "horizonator_unproject",
-    "horizonator_dem_init", "horizonator_dem_deinit", "horizonator_dem_sample",
-    "horizonator_dem_bounds_latlon_deg",
-    "horizonator_render_batch_device", "horizonator_render_batch", "horizonator_render_wedge_device",
-    "horizonator_download_mosaic", "horizonator_time_mosaic", "horizonator_last_render_stats",
-    "horizonator_profile_enable", "horizonator_profile_read",
-    "horizonator_host_alloc", "horizonator_host_free",
-    "horizonator_render_counters", "horizonator_horizon_profile_device", "horizonator_set_earth_curvature", "horizonator_set_seam_wrap",
-    "horizonator_peer_alloc", "horizonator_peer_open", "horizonator_peer_close", "horizonator_peer_free",
-    "horizonator_render_wedge_peers", "horizonator_peer_barrier",
-    "horizonator_render_wedge_host", "horizonator_host_register", "horizonator_host_unregister",
-    "horizonator_debug_device_math", "horizonator_set_lod",
-    "horizonator_viewshed_device", "horizonator_viewshed",
-    "horizonator_annotate_batch_device", "horizonator_annotate_batch",
-)
+EXPORTED_SYMBOLS = tuple(_signatures())
 
 if not os.path.exists(LIBRARY_PATH):
     raise ImportError(
@@ -179,6 +165,12 @@ lib = _declare(C.CDLL(LIBRARY_PATH))
 
 def _enc(s):
     return None if s is None else os.fsencode(s)
+
+
+def _check(fn, *args):
+    """Calls the library function fn; raises RuntimeError("<name>() failed") if it returns false."""
+    if not fn(*args):
+        raise RuntimeError("%s() failed" % fn.__name__)
 
 
 class horizonator:
@@ -200,13 +192,12 @@ class horizonator:
             raise RuntimeError("both render_radius_cells,render_radius_m cannot be >0")
         if width < 0 or height < 0:
             raise OverflowError("width, height must be unsigned")   # format "II"
-        if not lib.horizonator_init(C.byref(self._ctx), lat, lon, None,
-                                    int(width), int(height),
-                                    int(render_radius_cells), float(render_radius_m),
-                                    True, bool(render_texture), bool(SRTM1),
-                                    _enc(dir_dems), _enc(dir_tiles), _enc(tiles_name), _enc(tiles_url_fmt),
-                                    bool(allow_downloads)):
-            raise RuntimeError("horizonator_init() failed")
+        _check(lib.horizonator_init, C.byref(self._ctx), lat, lon, None,
+               int(width), int(height),
+               int(render_radius_cells), float(render_radius_m),
+               True, bool(render_texture), bool(SRTM1),
+               _enc(dir_dems), _enc(dir_tiles), _enc(tiles_name), _enc(tiles_url_fmt),
+               bool(allow_downloads))
 
     def __del__(self):
         ctx = getattr(self, "_ctx", None)
@@ -241,22 +232,18 @@ class horizonator:
             az_per_pixel = (az_deg1 - az_deg0) / float(W - 1)
             az_deg0 -= az_per_pixel / 2.
             az_deg1 += az_per_pixel / 2.
-        if not lib.horizonator_pan_zoom(C.byref(self._ctx), az_deg0, az_deg1):
-            raise RuntimeError("horizonator_pan_zoom() failed")
+        _check(lib.horizonator_pan_zoom, C.byref(self._ctx), az_deg0, az_deg1)
         if lat > -1000.:
-            if not lib.horizonator_move(C.byref(self._ctx), None, lat, lon):
-                raise RuntimeError("horizonator_move() failed")
-        if not lib.horizonator_set_zextents(C.byref(self._ctx), znear, zfar, znear_color, zfar_color):
-            raise RuntimeError("horizonator_set_zextents() failed")
+            _check(lib.horizonator_move, C.byref(self._ctx), None, lat, lon)
+        _check(lib.horizonator_set_zextents, C.byref(self._ctx), znear, zfar, znear_color, zfar_color)
         # fresh arrays per call like the reference (pywrap.c:234-250), but out of a recycling pool of page-locked
         # blocks: the results then arrive by DMA instead of through the driver's pageable staging (3x faster for
         # 15 MB), and a block goes back to the pool when the caller drops the array
         image = _pool.array((H, W, 3), np.uint8) if return_image else None
         ranges = _pool.array((H, W), np.float32) if return_range else None
-        if not lib.horizonator_render_offscreen(C.byref(self._ctx),
-                                                image.ctypes.data if image is not None else None,
-                                                ranges.ctypes.data if ranges is not None else None):
-            raise RuntimeError("horizonator_render_offscreen() failed")
+        _check(lib.horizonator_render_offscreen, C.byref(self._ctx),
+               image.ctypes.data if image is not None else None,
+               ranges.ctypes.data if ranges is not None else None)
         if return_image and not return_range:
             return image
         if return_range and not return_image:
@@ -291,8 +278,7 @@ class horizonator:
             znear_color = znear
         if zfar_color < 0.:
             zfar_color = zfar
-        if not lib.horizonator_set_zextents(C.byref(self._ctx), znear, zfar, znear_color, zfar_color):
-            raise RuntimeError("horizonator_set_zextents() failed")
+        _check(lib.horizonator_set_zextents, C.byref(self._ctx), znear, zfar, znear_color, zfar_color)
 
     def render_batch(self, views, return_image=True, return_range=True):
         """views: sequence of (lat, lon, az_deg0, az_deg1[, viewer_z]).  Host arrays (n,H,W,3), (n,H,W)."""
@@ -301,60 +287,51 @@ class horizonator:
         # overlap the next views' kernels (into pageable arrays each copy would go through the driver's staging)
         image = _pool.array((n, H, W, 3), np.uint8) if return_image else None
         ranges = _pool.array((n, H, W), np.float32) if return_range else None
-        if not lib.horizonator_render_batch(C.byref(self._ctx), n, self._views(views),
-                                            image.ctypes.data if image is not None else None,
-                                            ranges.ctypes.data if ranges is not None else None):
-            raise RuntimeError("horizonator_render_batch() failed")
+        _check(lib.horizonator_render_batch, C.byref(self._ctx), n, self._views(views),
+               image.ctypes.data if image is not None else None,
+               ranges.ctypes.data if ranges is not None else None)
         return image, ranges
 
     def render_batch_device(self, views, d_images=0, d_ranges=0, stream=0):
         """Device-pointer variant: d_images / d_ranges are integer device addresses (e.g. tensor.data_ptr()),
         stream an integer cudaStream_t (0 = the context's own stream, synchronous)."""
-        if not lib.horizonator_render_batch_device(C.byref(self._ctx), len(views), self._views(views),
-                                                   d_images or None, d_ranges or None, stream or None):
-            raise RuntimeError("horizonator_render_batch_device() failed")
+        _check(lib.horizonator_render_batch_device, C.byref(self._ctx), len(views), self._views(views),
+               d_images or None, d_ranges or None, stream or None)
 
     def render_wedge_device(self, x0, x1, d_image=0, d_ranges=0, stream=0):
-        if not lib.horizonator_render_wedge_device(C.byref(self._ctx), int(x0), int(x1),
-                                                   d_image or None, d_ranges or None, stream or None):
-            raise RuntimeError("horizonator_render_wedge_device() failed")
+        _check(lib.horizonator_render_wedge_device, C.byref(self._ctx), int(x0), int(x1),
+               d_image or None, d_ranges or None, stream or None)
 
     def render_wedge_host(self, x0, x1, image=None, ranges=None):
         """Columns [x0, x1) of the current view into FULL-size host arrays (H,W,3) uint8 / (H,W) float32."""
-        if not lib.horizonator_render_wedge_host(C.byref(self._ctx), int(x0), int(x1),
-                                                 image.ctypes.data if image is not None else None,
-                                                 ranges.ctypes.data if ranges is not None else None):
-            raise RuntimeError("horizonator_render_wedge_host() failed")
+        _check(lib.horizonator_render_wedge_host, C.byref(self._ctx), int(x0), int(x1),
+               image.ctypes.data if image is not None else None,
+               ranges.ctypes.data if ranges is not None else None)
 
     def set_seam_wrap(self, on=True):
         """Opt-in (off by default; the reference drops them): draw triangles across the +-180 degree seam at both
         edges of a full-circle panorama.  See horizonator-batch.h."""
-        if not lib.horizonator_set_seam_wrap(C.byref(self._ctx), bool(on)):
-            raise RuntimeError("horizonator_set_seam_wrap() failed")
+        _check(lib.horizonator_set_seam_wrap, C.byref(self._ctx), bool(on))
 
     def set_lod(self, max_cell_pixels=0.5):
         """Opt-in level of detail (0 = off, the default; the reference always draws every DEM cell): coarser far mesh
         where a coarser cell still is at most `max_cell_pixels` pixels across.  See horizonator-batch.h."""
-        if not lib.horizonator_set_lod(C.byref(self._ctx), float(max_cell_pixels)):
-            raise RuntimeError("horizonator_set_lod() failed")
+        _check(lib.horizonator_set_lod, C.byref(self._ctx), float(max_cell_pixels))
 
     def set_earth_curvature(self, on=True, refraction=0.13):
         """Opt-in accuracy mode (off by default; the reference is flat-earth): see horizonator-batch.h."""
-        if not lib.horizonator_set_earth_curvature(C.byref(self._ctx), bool(on), float(refraction)):
-            raise RuntimeError("horizonator_set_earth_curvature() failed")
+        _check(lib.horizonator_set_earth_curvature, C.byref(self._ctx), bool(on), float(refraction))
 
     # peer-memory assembly of wedge-sharded panoramas (horizonator-batch.h); used by sharding.PeerPanorama
     def peer_alloc(self, nbytes):
         """-> (device address, 64-byte handle) of a buffer other ranks can map."""
         ptr, handle = C.c_void_p(), (C.c_ubyte * 64)()
-        if not lib.horizonator_peer_alloc(C.byref(self._ctx), nbytes, C.byref(ptr), C.byref(handle)):
-            raise RuntimeError("horizonator_peer_alloc() failed")
+        _check(lib.horizonator_peer_alloc, C.byref(self._ctx), nbytes, C.byref(ptr), C.byref(handle))
         return ptr.value, bytes(handle)
 
     def peer_open(self, handle):
         ptr = C.c_void_p()
-        if not lib.horizonator_peer_open(C.byref(self._ctx), (C.c_ubyte * 64).from_buffer_copy(handle), C.byref(ptr)):
-            raise RuntimeError("horizonator_peer_open() failed")
+        _check(lib.horizonator_peer_open, C.byref(self._ctx), (C.c_ubyte * 64).from_buffer_copy(handle), C.byref(ptr))
         return ptr.value
 
     def peer_close(self, ptr):
@@ -366,67 +343,57 @@ class horizonator:
     def peer_barrier(self, rank, d_flags, epoch, stream=0):
         """GPU-side barrier between ranks (horizonator_peer_barrier); d_flags: every rank's flag block address."""
         arr = (C.c_void_p * len(d_flags))(*d_flags)
-        if not lib.horizonator_peer_barrier(C.byref(self._ctx), len(d_flags), int(rank), arr, int(epoch), stream or None):
-            raise RuntimeError("horizonator_peer_barrier() failed")
+        _check(lib.horizonator_peer_barrier, C.byref(self._ctx), len(d_flags), int(rank), arr, int(epoch), stream or None)
 
     def render_wedge_peers(self, x0, x1, d_images, d_ranges, stream=0):
         """d_images / d_ranges: sequences of device addresses of every rank's full image / range buffer (or None)."""
         n = len(d_images) if d_images is not None else len(d_ranges)
         ai = (C.c_void_p * n)(*d_images) if d_images is not None else None
         ar = (C.c_void_p * n)(*d_ranges) if d_ranges is not None else None
-        if not lib.horizonator_render_wedge_peers(C.byref(self._ctx), int(x0), int(x1), n, ai, ar, stream or None):
-            raise RuntimeError("horizonator_render_wedge_peers() failed")
+        _check(lib.horizonator_render_wedge_peers, C.byref(self._ctx), int(x0), int(x1), n, ai, ar, stream or None)
 
     def pan_zoom(self, az_deg0, az_deg1):
-        if not lib.horizonator_pan_zoom(C.byref(self._ctx), az_deg0, az_deg1):
-            raise RuntimeError("horizonator_pan_zoom() failed")
+        _check(lib.horizonator_pan_zoom, C.byref(self._ctx), az_deg0, az_deg1)
 
     def move(self, lat, lon, viewer_z=None):
         z = C.c_float(-1. if viewer_z is None else viewer_z)
-        if not lib.horizonator_move(C.byref(self._ctx), C.byref(z), lat, lon):
-            raise RuntimeError("horizonator_move() failed")
+        _check(lib.horizonator_move, C.byref(self._ctx), C.byref(z), lat, lon)
         return z.value
 
     def mosaic(self):
         """The decoded DEM square as the GPU holds it: (2R, 2R) int16, [j north][i east]."""
         n = 2 * self._ctx.dems.radius_cells
         out = np.empty((n, n), dtype=np.int16)
-        if not lib.horizonator_download_mosaic(C.byref(self._ctx), out.ctypes.data):
-            raise RuntimeError("horizonator_download_mosaic() failed")
+        _check(lib.horizonator_download_mosaic, C.byref(self._ctx), out.ctypes.data)
         return out
 
     def time_mosaic(self, reps=10):
         ms = C.c_float(0)
-        if not lib.horizonator_time_mosaic(C.byref(self._ctx), reps, C.byref(ms)):
-            raise RuntimeError("horizonator_time_mosaic() failed")
+        _check(lib.horizonator_time_mosaic, C.byref(self._ctx), reps, C.byref(ms))
         return ms.value
 
     def render_into(self, image, ranges):
         """horizonator_render_offscreen() with the current state into caller-owned arrays (either may be
         None): no allocation, and DMA speed when the arrays come from pinned_array()."""
-        if not lib.horizonator_render_offscreen(C.byref(self._ctx),
-                                                image.ctypes.data if image is not None else None,
-                                                ranges.ctypes.data if ranges is not None else None):
-            raise RuntimeError("horizonator_render_offscreen() failed")
+        _check(lib.horizonator_render_offscreen, C.byref(self._ctx),
+               image.ctypes.data if image is not None else None,
+               ranges.ctypes.data if ranges is not None else None)
 
     def profile(self, on=True):
         """Record CUDA events around every kernel of every render from now on (see profile_read)."""
-        if not lib.horizonator_profile_enable(C.byref(self._ctx), bool(on)):
-            raise RuntimeError("horizonator_profile_enable() failed")
+        _check(lib.horizonator_profile_enable, C.byref(self._ctx), bool(on))
 
     def profile_read(self):
         """Mean device ms per render of each kernel since the last read, and the number of renders."""
         ms = (C.c_float * 6)()
         n = C.c_int(0)
-        if not lib.horizonator_profile_read(C.byref(self._ctx), C.byref(ms), C.byref(n)):
-            raise RuntimeError("horizonator_profile_read() failed")
+        _check(lib.horizonator_profile_read, C.byref(self._ctx), C.byref(ms), C.byref(n))
         return {"prepare": ms[0], "near": ms[1], "big_near": ms[2], "march": ms[3], "big_far": ms[4],
                 "resolve": ms[5], "renders": n.value}
 
     def last_render_stats(self):
         out = (C.c_uint * 5)()
-        if not lib.horizonator_last_render_stats(C.byref(self._ctx), C.byref(out)):
-            raise RuntimeError("horizonator_last_render_stats() failed")
+        _check(lib.horizonator_last_render_stats, C.byref(self._ctx), C.byref(out))
         return {"big_entries": out[0], "big_capacity": out[1], "launches": out[2], "device": out[3],
                 "triangles_rasterised": out[4]}
 
@@ -437,15 +404,13 @@ class horizonator:
     def render_counters(self):
         """Culling counters of the most recent render (horizonator_render_counters)."""
         out = (C.c_uint * 16)()
-        if not lib.horizonator_render_counters(C.byref(self._ctx), C.byref(out)):
-            raise RuntimeError("horizonator_render_counters() failed")
+        _check(lib.horizonator_render_counters, C.byref(self._ctx), C.byref(out))
         return dict(zip(self.COUNTER_NAMES, out))
 
     def horizon_profile_device(self, d_ranges, n, d_rows, d_range, stream=0):
         """Per-column topmost terrain (row, range) of n device range images; all arguments device addresses."""
-        if not lib.horizonator_horizon_profile_device(C.byref(self._ctx), d_ranges, int(n), d_rows, d_range,
-                                                      stream or None):
-            raise RuntimeError("horizonator_horizon_profile_device() failed")
+        _check(lib.horizonator_horizon_profile_device, C.byref(self._ctx), d_ranges, int(n), d_rows, d_range,
+               stream or None)
 
     # viewsheds (horizonator-batch.h: which vertices of the loaded square each view sees)
     @property
@@ -466,18 +431,16 @@ class horizonator:
         w32 = (N + 31) // 32
         words = np.empty((n, N, w32), np.uint32)
         cnt = np.zeros((N, N), np.uint32) if counts else None
-        if not lib.horizonator_viewshed(C.byref(self._ctx), n, self._eyes(views), float(target_height),
-                                        words.ctypes.data, cnt.ctypes.data if counts else None):
-            raise RuntimeError("horizonator_viewshed() failed")
+        _check(lib.horizonator_viewshed, C.byref(self._ctx), n, self._eyes(views), float(target_height),
+               words.ctypes.data, cnt.ctypes.data if counts else None)
         bits = np.unpackbits(words.view(np.uint8), axis=-1, bitorder="little")[..., :N].astype(bool)
         return (bits, cnt) if counts else bits
 
     def viewshed_device(self, views, d_masks=0, d_counts=0, target_height=0., stream=0):
         """Device-pointer variant: d_masks (n, N, (N+31)//32) uint32 words, overwritten; d_counts (N, N) uint32,
         added to.  Integer device addresses, either may be 0 (not both); stream as render_batch_device."""
-        if not lib.horizonator_viewshed_device(C.byref(self._ctx), len(views), self._eyes(views), float(target_height),
-                                               d_masks or None, d_counts or None, stream or None):
-            raise RuntimeError("horizonator_viewshed_device() failed")
+        _check(lib.horizonator_viewshed_device, C.byref(self._ctx), len(views), self._eyes(views), float(target_height),
+               d_masks or None, d_counts or None, stream or None)
 
 
     # labels of points of interest (horizonator_annotate_batch*: which POIs each view sees, and where)
@@ -493,9 +456,8 @@ class horizonator:
         p = self.pois_array(pois)
         n, m = len(views), p.shape[0]
         out = _pool.array((n, m, 4), np.float32)
-        if not lib.horizonator_annotate_batch(C.byref(self._ctx), n, self._views(views), m, p.ctypes.data if m else None,
-                                              out.ctypes.data if out.size else None):
-            raise RuntimeError("horizonator_annotate_batch() failed")
+        _check(lib.horizonator_annotate_batch, C.byref(self._ctx), n, self._views(views), m, p.ctypes.data if m else None,
+               out.ctypes.data if out.size else None)
         return out.view(LABEL_DTYPE).reshape(n, m)
 
     def annotate_device(self, views, d_pois, d_labels, d_images=0, d_ranges=0, stream=0, m=None):
@@ -510,10 +472,9 @@ class horizonator:
             raise ValueError("annotate_device: m is needed when d_pois is an address")
         if hasattr(d_labels, "data_ptr"):
             d_labels = d_labels.data_ptr()
-        if not lib.horizonator_annotate_batch_device(C.byref(self._ctx), len(views), self._views(views), int(m),
-                                                     d_pois or None, d_labels or None, d_images or None, d_ranges or None,
-                                                     stream or None):
-            raise RuntimeError("horizonator_annotate_batch_device() failed")
+        _check(lib.horizonator_annotate_batch_device, C.byref(self._ctx), len(views), self._views(views), int(m),
+               d_pois or None, d_labels or None, d_images or None, d_ranges or None,
+               stream or None)
 
 
 class _PinnedBlock:

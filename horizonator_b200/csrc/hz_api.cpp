@@ -108,6 +108,24 @@ template<class H> bool empty_handle(const H& h, const char* what)
     return true;
 }
 
+// Device scratch that grows on demand: the buffer and how many elements it holds.  Before grow() the caller waits for
+// whatever may still use the old buffer.
+template<class T> struct GrowBuffer
+{
+    DevPtr<T> buf;
+    size_t cap = 0;
+    T* get() const { return buf.get(); }
+    // Replaces the buffer with one of n elements, releasing the old one first.  A failed cudaMalloc leaves it empty and
+    // its error cleared; the error is returned for the caller's message.
+    cudaError_t grow(size_t n)
+    {
+        buf = nullptr; cap = 0;
+        if(!(buf = make_device<T>(n))) return cudaGetLastError();
+        cap = n;
+        return cudaSuccess;
+    }
+};
+
 // ---- the render chain's configuration.  Each value won its sweep (profiles/); a new sweep edits a constant and
 // compares a second build of the library (build_library(extra_flags, name) + HORIZONATOR_LIBRARY).
 
@@ -217,8 +235,7 @@ struct ViewSet
     // POIs), and for the host-memory call the labels of one chunk, copied to the caller on the set's stream
     DevPtr<HzAnnotate>  d_annot;
     HostPtr<HzAnnotate> h_annot;       // pinned [PARAM_RING]
-    DevPtr<float4>      d_labels;
-    size_t labels_cap = 0;             // labels d_labels holds
+    GrowBuffer<float4>  d_labels;
 };
 
 struct Slot
@@ -274,14 +291,12 @@ struct Slot
     // viewsheds, allocated by the first viewshed call that needs them: the masks of one chunk of views for calls that
     // want only counts or want the masks in host memory, and the counts of the host-memory call.  A call's stream
     // waits for `vs_done` of the call before it, which may have been queued on another stream and use the same scratch.
-    DevPtr<uint32_t> d_vs_masks;
-    int              vs_mask_views = 0;
-    DevPtr<uint32_t> d_vs_counts;
-    EventHandle      vs_done;
+    GrowBuffer<uint32_t> d_vs_masks;
+    GrowBuffer<uint32_t> d_vs_counts;
+    EventHandle          vs_done;
 
     // labels (horizonator_annotate_batch): the POIs of the host-memory call, uploaded per call, made on first use
-    DevPtr<double>   d_pois;             // [pois_cap][3]
-    size_t           pois_cap = 0;
+    GrowBuffer<double>   d_pois;         // [POIs][3]
 };
 
 // raw pointers: a slot is deleted by horizonator_deinit(), never by a destructor at exit, when the CUDA runtime may
@@ -308,6 +323,19 @@ struct DeviceGuard
     }
     ~DeviceGuard() { if(prev >= 0) cudaSetDevice(prev); }
 };
+
+// The frame of an entry point that queues work for a context, once it has found the context's slot and checked its
+// arguments.  body(st) runs with the context's device current and queues the call's work on st: the caller's `stream`,
+// or, where that is null, the context's own, and the call then returns once that stream is idle (horizonator-batch.h).
+// The calls into host memory are of the second kind.
+template<class F> bool on_stream(const Slot& s, void* stream, F&& body)
+{
+    DeviceGuard g(s.device);
+    const cudaStream_t st = stream ? (cudaStream_t)stream : s.stream.get();
+    if(!body(st)) return false;
+    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
+    return true;
+}
 
 // The device buffers of a scratch, as (member, number of elements): those sized by the terrain unless `image_only`,
 // then, if the slot has a target, those sized by the image.  alloc_scratch() allocates them from this list, and
@@ -1269,12 +1297,11 @@ bool horizonator_redraw(const horizonator_context_t* ctx)
 {
     Slot* s = slot_of(ctx);
     if(s == nullptr) return false;
-    DeviceGuard g(s->device);
-    const Scratch& own = s->main.sc[0];
-    const OutSpec out = single_out(own.d_image.get(), own.d_ranges.get());
-    if(!enqueue_views(*s, s->main, 1, &s->view, 0, s->W, &out, s->stream.get())) return false;
-    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
-    return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        const Scratch& own = s->main.sc[0];
+        const OutSpec out = single_out(own.d_image.get(), own.d_ranges.get());
+        return enqueue_views(*s, s->main, 1, &s->view, 0, s->W, &out, st);
+    });
 }
 
 bool horizonator_render_offscreen(const horizonator_context_t* ctx, char* image, float* ranges)
@@ -1370,18 +1397,6 @@ struct AnnotReq
     float4* labels;              // [n][m]: device memory, or host memory when to_host
 };
 
-// makes sure a set's label scratch holds `count` labels (host-memory call only; those are synchronous, so nothing queued
-// still uses the old buffer once the set's stream is idle)
-static bool ensure_labels(ViewSet& set, cudaStream_t st, size_t count)
-{
-    if(set.labels_cap >= count) return true;
-    CUDA_TRY(cudaStreamSynchronize(st));
-    set.d_labels = nullptr; set.labels_cap = 0;
-    if(empty_handle(set.d_labels = make_device<float4>(count), "cudaMalloc(labels)")) return false;
-    set.labels_cap = count;
-    return true;
-}
-
 static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
                                 uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const AnnotReq* ann = nullptr)
 {
@@ -1435,8 +1450,15 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     if(!forked) { sets.push_back(&s->main); chunk = 1; }
     auto stream_of = [st](const ViewSet& set) { return set.stream ? set.stream.get() : st; };
 
+    // each set's label scratch for a chunk (host-memory call only; those are synchronous, so nothing queued still uses
+    // the old buffer once the set's stream is idle)
     for(ViewSet* set : sets)
-        if(ann && to_host && !ensure_labels(*set, stream_of(*set), (size_t)chunk * m_poi)) return false;
+        if(ann && to_host && set->d_labels.cap < (size_t)chunk * m_poi)
+        {
+            CUDA_TRY(cudaStreamSynchronize(stream_of(*set)));
+            const cudaError_t e = set->d_labels.grow((size_t)chunk * m_poi);
+            if(e != cudaSuccess) { MSG("CUDA error: cudaMalloc(labels) failed: %s", cudaGetErrorString(e)); return false; }
+        }
     if(forked)
     {
         CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
@@ -1515,17 +1537,14 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
     const int chunk = n < HZ_VS_MAX_VIEWS ? n : HZ_VS_MAX_VIEWS;
     if(!s->vs_done) { if(empty_handle(s->vs_done = make_event(), "cudaEventCreate")) return false; }
     else CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
-    if(d_masks == nullptr && s->vs_mask_views < chunk)
+    if(d_masks == nullptr && s->d_vs_masks.cap < (size_t)chunk * mwords)
     {
         CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
-        s->d_vs_masks = nullptr; s->vs_mask_views = 0;          // the smaller masks go before the larger ones come
-        if(!(s->d_vs_masks = make_device<uint32_t>((size_t)chunk * mwords)))
+        if(s->d_vs_masks.grow((size_t)chunk * mwords) != cudaSuccess)
         {
-            cudaGetLastError();
             MSG("Could not allocate the viewshed masks of %d views (%zu MB)", chunk, (size_t)chunk * mwords * 4 >> 20);
             return false;
         }
-        s->vs_mask_views = chunk;
     }
 
     HzViewshed p{};
@@ -1559,12 +1578,9 @@ bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const 
         MSG("horizonator_viewshed_device: neither masks nor counts asked for");
         return false;
     }
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    if(!viewshed_common(ctx, s, n, views, target_height_m, (uint32_t*)d_masks, (uint32_t*)d_counts, nullptr, st))
-        return false;
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        return viewshed_common(ctx, s, n, views, target_height_m, (uint32_t*)d_masks, (uint32_t*)d_counts, nullptr, st);
+    });
 }
 
 bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
@@ -1577,30 +1593,29 @@ bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizon
         MSG("horizonator_viewshed: neither masks nor counts asked for");
         return false;
     }
-    DeviceGuard g(s->device);
-    const size_t cells = (size_t)s->N * s->N;
-    if(counts && n > 0 && !s->d_vs_counts)
-    {
-        if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
-        if(!(s->d_vs_counts = make_device<uint32_t>(cells)))
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        const size_t cells = (size_t)s->N * s->N;
+        if(counts && n > 0 && s->d_vs_counts.cap < cells)
         {
+            if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
+            if(s->d_vs_counts.grow(cells) != cudaSuccess)
+            {
+                MSG("Could not allocate the viewshed counts (%zu MB)", cells * 4 >> 20);
+                return false;
+            }
+        }
+        // the counts' upload waits for whatever an earlier call still does with the same buffer
+        if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
+        if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts.get(), counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts.get() : nullptr, masks, st))
+        {
+            cudaStreamSynchronize(st);
             cudaGetLastError();
-            MSG("Could not allocate the viewshed counts (%zu MB)", cells * 4 >> 20);
             return false;
         }
-    }
-    // the counts' upload waits for whatever an earlier call still does with the same buffer
-    if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(s->stream.get(), s->vs_done.get(), 0));
-    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts.get(), counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream.get()));
-    if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts.get() : nullptr, masks, s->stream.get()))
-    {
-        cudaStreamSynchronize(s->stream.get());
-        cudaGetLastError();
-        return false;
-    }
-    if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts.get(), cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, s->stream.get()));
-    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
-    return true;
+        if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts.get(), cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        return true;
+    });
 }
 
 bool horizonator_render_batch_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
@@ -1608,11 +1623,9 @@ bool horizonator_render_batch_device(const horizonator_context_t* ctx, int n, co
 {
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    if(!render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st)) return false;
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        return render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st);
+    });
 }
 
 bool horizonator_render_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
@@ -1620,10 +1633,9 @@ bool horizonator_render_batch(const horizonator_context_t* ctx, int n, const hor
 {
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
-    DeviceGuard g(s->device);
-    if(!render_batch_common(ctx, s, n, views, (uint8_t*)images, ranges, true, s->stream.get())) return false;
-    CUDA_TRY(cudaStreamSynchronize(s->stream.get()));
-    return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        return render_batch_common(ctx, s, n, views, (uint8_t*)images, ranges, true, st);
+    });
 }
 
 // ---- labels of points of interest (horizonator-batch.h) ----------------------------------------------------------
@@ -1649,12 +1661,10 @@ bool horizonator_annotate_batch_device(const horizonator_context_t* ctx, int n, 
         MSG("horizonator_annotate_batch_device: d_pois must be 8-byte and d_labels 16-byte aligned");
         return false;
     }
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     const AnnotReq ann{ (const double*)d_pois, m, (float4*)d_labels };
-    if(!render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &ann)) return false;
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        return render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &ann);
+    });
 }
 
 bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
@@ -1663,26 +1673,24 @@ bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const h
     Slot* s = slot_of(ctx);
     if(s == nullptr || !annotate_args_ok("horizonator_annotate_batch", n, views, m, pois, labels)) return false;
     if(n == 0 || m == 0) return true;
-    DeviceGuard g(s->device);
-    cudaStream_t st = s->stream.get();
-    // the POIs go up once per call into the context's scratch (the call is synchronous: no earlier one still reads it)
-    if(s->pois_cap < (size_t)m)
-    {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        s->d_pois = nullptr; s->pois_cap = 0;
-        if(empty_handle(s->d_pois = make_device<double>(3 * (size_t)m), "cudaMalloc(POIs)")) return false;
-        s->pois_cap = (size_t)m;
-    }
-    CUDA_TRY(cudaMemcpyAsync(s->d_pois.get(), pois, (size_t)m * sizeof(horizonator_poi_t), cudaMemcpyHostToDevice, st));
-    const AnnotReq ann{ s->d_pois.get(), m, (float4*)labels };
-    if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &ann))
-    {
-        cudaStreamSynchronize(st);
-        cudaGetLastError();
-        return false;
-    }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        // the POIs go up once per call into the context's scratch (the call is synchronous: no earlier one still reads it)
+        if(s->d_pois.cap < 3 * (size_t)m)
+        {
+            CUDA_TRY(cudaStreamSynchronize(st));
+            const cudaError_t e = s->d_pois.grow(3 * (size_t)m);
+            if(e != cudaSuccess) { MSG("CUDA error: cudaMalloc(POIs) failed: %s", cudaGetErrorString(e)); return false; }
+        }
+        CUDA_TRY(cudaMemcpyAsync(s->d_pois.get(), pois, (size_t)m * sizeof(horizonator_poi_t), cudaMemcpyHostToDevice, st));
+        const AnnotReq ann{ s->d_pois.get(), m, (float4*)labels };
+        if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &ann))
+        {
+            cudaStreamSynchronize(st);
+            cudaGetLastError();
+            return false;
+        }
+        return true;
+    });
 }
 
 bool horizonator_render_wedge_device(const horizonator_context_t* ctx, int x0, int x1,
@@ -1690,12 +1698,8 @@ bool horizonator_render_wedge_device(const horizonator_context_t* ctx, int x0, i
 {
     Slot* s = slot_of(ctx);
     if(s == nullptr || !wedge_columns_ok(*s, x0, x1)) return false;
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
     const OutSpec out = single_out((uint8_t*)d_image, (float*)d_ranges);
-    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) { return enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st); });
 }
 
 bool horizonator_render_wedge_host(const horizonator_context_t* ctx, int x0, int x1, char* image, float* ranges)
@@ -1703,19 +1707,18 @@ bool horizonator_render_wedge_host(const horizonator_context_t* ctx, int x0, int
     Slot* s = slot_of(ctx);
     if(s == nullptr || !wedge_columns_ok(*s, x0, x1)) return false;
     if(image == nullptr && ranges == nullptr) return true;
-    DeviceGuard g(s->device);
-    cudaStream_t st = s->stream.get();
     // the context's own scratch serves as the slab [H][x1-x0]; from there straight into the caller's columns
     const size_t w = (size_t)(x1 - x0);
     const Scratch& own = s->main.sc[0];
     const OutSpec out = single_out(image ? own.d_image.get() : nullptr, ranges ? own.d_ranges.get() : nullptr);
-    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
-    if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, own.d_image.get(), w * 3, w * 3, (size_t)s->H,
-                                          cudaMemcpyDeviceToHost, st));
-    if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), own.d_ranges.get(), w * sizeof(float),
-                                          w * sizeof(float), (size_t)s->H, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
+        if(image)  CUDA_TRY(cudaMemcpy2DAsync(image + (size_t)x0 * 3, (size_t)s->W * 3, own.d_image.get(), w * 3, w * 3, (size_t)s->H,
+                                              cudaMemcpyDeviceToHost, st));
+        if(ranges) CUDA_TRY(cudaMemcpy2DAsync(ranges + x0, (size_t)s->W * sizeof(float), own.d_ranges.get(), w * sizeof(float),
+                                              w * sizeof(float), (size_t)s->H, cudaMemcpyDeviceToHost, st));
+        return true;
+    });
 }
 
 bool horizonator_host_register(void* p, size_t bytes)
@@ -1811,11 +1814,7 @@ bool horizonator_render_wedge_peers(const horizonator_context_t* ctx, int x0, in
             return false;
         }
     }
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    if(!enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st)) return false;
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) { return enqueue_views(*s, s->main, 1, &s->view, x0, x1, &out, st); });
 }
 
 bool horizonator_peer_barrier(const horizonator_context_t* ctx, int n_ranks, int rank, void* const* d_flags,
@@ -1830,11 +1829,10 @@ bool horizonator_peer_barrier(const horizonator_context_t* ctx, int n_ranks, int
         if(d_flags[r] == nullptr) return false;
         f.arrive[r] = (uint32_t*)d_flags[r];
     }
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    CUDA_TRY(hz_launch_peer_barrier(f, epoch, st));
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        CUDA_TRY(hz_launch_peer_barrier(f, epoch, st));
+        return true;
+    });
 }
 
 bool horizonator_set_seam_wrap(const horizonator_context_t* ctx, bool on)
@@ -2015,11 +2013,10 @@ bool horizonator_horizon_profile_device(const horizonator_context_t* ctx, const 
 {
     Slot* s = slot_of(ctx);
     if(s == nullptr || n < 0 || d_ranges == nullptr || d_rows == nullptr || d_range == nullptr) return false;
-    DeviceGuard g(s->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream.get();
-    CUDA_TRY(hz_launch_horizon((const float*)d_ranges, n, s->W, s->H, (int*)d_rows, (float*)d_range, st));
-    if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
-    return true;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        CUDA_TRY(hz_launch_horizon((const float*)d_ranges, n, s->W, s->H, (int*)d_rows, (float*)d_range, st));
+        return true;
+    });
 }
 
 } // extern "C"
