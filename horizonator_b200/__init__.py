@@ -86,6 +86,29 @@ class label_t(C.Structure):
 LABEL_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("range_m", np.float32), ("range_rendered_m", np.float32)])
 
 
+class skyline_sample_t(C.Structure):
+    """include/horizonator-batch.h: horizonator_skyline_sample_t (8 bytes)."""
+    _fields_ = [("dx", C.c_int32), ("y", C.c_float)]
+
+
+#: numpy dtype of skyline_sample_t: what skyline_samples() returns
+SKYLINE_SAMPLE_DTYPE = np.dtype([("dx", np.int32), ("y", np.float32)])
+
+
+def skyline_samples(rel_az_deg, el_deg, az_width_deg, width, height):
+    """An observed skyline given as angles -> its samples (SKYLINE_SAMPLE_DTYPE) for width x height panoramas of windows
+    az_width_deg (az_deg1 - az_deg0) wide: points rel_az_deg degrees right of the heading and el_deg above the
+    horizontal.  With p = az_width_deg / width degrees per column, dx = rint(rel_az_deg / p) and
+    y = (height - 1) / 2 - el_deg / p in double, rounded to float once (horizonator-batch.h)."""
+    rel = np.asarray(rel_az_deg, np.float64).ravel()
+    el = np.asarray(el_deg, np.float64).ravel()
+    p = float(az_width_deg) / width
+    out = np.empty(len(rel), SKYLINE_SAMPLE_DTYPE)
+    out["dx"] = np.rint(rel / p)
+    out["y"] = (height - 1) / 2. - el / p
+    return out
+
+
 def _signatures():
     """{symbol: (restype, argtypes)} of every function include/*.h declares."""
     P = C.POINTER
@@ -137,6 +160,8 @@ def _signatures():
         "horizonator_viewshed": (b, [ctx, i, P(view_t), f, vp, vp]),
         "horizonator_annotate_batch_device": (b, [ctx, i, P(view_t), i, vp, vp, vp, vp, vp]),
         "horizonator_annotate_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
+        "horizonator_skyline_match_device": (b, [ctx, i, P(view_t), vp, vp, i, vp, f, b, vp, vp]),
+        "horizonator_skyline_match": (b, [ctx, i, P(view_t), vp, vp, i, vp, f, b, vp]),
     }
 
 
@@ -475,6 +500,76 @@ class horizonator:
         _check(lib.horizonator_annotate_batch_device, C.byref(self._ctx), len(views), self._views(views), int(m),
                d_pois or None, d_labels or None, d_images or None, d_ranges or None,
                stream or None)
+
+    # skylines and their match against an observed skyline (horizonator_skyline_match*: where a photo was taken)
+    def skyline_samples(self, rel_az_deg, el_deg, az_width_deg):
+        """skyline_samples() for this context's W x H panoramas."""
+        return skyline_samples(rel_az_deg, el_deg, az_width_deg, self.width, self.height)
+
+    @staticmethod
+    def _samples(samples):
+        """SKYLINE_SAMPLE_DTYPE array, or a sequence of (dx, y) -> C-contiguous SKYLINE_SAMPLE_DTYPE array."""
+        a = np.asarray(samples)
+        if a.dtype == SKYLINE_SAMPLE_DTYPE:
+            return np.ascontiguousarray(a.ravel())
+        a = a.reshape(-1, 2)
+        out = np.empty(len(a), SKYLINE_SAMPLE_DTYPE)
+        out["dx"], out["y"] = a[:, 0], a[:, 1]
+        return out
+
+    def _skyline_call(self, views, samples, clip_rows, wrap, rows, rng, scores):
+        n, W = len(views), self.width
+        out = {k: _pool.array((n, W), dt) if want else None
+               for k, dt, want in (("rows", np.int32, rows), ("range", np.float32, rng), ("scores", np.float32, scores))}
+        s = self._samples(samples) if scores else None
+        addr = {k: (a.ctypes.data if a is not None and a.size else None) for k, a in out.items()}
+        _check(lib.horizonator_skyline_match, C.byref(self._ctx), n, self._views(views), addr["rows"], addr["range"],
+               len(s) if scores else 0, s.ctypes.data if scores and len(s) else None, float(clip_rows), bool(wrap),
+               addr["scores"])
+        return out
+
+    def skyline(self, views):
+        """views as render_batch takes them -> (rows (n, W) int32, range (n, W) float32): the topmost terrain pixel of
+        each column (image row, 0 = top) and its range, -1 / -1 for an all-sky column.  Only these leave the GPU."""
+        out = self._skyline_call(views, None, 1., False, True, True, False)
+        return out["rows"], out["range"]
+
+    def skyline_match(self, views, samples, clip_rows=8., wrap=True, rows=False):
+        """Scores (n, W) float32 of an observed skyline (samples: skyline_samples(), or (dx, y) pairs) against every
+        view at every heading column: the mean error in rows, each sample's clipped at clip_rows (horizonator-batch.h).
+        wrap: columns wrap around (full-circle windows).  rows=True: (scores, rows (n, W) int32)."""
+        out = self._skyline_call(views, samples, clip_rows, wrap, rows, False, True)
+        return (out["scores"], out["rows"]) if rows else out["scores"]
+
+    def skyline_match_device(self, views, d_samples, d_scores=0, d_rows=0, d_range=0, clip_rows=8., wrap=True, stream=0,
+                             m=None):
+        """Device-memory variant.  d_samples: an (m, 2) int32 CUDA tensor whose rows are (dx, y as float bits), an (m,)
+        int64 one, or an integer device address with `m` given; d_scores, d_rows, d_range: (n, W) float32 / int32 /
+        float32 CUDA tensors or integer addresses (0 = not written); stream as render_batch_device."""
+        if hasattr(d_samples, "data_ptr"):
+            if m is None:
+                m = d_samples.shape[0]
+            d_samples = d_samples.data_ptr()
+        if m is None:
+            m = 0
+        d_scores, d_rows, d_range = (a.data_ptr() if hasattr(a, "data_ptr") else a for a in (d_scores, d_rows, d_range))
+        _check(lib.horizonator_skyline_match_device, C.byref(self._ctx), len(views), self._views(views), d_rows or None,
+               d_range or None, int(m), d_samples or None, float(clip_rows), bool(wrap), d_scores or None, stream or None)
+
+    def locate(self, views, samples, top=10, clip_rows=8., wrap=True):
+        """Where and which way a photo was taken: the `top` best (view index, heading azimuth in degrees, score) of
+        skyline_match() over the candidate views and all their headings, best (smallest score) first; ties go to the
+        lower view index, then the lower heading column.  The heading of column h is az_deg0 + (h + 0.5) * p."""
+        scores = self.skyline_match(views, samples, clip_rows=clip_rows, wrap=wrap)
+        W = self.width
+        flat = scores.ravel()
+        order = np.argsort(flat, kind="stable")[:top]
+        out = []
+        for i in order:
+            k, h = divmod(int(i), W)
+            az0, az1 = float(np.float32(views[k][2])), float(np.float32(views[k][3]))
+            out.append((k, az0 + (h + 0.5) * (az1 - az0) / W, float(flat[i])))
+        return out
 
 
 class _PinnedBlock:

@@ -198,6 +198,41 @@ struct Scratch
     unsigned int last_epoch = 0;       // of the most recent render (horizonator_pick decodes main's keys with it)
 };
 
+// The stages of a render chain after its bands (launch_chain): k_resolve (images, range images), k_annotate (labels),
+// k_skyline (skylines) and k_skyline_score (their scores).  A captured chain is one combination.
+struct Stages
+{
+    bool resolve = false, annotate = false, skyline = false, score = false;
+    bool operator==(const Stages& o) const
+    {
+        return resolve == o.resolve && annotate == o.annotate && skyline == o.skyline && score == o.score;
+    }
+};
+
+// The per-chunk parameter block of a stage after the render chain (k_annotate's HzAnnotate, k_skyline's HzSkyline): a
+// pinned ring beside a set's h_views whose slot goes to one device address with them, so that a captured chain replays
+// for any inputs.  Made on first use.
+template<class T> struct StageBlock
+{
+    DevPtr<T>  d;
+    HostPtr<T> h;                      // pinned [PARAM_RING]
+    bool ensure(const char* d_what, const char* h_what)
+    {
+        if(d) return true;
+        DevPtr<T> dd = make_device<T>(1);
+        HostPtr<T> hh = make_host<T>(PARAM_RING);
+        if(empty_handle(dd, d_what) || empty_handle(hh, h_what)) return false;
+        d = std::move(dd); h = std::move(hh);
+        return true;
+    }
+    T* at(int slot) { return h.get() + slot; }
+    // the first `bytes` of the slot to the device, on st
+    cudaError_t upload(int slot, size_t bytes, cudaStream_t st)
+    {
+        return cudaMemcpyAsync(d.get(), at(slot), bytes, cudaMemcpyHostToDevice, st);
+    }
+};
+
 // Up to `cap` views that are rendered TOGETHER: one chain of kernel launches whose grids have a view dimension
 // (gridDim.y), each view with its own scratch.  The context's own view is a set of one; the batch calls use sets of
 // up to VIEWS_PER_SET, each with its own stream, so that the tail of one set's kernels overlaps another's.
@@ -226,16 +261,18 @@ struct ViewSet
     // the standard chain, captured on first use per (number of views, shape)
     // (several executable instances each, used in turn: an instance that is still in flight makes the next launch of
     // the SAME instance wait on the host)
-    // (variants: with k_resolve or without it -- labels only -- and with k_annotate after the chain or without it)
-    struct Graph { int m; bool big_per_band, resolve, annotate; std::vector<GraphExecHandle> exec; size_t next; int launches; };
+    // (variants: the stages after the bands, Stages)
+    struct Graph { int m; bool big_per_band; Stages stages; std::vector<GraphExecHandle> exec; size_t next; int launches; };
     std::vector<Graph> graphs;
     bool graph_failed = false;
-    // labels of points of interest (horizonator_annotate_batch*), made on first use: k_annotate's per-chunk block (a
-    // pinned ring beside h_views, copied with them to one device address, so that a captured chain replays for any
-    // POIs), and for the host-memory call the labels of one chunk, copied to the caller on the set's stream
-    DevPtr<HzAnnotate>  d_annot;
-    HostPtr<HzAnnotate> h_annot;       // pinned [PARAM_RING]
-    GrowBuffer<float4>  d_labels;
+    // the per-chunk blocks of labels of points of interest (horizonator_annotate_batch*) and of skylines
+    // (horizonator_skyline_match*)
+    StageBlock<HzAnnotate> annot;
+    StageBlock<HzSkyline>  skyline;
+    // made on first use: for the host-memory calls the labels or skylines of one chunk, copied to the caller on the set's
+    // stream; the skylines of one chunk that k_skyline_score reads
+    GrowBuffer<float4>  d_stage_out;
+    GrowBuffer<int16_t> d_sky;
 };
 
 struct Slot
@@ -295,8 +332,9 @@ struct Slot
     GrowBuffer<uint32_t> d_vs_counts;
     EventHandle          vs_done;
 
-    // labels (horizonator_annotate_batch): the POIs of the host-memory call, uploaded per call, made on first use
-    GrowBuffer<double>   d_pois;         // [POIs][3]
+    // the inputs of the host-memory calls (horizonator_annotate_batch: POIs, horizonator_skyline_match: samples),
+    // uploaded per call (upload_inputs), made on first use
+    GrowBuffer<double>   d_inputs;
 };
 
 // raw pointers: a slot is deleted by horizonator_deinit(), never by a destructor at exit, when the CUDA runtime may
@@ -558,8 +596,8 @@ bool big_after_every_band(const Slot& s, const ViewState& vs)
 }
 
 // the kernels of one render of m views, in order, reading their parameters from set.d_views; hv = the host copy of those
-bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool worst_case, bool resolve,
-                  bool annotate, cudaStream_t st, const EventHandle* ev, int* launches)
+bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool worst_case, const Stages& g,
+                  cudaStream_t st, const EventHandle* ev, int* launches)
 {
     const HzView* dv = set.d_views.get();
     int n = 0;
@@ -597,11 +635,13 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
     }
     if(ev) CUDA_TRY(cudaEventRecord(ev[5].get(), st));
     if(fork) CUDA_TRY(cudaStreamWaitEvent(st, set.ev_join.get(), 0));
-    if(resolve) { CUDA_TRY(hz_launch_resolve(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
+    if(g.resolve) { CUDA_TRY(hz_launch_resolve(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
     if(ev) CUDA_TRY(cudaEventRecord(ev[6].get(), st));
-    // the labels: after the join (the near pass's large triangles are in the visibility buffers), before the set's next
-    // chunk reuses those buffers (the same stream)
-    if(annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.d_annot.get(), m, st)); n++; }
+    // the labels and skylines: after the join (the near pass's large triangles are in the visibility buffers), before the
+    // set's next chunk reuses those buffers (the same stream)
+    if(g.annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.annot.d.get(), m, st)); n++; }
+    if(g.skyline) { CUDA_TRY(hz_launch_skyline(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.skyline.d.get(), m, st)); n++; }
+    if(g.score) { CUDA_TRY(hz_launch_skyline_score(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.skyline.d.get(), m, st)); n++; }
     *launches = n;
     return true;
 }
@@ -609,7 +649,7 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
 // Captures the standard chain (full width, vectorised resolve, grids sized for any eye position) for m views of the
 // set; every later standard render of m views is one cudaGraphLaunch after the parameter copy.  A dozen separate
 // launches cost more host time than the GPU needs for the render.
-ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, bool resolve, bool annotate)
+ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_band, const Stages& stages)
 {
     const StreamHandle cs = make_stream();
     if(!cs) { cudaGetLastError(); return nullptr; }
@@ -618,7 +658,7 @@ ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bo
     int launches = 0;
     if(ok)
     {
-        ok = launch_chain(s, set, hv, m, big_per_band, true, resolve, annotate, cs.get(), nullptr, &launches);
+        ok = launch_chain(s, set, hv, m, big_per_band, true, stages, cs.get(), nullptr, &launches);
         if(cudaStreamEndCapture(cs.get(), &captured) != cudaSuccess) ok = false;
     }
     const GraphHandle g(captured);
@@ -634,7 +674,7 @@ ViewSet::Graph* capture_graph(Slot& s, ViewSet& set, const HzView* hv, int m, bo
         MSG("CUDA graph capture of the render chain failed; launching the kernels one by one instead");
         return nullptr;
     }
-    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, resolve, annotate, std::move(exec), 0, launches });
+    set.graphs.push_back(ViewSet::Graph{ m, big_per_band, stages, std::move(exec), 0, launches });
     return &set.graphs.back();
 }
 
@@ -736,20 +776,18 @@ static_assert(sizeof(((HzAnnotate*)nullptr)->view) / sizeof(HzAnnotView) >= VIEW
 
 // Enqueues one render of columns [x0,x1) of m views (m <= what ensure_views() gave) on stream st: view k uses scratch
 // set.sc[k] and writes to outs[k] (device memory), and, with `ann`, the labels of the POIs for each view after the
-// render.  All views of one call must have the same kinds of output.
+// render, with `sky`, the chunk's skylines (and their scores) as that block says.  All views of one call must have the
+// same kinds of output.
 bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st,
-                   const AnnotSpec* ann = nullptr)
+                   const AnnotSpec* ann = nullptr, const HzSkyline* sky = nullptr)
 {
     if(s.W <= 0 || s.H <= 0 || m < 1 || m > (int)set.sc.size()) return false;
     const bool want_image = outs[0].image[0] != nullptr, want_ranges = outs[0].ranges[0] != nullptr;
-    const bool resolve = want_image || want_ranges, annotate = ann != nullptr;
-    if(annotate && !set.d_annot)
-    {
-        DevPtr<HzAnnotate> d = make_device<HzAnnotate>(1);
-        HostPtr<HzAnnotate> h = make_host<HzAnnotate>(PARAM_RING);
-        if(empty_handle(d, "cudaMalloc(annotate)") || empty_handle(h, "cudaMallocHost(annotate)")) return false;
-        set.d_annot = std::move(d); set.h_annot = std::move(h);
-    }
+    Stages stages;
+    stages.resolve = want_image || want_ranges; stages.annotate = ann != nullptr;
+    stages.skyline = sky != nullptr; stages.score = sky != nullptr && sky->scores != nullptr;
+    if(stages.annotate && !set.annot.ensure("cudaMalloc(annotate)", "cudaMallocHost(annotate)")) return false;
+    if(stages.skyline && !set.skyline.ensure("cudaMalloc(skyline)", "cudaMallocHost(skyline)")) return false;
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
     if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy.get(), 0));
 
@@ -814,9 +852,9 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
             vb.cell_diag2 = hk[0].cell_diag2 * (float)((1 << lod) * (1 << lod));
             lo = vb.ring_hi;
         }
-        // the row table of this view's window, unless the scratch still holds it from its previous render (the ranges and
-        // the labels' rendered ranges need it)
-        if((want_ranges || annotate) && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
+        // the row table of this view's window, unless the scratch still holds it from its previous render (the ranges, and
+        // the rendered ranges of the labels and skylines need it)
+        if((want_ranges || stages.annotate || stages.skyline) && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
         {
             float* h_row = set.h_tanel.get() + ((size_t)slot * set.cap + k) * s.H;
             memcpy(h_row, tanel_row(s, vs[k].az_deg0, vs[k].az_deg1), (size_t)s.H * sizeof(float));
@@ -825,26 +863,30 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         }
     }
     CUDA_TRY(cudaMemcpyAsync(set.d_views.get(), hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
-    if(annotate)
+    if(stages.annotate)
     {
-        HzAnnotate* ha = set.h_annot.get() + slot;
+        HzAnnotate* ha = set.annot.at(slot);
         ha->pois = ann->pois; ha->labels = ann->labels; ha->m = ann->m; ha->pad = 0;
         for(int k = 0; k < m; k++) ha->view[k] = ann->views[k];
-        CUDA_TRY(cudaMemcpyAsync(set.d_annot.get(), ha, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView),
-                                 cudaMemcpyHostToDevice, st));
+        CUDA_TRY(set.annot.upload(slot, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView), st));
+    }
+    if(stages.skyline)
+    {
+        *set.skyline.at(slot) = *sky;
+        CUDA_TRY(set.skyline.upload(slot, sizeof(HzSkyline), st));
     }
     CUDA_TRY(cudaEventRecord(set.ring_ev[slot].get(), st));
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
     const bool is_main = (&set == &s.main);
-    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (resolve || annotate) &&
-                          outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && (vectorisable || !resolve);
+    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (stages.resolve || stages.annotate || stages.skyline) &&
+                          outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && (vectorisable || !stages.resolve);
     if(standard && !set.graph_failed)
     {
         ViewSet::Graph* g = nullptr;
         for(ViewSet::Graph& c : set.graphs)
-            if(c.m == m && c.big_per_band == big_per_band && c.resolve == resolve && c.annotate == annotate) g = &c;
-        if(g == nullptr && (g = capture_graph(s, set, hv, m, big_per_band, resolve, annotate)) == nullptr) set.graph_failed = true;
+            if(c.m == m && c.big_per_band == big_per_band && c.stages == stages) g = &c;
+        if(g == nullptr && (g = capture_graph(s, set, hv, m, big_per_band, stages)) == nullptr) set.graph_failed = true;
         if(g != nullptr)
         {
             CUDA_TRY(cudaGraphLaunch(g->exec[g->next].get(), st));
@@ -870,7 +912,7 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     }
     int launches = 0;
     // grids sized for this view's eye tile only when there is just one view
-    if(!launch_chain(s, set, hv, m, big_per_band, m > 1, resolve, annotate, st, ev, &launches)) return false;
+    if(!launch_chain(s, set, hv, m, big_per_band, m > 1, stages, st, ev, &launches)) return false;
     CUDA_TRY(cudaEventRecord(set.busy.get(), st)); set.last_stream = st; set.busy_recorded = true;
     s.launches_last = launches;
     if(is_main) s.have_render = (x0 == 0 && x1 == s.W);
@@ -1396,9 +1438,23 @@ struct AnnotReq
     int m;
     float4* labels;              // [n][m]: device memory, or host memory when to_host
 };
+// sky: the skylines of every view (horizonator_skyline_match*), by k_skyline after each chunk's chain, and their scores
+// against the samples by k_skyline_score; into device memory, or (to_host) through the set's output scratch and copies
+// on its stream.
+struct SkyReq
+{
+    int*   rows;                 // [n][W] each, or null: device memory, or host memory when to_host
+    float* range;
+    float* scores;
+    const HzSkySample* d_samples;
+    int   m;
+    float clip;
+    bool  wrap;
+};
 
 static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
-                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const AnnotReq* ann = nullptr)
+                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const AnnotReq* ann = nullptr,
+                                const SkyReq* sky = nullptr)
 {
     const size_t px = (size_t)s->W * s->H;
     std::vector<ViewState> vs((size_t)n);
@@ -1450,15 +1506,27 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     if(!forked) { sets.push_back(&s->main); chunk = 1; }
     auto stream_of = [st](const ViewSet& set) { return set.stream ? set.stream.get() : st; };
 
-    // each set's label scratch for a chunk (host-memory call only; those are synchronous, so nothing queued still uses
-    // the old buffer once the set's stream is idle)
+    // each set's scratch for a chunk: the labels or the skylines of the host-memory calls (rows, range and scores, W * chunk
+    // words each, one after the other), the skylines the scorer reads.  Nothing queued still uses an old buffer once the
+    // set's stream is idle.
+    const size_t W = (size_t)s->W, sky_words = (size_t)chunk * W;
+    const size_t stage_out = !to_host ? 0 : ann ? (size_t)chunk * m_poi : sky ? (3 * sky_words + 3) / 4 : 0;
+    const size_t sky_rows = sky && sky->scores ? sky_words : 0;
     for(ViewSet* set : sets)
-        if(ann && to_host && set->d_labels.cap < (size_t)chunk * m_poi)
+    {
+        if(set->d_stage_out.cap < stage_out || set->d_sky.cap < sky_rows) CUDA_TRY(cudaStreamSynchronize(stream_of(*set)));
+        cudaError_t e = cudaSuccess;
+        if(set->d_stage_out.cap < stage_out && (e = set->d_stage_out.grow(stage_out)) != cudaSuccess)
         {
-            CUDA_TRY(cudaStreamSynchronize(stream_of(*set)));
-            const cudaError_t e = set->d_labels.grow((size_t)chunk * m_poi);
-            if(e != cudaSuccess) { MSG("CUDA error: cudaMalloc(labels) failed: %s", cudaGetErrorString(e)); return false; }
+            MSG("CUDA error: cudaMalloc(%s) failed: %s", ann ? "labels" : "skylines", cudaGetErrorString(e));
+            return false;
         }
+        if(set->d_sky.cap < sky_rows && (e = set->d_sky.grow(sky_rows)) != cudaSuccess)
+        {
+            MSG("CUDA error: cudaMalloc(skyline scratch) failed: %s", cudaGetErrorString(e));
+            return false;
+        }
+    }
     if(forked)
     {
         CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
@@ -1472,8 +1540,19 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
             outs[k] = single_out(images ? (to_host ? set.sc[k].d_image.get()  : images + (size_t)(k0 + k) * px * 3) : nullptr,
                                  ranges ? (to_host ? set.sc[k].d_ranges.get() : ranges + (size_t)(k0 + k) * px)     : nullptr);
         AnnotSpec a{};
-        if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? set.d_labels.get() : ann->labels + (size_t)k0 * m_poi, &av[k0] };
-        if(!enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), sst, ann ? &a : nullptr)) return false;
+        if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? set.d_stage_out.get() : ann->labels + (size_t)k0 * m_poi, &av[k0] };
+        HzSkyline k{};
+        const size_t at = (size_t)k0 * W;
+        if(sky)
+        {
+            float* const stage = (float*)set.d_stage_out.get();
+            k.rows   = !sky->rows   ? nullptr : to_host ? (int*)stage           : sky->rows + at;
+            k.range  = !sky->range  ? nullptr : to_host ? stage + sky_words     : sky->range + at;
+            k.scores = !sky->scores ? nullptr : to_host ? stage + 2 * sky_words : sky->scores + at;
+            k.sky = sky->scores ? set.d_sky.get() : nullptr;
+            k.samples = sky->d_samples; k.m = sky->m; k.clip = sky->clip; k.wrap = sky->wrap;
+        }
+        if(!enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), sst, ann ? &a : nullptr, sky ? &k : nullptr)) return false;
         for(int k = 0; k < m && to_host; k++)
         {
             if(images) CUDA_TRY(cudaMemcpyAsync(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3,
@@ -1484,6 +1563,10 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         if(ann && to_host)
             CUDA_TRY(cudaMemcpyAsync(ann->labels + (size_t)k0 * m_poi, a.labels, (size_t)m * m_poi * sizeof(float4),
                                      cudaMemcpyDeviceToHost, sst));
+        const size_t sky_bytes = (size_t)m * W * 4;
+        if(sky && to_host && k.rows)   CUDA_TRY(cudaMemcpyAsync(sky->rows + at, k.rows, sky_bytes, cudaMemcpyDeviceToHost, sst));
+        if(sky && to_host && k.range)  CUDA_TRY(cudaMemcpyAsync(sky->range + at, k.range, sky_bytes, cudaMemcpyDeviceToHost, sst));
+        if(sky && to_host && k.scores) CUDA_TRY(cudaMemcpyAsync(sky->scores + at, k.scores, sky_bytes, cudaMemcpyDeviceToHost, sst));
         return true;
     };
     bool ok = true;
@@ -1638,6 +1721,21 @@ bool horizonator_render_batch(const horizonator_context_t* ctx, int n, const hor
     });
 }
 
+// The inputs of a host-memory call (POIs, skyline samples) go up once per call into the context's scratch, s.d_inputs
+// (the calls are synchronous: no earlier one still reads it).
+static bool upload_inputs(Slot& s, cudaStream_t st, const void* src, size_t bytes, const char* what)
+{
+    const size_t words = (bytes + sizeof(double) - 1) / sizeof(double);
+    if(s.d_inputs.cap < words)
+    {
+        CUDA_TRY(cudaStreamSynchronize(st));
+        const cudaError_t e = s.d_inputs.grow(words);
+        if(e != cudaSuccess) { MSG("CUDA error: cudaMalloc(%s) failed: %s", what, cudaGetErrorString(e)); return false; }
+    }
+    CUDA_TRY(cudaMemcpyAsync(s.d_inputs.get(), src, bytes, cudaMemcpyHostToDevice, st));
+    return true;
+}
+
 // ---- labels of points of interest (horizonator-batch.h) ----------------------------------------------------------
 
 // the argument rules of both annotate calls; false: nothing may be done
@@ -1674,16 +1772,86 @@ bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const h
     if(s == nullptr || !annotate_args_ok("horizonator_annotate_batch", n, views, m, pois, labels)) return false;
     if(n == 0 || m == 0) return true;
     return on_stream(*s, nullptr, [&](cudaStream_t st) {
-        // the POIs go up once per call into the context's scratch (the call is synchronous: no earlier one still reads it)
-        if(s->d_pois.cap < 3 * (size_t)m)
-        {
-            CUDA_TRY(cudaStreamSynchronize(st));
-            const cudaError_t e = s->d_pois.grow(3 * (size_t)m);
-            if(e != cudaSuccess) { MSG("CUDA error: cudaMalloc(POIs) failed: %s", cudaGetErrorString(e)); return false; }
-        }
-        CUDA_TRY(cudaMemcpyAsync(s->d_pois.get(), pois, (size_t)m * sizeof(horizonator_poi_t), cudaMemcpyHostToDevice, st));
-        const AnnotReq ann{ s->d_pois.get(), m, (float4*)labels };
+        if(!upload_inputs(*s, st, pois, (size_t)m * sizeof(horizonator_poi_t), "POIs")) return false;
+        const AnnotReq ann{ s->d_inputs.get(), m, (float4*)labels };
         if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &ann))
+        {
+            cudaStreamSynchronize(st);
+            cudaGetLastError();
+            return false;
+        }
+        return true;
+    });
+}
+
+// ---- skylines and their match against an observed skyline (horizonator-batch.h) ---------------------------------
+
+static_assert(sizeof(HzSkySample) == sizeof(horizonator_skyline_sample_t) && offsetof(horizonator_skyline_sample_t, y) == 4,
+              "HzSkySample: horizonator_skyline_sample_t");
+
+// the argument rules of both skyline calls; false: nothing may be done
+static bool skyline_args_ok(const char* fn, const Slot& s, int n, const horizonator_view_t* views, const void* rows,
+                            const void* range, int m, const void* samples, float clip_rows, const void* scores)
+{
+    if(n < 0) { MSG("%s: negative count n = %d", fn, n); return false; }
+    if(n == 0) return true;
+    if(views == nullptr) { MSG("%s: views are required", fn); return false; }
+    if(rows == nullptr && range == nullptr && scores == nullptr) { MSG("%s: neither rows, range nor scores asked for", fn); return false; }
+    if(scores == nullptr) return true;
+    if(m < 1 || samples == nullptr || !(std::isfinite(clip_rows) && clip_rows > 0.f))
+    {
+        MSG("%s: scores need m >= 1 samples and a finite clip_rows > 0 (m = %d, clip_rows = %g)", fn, m, (double)clip_rows);
+        return false;
+    }
+    if(s.H > 32767) { MSG("%s: scores need an image at most 32767 rows high (H = %d)", fn, s.H); return false; }
+    return true;
+}
+
+// the scorer's shared memory for the context's width, on the current device, before anything is queued
+static bool skyline_score_ready(const char* fn, const Slot& s)
+{
+    const cudaError_t e = hz_skyline_score_setup(s.W);
+    if(e == cudaSuccess) return true;
+    cudaGetLastError();
+    MSG("%s: scores of a panorama %d columns wide do not fit the scorer's shared memory: %s", fn, s.W, cudaGetErrorString(e));
+    return false;
+}
+
+bool horizonator_skyline_match_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                      int* d_rows, float* d_range,
+                                      int m, const horizonator_skyline_sample_t* d_samples,
+                                      float clip_rows, bool wrap, float* d_scores, void* stream)
+{
+    static const char* fn = "horizonator_skyline_match_device";
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !skyline_args_ok(fn, *s, n, views, d_rows, d_range, m, d_samples, clip_rows, d_scores)) return false;
+    if(n == 0) return true;
+    if((((uintptr_t)d_rows | (uintptr_t)d_range | (uintptr_t)d_scores) & 3) != 0 || (d_scores && ((uintptr_t)d_samples & 7) != 0))
+    {
+        MSG("%s: d_rows, d_range and d_scores must be 4-byte and d_samples 8-byte aligned", fn);
+        return false;
+    }
+    const SkyReq sky{ d_rows, d_range, d_scores, (const HzSkySample*)d_samples, m, clip_rows, wrap };
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        if(d_scores && !skyline_score_ready(fn, *s)) return false;
+        return render_batch_common(ctx, s, n, views, nullptr, nullptr, false, st, nullptr, &sky);
+    });
+}
+
+bool horizonator_skyline_match(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                               int* rows, float* range,
+                               int m, const horizonator_skyline_sample_t* samples,
+                               float clip_rows, bool wrap, float* scores)
+{
+    static const char* fn = "horizonator_skyline_match";
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !skyline_args_ok(fn, *s, n, views, rows, range, m, samples, clip_rows, scores)) return false;
+    if(n == 0) return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        if(scores && !(skyline_score_ready(fn, *s) && upload_inputs(*s, st, samples, (size_t)m * sizeof(HzSkySample), "samples")))
+            return false;
+        const SkyReq sky{ rows, range, scores, (const HzSkySample*)s->d_inputs.get(), m, clip_rows, wrap };
+        if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, nullptr, &sky))
         {
             cudaStreamSynchronize(st);
             cudaGetLastError();

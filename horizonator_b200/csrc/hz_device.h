@@ -222,6 +222,31 @@ struct HzAnnotate
 };
 // after the render chain of a chunk (its visibility buffers and tan(elevation) rows), on the same stream
 cudaError_t hz_launch_annotate(const HzView& v, const HzView* d_v, const HzAnnotate* d_a, int nviews, cudaStream_t stream);
+// ---- skylines and their match against an observed one (horizonator_skyline_match*: the rule is in
+// include/horizonator-batch.h) ------------------------------------------------------------------------------------
+struct alignas(8) HzSkySample { int32_t dx; float y; };    // horizonator_skyline_sample_t
+// The per-chunk block, copied to the device with the HzView variants like HzAnnotate.  View k of the chunk writes
+// column c to rows / range / scores [k * W + c]; any of them may be null.  sky: the chunk's skylines for k_skyline_score
+// ([views][W] image rows, -1 = all sky), null when no scores are asked for.
+struct HzSkyline
+{
+    int*               rows;
+    float*             range;
+    float*             scores;
+    int16_t*           sky;
+    const HzSkySample* samples;   // [m]
+    int                m;
+    float              clip;      // clip_rows
+    int                wrap;
+    int                pad;
+};
+// after the render chain of a chunk, in place of k_resolve: the topmost terrain pixel of every column
+cudaError_t hz_launch_skyline(const HzView& v, const HzView* d_v, const HzSkyline* d_s, int nviews, cudaStream_t stream);
+// after hz_launch_skyline: scores[k * W + h] for every heading column h
+cudaError_t hz_launch_skyline_score(const HzView& v, const HzView* d_v, const HzSkyline* d_s, int nviews, cudaStream_t stream);
+// Lets k_skyline_score stage W skyline rows in shared memory on the current device; an error if W is too wide for that
+// (beyond about 110 000 columns).  Called before any scores are queued, outside graph capture.
+cudaError_t hz_skyline_score_setup(int W);
 // ---- viewsheds (horizonator_viewshed*: the definition is in include/horizonator-batch.h) ------
 constexpr int HZ_VS_MAX_VIEWS = 64;     // views per k_viewshed launch (gridDim.y); their eyes travel in the parameters
 struct HzViewshedEye { float vci, vcj, vz, cos_lat; };     // compute_move()'s eye, float as there

@@ -22,6 +22,8 @@
 //   k_horizon  (extra)   range image -> per-column topmost terrain row and its range
 //   k_annotate (labels)  points of interest -> marker position and the matched rendered range, read from the
 //                        visibility buffers of the views just rendered                     annotator.c:280-348
+//   k_skyline, k_skyline_score (skylines)  the topmost terrain pixel of every column, read from the visibility buffers;
+//                        the match of those skylines against an observed one at every heading
 //   k_viewshed, k_viewshed_count (viewsheds)  R2 ray casting over the DEM square, one thread per ray -> bit masks;
 //                        masks -> per-vertex counts of the views that see it
 //
@@ -80,15 +82,22 @@ static unsigned int hz_grid(const HzView& v, unsigned int ctas_per_sm, int nview
 }
 
 template <typename... KArgs, typename... Args>
-static cudaError_t hz_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args&&... args)
+static cudaError_t hz_launch_smem(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                                  Args&&... args)
 {
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = stream;
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+template <typename... KArgs, typename... Args>
+static cudaError_t hz_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args&&... args)
+{
+    return hz_launch_smem(kernel, grid, block, 0, stream, static_cast<Args&&>(args)...);
 }
 
 // ================================================================================================
@@ -2185,6 +2194,125 @@ cudaError_t hz_launch_annotate(const HzView& v, const HzView* d_v, const HzAnnot
 {
     (void)v;
     return hz_launch(k_annotate, dim3(HZ_ANNOT_CTAS, (unsigned)nviews), dim3(HZ_CTA_THREADS), stream, d_v, d_a);
+}
+
+// ================================================================================================
+// k_skyline, k_skyline_score: the skyline of each view read straight from its visibility buffer, and its match against
+// an observed skyline at every heading (include/horizonator-batch.h states the rule)
+// ================================================================================================
+
+// One thread per (view, column), gridDim.y = view of the chunk; a warp takes 32 adjacent columns, so that the key reads
+// of a row are coalesced.  The column is walked from GL row H-1 (the top image row) downwards; 8-row groups whose 8x8
+// block was not drawn into this render (touched flag of the span grid) are skipped as k_resolve4 skips them -- most of a
+// panorama is sky.  A pixel is terrain where k_horizon would find it so in the range image: its range, converted by
+// hz_range_of_q() as k_resolve converts it, is > 0.  Register budget: launch_bounds(256) alone; it needs few.
+__global__ void __launch_bounds__(HZ_CTA_THREADS)
+k_skyline(const HzView* __restrict__ V, const HzSkyline* __restrict__ S)
+{
+    HZ_KERNEL_PROLOGUE(V, P);
+    const int W = P.W, H = P.H;
+    const int c = blockIdx.x * HZ_CTA_THREADS + threadIdx.x;
+    if(c >= W) return;
+    const unsigned int ep = P.epoch;
+    const float znear = P.znear, zfar = P.zfar;
+    const unsigned long long* const col = P.vis + c;
+    const uint8_t* const flags = P.hiz_flags + c / HZ_SPAN_KEYS;
+    const unsigned int spans = hz_spans((unsigned int)W);
+    int row = -1;
+    float range = -1.0f;
+    for(int g = (H - 1) / HZ_SPAN_KEYS; g >= 0 && row < 0; g--)
+    {
+        if(!(__ldg(flags + (size_t)g * spans) & HZ_FLAG_TOUCHED)) continue;
+        const int top = min(H - 1, g * HZ_SPAN_KEYS + HZ_SPAN_KEYS - 1);
+        for(int gl = top; gl >= g * HZ_SPAN_KEYS; gl--)
+        {
+            const unsigned int q = hz_key_q(__ldcs(col + (size_t)gl * (size_t)W), ep);
+            if(q == HZ_Q_MAX) continue;
+            const float r = hz_range_of_q(q, __ldg(P.tanel + gl), znear, zfar);
+            if(r > 0.0f) { row = H - 1 - gl; range = r; break; }
+        }
+    }
+    const size_t o = (size_t)blockIdx.y * (size_t)W + (size_t)c;
+    const HzSkyline& s = *S;
+    if(s.rows)   s.rows[o] = row;
+    if(s.range)  s.range[o] = range;
+    if(s.sky)    s.sky[o] = (int16_t)row;
+}
+
+cudaError_t hz_launch_skyline(const HzView& v, const HzView* d_v, const HzSkyline* d_s, int nviews, cudaStream_t stream)
+{
+    const unsigned int parts = (unsigned int)((v.W + HZ_CTA_THREADS - 1) / HZ_CTA_THREADS);
+    return hz_launch(k_skyline, dim3(parts, (unsigned)nviews), dim3(HZ_CTA_THREADS), stream, d_v, d_s);
+}
+
+#define HZ_SKY_TILE 512             /* samples staged in shared memory per round */
+
+// One thread per (view, heading column h), grid (ceil(W / 256), views).  The CTA stages its view's W skyline rows in
+// shared memory (dynamic, 2 W bytes: 72 KB at W = 36 000), then the samples in tiles of HZ_SKY_TILE, each reduced once
+// per CTA to a column offset in [0, W) (wrap) or clamped to [-W, W] (no wrap: every offset beyond is missing from every
+// heading alike).  Each thread then adds the samples' errors in sample order, so the fp32 sum is the rule's.  Consecutive
+// threads read consecutive skyline entries and the same sample (a broadcast): no bank conflicts.  Register budget:
+// 8 CTAs of 256 threads per SM, 32 registers (ptxas -v: no spills).
+__global__ void __launch_bounds__(HZ_CTA_THREADS, 8)
+k_skyline_score(const HzView* __restrict__ V, const HzSkyline* __restrict__ S)
+{
+    HZ_KERNEL_PROLOGUE(V, P);
+    extern __shared__ int16_t s_sky[];                  // [W]
+    __shared__ int2 s_smp[HZ_SKY_TILE];                 // (column offset, y as bits)
+    const int W = P.W, m = S->m;
+    const float clip = S->clip;
+    const bool wrap = S->wrap != 0;
+    const HzSkySample* const samples = S->samples;
+    const int16_t* const sky = S->sky + (size_t)blockIdx.y * (size_t)W;
+    for(int c = threadIdx.x; c < W; c += HZ_CTA_THREADS) s_sky[c] = sky[c];
+    const int h = blockIdx.x * HZ_CTA_THREADS + threadIdx.x;
+    float sum = 0.0f;
+    for(int i0 = 0; i0 < m; i0 += HZ_SKY_TILE)
+    {
+        const int nt = min(HZ_SKY_TILE, m - i0);
+        __syncthreads();                                // the previous tile is used up (first round: nothing)
+        for(int i = threadIdx.x; i < nt; i += HZ_CTA_THREADS)
+        {
+            const HzSkySample t = samples[i0 + i];
+            const int dx = wrap ? ((t.dx % W) + W) % W : max(-W, min(W, t.dx));
+            s_smp[i] = make_int2(dx, __float_as_int(t.y));
+        }
+        __syncthreads();                                // (first round: the skyline rows too)
+        if(h < W)
+            for(int i = 0; i < nt; i++)
+            {
+                const int2 t = s_smp[i];
+                int c = h + t.x;
+                if(wrap && c >= W) c -= W;
+                const int s = (c >= 0 && c < W) ? (int)s_sky[c] : -1;
+                const float d = s < 0 ? clip : fminf(fabsf(((float)s - 0.5f) - __int_as_float(t.y)), clip);
+                sum = sum + d;
+            }
+    }
+    if(h < W) S->scores[(size_t)blockIdx.y * (size_t)W + (size_t)h] = sum / (float)m;
+}
+
+static size_t hz_skyline_score_smem(int W) { return (size_t)W * sizeof(int16_t); }
+
+cudaError_t hz_skyline_score_setup(int W)
+{
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    cudaError_t e;
+    if((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    if((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+    if((e = cudaFuncGetAttributes(&fa, k_skyline_score)) != cudaSuccess) return e;
+    const size_t bytes = hz_skyline_score_smem(W);
+    if(W <= 0 || bytes + fa.sharedSizeBytes > (size_t)optin) return cudaErrorInvalidValue;
+    if((int)bytes <= fa.maxDynamicSharedSizeBytes) return cudaSuccess;
+    return cudaFuncSetAttribute(k_skyline_score, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
+cudaError_t hz_launch_skyline_score(const HzView& v, const HzView* d_v, const HzSkyline* d_s, int nviews, cudaStream_t stream)
+{
+    const unsigned int parts = (unsigned int)((v.W + HZ_CTA_THREADS - 1) / HZ_CTA_THREADS);
+    return hz_launch_smem(k_skyline_score, dim3(parts, (unsigned)nviews), dim3(HZ_CTA_THREADS), hz_skyline_score_smem(v.W),
+                          stream, d_v, d_s);
 }
 
 // ================================================================================================

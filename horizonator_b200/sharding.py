@@ -8,7 +8,8 @@ collective on the data path of a render:
   rank loads for itself.  Viewpoints are block-partitioned; outputs stay sharded on the rank that made them.
   Only reduced products (horizon profiles, a few bytes per image column) are gathered.  Viewsheds partition the same
   way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).  Labels of
-  points of interest too: 16 bytes per (view, POI) are gathered (annotate_sharded).
+  points of interest too: 16 bytes per (view, POI) are gathered (annotate_sharded), and the scores of an observed
+  skyline, 4 bytes per (view, heading column) (skyline_match_sharded).
 * azimuth wedges  -- one giant panorama: rank g renders columns [edges[g], edges[g+1]), bit-identical to the same
   columns of an unsharded render.  PeerPanorama fuses the exchange into the renderer: each rank's resolve kernel
   stores its wedge straight into every rank's full panorama over NVLink (peer memory), a barrier is the only
@@ -17,6 +18,7 @@ collective on the data path of a render:
 Everything here except the two render_* drivers is device-agnostic tensor code, so the world_size-2 gloo tests
 exercise exactly what runs over NCCL.
 """
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -349,3 +351,19 @@ def annotate_sharded(h, views, pois, group=None):
     if hi > lo and p.shape[0] > 0:
         h.annotate_device(views[lo:hi], p, labels, stream=torch.cuda.current_stream().cuda_stream)
     return gather_blocks(labels, len(views), group)
+
+
+def skyline_match_sharded(h, views, samples, group=None, clip_rows=8., wrap=True):
+    """Scores of an observed skyline against a viewpoint batch over the ranks: `views` block-partitioned, this rank's
+    share scored on its own GPU without writing any panorama (horizonator_skyline_match_device), and the scores
+    gathered.  samples: as h.skyline_match() takes them.  Returns the (n, W) float32 CUDA tensor of all views' scores on
+    every rank.  All ranks must hold contexts of the same DEM square and size."""
+    world, rank = _world(group)
+    lo, hi = block_partition(len(views), world, rank)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    s = torch.as_tensor(h._samples(samples).view(np.int32).reshape(-1, 2), device=dev)
+    scores = torch.empty((hi - lo, h.width), dtype=torch.float32, device=dev)
+    if hi > lo:
+        h.skyline_match_device(views[lo:hi], s, scores, clip_rows=clip_rows, wrap=wrap,
+                               stream=torch.cuda.current_stream().cuda_stream)
+    return gather_blocks(scores, len(views), group)

@@ -244,6 +244,50 @@ bool horizonator_annotate_batch_device(const horizonator_context_t* ctx,
 bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
                                 int m, const horizonator_poi_t* pois, horizonator_label_t* labels);
 
+/* Skylines, and their match against an observed skyline: for each of n views, the topmost terrain pixel of every
+ * column, and how well the skyline traced from a photo fits that view at every heading -- the search for where a photo
+ * was taken and which way it looks, over batches of candidate eyes, on the GPU.
+ *
+ * Render: each view is rendered exactly as horizonator_render_batch_device() renders it (the same chunks, captured
+ * graphs, the context's z extents and size, and the same opt-in modes: earth curvature, seam wrap, level of detail);
+ * terrain beyond zfar is sky, as in the image.  No image and no range image is written.
+ * Rows and range: rows[k * W + c] is the image row (0 = top) of the topmost terrain pixel of column c of view k, or -1
+ * if the column is all sky; range[k * W + c] is that pixel's range, or -1.  Both are bit-identical to
+ * horizonator_horizon_profile_device() applied to the range image of the same render.
+ * Samples: a sample (dx, y) says that dx columns right of the heading column the observed skyline lies at pixel
+ * coordinate y (pixel centres at integer y, 0 = top: the y of horizonator_project()).  From angles: with
+ * p = (az_deg1 - az_deg0) / W degrees per column, a skyline point rel_az_deg right of the heading and el_deg above the
+ * horizontal is dx = rint(rel_az_deg / p), y = (H - 1) / 2 - el_deg / p, evaluated in double and rounded to float once
+ * -- horizonator_project()'s y at the same angle, since x and y share one angular scale.
+ * Score, for view k and every heading column h in [0, W), whose heading is the azimuth of its centre,
+ * az_deg0 + (h + 0.5) * p:
+ *   - c_i = h + dx_i; with `wrap` taken modulo W (non-negative; meant for full-circle windows), without it a c_i
+ *     outside [0, W) is missing;
+ *   - d_i = fminf(fabsf(((float)s - 0.5f) - y_i), clip_rows) with s = rows[k][c_i] (the rendered skyline's edge lies
+ *     half a row above its topmost terrain pixel); an all-sky (s = -1) or missing column gives d_i = clip_rows;
+ *   - scores[k * W + h] = (d_0 + d_1 + ... + d_{m-1}) / (float)m, the fp32 sum in that order, every operation rounded
+ *     once: the scores are reproducible exactly.  0 is a perfect fit; clip_rows is the worst.
+ * Arguments: views in host memory; any of rows, range and scores may be NULL, not all three; scores need m >= 1, the
+ * samples and a finite clip_rows > 0, and an image at most 32767 rows high and (shared memory) about 110 000 columns
+ * wide; without scores m, samples, clip_rows and wrap are ignored.  n == 0: nothing is done, true.  Bad arguments:
+ * false, nothing is written.  Each output takes n * W * 4 bytes.
+ */
+typedef struct { int32_t dx; float y; } horizonator_skyline_sample_t;     /* 8 bytes */
+
+/* d_rows, d_range, d_scores (4-byte aligned) and d_samples (8-byte aligned): DEVICE memory.  Stream as for the batch
+ * render. */
+bool horizonator_skyline_match_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                      int* d_rows, float* d_range,
+                                      int m, const horizonator_skyline_sample_t* d_samples,
+                                      float clip_rows, bool wrap, float* d_scores, void* stream);
+
+/* Same with everything in HOST memory, synchronous; only the n * W * (4 to 12) bytes asked for cross the bus (into
+ * page-locked memory by DMA; see horizonator_host_alloc()). */
+bool horizonator_skyline_match(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                               int* rows, float* range,
+                               int m, const horizonator_skyline_sample_t* samples,
+                               float clip_rows, bool wrap, float* scores);
+
 /* Per-kernel device times.  While enabled, every render records CUDA events around each of
  * its kernels on the stream it runs on.  horizonator_profile_read() waits for them and reports
  * the MEAN duration in milliseconds per render of: out_ms[0] k_prepare (clear + axis tables),
