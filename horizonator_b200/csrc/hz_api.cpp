@@ -209,29 +209,14 @@ struct Stages
     }
 };
 
-// The per-chunk parameter block of a stage after the render chain (k_annotate's HzAnnotate, k_skyline's HzSkyline): a
-// pinned ring beside a set's h_views whose slot goes to one device address with them, so that a captured chain replays
-// for any inputs.  Made on first use.
-template<class T> struct StageBlock
+// The per-chunk parameters of the stages after the bands: k_skyline's and k_skyline_score's HzSkyline, k_annotate's
+// HzAnnotate.  A chunk uploads only the parts its stages read (enqueue_views).
+struct ChunkBlock
 {
-    DevPtr<T>  d;
-    HostPtr<T> h;                      // pinned [PARAM_RING]
-    bool ensure(const char* d_what, const char* h_what)
-    {
-        if(d) return true;
-        DevPtr<T> dd = make_device<T>(1);
-        HostPtr<T> hh = make_host<T>(PARAM_RING);
-        if(empty_handle(dd, d_what) || empty_handle(hh, h_what)) return false;
-        d = std::move(dd); h = std::move(hh);
-        return true;
-    }
-    T* at(int slot) { return h.get() + slot; }
-    // the first `bytes` of the slot to the device, on st
-    cudaError_t upload(int slot, size_t bytes, cudaStream_t st)
-    {
-        return cudaMemcpyAsync(d.get(), at(slot), bytes, cudaMemcpyHostToDevice, st);
-    }
+    HzSkyline  sky;
+    HzAnnotate annot;
 };
+static_assert(sizeof(((HzAnnotate*)nullptr)->view) / sizeof(HzAnnotView) >= VIEWS_PER_SET, "HzAnnotate: a view set's views");
 
 // Up to `cap` views that are rendered TOGETHER: one chain of kernel launches whose grids have a view dimension
 // (gridDim.y), each view with its own scratch.  The context's own view is a set of one; the batch calls use sets of
@@ -248,6 +233,10 @@ struct ViewSet
     // copies it over (the ring lets several renders be queued without waiting)
     DevPtr<HzView>  d_views;           // [cap][HZ_V_COUNT]
     HostPtr<HzView> h_views;           // pinned [PARAM_RING][cap][HZ_V_COUNT]
+    // the stages' parameters go the same way, in the same slot; d_chunk keeps its address while the set lives (captured
+    // chains hold it)
+    DevPtr<ChunkBlock>  d_chunk;
+    HostPtr<ChunkBlock> h_chunk;       // pinned [PARAM_RING]
     HostPtr<float>  h_tanel;           // pinned [PARAM_RING][cap][H] (alloc_set_target)
     EventHandle ring_ev[PARAM_RING];
     int ring_next = 0;
@@ -265,14 +254,10 @@ struct ViewSet
     struct Graph { int m; bool big_per_band; Stages stages; std::vector<GraphExecHandle> exec; size_t next; int launches; };
     std::vector<Graph> graphs;
     bool graph_failed = false;
-    // the per-chunk blocks of labels of points of interest (horizonator_annotate_batch*) and of skylines
-    // (horizonator_skyline_match*)
-    StageBlock<HzAnnotate> annot;
-    StageBlock<HzSkyline>  skyline;
-    // made on first use: for the host-memory calls the labels or skylines of one chunk, copied to the caller on the set's
-    // stream; the skylines of one chunk that k_skyline_score reads
-    GrowBuffer<float4>  d_stage_out;
-    GrowBuffer<int16_t> d_sky;
+    // grown on demand: the outputs of one chunk's stages that do not go straight to the caller's device memory
+    // (render_batch_common's output plan) -- those of the host-memory calls, copied to the caller on the set's stream,
+    // and the skylines k_skyline_score reads
+    GrowBuffer<float4> d_stage;
 };
 
 struct Slot
@@ -365,12 +350,17 @@ struct DeviceGuard
 // The frame of an entry point that queues work for a context, once it has found the context's slot and checked its
 // arguments.  body(st) runs with the context's device current and queues the call's work on st: the caller's `stream`,
 // or, where that is null, the context's own, and the call then returns once that stream is idle (horizonator-batch.h).
-// The calls into host memory are of the second kind.
+// The calls into host memory are of the second kind; when such a call fails it still waits, so that nothing it queued
+// writes into the caller's memory after it has returned, and clears the error.
 template<class F> bool on_stream(const Slot& s, void* stream, F&& body)
 {
     DeviceGuard g(s.device);
     const cudaStream_t st = stream ? (cudaStream_t)stream : s.stream.get();
-    if(!body(st)) return false;
+    if(!body(st))
+    {
+        if(stream == nullptr) { cudaStreamSynchronize(st); cudaGetLastError(); }
+        return false;
+    }
     if(stream == nullptr) CUDA_TRY(cudaStreamSynchronize(st));
     return true;
 }
@@ -475,7 +465,9 @@ bool alloc_set(ViewSet& out, int cap, bool batch)
     vs.cap = cap; vs.batch = batch;
     vs.d_views = make_device<HzView>((size_t)cap * HZ_V_COUNT);
     vs.h_views = make_host<HzView>((size_t)PARAM_RING * cap * HZ_V_COUNT);
-    bool ok = vs.d_views && vs.h_views;
+    vs.d_chunk = make_device<ChunkBlock>(1);
+    vs.h_chunk = make_host<ChunkBlock>(PARAM_RING);
+    bool ok = vs.d_views && vs.h_views && vs.d_chunk && vs.h_chunk;
     for(EventHandle& e : vs.ring_ev) ok = ok && (e = make_event());
     ok = ok && (vs.busy = make_event()) && (vs.side = make_stream()) && (vs.ev_fork = make_event()) && (vs.ev_join = make_event());
     if(batch) ok = ok && (vs.stream = make_stream()) && (vs.done = make_event());
@@ -639,9 +631,10 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
     if(ev) CUDA_TRY(cudaEventRecord(ev[6].get(), st));
     // the labels and skylines: after the join (the near pass's large triangles are in the visibility buffers), before the
     // set's next chunk reuses those buffers (the same stream)
-    if(g.annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.annot.d.get(), m, st)); n++; }
-    if(g.skyline) { CUDA_TRY(hz_launch_skyline(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.skyline.d.get(), m, st)); n++; }
-    if(g.score) { CUDA_TRY(hz_launch_skyline_score(hv[HZ_V_NEAR], dv + HZ_V_NEAR, set.skyline.d.get(), m, st)); n++; }
+    const ChunkBlock* d = set.d_chunk.get();
+    if(g.annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->annot, m, st)); n++; }
+    if(g.skyline) { CUDA_TRY(hz_launch_skyline(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->sky, m, st)); n++; }
+    if(g.score) { CUDA_TRY(hz_launch_skyline_score(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->sky, m, st)); n++; }
     *launches = n;
     return true;
 }
@@ -763,31 +756,20 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
     for(int d = 0; d < out.n; d++) { v.out_image[d] = out.image[d]; v.out_ranges[d] = out.ranges[d]; }
 }
 
-// The labels of a chunk's views (k_annotate): the POIs (device), how many, where the label of the chunk's first view and
-// POI 0 goes (device; view k's follow m labels further per view), and the per-view inputs of the projection.
-struct AnnotSpec
-{
-    const double* pois;
-    int m;
-    float4* labels;
-    const HzAnnotView* views;
-};
-static_assert(sizeof(((HzAnnotate*)nullptr)->view) / sizeof(HzAnnotView) >= VIEWS_PER_SET, "HzAnnotate: a view set's views");
-
 // Enqueues one render of columns [x0,x1) of m views (m <= what ensure_views() gave) on stream st: view k uses scratch
-// set.sc[k] and writes to outs[k] (device memory), and, with `ann`, the labels of the POIs for each view after the
-// render, with `sky`, the chunk's skylines (and their scores) as that block says.  All views of one call must have the
-// same kinds of output.
+// set.sc[k] and writes to outs[k] (device memory), and, with `blk`, the stages after the render that it asks for: the
+// labels where blk->annot.labels is set (blk->annot.view[k] for view k), the skylines where blk->sky has a destination,
+// and their scores with blk->sky.scores.  All views of one call must have the same kinds of output.
 bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st,
-                   const AnnotSpec* ann = nullptr, const HzSkyline* sky = nullptr)
+                   const ChunkBlock* blk = nullptr)
 {
     if(s.W <= 0 || s.H <= 0 || m < 1 || m > (int)set.sc.size()) return false;
     const bool want_image = outs[0].image[0] != nullptr, want_ranges = outs[0].ranges[0] != nullptr;
     Stages stages;
-    stages.resolve = want_image || want_ranges; stages.annotate = ann != nullptr;
-    stages.skyline = sky != nullptr; stages.score = sky != nullptr && sky->scores != nullptr;
-    if(stages.annotate && !set.annot.ensure("cudaMalloc(annotate)", "cudaMallocHost(annotate)")) return false;
-    if(stages.skyline && !set.skyline.ensure("cudaMalloc(skyline)", "cudaMallocHost(skyline)")) return false;
+    stages.resolve = want_image || want_ranges;
+    stages.annotate = blk && blk->annot.labels;
+    stages.skyline = blk && (blk->sky.rows || blk->sky.range || blk->sky.scores);
+    stages.score = blk && blk->sky.scores;
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
     if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy.get(), 0));
 
@@ -863,18 +845,14 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
         }
     }
     CUDA_TRY(cudaMemcpyAsync(set.d_views.get(), hv, (size_t)m * HZ_V_COUNT * sizeof(HzView), cudaMemcpyHostToDevice, st));
-    if(stages.annotate)
-    {
-        HzAnnotate* ha = set.annot.at(slot);
-        ha->pois = ann->pois; ha->labels = ann->labels; ha->m = ann->m; ha->pad = 0;
-        for(int k = 0; k < m; k++) ha->view[k] = ann->views[k];
-        CUDA_TRY(set.annot.upload(slot, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView), st));
-    }
-    if(stages.skyline)
-    {
-        *set.skyline.at(slot) = *sky;
-        CUDA_TRY(set.skyline.upload(slot, sizeof(HzSkyline), st));
-    }
+    // the first `bytes` of a part of the stages' block, through the ring slot
+    auto upload = [&](auto ChunkBlock::*part, size_t bytes) {
+        void* const h = &(set.h_chunk.get()[slot].*part);
+        memcpy(h, &(blk->*part), bytes);
+        return cudaMemcpyAsync(&(set.d_chunk.get()->*part), h, bytes, cudaMemcpyHostToDevice, st);
+    };
+    if(stages.annotate) CUDA_TRY(upload(&ChunkBlock::annot, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView)));
+    if(stages.skyline)  CUDA_TRY(upload(&ChunkBlock::sky, sizeof(HzSkyline)));
     CUDA_TRY(cudaEventRecord(set.ring_ev[slot].get(), st));
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
@@ -1430,31 +1408,25 @@ bool horizonator_unproject(float* lat, float* lon, int x, int y,
 // kernels overlap another chunk's.  The sets start after everything already queued on `st`, and `st` continues after
 // all of them.  to_host: outputs go through the views' scratch and device->host copies on the set's stream, which
 // overlap the other sets' kernels.
-// ann: the labels of m POIs for every view as well (horizonator_annotate_batch*), by k_annotate after each chunk's chain;
-// into device memory, or (to_host) through the set's label scratch and a copy on its stream.
-struct AnnotReq
+// req: the stages after each chunk's chain as well, into device memory or (to_host) host memory: the labels of n_pois
+// POIs for every view (horizonator_annotate_batch*) by k_annotate; the skylines of every view
+// (horizonator_skyline_match*) by k_skyline, and their scores against the samples by k_skyline_score.
+struct StageReq
 {
-    const double* d_pois;
-    int m;
-    float4* labels;              // [n][m]: device memory, or host memory when to_host
-};
-// sky: the skylines of every view (horizonator_skyline_match*), by k_skyline after each chunk's chain, and their scores
-// against the samples by k_skyline_score; into device memory, or (to_host) through the set's output scratch and copies
-// on its stream.
-struct SkyReq
-{
-    int*   rows;                 // [n][W] each, or null: device memory, or host memory when to_host
-    float* range;
-    float* scores;
-    const HzSkySample* d_samples;
-    int   m;
-    float clip;
-    bool  wrap;
+    const double*      pois;         // device memory
+    int                n_pois;
+    float4*            labels;       // [n][n_pois], or null: no labels
+    int*               rows;         // [n][W] each, or null
+    float*             range;
+    float*             scores;
+    const HzSkySample* samples;      // [n_samples], device memory
+    int                n_samples;
+    float              clip;
+    bool               wrap;
 };
 
 static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
-                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const AnnotReq* ann = nullptr,
-                                const SkyReq* sky = nullptr)
+                                uint8_t* images, float* ranges, bool to_host, cudaStream_t st, const StageReq* req = nullptr)
 {
     const size_t px = (size_t)s->W * s->H;
     std::vector<ViewState> vs((size_t)n);
@@ -1465,15 +1437,6 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         vs[k].az_deg0 = views[k].az_deg0; vs[k].az_deg1 = views[k].az_deg1;
     }
     if(n == 0) return true;
-    // the projection's inputs per view, as write_labels() of the command-line tool forms them (horizonator-batch.h)
-    std::vector<HzAnnotView> av(ann ? (size_t)n : 0);
-    for(size_t k = 0; k < av.size(); k++)
-    {
-        const double lat = (double)views[k].lat;
-        av[k] = HzAnnotView{ lat, (double)views[k].lon, cos(lat * M_PI / 180.), (double)vs[k].viewer_z,
-                             (double)views[k].az_deg0 * M_PI / 180., (double)views[k].az_deg1 * M_PI / 180. };
-    }
-    const size_t m_poi = ann ? (size_t)ann->m : 0;
 
     // chunk size: the views spread evenly over the batch sets, at most VIEWS_PER_SET each, at most what fits in memory
     int n_sets = 0, chunk = 0;
@@ -1506,24 +1469,41 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     if(!forked) { sets.push_back(&s->main); chunk = 1; }
     auto stream_of = [st](const ViewSet& set) { return set.stream ? set.stream.get() : st; };
 
-    // each set's scratch for a chunk: the labels or the skylines of the host-memory calls (rows, range and scores, W * chunk
-    // words each, one after the other), the skylines the scorer reads.  Nothing queued still uses an old buffer once the
-    // set's stream is idle.
-    const size_t W = (size_t)s->W, sky_words = (size_t)chunk * W;
-    const size_t stage_out = !to_host ? 0 : ann ? (size_t)chunk * m_poi : sky ? (3 * sky_words + 3) / 4 : 0;
-    const size_t sky_rows = sky && sky->scores ? sky_words : 0;
+    // The output plan of the stages' outputs that are sized by the chunk: per view, the labels, the skylines' rows, range
+    // and scores, and the int16 skylines k_skyline_score reads, which the caller does not get.  An output the caller
+    // does not get, or gets in host memory, is staged: it goes into the set's staging buffer (each output 16-byte
+    // aligned, for the float4 labels) and from there to the caller after the chunk.  The others go straight to the
+    // caller's device memory.
+    const StageReq r = req ? *req : StageReq{};
+    const size_t W = (size_t)s->W;
+    struct ChunkOut { char* caller; size_t per_view; bool staged; size_t at; };   // at: offset in the staging buffer
+    enum { LABELS, ROWS, RANGE, SCORES, SKY, N_OUT };
+    ChunkOut plan[N_OUT] = {
+        { (char*)r.labels, r.labels ? (size_t)r.n_pois * sizeof(float4) : 0 },
+        { (char*)r.rows,   r.rows   ? W * sizeof(int)     : 0 },
+        { (char*)r.range,  r.range  ? W * sizeof(float)   : 0 },
+        { (char*)r.scores, r.scores ? W * sizeof(float)   : 0 },
+        { nullptr,         r.scores ? W * sizeof(int16_t) : 0 },
+    };
+    size_t staged = 0;
+    for(ChunkOut& o : plan)
+        if(o.per_view > 0 && (to_host || o.caller == nullptr))
+        {
+            o.staged = true; o.at = staged;
+            staged += ((size_t)chunk * o.per_view + 15) & ~(size_t)15;
+        }
+    // (nothing queued still uses an old buffer once the set's stream is idle; a failed growth is named after what the
+    // buffer stages: labels, skylines for the caller, or only the scorer's skylines)
+    const char* staged_what = plan[LABELS].staged ? "labels" :
+                              plan[ROWS].staged || plan[RANGE].staged || plan[SCORES].staged ? "skylines" : "skyline scratch";
     for(ViewSet* set : sets)
     {
-        if(set->d_stage_out.cap < stage_out || set->d_sky.cap < sky_rows) CUDA_TRY(cudaStreamSynchronize(stream_of(*set)));
-        cudaError_t e = cudaSuccess;
-        if(set->d_stage_out.cap < stage_out && (e = set->d_stage_out.grow(stage_out)) != cudaSuccess)
+        if(set->d_stage.cap * sizeof(float4) >= staged) continue;
+        CUDA_TRY(cudaStreamSynchronize(stream_of(*set)));
+        const cudaError_t e = set->d_stage.grow(staged / sizeof(float4));
+        if(e != cudaSuccess)
         {
-            MSG("CUDA error: cudaMalloc(%s) failed: %s", ann ? "labels" : "skylines", cudaGetErrorString(e));
-            return false;
-        }
-        if(set->d_sky.cap < sky_rows && (e = set->d_sky.grow(sky_rows)) != cudaSuccess)
-        {
-            MSG("CUDA error: cudaMalloc(skyline scratch) failed: %s", cudaGetErrorString(e));
+            MSG("CUDA error: cudaMalloc(%s) failed: %s", staged_what, cudaGetErrorString(e));
             return false;
         }
     }
@@ -1532,27 +1512,36 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         CUDA_TRY(cudaEventRecord(s->fork_ev.get(), st));
         for(ViewSet* set : sets) CUDA_TRY(cudaStreamWaitEvent(set->stream.get(), s->fork_ev.get(), 0));
     }
-    // views [k0, k0+m) on one set: the chain, then (to_host) the copies of their outputs out of the set's scratch
+    // views [k0, k0+m) on one set: the chain and its stages, then (to_host) the copies of their outputs out of the views'
+    // scratch and the set's staging buffer
     std::vector<OutSpec> outs((size_t)chunk);
     auto enqueue_chunk = [&](ViewSet& set, int k0, int m) {
         const cudaStream_t sst = stream_of(set);
         for(int k = 0; k < m; k++)
             outs[k] = single_out(images ? (to_host ? set.sc[k].d_image.get()  : images + (size_t)(k0 + k) * px * 3) : nullptr,
                                  ranges ? (to_host ? set.sc[k].d_ranges.get() : ranges + (size_t)(k0 + k) * px)     : nullptr);
-        AnnotSpec a{};
-        if(ann) a = AnnotSpec{ ann->d_pois, ann->m, to_host ? set.d_stage_out.get() : ann->labels + (size_t)k0 * m_poi, &av[k0] };
-        HzSkyline k{};
-        const size_t at = (size_t)k0 * W;
-        if(sky)
+        char* dst[N_OUT];
+        for(int i = 0; i < N_OUT; i++)
         {
-            float* const stage = (float*)set.d_stage_out.get();
-            k.rows   = !sky->rows   ? nullptr : to_host ? (int*)stage           : sky->rows + at;
-            k.range  = !sky->range  ? nullptr : to_host ? stage + sky_words     : sky->range + at;
-            k.scores = !sky->scores ? nullptr : to_host ? stage + 2 * sky_words : sky->scores + at;
-            k.sky = sky->scores ? set.d_sky.get() : nullptr;
-            k.samples = sky->d_samples; k.m = sky->m; k.clip = sky->clip; k.wrap = sky->wrap;
+            const ChunkOut& o = plan[i];
+            dst[i] = o.per_view == 0 ? nullptr : o.staged ? (char*)set.d_stage.get() + o.at : o.caller + (size_t)k0 * o.per_view;
         }
-        if(!enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), sst, ann ? &a : nullptr, sky ? &k : nullptr)) return false;
+        ChunkBlock blk;                    // (a call without stages renders only: the block is neither filled nor read)
+        if(req)
+        {
+            blk.sky = HzSkyline{ (int*)dst[ROWS], (float*)dst[RANGE], (float*)dst[SCORES], (int16_t*)dst[SKY],
+                                 r.samples, r.n_samples, r.clip, r.wrap, 0 };
+            blk.annot.pois = r.pois; blk.annot.labels = (float4*)dst[LABELS]; blk.annot.m = r.n_pois; blk.annot.pad = 0;
+            for(int k = 0; k < m && r.labels; k++)
+            {
+                // the projection's inputs, as write_labels() of the command-line tool forms them (horizonator-batch.h)
+                const horizonator_view_t& v = views[k0 + k];
+                const double lat = (double)v.lat;
+                blk.annot.view[k] = HzAnnotView{ lat, (double)v.lon, cos(lat * M_PI / 180.), (double)vs[k0 + k].viewer_z,
+                                                 (double)v.az_deg0 * M_PI / 180., (double)v.az_deg1 * M_PI / 180. };
+            }
+        }
+        if(!enqueue_views(*s, set, m, &vs[k0], 0, s->W, outs.data(), sst, req ? &blk : nullptr)) return false;
         for(int k = 0; k < m && to_host; k++)
         {
             if(images) CUDA_TRY(cudaMemcpyAsync(images + (size_t)(k0 + k) * px * 3, set.sc[k].d_image.get(), px * 3,
@@ -1560,18 +1549,25 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
             if(ranges) CUDA_TRY(cudaMemcpyAsync(ranges + (size_t)(k0 + k) * px, set.sc[k].d_ranges.get(), px * sizeof(float),
                                                 cudaMemcpyDeviceToHost, sst));
         }
-        if(ann && to_host)
-            CUDA_TRY(cudaMemcpyAsync(ann->labels + (size_t)k0 * m_poi, a.labels, (size_t)m * m_poi * sizeof(float4),
-                                     cudaMemcpyDeviceToHost, sst));
-        const size_t sky_bytes = (size_t)m * W * 4;
-        if(sky && to_host && k.rows)   CUDA_TRY(cudaMemcpyAsync(sky->rows + at, k.rows, sky_bytes, cudaMemcpyDeviceToHost, sst));
-        if(sky && to_host && k.range)  CUDA_TRY(cudaMemcpyAsync(sky->range + at, k.range, sky_bytes, cudaMemcpyDeviceToHost, sst));
-        if(sky && to_host && k.scores) CUDA_TRY(cudaMemcpyAsync(sky->scores + at, k.scores, sky_bytes, cudaMemcpyDeviceToHost, sst));
+        for(int i = 0; i < N_OUT; i++)
+            if(plan[i].staged && plan[i].caller)
+                CUDA_TRY(cudaMemcpyAsync(plan[i].caller + (size_t)k0 * plan[i].per_view, dst[i], (size_t)m * plan[i].per_view,
+                                         cudaMemcpyDeviceToHost, sst));
+        return true;
+    };
+    // `st` continues after all the sets
+    auto join = [&] {
+        for(ViewSet* set : sets)
+        {
+            CUDA_TRY(cudaEventRecord(set->done.get(), set->stream.get()));
+            CUDA_TRY(cudaStreamWaitEvent(st, set->done.get(), 0));
+        }
         return true;
     };
     bool ok = true;
     for(int k0 = 0, c = 0; k0 < n && ok; k0 += chunk, c++)
         ok = enqueue_chunk(*sets[(size_t)c % sets.size()], k0, n - k0 < chunk ? n - k0 : chunk);
+    ok = ok && (!forked || join());
     if(!forked) s->have_render = false;     // the context's visibility buffer no longer holds the context's own view
     if(!ok)
     {
@@ -1580,12 +1576,6 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         cudaGetLastError();
         return false;
     }
-    if(forked)
-        for(ViewSet* set : sets)
-        {
-            CUDA_TRY(cudaEventRecord(set->done.get(), set->stream.get()));
-            CUDA_TRY(cudaStreamWaitEvent(st, set->done.get(), 0));
-        }
     return true;
 }
 
@@ -1691,11 +1681,7 @@ bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizon
         if(counts && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
         if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_counts.get(), counts, cells * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts.get() : nullptr, masks, st))
-        {
-            cudaStreamSynchronize(st);
-            cudaGetLastError();
             return false;
-        }
         if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts.get(), cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         return true;
     });
@@ -1759,9 +1745,9 @@ bool horizonator_annotate_batch_device(const horizonator_context_t* ctx, int n, 
         MSG("horizonator_annotate_batch_device: d_pois must be 8-byte and d_labels 16-byte aligned");
         return false;
     }
-    const AnnotReq ann{ (const double*)d_pois, m, (float4*)d_labels };
+    const StageReq req{ (const double*)d_pois, m, (float4*)d_labels };
     return on_stream(*s, stream, [&](cudaStream_t st) {
-        return render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &ann);
+        return render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &req);
     });
 }
 
@@ -1773,14 +1759,8 @@ bool horizonator_annotate_batch(const horizonator_context_t* ctx, int n, const h
     if(n == 0 || m == 0) return true;
     return on_stream(*s, nullptr, [&](cudaStream_t st) {
         if(!upload_inputs(*s, st, pois, (size_t)m * sizeof(horizonator_poi_t), "POIs")) return false;
-        const AnnotReq ann{ s->d_inputs.get(), m, (float4*)labels };
-        if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &ann))
-        {
-            cudaStreamSynchronize(st);
-            cudaGetLastError();
-            return false;
-        }
-        return true;
+        const StageReq req{ s->d_inputs.get(), m, (float4*)labels };
+        return render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &req);
     });
 }
 
@@ -1831,10 +1811,10 @@ bool horizonator_skyline_match_device(const horizonator_context_t* ctx, int n, c
         MSG("%s: d_rows, d_range and d_scores must be 4-byte and d_samples 8-byte aligned", fn);
         return false;
     }
-    const SkyReq sky{ d_rows, d_range, d_scores, (const HzSkySample*)d_samples, m, clip_rows, wrap };
+    const StageReq req{ nullptr, 0, nullptr, d_rows, d_range, d_scores, (const HzSkySample*)d_samples, m, clip_rows, wrap };
     return on_stream(*s, stream, [&](cudaStream_t st) {
         if(d_scores && !skyline_score_ready(fn, *s)) return false;
-        return render_batch_common(ctx, s, n, views, nullptr, nullptr, false, st, nullptr, &sky);
+        return render_batch_common(ctx, s, n, views, nullptr, nullptr, false, st, &req);
     });
 }
 
@@ -1850,14 +1830,8 @@ bool horizonator_skyline_match(const horizonator_context_t* ctx, int n, const ho
     return on_stream(*s, nullptr, [&](cudaStream_t st) {
         if(scores && !(skyline_score_ready(fn, *s) && upload_inputs(*s, st, samples, (size_t)m * sizeof(HzSkySample), "samples")))
             return false;
-        const SkyReq sky{ rows, range, scores, (const HzSkySample*)s->d_inputs.get(), m, clip_rows, wrap };
-        if(!render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, nullptr, &sky))
-        {
-            cudaStreamSynchronize(st);
-            cudaGetLastError();
-            return false;
-        }
-        return true;
+        const StageReq req{ nullptr, 0, nullptr, rows, range, scores, (const HzSkySample*)s->d_inputs.get(), m, clip_rows, wrap };
+        return render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &req);
     });
 }
 

@@ -34,6 +34,14 @@ def test_batch_calls_without_memory_for_a_set_equal_lone_renders(tiles_c1):
         h.render_into(want_i[k], want_r[k])
     assert (want_r > 0).any()
     lone_launches = h.last_render_stats()["launches"]
+    # the skylines of the lone renders (horizon_profile_device()'s rule: the topmost pixel with a range > 0), and an
+    # observed skyline made of view 0's: every third column from 1000 on
+    terrain = want_r > 0
+    want_rows = np.where(terrain.any(axis=1), terrain.argmax(axis=1), -1).astype(np.int32)
+    want_range = np.where(want_rows >= 0, np.take_along_axis(want_r, np.maximum(want_rows, 0)[:, None, :], 1)[:, 0],
+                          -1).astype(np.float32)
+    samples = [(c - 1000, float(want_rows[0, c]) + 0.25) for c in range(1000, 1600, 3) if want_rows[0, c] >= 0]
+    assert samples
     di = torch.zeros((n, H, W, 3), dtype=torch.uint8, device="cuda")
     dr = torch.zeros((n, H, W), dtype=torch.float32, device="cuda")
     torch.cuda.synchronize()
@@ -49,14 +57,24 @@ def test_batch_calls_without_memory_for_a_set_equal_lone_renders(tiles_c1):
         h.render_batch_device(VIEWS, di.data_ptr(), dr.data_ptr())
         assert h.last_render_stats()["launches"] == lone_launches
         labels = h.annotate(VIEWS, pois)
+        rows, rng = h.skyline(VIEWS)
+        scores, score_rows = h.skyline_match(VIEWS, samples, rows=True)
+        match_launches = h.last_render_stats()["launches"]
     finally:
         del hold
         torch.cuda.empty_cache()
 
     assert np.array_equal(bi, want_i) and np.array_equal(br, want_r)
     assert np.array_equal(di.cpu().numpy(), want_i) and np.array_equal(dr.cpu().numpy(), want_r)
-    # the same call with memory to spare renders on a batch set (the batch chain: more launches)
+    assert np.array_equal(rows, want_rows) and np.array_equal(rng.view(np.uint32), want_range.view(np.uint32))
+    assert np.array_equal(score_rows, want_rows)
+    # the same calls with memory to spare render on the batch sets (the batch chain: more launches)
     want_labels = h.annotate(VIEWS, pois)
     assert h.last_render_stats()["launches"] != lone_launches
     assert (want_labels["range_rendered_m"] > 0).any()
     assert np.array_equal(labels.view(np.uint32), want_labels.view(np.uint32))
+    assert all(np.array_equal(a, b) for a, b in zip(h.skyline(VIEWS), (rows, rng)))
+    want_scores, _ = h.skyline_match(VIEWS, samples, rows=True)
+    assert h.last_render_stats()["launches"] != match_launches
+    assert (want_scores[0] < 1.).any()
+    assert np.array_equal(scores.view(np.uint32), want_scores.view(np.uint32))
