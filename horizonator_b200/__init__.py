@@ -95,6 +95,22 @@ class skyline_sample_t(C.Structure):
 SKYLINE_SAMPLE_DTYPE = np.dtype([("dx", np.int32), ("y", np.float32)])
 
 
+class pixel_t(C.Structure):
+    """include/horizonator-batch.h: horizonator_pixel_t (8 bytes): column, row (0 = top)."""
+    _fields_ = [("x", C.c_int32), ("y", C.c_int32)]
+
+
+class ground_t(C.Structure):
+    """include/horizonator-batch.h: horizonator_ground_t (32 bytes)."""
+    _fields_ = [("lat", C.c_double), ("lon", C.c_double), ("ele_m", C.c_float), ("range_m", C.c_float),
+                ("distance_m", C.c_float), ("triangle", C.c_uint32)]
+
+
+#: numpy dtype of ground_t: what pick() returns.  Sky: triangle 0xFFFFFFFF, range_m -1, the rest NaN.
+GROUND_DTYPE = np.dtype([("lat", np.float64), ("lon", np.float64), ("ele_m", np.float32), ("range_m", np.float32),
+                         ("distance_m", np.float32), ("triangle", np.uint32)])
+
+
 def skyline_samples(rel_az_deg, el_deg, az_width_deg, width, height):
     """An observed skyline given as angles -> its samples (SKYLINE_SAMPLE_DTYPE) for width x height panoramas of windows
     az_width_deg (az_deg1 - az_deg0) wide: points rel_az_deg degrees right of the heading and el_deg above the
@@ -162,6 +178,8 @@ def _signatures():
         "horizonator_annotate_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
         "horizonator_skyline_match_device": (b, [ctx, i, P(view_t), vp, vp, i, vp, f, b, vp, vp]),
         "horizonator_skyline_match": (b, [ctx, i, P(view_t), vp, vp, i, vp, f, b, vp]),
+        "horizonator_pick_batch_device": (b, [ctx, i, P(view_t), i, vp, vp, vp, vp, vp]),
+        "horizonator_pick_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
     }
 
 
@@ -570,6 +588,46 @@ class horizonator:
             az0, az1 = float(np.float32(views[k][2])), float(np.float32(views[k][3]))
             out.append((k, az0 + (h + 0.5) * (az1 - az0) / W, float(flat[i])))
         return out
+
+    # ground points of rendered pixels (horizonator_pick_batch*: what is at this pixel)
+    def pick(self, views, pixels):
+        """views as render_batch takes them; pixels: (m, 2) (x, y) pairs asked of every view, or (n, m, 2) per view (x
+        column, y row, 0 = top).  Returns an (n, m) structured array (GROUND_DTYPE): lat, lon, ele_m, distance_m of the
+        ground point the pixel shows, range_m (bit-identical to the range image) and the triangle number; sky: triangle
+        0xFFFFFFFF, range_m -1, the rest NaN (horizonator-batch.h).  Only the ground points leave the GPU."""
+        n = len(views)
+        px = np.asarray(pixels, dtype=np.int32)
+        px = px.reshape(-1, 2) if px.ndim < 3 else px
+        px = np.ascontiguousarray(np.broadcast_to(px, (n,) + px.shape[-2:]))
+        m = px.shape[1]
+        out = _pool.array((n, m), GROUND_DTYPE)
+        _check(lib.horizonator_pick_batch, C.byref(self._ctx), n, self._views(views), m,
+               px.ctypes.data if px.size else None, out.ctypes.data if out.size else None)
+        return out
+
+    def ground(self, views):
+        """The ground point of every pixel: (lat, lon, ele, range), each (n, H, W) in image order (float64, float64,
+        float32, float32; sky: NaN, NaN, NaN, -1).  n * H * W * 32 bytes cross the bus."""
+        n = len(views)
+        g = _pool.array((n, self.height, self.width), GROUND_DTYPE)
+        _check(lib.horizonator_pick_batch, C.byref(self._ctx), n, self._views(views), 0, None,
+               g.ctypes.data if g.size else None)
+        return g["lat"], g["lon"], g["ele_m"], g["range_m"]
+
+    def pick_device(self, views, d_pixels, d_ground, d_images=0, d_ranges=0, stream=0, m=None):
+        """Device-memory variant.  d_pixels: an (n, m, 2) int32 CUDA tensor, an integer device address with `m` given,
+        or None / 0 for every pixel; d_ground: a CUDA tensor or address of n * m (or n * H * W) ground_t, e.g. an
+        (n, m, 32) uint8 tensor (.cpu().numpy().view(GROUND_DTYPE) reads it); d_images / d_ranges as render_batch_device
+        (0 = not written); stream as render_batch_device."""
+        if hasattr(d_pixels, "data_ptr"):
+            if m is None:
+                m = d_pixels.shape[-2]
+            d_pixels = d_pixels.data_ptr()
+        if hasattr(d_ground, "data_ptr"):
+            d_ground = d_ground.data_ptr()
+        d_images, d_ranges = (a.data_ptr() if hasattr(a, "data_ptr") else a for a in (d_images, d_ranges))
+        _check(lib.horizonator_pick_batch_device, C.byref(self._ctx), len(views), self._views(views),
+               int(m or 0), d_pixels or None, d_ground or None, d_images or None, d_ranges or None, stream or None)
 
 
 class _PinnedBlock:

@@ -198,23 +198,24 @@ struct Scratch
     unsigned int last_epoch = 0;       // of the most recent render (horizonator_pick decodes main's keys with it)
 };
 
-// The stages of a render chain after its bands (launch_chain): k_resolve (images, range images), k_annotate (labels),
-// k_skyline (skylines) and k_skyline_score (their scores).  A captured chain is one combination.
+// The stages of a render chain after its bands (launch_chain): k_resolve (images, range images), k_pick (ground points),
+// k_annotate (labels), k_skyline (skylines) and k_skyline_score (their scores).  A captured chain is one combination.
 struct Stages
 {
-    bool resolve = false, annotate = false, skyline = false, score = false;
+    bool resolve = false, annotate = false, skyline = false, score = false, pick = false;
     bool operator==(const Stages& o) const
     {
-        return resolve == o.resolve && annotate == o.annotate && skyline == o.skyline && score == o.score;
+        return resolve == o.resolve && annotate == o.annotate && skyline == o.skyline && score == o.score && pick == o.pick;
     }
 };
 
 // The per-chunk parameters of the stages after the bands: k_skyline's and k_skyline_score's HzSkyline, k_annotate's
-// HzAnnotate.  A chunk uploads only the parts its stages read (enqueue_views).
+// HzAnnotate, k_pick's HzPick.  A chunk uploads only the parts its stages read (enqueue_views).
 struct ChunkBlock
 {
     HzSkyline  sky;
     HzAnnotate annot;
+    HzPick     pick;
 };
 static_assert(sizeof(((HzAnnotate*)nullptr)->view) / sizeof(HzAnnotView) >= VIEWS_PER_SET, "HzAnnotate: a view set's views");
 
@@ -629,9 +630,10 @@ bool launch_chain(Slot& s, ViewSet& set, const HzView* hv, int m, bool big_per_b
     if(fork) CUDA_TRY(cudaStreamWaitEvent(st, set.ev_join.get(), 0));
     if(g.resolve) { CUDA_TRY(hz_launch_resolve(hv[HZ_V_NEAR], dv + HZ_V_NEAR, m, st)); n++; }
     if(ev) CUDA_TRY(cudaEventRecord(ev[6].get(), st));
-    // the labels and skylines: after the join (the near pass's large triangles are in the visibility buffers), before the
-    // set's next chunk reuses those buffers (the same stream)
+    // the ground points, labels and skylines: after the join (the near pass's large triangles are in the visibility
+    // buffers), before the set's next chunk reuses those buffers (the same stream)
     const ChunkBlock* d = set.d_chunk.get();
+    if(g.pick) { CUDA_TRY(hz_launch_pick(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->pick, m, st)); n++; }
     if(g.annotate) { CUDA_TRY(hz_launch_annotate(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->annot, m, st)); n++; }
     if(g.skyline) { CUDA_TRY(hz_launch_skyline(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->sky, m, st)); n++; }
     if(g.score) { CUDA_TRY(hz_launch_skyline_score(hv[HZ_V_NEAR], dv + HZ_V_NEAR, &d->sky, m, st)); n++; }
@@ -759,7 +761,8 @@ void fill_view(const Slot& s, const ViewSet& set, const Scratch& sc, const ViewS
 // Enqueues one render of columns [x0,x1) of m views (m <= what ensure_views() gave) on stream st: view k uses scratch
 // set.sc[k] and writes to outs[k] (device memory), and, with `blk`, the stages after the render that it asks for: the
 // labels where blk->annot.labels is set (blk->annot.view[k] for view k), the skylines where blk->sky has a destination,
-// and their scores with blk->sky.scores.  All views of one call must have the same kinds of output.
+// their scores with blk->sky.scores, and the ground points where blk->pick.ground is set.  All views of one call must
+// have the same kinds of output.
 bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, int x1, const OutSpec* outs, cudaStream_t st,
                    const ChunkBlock* blk = nullptr)
 {
@@ -770,6 +773,7 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     stages.annotate = blk && blk->annot.labels;
     stages.skyline = blk && (blk->sky.rows || blk->sky.range || blk->sky.scores);
     stages.score = blk && blk->sky.scores;
+    stages.pick = blk && blk->pick.ground;
     // a set serves one render at a time: if its previous render went to another stream, wait for that one
     if(set.busy_recorded && set.last_stream != st) CUDA_TRY(cudaStreamWaitEvent(st, set.busy.get(), 0));
 
@@ -835,8 +839,8 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
             lo = vb.ring_hi;
         }
         // the row table of this view's window, unless the scratch still holds it from its previous render (the ranges, and
-        // the rendered ranges of the labels and skylines need it)
-        if((want_ranges || stages.annotate || stages.skyline) && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
+        // the rendered ranges of the labels, skylines and ground points need it)
+        if((want_ranges || stages.annotate || stages.skyline || stages.pick) && !sc.tanel_key.is(vs[k].az_deg1 - vs[k].az_deg0, s.W, s.H))
         {
             float* h_row = set.h_tanel.get() + ((size_t)slot * set.cap + k) * s.H;
             memcpy(h_row, tanel_row(s, vs[k].az_deg0, vs[k].az_deg1), (size_t)s.H * sizeof(float));
@@ -853,11 +857,12 @@ bool enqueue_views(Slot& s, ViewSet& set, int m, const ViewState* vs, int x0, in
     };
     if(stages.annotate) CUDA_TRY(upload(&ChunkBlock::annot, offsetof(HzAnnotate, view) + (size_t)m * sizeof(HzAnnotView)));
     if(stages.skyline)  CUDA_TRY(upload(&ChunkBlock::sky, sizeof(HzSkyline)));
+    if(stages.pick)     CUDA_TRY(upload(&ChunkBlock::pick, sizeof(HzPick)));
     CUDA_TRY(cudaEventRecord(set.ring_ev[slot].get(), st));
 
     // ---- the kernels: a replay of the captured graph where the chain has its standard shape, one by one otherwise
     const bool is_main = (&set == &s.main);
-    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (stages.resolve || stages.annotate || stages.skyline) &&
+    const bool standard = !s.profiling && x0 == 0 && x1 == s.W && (stages.resolve || stages.annotate || stages.skyline || stages.pick) &&
                           outs[0].n == 1 && hv[0].out_stride == s.W && outs[0].x_off == 0 && (vectorisable || !stages.resolve);
     if(standard && !set.graph_failed)
     {
@@ -1410,7 +1415,8 @@ bool horizonator_unproject(float* lat, float* lon, int x, int y,
 // overlap the other sets' kernels.
 // req: the stages after each chunk's chain as well, into device memory or (to_host) host memory: the labels of n_pois
 // POIs for every view (horizonator_annotate_batch*) by k_annotate; the skylines of every view
-// (horizonator_skyline_match*) by k_skyline, and their scores against the samples by k_skyline_score.
+// (horizonator_skyline_match*) by k_skyline, and their scores against the samples by k_skyline_score; the ground points
+// of n_pixels pixels of every view, or of all its pixels (horizonator_pick_batch*), by k_pick.
 struct StageReq
 {
     const double*      pois;         // device memory
@@ -1423,6 +1429,9 @@ struct StageReq
     int                n_samples;
     float              clip;
     bool               wrap;
+    const HzPickPixel* pixels;       // [n][n_pixels], device memory; null: every pixel
+    int                n_pixels;
+    HzGround*          ground;       // [n][n_pixels] or [n][H][W], or null: no ground points
 };
 
 static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
@@ -1477,13 +1486,14 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
     const StageReq r = req ? *req : StageReq{};
     const size_t W = (size_t)s->W;
     struct ChunkOut { char* caller; size_t per_view; bool staged; size_t at; };   // at: offset in the staging buffer
-    enum { LABELS, ROWS, RANGE, SCORES, SKY, N_OUT };
+    enum { LABELS, ROWS, RANGE, SCORES, SKY, GROUND, N_OUT };
     ChunkOut plan[N_OUT] = {
         { (char*)r.labels, r.labels ? (size_t)r.n_pois * sizeof(float4) : 0 },
         { (char*)r.rows,   r.rows   ? W * sizeof(int)     : 0 },
         { (char*)r.range,  r.range  ? W * sizeof(float)   : 0 },
         { (char*)r.scores, r.scores ? W * sizeof(float)   : 0 },
         { nullptr,         r.scores ? W * sizeof(int16_t) : 0 },
+        { (char*)r.ground, r.ground ? (r.pixels ? (size_t)r.n_pixels : W * (size_t)s->H) * sizeof(HzGround) : 0 },
     };
     size_t staged = 0;
     for(ChunkOut& o : plan)
@@ -1494,7 +1504,7 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
         }
     // (nothing queued still uses an old buffer once the set's stream is idle; a failed growth is named after what the
     // buffer stages: labels, skylines for the caller, or only the scorer's skylines)
-    const char* staged_what = plan[LABELS].staged ? "labels" :
+    const char* staged_what = plan[GROUND].staged ? "ground points" : plan[LABELS].staged ? "labels" :
                               plan[ROWS].staged || plan[RANGE].staged || plan[SCORES].staged ? "skylines" : "skyline scratch";
     for(ViewSet* set : sets)
     {
@@ -1532,6 +1542,10 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
             blk.sky = HzSkyline{ (int*)dst[ROWS], (float*)dst[RANGE], (float*)dst[SCORES], (int16_t*)dst[SKY],
                                  r.samples, r.n_samples, r.clip, r.wrap, 0 };
             blk.annot.pois = r.pois; blk.annot.labels = (float4*)dst[LABELS]; blk.annot.m = r.n_pois; blk.annot.pad = 0;
+            const horizonator_dem_context_t& dem = ctx->dems;
+            blk.pick = HzPick{ r.pixels ? r.pixels + (size_t)k0 * r.n_pixels : nullptr, (HzGround*)dst[GROUND], r.n_pixels,
+                               dem.origin_dem_lon_lat[0], dem.origin_dem_lon_lat[1], dem.origin_dem_cellij[0],
+                               dem.origin_dem_cellij[1], dem.cells_per_deg };
             for(int k = 0; k < m && r.labels; k++)
             {
                 // the projection's inputs, as write_labels() of the command-line tool forms them (horizonator-batch.h)
@@ -1831,6 +1845,55 @@ bool horizonator_skyline_match(const horizonator_context_t* ctx, int n, const ho
         if(scores && !(skyline_score_ready(fn, *s) && upload_inputs(*s, st, samples, (size_t)m * sizeof(HzSkySample), "samples")))
             return false;
         const StageReq req{ nullptr, 0, nullptr, rows, range, scores, (const HzSkySample*)s->d_inputs.get(), m, clip_rows, wrap };
+        return render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &req);
+    });
+}
+
+// ---- ground points of rendered pixels (horizonator-batch.h) ------------------------------------------------------
+
+static_assert(sizeof(HzPickPixel) == sizeof(horizonator_pixel_t) && offsetof(horizonator_pixel_t, y) == 4,
+              "HzPickPixel: horizonator_pixel_t");
+static_assert(sizeof(HzGround) == sizeof(horizonator_ground_t) && offsetof(horizonator_ground_t, ele_m) == 16 &&
+              offsetof(horizonator_ground_t, triangle) == 28, "HzGround: horizonator_ground_t");
+
+// the argument rules of both pick calls; false: nothing may be done
+static bool pick_args_ok(const char* fn, int n, const horizonator_view_t* views, int m, const void* pixels, const void* ground)
+{
+    if(n < 0 || m < 0) { MSG("%s: negative count (n = %d, m = %d)", fn, n, m); return false; }
+    if(n == 0 || (pixels && m == 0)) return true;
+    if(views == nullptr || ground == nullptr) { MSG("%s: views and ground are required", fn); return false; }
+    if((((uintptr_t)pixels | (uintptr_t)ground) & 7) != 0) { MSG("%s: pixels and ground must be 8-byte aligned", fn); return false; }
+    return true;
+}
+
+bool horizonator_pick_batch_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                   int m, const horizonator_pixel_t* d_pixels, horizonator_ground_t* d_ground,
+                                   void* d_images, void* d_ranges, void* stream)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !pick_args_ok("horizonator_pick_batch_device", n, views, m, d_pixels, d_ground)) return false;
+    if(n == 0 || (d_pixels && m == 0)) return true;
+    StageReq req{};
+    req.pixels = (const HzPickPixel*)d_pixels; req.n_pixels = d_pixels ? m : 0; req.ground = (HzGround*)d_ground;
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        return render_batch_common(ctx, s, n, views, (uint8_t*)d_images, (float*)d_ranges, false, st, &req);
+    });
+}
+
+bool horizonator_pick_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                            int m, const horizonator_pixel_t* pixels, horizonator_ground_t* ground)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || !pick_args_ok("horizonator_pick_batch", n, views, m, pixels, ground)) return false;
+    if(n == 0 || (pixels && m == 0)) return true;
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        StageReq req{};
+        req.ground = (HzGround*)ground;
+        if(pixels)
+        {
+            if(!upload_inputs(*s, st, pixels, (size_t)n * m * sizeof(horizonator_pixel_t), "pixels")) return false;
+            req.pixels = (const HzPickPixel*)s->d_inputs.get(); req.n_pixels = m;
+        }
         return render_batch_common(ctx, s, n, views, nullptr, nullptr, true, st, &req);
     });
 }

@@ -247,6 +247,22 @@ cudaError_t hz_launch_skyline_score(const HzView& v, const HzView* d_v, const Hz
 // Lets k_skyline_score stage W skyline rows in shared memory on the current device; an error if W is too wide for that
 // (beyond about 110 000 columns).  Called before any scores are queued, outside graph capture.
 cudaError_t hz_skyline_score_setup(int W);
+// ---- ground points of rendered pixels (horizonator_pick_batch*: the rule is in include/horizonator-batch.h) --------
+struct alignas(8) HzPickPixel { int32_t x, y; };                                       // horizonator_pixel_t
+struct alignas(8) HzGround { double lat, lon; float ele_m, range_m, distance_m; uint32_t triangle; };   // horizonator_ground_t
+// The per-chunk block, copied to the device with the HzView variants like HzAnnotate.  View k of the chunk reads
+// pixels[k * m + i] and writes ground[k * m + i]; in whole-image mode (pixels null) it writes ground[(k * H + y) * W + x]
+// for every pixel.  The DEM geometry: cell (i, j) of the mosaic is at longitude lon_deg + (cell_i + i) / cpd, latitude
+// lat_deg + (cell_j + j) / cpd (horizonator_dem_context_t's origin fields).
+struct HzPick
+{
+    const HzPickPixel* pixels;
+    HzGround*          ground;
+    int                m;
+    int                lon_deg, lat_deg, cell_i, cell_j, cpd;
+};
+// after the render chain of a chunk, in place of k_resolve or after it
+cudaError_t hz_launch_pick(const HzView& v, const HzView* d_v, const HzPick* d_p, int nviews, cudaStream_t stream);
 // ---- viewsheds (horizonator_viewshed*: the definition is in include/horizonator-batch.h) ------
 constexpr int HZ_VS_MAX_VIEWS = 64;     // views per k_viewshed launch (gridDim.y); their eyes travel in the parameters
 struct HzViewshedEye { float vci, vcj, vz, cos_lat; };     // compute_move()'s eye, float as there

@@ -24,6 +24,7 @@
 //                        visibility buffers of the views just rendered                     annotator.c:280-348
 //   k_skyline, k_skyline_score (skylines)  the topmost terrain pixel of every column, read from the visibility buffers;
 //                        the match of those skylines against an observed one at every heading
+//   k_pick     (ground points)  the ground point under rendered pixels, from the triangle number in each pixel's key
 //   k_viewshed, k_viewshed_count (viewsheds)  R2 ray casting over the DEM square, one thread per ray -> bit masks;
 //                        masks -> per-vertex counts of the views that see it
 //
@@ -36,6 +37,7 @@
 #include "hz_project.h"
 
 #include <cfloat>
+#include <climits>
 #include <cstdint>
 #include <cstdlib>
 
@@ -324,6 +326,9 @@ struct HzTri
 
 enum { HZ_SETUP_NOTHING = 0, HZ_SETUP_OK = 1, HZ_SETUP_TOO_WIDE = -1, HZ_SETUP_QUEUE_FULL = -2 };
 
+// viewport transform (F1): gl_Position -> window coordinate, half = half the target's width or height
+__device__ __forceinline__ float hz_viewport(float ndc, float half) { return ndc * half + half; }
+
 // geometry.glsl:21-27, guard band, back-face cull, bounding box.  HZ_SETUP_OK, or why the triangle produces nothing.
 __device__ __forceinline__ int
 hz_tri_bounds(const HzView& P, const HzVtx& a, const HzVtx& b, const HzVtx& c, HzTri& T)
@@ -333,9 +338,9 @@ hz_tri_bounds(const HzView& P, const HzVtx& a, const HzVtx& b, const HzVtx& c, H
     if(xmax - xmin > 0.5f) return HZ_SETUP_TOO_WIDE;                         // geometry.glsl:21-27
 
     const float halfW = 0.5f * (float)P.W, halfH = 0.5f * (float)P.H;
-    T.xw0 = a.xn * halfW + halfW; T.yw0 = a.yn * halfH + halfH;              // viewport transform (F1)
-    T.xw1 = b.xn * halfW + halfW; T.yw1 = b.yn * halfH + halfH;
-    T.xw2 = c.xn * halfW + halfW; T.yw2 = c.yn * halfH + halfH;
+    T.xw0 = hz_viewport(a.xn, halfW); T.yw0 = hz_viewport(a.yn, halfH);
+    T.xw1 = hz_viewport(b.xn, halfW); T.yw1 = hz_viewport(b.yn, halfH);
+    T.xw2 = hz_viewport(c.xn, halfW); T.yw2 = hz_viewport(c.yn, halfH);
     if(!(fabsf(T.xw0) < HZ_GUARD_PX && fabsf(T.yw0) < HZ_GUARD_PX &&
          fabsf(T.xw1) < HZ_GUARD_PX && fabsf(T.yw1) < HZ_GUARD_PX &&
          fabsf(T.xw2) < HZ_GUARD_PX && fabsf(T.yw2) < HZ_GUARD_PX)) return HZ_SETUP_NOTHING;   // F5
@@ -400,12 +405,12 @@ hz_tri_planes(const HzView& P, HzTri& T,
 // for a triangle that straddles the +-pi seam of the window and is therefore "too wide" as it stands: the same
 // triangle with its left-hand vertices moved one period to the right (1), and that moved one period to the left (2)
 // -- its two appearances at the right and left edge of a full-circle panorama.
-__device__ __forceinline__ int hz_tri_setup(const HzView& P, unsigned int id, int copy, HzTri& T)
+// The vertices of triangle `id` (mesh rows vj, columns vi), their metres from the eye (e, n) and projections v -- copy
+// as in hz_tri_setup.  k_pick recomputes a drawn triangle's vertices with it.
+__device__ __forceinline__ void hz_tri_project(const HzView& P, unsigned int id, int copy, int vj[3], int vi[3], float e[3],
+                                               float n[3], HzVtx v[3])
 {
-    int vj[3], vi[3];
     hz_tri_vertices(id, P.N, vj, vi);
-    float e[3], n[3];
-    HzVtx v[3];
     #pragma unroll
     for(int k = 0; k < 3; k++)
     {
@@ -416,6 +421,14 @@ __device__ __forceinline__ int hz_tri_setup(const HzView& P, unsigned int id, in
         if(copy >= 1 && v[k].xn < 0.0f) v[k].xn += P.seam_period;
         if(copy == 2) v[k].xn -= P.seam_period;
     }
+}
+
+__device__ __forceinline__ int hz_tri_setup(const HzView& P, unsigned int id, int copy, HzTri& T)
+{
+    int vj[3], vi[3];
+    float e[3], n[3];
+    HzVtx v[3];
+    hz_tri_project(P, id, copy, vj, vi, e, n, v);
     const int st = hz_tri_bounds(P, v[0], v[1], v[2], T);
     if(st != HZ_SETUP_OK) return st;
     T.id = id;
@@ -2313,6 +2326,127 @@ cudaError_t hz_launch_skyline_score(const HzView& v, const HzView* d_v, const Hz
     const unsigned int parts = (unsigned int)((v.W + HZ_CTA_THREADS - 1) / HZ_CTA_THREADS);
     return hz_launch_smem(k_skyline_score, dim3(parts, (unsigned)nviews), dim3(HZ_CTA_THREADS), hz_skyline_score_smem(v.W),
                           stream, d_v, d_s);
+}
+
+// ================================================================================================
+// k_pick: the ground point under rendered pixels, from the triangle number in each pixel's key (include/horizonator-batch.h
+// states the rule; oracle/pick.py restates it)
+// ================================================================================================
+
+#define HZ_PICK_CTAS 64             /* CTAs per view: a fixed grid, so that one captured chain serves any number of pixels */
+
+// Ground point of the pixel at column x, image row y (0 = top) of the view; lod_from[l]: the first ring of tiles meshed
+// at level l or coarser.
+__device__ __forceinline__ void hz_pick_pixel(const HzView& P, const HzPick& K, const int* lod_from, int x, int y, HzGround* g)
+{
+    const int W = P.W, H = P.H;
+    const int gl = H - 1 - (y < 0 ? 0 : y);                                  // GL row (0 = bottom)
+    unsigned int q = HZ_Q_MAX;
+    unsigned long long key = HZ_KEY_CLEAR;
+    // outside the image, or in an 8x8 block nothing was drawn into (k_resolve4's shortcut): sky
+    if(x >= 0 && x < W && y >= 0 && y < H &&
+       (__ldg(P.hiz_flags + (size_t)(gl / HZ_SPAN_KEYS) * hz_spans((unsigned int)W) + x / HZ_SPAN_KEYS) & HZ_FLAG_TOUCHED))
+    {
+        key = __ldcs(P.vis + (size_t)gl * (size_t)W + (size_t)x);
+        q = hz_key_q(key, P.epoch);
+    }
+    if(q == HZ_Q_MAX)
+    {
+        const double nan = __longlong_as_double(0x7FF8000000000000ll);
+        g->lat = nan; g->lon = nan;
+        *(uint2*)&g->ele_m = make_uint2(0x7FC00000u, __float_as_uint(-1.0f));
+        *(uint2*)&g->distance_m = make_uint2(0x7FC00000u, 0xFFFFFFFFu);
+        return;
+    }
+    const float range = hz_range_of_q(q, __ldg(P.tanel + gl), P.znear, P.zfar);
+    // The key keeps the low 29 bits of the triangle number; the level of detail is that of the band whose rings hold the
+    // tile of the triangle's vertex 0 (the near pass is never coarsened, and the bands' ring ranges do not overlap)
+    unsigned int id = (unsigned int)(key >> 8) & HZ_ID_CELL_MASK;
+    {
+        const unsigned int cell = id >> 1;
+        const int j = (int)(cell / (unsigned int)(P.N - 1)), i = (int)(cell % (unsigned int)(P.N - 1));
+        const int ring = max(abs(i / HZ_TILE_CELLS - P.eye_ti), abs(j / HZ_TILE_CELLS - P.eye_tj));
+        unsigned int lod = 0;
+        while(lod < HZ_MAX_LOD && ring >= lod_from[lod + 1]) lod++;
+        id |= lod << HZ_ID_LOD_SHIFT;
+    }
+    // the triangle's unsnapped window positions as hz_tri_setup computes them; with the seam wrap, the copy whose x-range
+    // holds the pixel centre
+    int vj[3], vi[3];
+    float e[3], n[3];
+    HzVtx v[3];
+    const float halfW = 0.5f * (float)W, halfH = 0.5f * (float)H;
+    const double cx = (double)x + 0.5, cy = (double)gl + 0.5;
+    hz_tri_project(P, id, 0, vj, vi, e, n, v);
+    if(P.seam_period > 0.0f && fmaxf(fmaxf(v[0].xn, v[1].xn), v[2].xn) - fminf(fminf(v[0].xn, v[1].xn), v[2].xn) > 0.5f)
+    {
+        hz_tri_project(P, id, 1, vj, vi, e, n, v);
+        const float x0 = hz_viewport(v[0].xn, halfW), x1 = hz_viewport(v[1].xn, halfW), x2 = hz_viewport(v[2].xn, halfW);
+        if(!((double)fminf(fminf(x0, x1), x2) <= cx && cx <= (double)fmaxf(fmaxf(x0, x1), x2)))
+            hz_tri_project(P, id, 2, vj, vi, e, n, v);
+    }
+    const double x0 = hz_viewport(v[0].xn, halfW), y0 = hz_viewport(v[0].yn, halfH);
+    const double x1 = hz_viewport(v[1].xn, halfW), y1 = hz_viewport(v[1].yn, halfH);
+    const double x2 = hz_viewport(v[2].xn, halfW), y2 = hz_viewport(v[2].yn, halfH);
+    // barycentric weights of the pixel centre, double, not clamped (-fmad=false: every operation rounded once)
+    const double d  = (x1 - x0) * (y2 - y0) - (x2 - x0) * (y1 - y0);
+    const double b1 = ((cx - x0) * (y2 - y0) - (x2 - x0) * (cy - y0)) / d;
+    const double b2 = ((x1 - x0) * (cy - y0) - (cx - x0) * (y1 - y0)) / d;
+    const double b0 = 1.0 - b1 - b2;
+    const double ci = b0 * (double)vi[0] + b1 * (double)vi[1] + b2 * (double)vi[2];
+    const double cj = b0 * (double)vj[0] + b1 * (double)vj[1] + b2 * (double)vj[2];
+    const double ge = b0 * (double)e[0] + b1 * (double)e[1] + b2 * (double)e[2];
+    const double gn = b0 * (double)n[0] + b1 * (double)n[1] + b2 * (double)n[2];
+    const double z  = b0 * (double)v[0].z + b1 * (double)v[1].z + b2 * (double)v[2].z;
+    g->lat = (double)K.lat_deg + ((double)K.cell_j + cj) / (double)K.cpd;
+    g->lon = (double)K.lon_deg + ((double)K.cell_i + ci) / (double)K.cpd;
+    *(uint2*)&g->ele_m = make_uint2(__float_as_uint((float)z), __float_as_uint(range));
+    *(uint2*)&g->distance_m = make_uint2(__float_as_uint((float)sqrt(ge * ge + gn * gn)), id);
+}
+
+// One thread per (view, pixel), gridDim.y = view of the chunk.  Query mode: the pixels strided over the view's CTAs.
+// Whole-image mode: the CTAs stride over the image rows and a warp takes 32 adjacent pixels of a row, so that its key
+// reads and its stores are coalesced.  Register budget: 4 CTAs of 256 threads per SM, 64 registers.
+__global__ void __launch_bounds__(HZ_CTA_THREADS, 4)
+k_pick(const HzView* __restrict__ V, const HzPick* __restrict__ K)
+{
+    HZ_KERNEL_PROLOGUE(V, P);
+    __shared__ int s_lod_from[HZ_MAX_LOD + 1];
+    if(threadIdx.x <= HZ_MAX_LOD) s_lod_from[threadIdx.x] = threadIdx.x == 0 ? 0 : INT_MAX;
+    __syncthreads();
+    if(threadIdx.x < HZ_MAX_BANDS)
+    {
+        const HzView& b = V[blockIdx.y * HZ_V_COUNT + HZ_V_BAND0 + threadIdx.x];
+        if(b.ring_lo < b.ring_hi)
+            for(int l = 1; l <= b.lod; l++) atomicMin(s_lod_from + l, b.ring_lo);
+    }
+    __syncthreads();
+    const HzPick& k = *K;
+    const int W = P.W, H = P.H;
+    if(k.pixels == nullptr)
+    {
+        HzGround* const ground = k.ground + (size_t)blockIdx.y * (size_t)H * (size_t)W;
+        for(int y = blockIdx.x; y < H; y += gridDim.x)
+            for(int x = threadIdx.x; x < W; x += HZ_CTA_THREADS)
+                hz_pick_pixel(P, k, s_lod_from, x, y, ground + (size_t)y * W + x);
+    }
+    else
+    {
+        const int m = k.m;
+        const HzPickPixel* const pixels = k.pixels + (size_t)blockIdx.y * (size_t)m;
+        HzGround* const ground = k.ground + (size_t)blockIdx.y * (size_t)m;
+        for(int i = blockIdx.x * HZ_CTA_THREADS + threadIdx.x; i < m; i += gridDim.x * HZ_CTA_THREADS)
+        {
+            const HzPickPixel p = pixels[i];
+            hz_pick_pixel(P, k, s_lod_from, p.x, p.y, ground + i);
+        }
+    }
+}
+
+cudaError_t hz_launch_pick(const HzView& v, const HzView* d_v, const HzPick* d_p, int nviews, cudaStream_t stream)
+{
+    (void)v;
+    return hz_launch(k_pick, dim3(HZ_PICK_CTAS, (unsigned)nviews), dim3(HZ_CTA_THREADS), stream, d_v, d_p);
 }
 
 // ================================================================================================

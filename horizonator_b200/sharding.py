@@ -9,7 +9,8 @@ collective on the data path of a render:
   Only reduced products (horizon profiles, a few bytes per image column) are gathered.  Viewsheds partition the same
   way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).  Labels of
   points of interest too: 16 bytes per (view, POI) are gathered (annotate_sharded), and the scores of an observed
-  skyline, 4 bytes per (view, heading column) (skyline_match_sharded).
+  skyline, 4 bytes per (view, heading column) (skyline_match_sharded), and the ground points of pixels, 32 bytes
+  per (view, pixel) (pick_sharded).
 * azimuth wedges  -- one giant panorama: rank g renders columns [edges[g], edges[g+1]), bit-identical to the same
   columns of an unsharded render.  PeerPanorama fuses the exchange into the renderer: each rank's resolve kernel
   stores its wedge straight into every rank's full panorama over NVLink (peer memory), a barrier is the only
@@ -367,3 +368,19 @@ def skyline_match_sharded(h, views, samples, group=None, clip_rows=8., wrap=True
         h.skyline_match_device(views[lo:hi], s, scores, clip_rows=clip_rows, wrap=wrap,
                                stream=torch.cuda.current_stream().cuda_stream)
     return gather_blocks(scores, len(views), group)
+
+
+def pick_sharded(h, views, pixels, group=None):
+    """Ground points of pixels over the ranks: `views` block-partitioned, this rank's share picked on its own GPU
+    without writing any panorama (horizonator_pick_batch_device), and the ground points gathered.  pixels: an (m, 2)
+    array of (x, y) asked of every view.  Returns an (n, m, 32) uint8 CUDA tensor of all views' ground_t on every rank
+    (.cpu().numpy().view(GROUND_DTYPE) reads it).  All ranks must hold contexts of the same DEM square and size."""
+    world, rank = _world(group)
+    lo, hi = block_partition(len(views), world, rank)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    px = np.ascontiguousarray(np.asarray(pixels, np.int32).reshape(-1, 2))
+    d_px = torch.as_tensor(np.broadcast_to(px, (hi - lo,) + px.shape).copy(), device=dev)
+    ground = torch.empty((hi - lo, px.shape[0], 32), dtype=torch.uint8, device=dev)
+    if hi > lo and px.shape[0] > 0:
+        h.pick_device(views[lo:hi], d_px, ground, stream=torch.cuda.current_stream().cuda_stream)
+    return gather_blocks(ground, len(views), group)

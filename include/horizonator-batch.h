@@ -288,6 +288,71 @@ bool horizonator_skyline_match(const horizonator_context_t* ctx, int n, const ho
                                int m, const horizonator_skyline_sample_t* samples,
                                float clip_rows, bool wrap, float* scores);
 
+/* What is at this pixel: for each of n views and each of m pixels (or every pixel), the ground point the pixel shows --
+ * its latitude, longitude, height and distance, the triangle of the DEM mesh it lies on, and the pixel's range -- read
+ * from the triangle number each visibility key of the render holds.
+ *
+ * Render: each view is rendered exactly as horizonator_render_batch_device() renders it (the same chunks, captured
+ * graphs, the context's z extents and size, and the same opt-in modes: earth curvature, seam wrap, level of detail).
+ * Images and range images are written only where d_images / d_ranges are given.
+ * DEM geometry (dem.h): mesh vertex (i, j) -- column i east, row j north, as horizonator_download_mosaic() indexes the
+ * square -- lies at
+ *     lon = origin_dem_lon_lat[0] + (origin_dem_cellij[0] + i) / cells_per_deg
+ *     lat = origin_dem_lon_lat[1] + (origin_dem_cellij[1] + j) / cells_per_deg
+ * evaluated in double with i, j real (the fields are those of ctx->dems).
+ * Per pixel (x, y) of view k (x column, y row, 0 = top, as the image):
+ *   - The key at GL row H-1-y, column x decides.  Sky -- nothing of this render drawn there, or (x, y) outside the
+ *     image -- gives triangle = 0xFFFFFFFF, range_m = -1 and lat = lon = ele_m = distance_m = NaN.
+ *   - range_m: the pixel's range, bit-identical to the range image of the same render.
+ *   - triangle: the number of the triangle drawn there, as the reference numbers them (horizonator-lib.c:496-508:
+ *     2 * (j * (N - 1) + i) + half, N = 2 * radius_cells, (j, i) its first vertex), with the level of detail of the
+ *     band it was drawn in in bits [30:29] (0 without horizonator_set_lod(); level l: vertices 2^l cells apart, half 0
+ *     = (j,i), (j+s,i+s), (j+s,i) and half 1 = (j,i), (j,i+s), (j+s,i+s), s = 2^l).  The level is that of the band of
+ *     rings of 32x32-cell tiles around the eye's tile that holds the tile of (j, i); bands do not overlap, so it is
+ *     unique.
+ *   - Ground point: the three vertices' window positions as the renderer computes them before snapping (float,
+ *     vertex.glsl and the viewport transform; with the seam wrap the copy of the triangle whose x-range holds the pixel
+ *     centre); the barycentric weights (b0, b1, b2) of the pixel centre (cx, cy) = (x + 0.5, H - 1 - y + 0.5) from them,
+ *     in double, not clamped:
+ *         d  = (x1 - x0) * (y2 - y0) - (x2 - x0) * (y1 - y0)
+ *         b1 = ((cx - x0) * (y2 - y0) - (x2 - x0) * (cy - y0)) / d
+ *         b2 = ((x1 - x0) * (cy - y0) - (cx - x0) * (y1 - y0)) / d
+ *         b0 = 1 - b1 - b2
+ *     and with S(a) = b0 * a0 + b1 * a1 + b2 * a2: i = S(vertex columns), j = S(vertex rows) -> lat, lon by the DEM
+ *     geometry; ele_m = S(terrain heights) (the true height, not the apparent one of the opt-in curvature);
+ *     distance_m = sqrt(E * E + N * N) with E, N = S of the vertices' metres east / north of the eye as the renderer
+ *     computes them (float, vertex.glsl:128-130).  All in double, every operation rounded once in the order written;
+ *     ele_m and distance_m rounded to float once.
+ * Limits: the point is the screen-space interpolation GL gives an attribute over the triangle (what the reference's
+ * texture mode does with its per-vertex texture coordinate, vertex.glsl:116-126), not the intersection of the pixel's
+ * ray with the surface.  The rasteriser decides coverage on positions snapped to 1/256 pixel, so at a silhouette a
+ * weight can lie up to about 1/256 pixel's worth outside [0, 1].  Whole-image output takes H * W * 32 bytes per view
+ * (69 MB at 3600 x 600).
+ * Arguments: views in host memory.  pixels (8-byte aligned): [n][m]; NULL: every pixel, the output is then [n][H][W]
+ * in image order and m (>= 0) is not used.  ground (8-byte aligned): [n][m] or [n][H][W].  n == 0, or m == 0 with
+ * pixels given: nothing is done, true.  n < 0, m < 0, NULL views or ground otherwise, or misaligned pointers: false,
+ * nothing is written. */
+typedef struct { int32_t x, y; } horizonator_pixel_t;     /* 8 bytes: column, row (0 = top), as the image */
+typedef struct
+{
+    double   lat, lon;
+    float    ele_m, range_m, distance_m;
+    uint32_t triangle;
+} horizonator_ground_t;                                    /* 32 bytes */
+
+/* d_pixels, d_ground: DEVICE memory; d_images / d_ranges as in horizonator_render_batch_device(), either or both may be
+ * NULL.  Stream as for the batch render. */
+bool horizonator_pick_batch_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                   int m, const horizonator_pixel_t* d_pixels, horizonator_ground_t* d_ground,
+                                   void* d_images, void* d_ranges, void* stream);
+
+/* Same with pixels and ground in HOST memory, synchronous; no panorama is written, and only the ground points cross
+ * the bus (into page-locked memory by DMA; see horizonator_host_alloc()).  Unlike horizonator_pick() (horizonator.h),
+ * which unprojects one pixel of the context's last render treating its depth as a horizontal distance, this reads the
+ * exact triangle. */
+bool horizonator_pick_batch(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                            int m, const horizonator_pixel_t* pixels, horizonator_ground_t* ground);
+
 /* Per-kernel device times.  While enabled, every render records CUDA events around each of
  * its kernels on the stream it runs on.  horizonator_profile_read() waits for them and reports
  * the MEAN duration in milliseconds per render of: out_ms[0] k_prepare (clear + axis tables),
