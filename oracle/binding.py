@@ -97,6 +97,12 @@ class Oracle:
             L.oracle_set_threads.argtypes = [vp, i]
             L.oracle_set_curvature.argtypes = [vp, f]
             L.oracle_set_seam_wrap.argtypes = [vp, b]
+            L.oracle_vertex_stage.restype = f
+            L.oracle_vertex_stage.argtypes = [vp, vp]
+            L.oracle_read_keys.restype = b
+            L.oracle_read_keys.argtypes = [vp, i, i, f, f, f, f, vp, vp]
+            L.glp_draw_keys.restype = i
+            L.glp_draw_keys.argtypes = [vp, i, i, vp, i, f, vp, i]
             cls._lib = L
         return cls._lib
 
@@ -152,8 +158,7 @@ class Oracle:
         L = self.lib()
         return np.array([[L.oracle_dem_sample(self.h, i, j) for i in range(n)] for j in range(n)], dtype=np.int16)
 
-    def render(self, az_deg0, az_deg1, lat=-1000., lon=-1000., znear=100., zfar=40000.,
-               znear_color=-1., zfar_color=-1.):
+    def _set_view(self, az_deg0, az_deg1, lat, lon, znear, zfar, znear_color, zfar_color):
         L = self.lib()
         if znear_color < 0:
             znear_color = znear
@@ -164,10 +169,69 @@ class Oracle:
             self.move(lat, lon)
         if not L.oracle_set_zextents(self.h, znear, zfar, znear_color, zfar_color):
             raise RuntimeError("oracle_set_zextents() failed")
+
+    def vertex_stage(self, az_deg0, az_deg1, lat=-1000., lon=-1000., znear=100., zfar=40000.,
+                     znear_color=-1., zfar_color=-1.):
+        """This oracle's vertex stage for the view render() would draw: (glp_vtx_t records [j * N + i], seam period)"""
+        self._set_view(az_deg0, az_deg1, lat, lon, znear, zfar, znear_color, zfar_color)
+        n = 2 * self.dem_geometry()["radius_cells"]
+        from oracle.vertex import VTX
+        vtx = np.empty(n * n, VTX)
+        period = self.lib().oracle_vertex_stage(self.h, vtx.ctypes.data)
+        return vtx, period
+
+    def render(self, az_deg0, az_deg1, lat=-1000., lon=-1000., znear=100., zfar=40000.,
+               znear_color=-1., zfar_color=-1.):
+        L = self.lib()
+        self._set_view(az_deg0, az_deg1, lat, lon, znear, zfar, znear_color, zfar_color)
         image = np.empty((self.H, self.W, 3), np.uint8)
         ranges = np.empty((self.H, self.W), np.float32)
         assert L.oracle_render_offscreen(self.h, image.ctypes.data, ranges.ctypes.data)
         return image, ranges
+
+
+KEY_Q_SHIFT, KEY_ID_MASK, Z24_MAX = 37, 0x1FFFFFFF, 0xFFFFFF     # oracle/gl_pipeline.h
+
+
+def draw_keys(vtx, N, W, H, seam_period=0.0, levels=None, threads=None):
+    """glp_draw_keys(): the visibility key of every pixel ((H, W) uint64, GL row order, bottom row first) of every
+    triangle of the N x N vertices vtx (oracle.vertex.VTX records [j * N + i]), unculled; levels: int8 [tj][ti] level
+    of detail per tile (oracle.vertex.tile_levels), None = the reference's mesh"""
+    from oracle.vertex import VTX, n_tiles
+    vtx = np.ascontiguousarray(vtx, VTX)
+    assert vtx.shape == (N * N,)
+    if levels is not None:
+        levels = np.ascontiguousarray(levels, np.int8)
+        assert levels.shape == (n_tiles(N), n_tiles(N))
+    keys = np.empty((H, W), np.uint64)
+    assert Oracle.lib().glp_draw_keys(keys.ctypes.data, W, H, vtx.ctypes.data, N, seam_period,
+                                      None if levels is None else levels.ctypes.data, threads or os.cpu_count() or 1)
+    return keys
+
+
+def read_keys(keys, az_deg0, az_deg1, znear, zfar):
+    """image (H, W, 3) and ranges (H, W) of keys, top row first, by oracle_render_offscreen()'s read-back"""
+    H, W = keys.shape
+    keys = np.ascontiguousarray(keys, np.uint64)
+    image = np.empty((H, W, 3), np.uint8)
+    ranges = np.empty((H, W), np.float32)
+    assert Oracle.lib().oracle_read_keys(keys.ctypes.data, W, H, az_deg0, az_deg1, znear, zfar, image.ctypes.data,
+                                         ranges.ctypes.data)
+    return image, ranges
+
+
+def key_triangles(keys, N, levels=None):
+    """(H, W) uint32, top row first: the triangle number each key holds, with the level of detail of its cell's tile
+    in bits [30:29] as horizonator_pick_batch() reports it; 0xFFFFFFFF where nothing was drawn"""
+    from oracle.vertex import LOD_SHIFT, TILE_CELLS
+    keys = keys[::-1]
+    sky = (keys >> np.uint64(KEY_Q_SHIFT)) >= Z24_MAX
+    tri = ((keys >> np.uint64(8)) & np.uint64(KEY_ID_MASK)).astype(np.uint32)
+    if levels is not None:
+        cell = tri >> 1
+        tj, ti = (cell // (N - 1)) // TILE_CELLS, (cell % (N - 1)) // TILE_CELLS
+        tri |= levels[np.where(sky, 0, tj), np.where(sky, 0, ti)].astype(np.uint32) << LOD_SHIFT
+    return np.where(sky, np.uint32(0xFFFFFFFF), tri)
 
 
 class Reference:

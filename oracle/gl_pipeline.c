@@ -134,13 +134,6 @@ void glp_read_depth_float(const glp_framebuffer_t* fb, int x, int y, int w, int 
 
 /* ---------------------------------------------------------------- primitive stages */
 
-typedef struct
-{
-    float x_ndc;         /* for the geometry stage */
-    float xw, yw, zw;    /* window coordinates (F1) */
-    float r;
-} glp_vtx_t;
-
 #define SUBPIXEL   256
 #define GUARD_PX   2097152.0f   /* 2^21 (F5) */
 
@@ -151,9 +144,18 @@ static inline int64_t snap(float a)                                          /* 
     return (int64_t)t;
 }
 
-/* pixel target: (q<<8)|r8 per pixel, so a private buffer is one word per pixel */
+/* Where draw_one writes a fragment.  zr != NULL: (q<<8)|r8 per pixel under GL_LESS, so a private buffer is one word
+ * per pixel.  Otherwise keys: the visibility key of triangle `id` (see GLP_KEY_Q_SHIFT), kept where it is the
+ * minimum. */
+typedef struct
+{
+    uint32_t* zr;
+    uint64_t* keys;
+    uint64_t  id;
+} glp_target_t;
+
 static inline void
-draw_one(uint32_t* zr, int W, int H, const glp_vtx_t* v0, const glp_vtx_t* v1, const glp_vtx_t* v2, float seam_period)
+draw_one(const glp_target_t* tg, int W, int H, const glp_vtx_t* v0, const glp_vtx_t* v1, const glp_vtx_t* v2, float seam_period)
 {
     /* geometry.glsl:21-27 */
     float xmax = fmaxf(fmaxf(v0->x_ndc, v1->x_ndc), v2->x_ndc);
@@ -174,7 +176,7 @@ draw_one(uint32_t* zr, int W, int H, const glp_vtx_t* v0, const glp_vtx_t* v1, c
                     if(copy == 2) c[k].x_ndc -= seam_period;
                     c[k].xw = c[k].x_ndc * halfW + halfW;
                 }
-                draw_one(zr, W, H, &c[0], &c[1], &c[2], 0.0f);
+                draw_one(tg, W, H, &c[0], &c[1], &c[2], 0.0f);
             }
         }
         return;
@@ -249,13 +251,19 @@ draw_one(uint32_t* zr, int W, int H, const glp_vtx_t* v0, const glp_vtx_t* v1, c
             if(!(zw >= 0.0f && zw <= 1.0f)) continue;                       /* F5 */
 
             const uint32_t q = (uint32_t)((double)zw * (double)GLP_Z24_MAX + 0.5);   /* F7 */
-            uint32_t* dst = &zr[(size_t)py * W + px];
-            if(!(q < (*dst >> 8))) continue;                                /* GL_LESS */
+            const size_t p = (size_t)py * W + px;
+            if(tg->zr ? !(q < (tg->zr[p] >> 8))                             /* GL_LESS */
+                      : (q >= GLP_Z24_MAX || q > (uint32_t)(tg->keys[p] >> GLP_KEY_Q_SHIFT))) continue;
 
             float r = v0->r + (drdx * ddx + drdy * ddy);                    /* fragment.glsl:16 */
             r = fmaxf(fminf(r, 1.0f), 0.0f);
             const uint32_t r8 = (uint32_t)(r * 255.0f + 0.5f);              /* F8 */
-            *dst = (q << 8) | r8;
+            if(tg->zr) tg->zr[p] = (q << 8) | r8;
+            else
+            {
+                const uint64_t key = ((uint64_t)q << GLP_KEY_Q_SHIFT) | (tg->id << 8) | r8;
+                if(key < tg->keys[p]) tg->keys[p] = key;
+            }
         }
     }
 }
@@ -276,29 +284,20 @@ triangle_indices(const uint32_t* indices, int64_t t, int gw, int64_t* i0, int64_
     else             { *i1 = j * gw + (i + 1);       *i2 = (j + 1) * gw + (i + 1); }
 }
 
-void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
-                        const int16_t* vertices_ijz, int64_t nvertices,
-                        const uint32_t* indices, int64_t ntriangles,
-                        int grid_width, int nthreads)
+/* period of x_ndc for the opt-in seam wrap: az_ndc_per_rad (vertex.glsl:139-150) * 2*pi; 0 without it */
+float glp_seam_period(const glp_uniforms_t* u)
 {
-    const int W = fb->width, H = fb->height;
-    if(nthreads < 1) nthreads = 1;
+    if(!u->seam_wrap) return 0.0f;
+    float az_rad0 = glsl_radians(u->az_deg0), az_rad1 = glsl_radians(u->az_deg1);
+    az_rad1 = unwrap_near_rad(az_rad1 - az_rad0, pi) + az_rad0;
+    return 2.0f / (az_rad1 - az_rad0) * 2.f * pi;
+}
 
-    glp_vtx_t* vtx = (glp_vtx_t*)malloc((size_t)nvertices * sizeof(glp_vtx_t));
-    if(!vtx) return;
-
+void glp_vertices(const glp_uniforms_t* u, const int16_t* vertices_ijz, int64_t nvertices, int W, int H,
+                  glp_vtx_t* vtx, int nthreads)
+{
     const float halfW = 0.5f * (float)W, halfH = 0.5f * (float)H;
-
-    /* period of x_ndc for the opt-in seam wrap: az_ndc_per_rad (vertex.glsl:139-150) * 2*pi */
-    float seam_period = 0.0f;
-    if(u->seam_wrap)
-    {
-        float az_rad0 = glsl_radians(u->az_deg0), az_rad1 = glsl_radians(u->az_deg1);
-        az_rad1 = unwrap_near_rad(az_rad1 - az_rad0, pi) + az_rad0;
-        seam_period = 2.0f / (az_rad1 - az_rad0) * 2.f * pi;
-    }
-
-    #pragma omp parallel for num_threads(nthreads) schedule(static)
+    #pragma omp parallel for num_threads(nthreads < 1 ? 1 : nthreads) schedule(static)
     for(int64_t v = 0; v < nvertices; v++)
     {
         glp_vsout_t o;
@@ -311,6 +310,20 @@ void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
         vtx[v].zw = o.z_ndc * 0.5f + 0.5f;
         vtx[v].r  = o.r;
     }
+}
+
+void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
+                        const int16_t* vertices_ijz, int64_t nvertices,
+                        const uint32_t* indices, int64_t ntriangles,
+                        int grid_width, int nthreads)
+{
+    const int W = fb->width, H = fb->height;
+    if(nthreads < 1) nthreads = 1;
+
+    glp_vtx_t* vtx = (glp_vtx_t*)malloc((size_t)nvertices * sizeof(glp_vtx_t));
+    if(!vtx) return;
+    glp_vertices(u, vertices_ijz, nvertices, W, H, vtx, nthreads);
+    const float seam_period = glp_seam_period(u);
 
     const size_t npix = (size_t)W * H;
 
@@ -321,11 +334,12 @@ void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
 
     if(nthreads == 1)
     {
+        const glp_target_t tg = { target, NULL, 0 };
         for(int64_t t = 0; t < ntriangles; t++)
         {
             int64_t i0, i1, i2;
             triangle_indices(indices, t, grid_width, &i0, &i1, &i2);
-            draw_one(target, W, H, &vtx[i0], &vtx[i1], &vtx[i2], seam_period);
+            draw_one(&tg, W, H, &vtx[i0], &vtx[i1], &vtx[i2], seam_period);
         }
     }
     else
@@ -341,12 +355,13 @@ void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
             uint32_t* mine = (uint32_t*)malloc(npix * sizeof(uint32_t));
             for(size_t p = 0; p < npix; p++) mine[p] = (GLP_Z24_MAX << 8);
             priv[tid] = mine;
+            const glp_target_t tg = { mine, NULL, 0 };
             const int64_t t0 = ntriangles * tid / nt, t1 = ntriangles * (tid + 1) / nt;
             for(int64_t t = t0; t < t1; t++)
             {
                 int64_t i0, i1, i2;
                 triangle_indices(indices, t, grid_width, &i0, &i1, &i2);
-                draw_one(mine, W, H, &vtx[i0], &vtx[i1], &vtx[i2], seam_period);
+                draw_one(&tg, W, H, &vtx[i0], &vtx[i1], &vtx[i2], seam_period);
             }
         }
         /* merge in draw order with the same strict LESS */
@@ -373,4 +388,81 @@ void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
 
     free(target);
     free(vtx);
+}
+
+int glp_draw_keys(uint64_t* keys, int W, int H, const glp_vtx_t* vtx, int N, float seam_period,
+                  const int8_t* tile_levels, int nthreads)
+{
+    if(nthreads < 1) nthreads = 1;
+    const size_t npix = (size_t)W * H;
+    const int nt = (N - 1 + GLP_TILE_CELLS - 1) / GLP_TILE_CELLS;
+    uint64_t** priv = (uint64_t**)calloc(nthreads, sizeof(uint64_t*));
+    if(!priv) return 0;
+    int ok = 1;
+    #pragma omp parallel num_threads(nthreads)
+    {
+#ifdef _OPENMP
+        const int tid = omp_get_thread_num();
+#else
+        const int tid = 0;
+#endif
+        uint64_t* mine = (uint64_t*)malloc(npix * sizeof(uint64_t));
+        if(!mine) ok = 0;
+        else for(size_t p = 0; p < npix; p++) mine[p] = GLP_KEY_CLEAR;
+        priv[tid] = mine;
+        #pragma omp for schedule(dynamic, 1)
+        for(int tj = 0; tj < nt; tj++)
+        {
+            if(!mine) continue;
+            for(int ti = 0; ti < nt; ti++)
+            {
+                const int l = tile_levels ? tile_levels[(size_t)tj * nt + ti] : 0, s = 1 << l;
+                /* the last (N - 1) mod s cells of a row or column are not drawn at level l */
+                const int jend = GLP_TILE_CELLS * (tj + 1) < N - s ? GLP_TILE_CELLS * (tj + 1) : N - s;
+                const int iend = GLP_TILE_CELLS * (ti + 1) < N - s ? GLP_TILE_CELLS * (ti + 1) : N - s;
+                for(int j = GLP_TILE_CELLS * tj; j < jend; j += s)
+                    for(int i = GLP_TILE_CELLS * ti; i < iend; i += s)
+                    {
+                        const glp_vtx_t* a = vtx + (size_t)j * N + i;             /* (j, i) */
+                        const glp_vtx_t* b = a + s;                               /* (j, i+s) */
+                        const glp_vtx_t* c = a + (size_t)s * N;                   /* (j+s, i) */
+                        const glp_vtx_t* d = c + s;                               /* (j+s, i+s) */
+                        const uint64_t cell = (uint64_t)j * (uint64_t)(N - 1) + (uint64_t)i;
+                        /* horizonator-lib.c:496-508 with vertices s apart: (j,i),(j+s,i+s),(j+s,i) and (j,i),(j,i+s),(j+s,i+s) */
+                        const glp_target_t t0 = { NULL, mine, (2 * cell) & GLP_KEY_ID_MASK };
+                        const glp_target_t t1 = { NULL, mine, (2 * cell + 1) & GLP_KEY_ID_MASK };
+                        draw_one(&t0, W, H, a, d, c, seam_period);
+                        draw_one(&t1, W, H, a, b, d, seam_period);
+                    }
+            }
+        }
+    }
+    if(ok)
+    {
+        /* the minimum over all fragments: the order of the triangles, and so the number of threads, cannot matter */
+        #pragma omp parallel for num_threads(nthreads) schedule(static)
+        for(size_t p = 0; p < npix; p++)
+        {
+            uint64_t cur = GLP_KEY_CLEAR;
+            for(int k = 0; k < nthreads; k++)
+                if(priv[k] && priv[k][p] < cur) cur = priv[k][p];
+            keys[p] = cur;
+        }
+    }
+    for(int k = 0; k < nthreads; k++) free(priv[k]);
+    free(priv);
+    return ok;
+}
+
+void glp_keys_to_framebuffer(const uint64_t* keys, glp_framebuffer_t* fb)
+{
+    glp_clear(fb);
+    const size_t n = (size_t)fb->width * fb->height;
+    for(size_t p = 0; p < n; p++)
+    {
+        const uint32_t q = (uint32_t)(keys[p] >> GLP_KEY_Q_SHIFT);
+        if(q >= GLP_Z24_MAX) continue;
+        fb->z24[p] = q;
+        fb->rgb[3*p+0] = (uint8_t)(keys[p] & 0xFF); fb->rgb[3*p+1] = 0; fb->rgb[3*p+2] = 0;
+    }
 }

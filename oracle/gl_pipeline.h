@@ -67,6 +67,24 @@ typedef struct
 
 #define GLP_Z24_MAX 0xFFFFFFu
 
+/* one vertex after the vertex stage and the viewport transform (F1): gl_Position.x for the geometry stage, the window
+ * coordinates, and the red channel */
+typedef struct
+{
+    float x_ndc;
+    float xw, yw, zw;
+    float r;
+} glp_vtx_t;
+
+/* Visibility key of glp_draw_keys(), one per pixel: the renderer's (horizonator_b200/csrc/hz_device.h) without its
+ * epoch bits.  [60:37] q (F7), [36:8] triangle number & GLP_KEY_ID_MASK, [7:0] r8 (F8).  The minimum over a pixel's
+ * fragments is GL_LESS in draw order (nearest q, equal q: lowest triangle number); a fragment with q = GLP_Z24_MAX
+ * cannot pass GL_LESS against the cleared depth and is dropped. */
+#define GLP_KEY_Q_SHIFT 37
+#define GLP_KEY_ID_MASK 0x1FFFFFFFull
+#define GLP_KEY_CLEAR   0x1FFFFFFFFFFFFFFFull    /* nothing drawn: q = GLP_Z24_MAX */
+#define GLP_TILE_CELLS  32                       /* tiles of the level-of-detail rule (HZ_TILE_CELLS) */
+
 void glp_vertex_stage(const glp_uniforms_t* u, float vi, float vj, float vz, glp_vsout_t* out);
 
 int  glp_framebuffer_alloc(glp_framebuffer_t* fb, int width, int height);
@@ -86,6 +104,24 @@ void glp_draw_triangles(glp_framebuffer_t* fb, const glp_uniforms_t* u,
                         const int16_t* vertices_ijz, int64_t nvertices,
                         const uint32_t* indices, int64_t ntriangles,
                         int grid_width, int nthreads);
+
+/* the vertex stage and the viewport transform of glp_draw_triangles() for nvertices int16 (i,j,z) vertices */
+void glp_vertices(const glp_uniforms_t* u, const int16_t* vertices_ijz, int64_t nvertices, int W, int H,
+                  glp_vtx_t* vtx, int nthreads);
+/* period of x_ndc of the opt-in seam wrap, 0 when it is off */
+float glp_seam_period(const glp_uniforms_t* u);
+
+/* Every triangle of the dense grid of N x N vertices vtx[j * N + i], rasterised by the same rules F2-F8 as
+ * glp_draw_triangles() (and the seam copies when seam_period > 0), into one visibility key per pixel of a W x H
+ * target, bottom row first.  No culling of any kind.  tile_levels == NULL: the reference's mesh.  Otherwise the
+ * level of detail l of each tile of GLP_TILE_CELLS x GLP_TILE_CELLS cells, [tj][ti] over ceil((N-1)/32) tiles per
+ * side: the tile draws its cells (j, i) with j and i multiples of s = 2^l and at most N-1-s, triangles of vertices s
+ * apart, numbered like the cell (j, i) of the dense grid.  Threads draw into private buffers that are merged by min(),
+ * so the result does not depend on nthreads.  0 if memory ran out. */
+int glp_draw_keys(uint64_t* keys, int W, int H, const glp_vtx_t* vtx, int N, float seam_period,
+                  const int8_t* tile_levels, int nthreads);
+/* the framebuffer as GL would hold it after drawing those keys' fragments into a cleared one */
+void glp_keys_to_framebuffer(const uint64_t* keys, glp_framebuffer_t* fb);
 
 /* glReadPixels(GL_BGR, GL_UNSIGNED_BYTE), pack alignment 1, bottom row first */
 void glp_read_bgr(const glp_framebuffer_t* fb, uint8_t* out);

@@ -212,20 +212,14 @@ void oracle_get_viewer(const oracle_context_t* c, float o[4])
     o[0] = c->u.viewer_cell_i; o[1] = c->u.viewer_cell_j; o[2] = c->u.viewer_z; o[3] = c->u.cos_viewer_lat;
 }
 
-/* horizonator-lib.c:911-1051 */
-bool oracle_render_offscreen(oracle_context_t* c, char* image, float* ranges)
+/* horizonator-lib.c:936-1048: image and ranges out of the framebuffer, top row first */
+static void read_back(const glp_framebuffer_t* fb, const glp_uniforms_t* u, char* image, float* ranges)
 {
-    const int W = c->W, H = c->H, N = 2 * c->R;
-
-    /* :887-899 redraw: clear, then every triangle of the dense grid in index order */
-    glp_clear(&c->fb);
-    glp_draw_triangles(&c->fb, &c->u, c->vertices, (int64_t)N * N,
-                       NULL, (int64_t)2 * (N - 1) * (N - 1), N, c->nthreads);
-
+    const int W = fb->width, H = fb->height;
     if(image)                                                       /* :936-959 */
     {
         uint8_t* tmp = (uint8_t*)malloc((size_t)W * H * 3);
-        glp_read_bgr(&c->fb, tmp);
+        glp_read_bgr(fb, tmp);
         for(int y = 0; y < H; y++)   /* GL row y -> image row H-1-y */
             memcpy(image + (size_t)(H - 1 - y) * W * 3, tmp + (size_t)y * W * 3, (size_t)W * 3);
         free(tmp);
@@ -233,10 +227,10 @@ bool oracle_render_offscreen(oracle_context_t* c, char* image, float* ranges)
     if(ranges)                                                      /* :960-1048 */
     {
         float* depth = (float*)malloc((size_t)W * H * sizeof(float));
-        glp_read_depth_float(&c->fb, 0, 0, W, H, depth);
+        glp_read_depth_float(fb, 0, 0, W, H, depth);
 
-        const float az_deg0 = c->u.az_deg0, az_deg1 = c->u.az_deg1;
-        const float znear = c->u.znear, zfar = c->u.zfar;
+        const float az_deg0 = u->az_deg0, az_deg1 = u->az_deg1;
+        const float znear = u->znear, zfar = u->zfar;
         const float aspect = (float)W / (float)H;                   /* :1006 */
 
         for(int y = 0; y < H; y++)   /* y = GL row */
@@ -264,6 +258,39 @@ bool oracle_render_offscreen(oracle_context_t* c, char* image, float* ranges)
         }
         free(depth);
     }
+}
+
+/* horizonator-lib.c:911-1051 */
+bool oracle_render_offscreen(oracle_context_t* c, char* image, float* ranges)
+{
+    const int N = 2 * c->R;
+
+    /* :887-899 redraw: clear, then every triangle of the dense grid in index order */
+    glp_clear(&c->fb);
+    glp_draw_triangles(&c->fb, &c->u, c->vertices, (int64_t)N * N,
+                       NULL, (int64_t)2 * (N - 1) * (N - 1), N, c->nthreads);
+    read_back(&c->fb, &c->u, image, ranges);
+    return true;
+}
+
+float oracle_vertex_stage(const oracle_context_t* c, glp_vtx_t* out)
+{
+    const int N = 2 * c->R;
+    glp_vertices(&c->u, c->vertices, (int64_t)N * N, c->W, c->H, out, c->nthreads);
+    return glp_seam_period(&c->u);
+}
+
+bool oracle_read_keys(const uint64_t* keys, int W, int H, float az_deg0, float az_deg1, float znear, float zfar,
+                      char* image, float* ranges)
+{
+    glp_framebuffer_t fb;
+    if(!glp_framebuffer_alloc(&fb, W, H)) return false;
+    glp_uniforms_t u;
+    memset(&u, 0, sizeof(u));
+    u.az_deg0 = az_deg0; u.az_deg1 = az_deg1; u.znear = znear; u.zfar = zfar;
+    glp_keys_to_framebuffer(keys, &fb);
+    read_back(&fb, &u, image, ranges);
+    glp_framebuffer_free(&fb);
     return true;
 }
 

@@ -19,6 +19,8 @@
 #include <stdbool.h>
 #include <stdint.h>
 
+#include "gl_pipeline.h"
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -54,6 +56,16 @@ void oracle_set_seam_wrap(oracle_context_t* ctx, bool on);
 
 /* number of OpenMP threads the draw uses (1 = strictly serial). Default 1. */
 void oracle_set_threads(oracle_context_t* ctx, int nthreads);
+
+/* The exact reference of the renderer (tests/test_exact_reference.py, tests/test_gpu_exact.py): visibility keys drawn
+ * by glp_draw_keys() from any vertex stage, read back by the code of oracle_render_offscreen().
+ * oracle_vertex_stage: this oracle's own vertex stage for the context's (2R)^2 vertices, j outer -> out; returns the
+ * seam period (0 without the seam wrap).
+ * oracle_read_keys: image and ranges (either may be NULL) of a W x H target of keys, bottom row first, as
+ * oracle_render_offscreen() reads them out of its framebuffer for that window and z extents. */
+float oracle_vertex_stage(const oracle_context_t* ctx, glp_vtx_t* out);
+bool  oracle_read_keys(const uint64_t* keys, int W, int H, float az_deg0, float az_deg1, float znear, float zfar,
+                       char* image, float* ranges);
 
 #ifdef __cplusplus
 }
