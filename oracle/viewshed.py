@@ -59,6 +59,37 @@ def lib():
     return _LIB
 
 
+def _cell(x, origin_deg, cells_per_deg, origin_cell):
+    """compute_move's cell coordinate of the float32 angle x (oracle/vertex.py eye())"""
+    F = np.float32
+    return F(F(F(F(x) - F(origin_deg)) * F(cells_per_deg)) - F(origin_cell))
+
+
+def _angle(target, origin_deg, cells_per_deg, origin_cell, below):
+    """The smallest float32 angle whose cell coordinate is >= target, or (below) the largest one whose coordinate is
+    < target; the coordinate does not decrease with the angle."""
+    f = lambda x: _cell(x, origin_deg, cells_per_deg, origin_cell)
+    x = np.float32(origin_deg + (float(target) + origin_cell) / cells_per_deg)
+    while f(x) < target:
+        x = np.nextafter(x, np.float32(np.inf))
+    while f(np.nextafter(x, np.float32(-np.inf))) >= target:
+        x = np.nextafter(x, np.float32(-np.inf))
+    return np.nextafter(x, np.float32(-np.inf)) if below else x
+
+
+def eye_at(oracle, ci, cj):
+    """(lat, lon), float32 values, of an eye at cell coordinates (ci, cj) of `oracle`'s square.  Each coordinate is a
+    number (the smallest reachable coordinate >= it: itself where it is reachable) or ("below", t) (the largest
+    reachable coordinate < t).  The caller checks through oracle.viewer() what the eye came to."""
+    g = oracle.dem_geometry()
+    (lon0, lat0), (i0, j0), cpd = g["origin_dem_lon_lat"], g["origin_dem_cellij"], g["cells_per_deg"]
+
+    def one(c, origin_deg, origin_cell):
+        below = isinstance(c, tuple)
+        return float(_angle(c[1] if below else c, origin_deg, cpd, origin_cell, below))
+    return one(cj, lat0, j0), one(ci, lon0, i0)
+
+
 def unpack_mask(words):
     """(..., N, W32) uint32 viewshed words -> (..., N, N) bool (cell i of row j = bit i & 31 of word [j][i >> 5])."""
     words = np.ascontiguousarray(words, dtype="<u4")

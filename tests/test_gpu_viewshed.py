@@ -100,6 +100,7 @@ def test_counts_are_the_sum_of_the_masks_and_accumulate(hz, tiles_c1):
     views = [(C1_LAT + 0.01 * k, C1_LON - 0.007 * k) for k in range(-4, 5)]
     masks = torch.empty((len(views), N, (N + 31) // 32), dtype=torch.int32, device="cuda")
     counts = torch.zeros((N, N), dtype=torch.int32, device="cuda")
+    torch.cuda.synchronize()                        # the context's own stream does not wait for torch's fill
     h.viewshed_device(views, d_masks=masks.data_ptr(), d_counts=counts.data_ptr())
     m = unpack_mask(masks.cpu().numpy().view(np.uint32))
     want = m.sum(axis=0)
@@ -117,6 +118,7 @@ def test_degenerate_and_invalid_arguments_write_nothing(hz, tiles_c1):
     ctx = C.byref(h.context)
     masks = torch.full((2, N, (N + 31) // 32), 0x5A5A5A5A, dtype=torch.int32, device="cuda")
     counts = torch.full((N, N), 7, dtype=torch.int32, device="cuda")
+    torch.cuda.synchronize()
     lib = hz.lib
     ok = [(C1_LAT, C1_LON)]
     assert lib.horizonator_viewshed_device(ctx, 0, h._eyes(ok), 0., masks.data_ptr(), counts.data_ptr(), None)
