@@ -174,6 +174,8 @@ def _signatures():
         "horizonator_profile_read": (b, [ctx, P(f * 6), P(i)]),
         "horizonator_viewshed_device": (b, [ctx, i, P(view_t), f, vp, vp, vp]),
         "horizonator_viewshed": (b, [ctx, i, P(view_t), f, vp, vp]),
+        "horizonator_viewshed_heights_device": (b, [ctx, i, P(view_t), vp, vp, vp]),
+        "horizonator_viewshed_heights": (b, [ctx, i, P(view_t), vp, vp]),
         "horizonator_annotate_batch_device": (b, [ctx, i, P(view_t), i, vp, vp, vp, vp, vp]),
         "horizonator_annotate_batch": (b, [ctx, i, P(view_t), i, vp, vp]),
         "horizonator_skyline_match_device": (b, [ctx, i, P(view_t), vp, vp, i, vp, f, b, vp, vp]),
@@ -484,6 +486,32 @@ class horizonator:
         added to.  Integer device addresses, either may be 0 (not both); stream as render_batch_device."""
         _check(lib.horizonator_viewshed_device, C.byref(self._ctx), len(views), self._eyes(views), float(target_height),
                d_masks or None, d_counts or None, stream or None)
+
+    def viewshed_heights(self, views, least=False):
+        """Host arrays: heights (n, N, N) float32, [j north][i east], how far above the ground a point at each vertex
+        must rise for the view to see it (+0 where the ground itself is seen, +inf where no ray reaches the vertex);
+        with least=True also (N, N) float32, the least of them over the views (horizonator-batch.h)."""
+        n, N = len(views), self.size
+        h = np.empty((n, N, N), np.float32)
+        lst = np.full((N, N), np.inf, np.float32) if least else None
+        _check(lib.horizonator_viewshed_heights, C.byref(self._ctx), n, self._eyes(views), h.ctypes.data,
+               lst.ctypes.data if least else None)
+        return (h, lst) if least else h
+
+    def viewshed_least_height(self, views):
+        """(N, N) float32: for every vertex the least height above the ground at which any of the views sees a point
+        there -- below it the point stays hidden from all of them.  No per-view array is made."""
+        N = self.size
+        lst = np.full((N, N), np.inf, np.float32)
+        _check(lib.horizonator_viewshed_heights, C.byref(self._ctx), len(views), self._eyes(views), None,
+               lst.ctypes.data)
+        return lst
+
+    def viewshed_heights_device(self, views, d_heights=0, d_least=0, stream=0):
+        """Device-pointer variant: d_heights (n, N, N) float32, overwritten; d_least (N, N) float32, min-folded (fill
+        it with +inf first).  Integer device addresses, either may be 0 (not both); stream as render_batch_device."""
+        _check(lib.horizonator_viewshed_heights_device, C.byref(self._ctx), len(views), self._eyes(views),
+               d_heights or None, d_least or None, stream or None)
 
 
     # labels of points of interest (horizonator_annotate_batch*: which POIs each view sees, and where)

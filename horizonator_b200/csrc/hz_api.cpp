@@ -312,10 +312,12 @@ struct Slot
     size_t prof_used = 0;
 
     // viewsheds, allocated by the first viewshed call that needs them: the masks of one chunk of views for calls that
-    // want only counts or want the masks in host memory, and the counts of the host-memory call.  A call's stream
-    // waits for `vs_done` of the call before it, which may have been queued on another stream and use the same scratch.
+    // want only counts or want the masks in host memory (or, for the host-memory heights call, the per-view heights of
+    // one chunk), the counts of the host-memory call and its least heights.  A call's stream waits for `vs_done` of the
+    // call before it, which may have been queued on another stream and use the same scratch.
     GrowBuffer<uint32_t> d_vs_masks;
     GrowBuffer<uint32_t> d_vs_counts;
+    GrowBuffer<uint32_t> d_vs_least;
     EventHandle          vs_done;
 
     // the inputs of the host-memory calls (horizonator_annotate_batch: POIs, horizonator_skyline_match: samples),
@@ -1595,15 +1597,29 @@ static bool render_batch_common(const horizonator_context_t* ctx, Slot* s, int n
 
 // ---- viewsheds (horizonator-batch.h) -------------------------------------------------------------------------------
 //
-// The views go in chunks of up to HZ_VS_MAX_VIEWS, each one k_viewshed launch (gridDim.y = view) into its masks --
-// the caller's, or the scratch when the masks are not wanted in device memory -- then k_viewshed_count into the
-// counts and/or a copy of the masks to host memory, all on `st`.
+// Masks: the views go in chunks of up to HZ_VS_MAX_VIEWS, each one k_viewshed launch (gridDim.y = view) into its
+// masks -- the caller's, or the scratch when the masks are not wanted in device memory -- then k_viewshed_count into
+// the counts and/or a copy of the masks to host memory, all on `st`.
+// Heights (`heights`; d_masks / d_counts / h_masks then stand for the per-view heights in device memory, the least
+// heights and the per-view heights in host memory): the same chunks, each one k_viewshed_heights launch.  Per-view
+// heights go to the caller's device array or the scratch, filled with +inf first, and k_viewshed_least folds them
+// into the least heights; without per-view heights the walk's minima go straight into the least heights.  The
+// scratch holds at most HZ_VS_HEIGHTS_SCRATCH bytes, so the host call's chunks may be smaller.
+constexpr size_t HZ_VS_HEIGHTS_SCRATCH = (size_t)2 << 30;
+
 static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, const horizonator_view_t* views,
                             float target_height, uint32_t* d_masks, uint32_t* d_counts, uint32_t* h_masks,
-                            cudaStream_t st)
+                            cudaStream_t st, bool heights = false)
 {
     const int N = s->N, w32 = (N + 31) / 32;
-    const size_t mwords = (size_t)N * w32;
+    const size_t cells = (size_t)N * N;
+    // per view: the words of a mask, or the cells of a view's heights
+    const size_t mwords = heights ? cells : (size_t)N * w32;
+    if(heights && cells >= 0xffffffffu)
+    {
+        MSG("viewshed heights: a square of %d x %d vertices is too large (N * N must be below 2^32 - 1)", N, N);
+        return false;
+    }
     std::vector<HzViewshedEye> eyes((size_t)n);
     for(int k = 0; k < n; k++)
     {
@@ -1621,15 +1637,24 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
     }
     if(n == 0) return true;
 
-    const int chunk = n < HZ_VS_MAX_VIEWS ? n : HZ_VS_MAX_VIEWS;
+    // the heights' scratch (per-view heights into host memory) is bounded; the least-only walk needs none
+    const bool per_view = !heights || d_masks != nullptr || h_masks != nullptr;
+    int cap = HZ_VS_MAX_VIEWS;
+    if(heights && d_masks == nullptr && h_masks != nullptr)
+    {
+        const size_t fit = HZ_VS_HEIGHTS_SCRATCH / (mwords * sizeof(uint32_t));
+        cap = fit < 1 ? 1 : (fit < (size_t)cap ? (int)fit : cap);
+    }
+    const int chunk = n < cap ? n : cap;
     if(!s->vs_done) { if(empty_handle(s->vs_done = make_event(), "cudaEventCreate")) return false; }
     else CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
-    if(d_masks == nullptr && s->d_vs_masks.cap < (size_t)chunk * mwords)
+    if(per_view && d_masks == nullptr && s->d_vs_masks.cap < (size_t)chunk * mwords)
     {
         CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
         if(s->d_vs_masks.grow((size_t)chunk * mwords) != cudaSuccess)
         {
-            MSG("Could not allocate the viewshed masks of %d views (%zu MB)", chunk, (size_t)chunk * mwords * 4 >> 20);
+            MSG("Could not allocate the viewshed %s of %d views (%zu MB)", heights ? "heights" : "masks", chunk,
+                (size_t)chunk * mwords * 4 >> 20);
             return false;
         }
     }
@@ -1644,9 +1669,25 @@ static bool viewshed_common(const horizonator_context_t* ctx, Slot* s, int n, co
         const int m = n - k0 < chunk ? n - k0 : chunk;
         p.masks = d_masks ? d_masks + (size_t)k0 * mwords : s->d_vs_masks.get();
         for(int k = 0; k < m; k++) p.eye[k] = eyes[(size_t)(k0 + k)];
-        CUDA_TRY(cudaMemsetAsync(p.masks, 0, (size_t)m * mwords * sizeof(uint32_t), st));
-        CUDA_TRY(hz_launch_viewshed(p, m, st));
-        if(d_counts) CUDA_TRY(hz_launch_viewshed_count(p.masks, m, N, w32, d_counts, st));
+        if(heights && !per_view)
+        {
+            p.heights = d_counts; p.heights_stride = 0;
+            CUDA_TRY(hz_launch_viewshed_heights(p, m, st));
+            continue;
+        }
+        if(heights)
+        {
+            p.heights = p.masks; p.heights_stride = mwords;
+            CUDA_TRY(hz_launch_fill_u32(p.heights, (size_t)m * mwords, 0x7f800000u, st));         // +inf
+            CUDA_TRY(hz_launch_viewshed_heights(p, m, st));
+            if(d_counts) CUDA_TRY(hz_launch_viewshed_least(p.heights, m, cells, d_counts, st));
+        }
+        else
+        {
+            CUDA_TRY(cudaMemsetAsync(p.masks, 0, (size_t)m * mwords * sizeof(uint32_t), st));
+            CUDA_TRY(hz_launch_viewshed(p, m, st));
+            if(d_counts) CUDA_TRY(hz_launch_viewshed_count(p.masks, m, N, w32, d_counts, st));
+        }
         if(h_masks)
             CUDA_TRY(cudaMemcpyAsync(h_masks + (size_t)k0 * mwords, p.masks, (size_t)m * mwords * sizeof(uint32_t),
                                      cudaMemcpyDeviceToHost, st));
@@ -1697,6 +1738,53 @@ bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizon
         if(!viewshed_common(ctx, s, n, views, target_height_m, nullptr, counts ? s->d_vs_counts.get() : nullptr, masks, st))
             return false;
         if(counts && n > 0) CUDA_TRY(cudaMemcpyAsync(counts, s->d_vs_counts.get(), cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        return true;
+    });
+}
+
+bool horizonator_viewshed_heights_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                         float* d_heights, float* d_least, void* stream)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
+    if(d_heights == nullptr && d_least == nullptr)
+    {
+        MSG("horizonator_viewshed_heights_device: neither heights nor least asked for");
+        return false;
+    }
+    return on_stream(*s, stream, [&](cudaStream_t st) {
+        return viewshed_common(ctx, s, n, views, 0.f, (uint32_t*)d_heights, (uint32_t*)d_least, nullptr, st, true);
+    });
+}
+
+bool horizonator_viewshed_heights(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                  float* heights, float* least)
+{
+    Slot* s = slot_of(ctx);
+    if(s == nullptr || n < 0 || (n > 0 && views == nullptr)) return false;
+    if(heights == nullptr && least == nullptr)
+    {
+        MSG("horizonator_viewshed_heights: neither heights nor least asked for");
+        return false;
+    }
+    return on_stream(*s, nullptr, [&](cudaStream_t st) {
+        const size_t cells = (size_t)s->N * s->N;
+        if(least && n > 0 && s->d_vs_least.cap < cells)
+        {
+            if(s->vs_done) CUDA_TRY(cudaEventSynchronize(s->vs_done.get()));
+            if(s->d_vs_least.grow(cells) != cudaSuccess)
+            {
+                MSG("Could not allocate the viewshed least heights (%zu MB)", cells * 4 >> 20);
+                return false;
+            }
+        }
+        // the upload waits for whatever an earlier call still does with the same buffer
+        if(least && n > 0 && s->vs_done) CUDA_TRY(cudaStreamWaitEvent(st, s->vs_done.get(), 0));
+        if(least && n > 0) CUDA_TRY(cudaMemcpyAsync(s->d_vs_least.get(), least, cells * sizeof(float), cudaMemcpyHostToDevice, st));
+        if(!viewshed_common(ctx, s, n, views, 0.f, nullptr, least ? s->d_vs_least.get() : nullptr, (uint32_t*)heights, st,
+                            true))
+            return false;
+        if(least && n > 0) CUDA_TRY(cudaMemcpyAsync(least, s->d_vs_least.get(), cells * sizeof(float), cudaMemcpyDeviceToHost, st));
         return true;
     });
 }

@@ -274,8 +274,19 @@ struct HzViewshed
     float deg_per_cell, curvature, target_height;
     uint32_t* masks;             // view y's mask at masks + y * N * w32, zeroed before the launch
     HzViewshedEye eye[HZ_VS_MAX_VIEWS];
+    // k_viewshed_heights only (after the eyes, so that k_viewshed's parameters sit where they always did): view y's
+    // heights, float patterns, at heights + y * heights_stride, min-folded (0: every view into one N x N array)
+    uint32_t* heights;
+    size_t    heights_stride;
 };
 cudaError_t hz_launch_viewshed(const HzViewshed& p, int nviews, cudaStream_t stream);
+// the heights of the same walk (horizonator_viewshed_heights*); N * N must be below 2^32 - 1
+cudaError_t hz_launch_viewshed_heights(const HzViewshed& p, int nviews, cudaStream_t stream);
+// least[c] = min(least[c], heights[v * cells + c] for v < nviews), on the 32-bit patterns
+cudaError_t hz_launch_viewshed_least(const uint32_t* heights, int nviews, size_t cells, uint32_t* least,
+                                     cudaStream_t stream);
+// out[0 .. n) = value
+cudaError_t hz_launch_fill_u32(uint32_t* out, size_t n, uint32_t value, cudaStream_t stream);
 // counts[j * N + i] += the number of the nviews masks (N * w32 words apart) with cell (i, j) set
 cudaError_t hz_launch_viewshed_count(const uint32_t* masks, int nviews, int N, int w32, uint32_t* counts,
                                      cudaStream_t stream);

@@ -27,6 +27,8 @@
 //   k_pick     (ground points)  the ground point under rendered pixels, from the triangle number in each pixel's key
 //   k_viewshed, k_viewshed_count (viewsheds)  R2 ray casting over the DEM square, one thread per ray -> bit masks;
 //                        masks -> per-vertex counts of the views that see it
+//   k_viewshed_heights, k_viewshed_least, k_fill_u32 (viewshed heights)  the same walk -> per vertex the least height
+//                        above the ground at which it is seen; per-view heights -> their minimum over the views
 //
 // The mesh is never materialised: triangle t of the reference's index buffer is (cell = t>>1, half = t&1)
 // and its vertices are read straight from the int16 mosaic.
@@ -2485,21 +2487,40 @@ __device__ __forceinline__ void hz_vs_collect(uint32_t*& pend, uint32_t& pbits, 
 #define HZ_VS_WARPS  4     /* warps per CTA */
 #define HZ_VS_UNROLL 4     /* steps whose heights are loaded before the first of them is evaluated */
 
+// The heights walk's output (horizonator_viewshed_heights*): every lane of the warp calls it at the same step, `cell`
+// = j * N + i of the vertex its step decides or HZ_VS_NO_CELL, `e` that step's height (>= +0).  Lanes deciding the same vertex
+// merge first (near the eye many rays share one), so one atomicMin per distinct address; the minimum is taken on the
+// 32-bit patterns, which order like the floats for values >= +0 and +inf.
+#define HZ_VS_NO_CELL 0xffffffffu   /* N * N < 2^32 - 1: the host refuses larger squares for heights */
+__device__ __forceinline__ void hz_vs_height_min(uint32_t* out, uint32_t cell, float e)
+{
+    const unsigned int fm = __ballot_sync(0xffffffffu, cell != HZ_VS_NO_CELL);
+    if(cell != HZ_VS_NO_CELL)
+    {
+        const unsigned int peers = __match_any_sync(fm, cell);
+        const unsigned int v = __reduce_min_sync(peers, __float_as_uint(e));
+        if((threadIdx.x & 31) == (unsigned int)(__ffs(peers) - 1)) atomicMin(out + cell, v);
+    }
+}
+
 // One thread per ray, gridDim.y = view.  The 4N-4 rays go to warps side by side: bottom row, top row, left column,
 // right column (without the corners), each side padded to whole warps, so that a warp holds 32 adjacent rays.  A
 // warp's rays run for a common number of steps (each lane's own count masks the rest): a side's rays that step
 // along the same axis all end on the same column or row, and the collective hand-on of mask bits needs every lane.
-__global__ void __launch_bounds__(HZ_VS_WARPS * 32)
-k_viewshed(const __grid_constant__ HzViewshed p)
+// HEIGHTS = false: the mask (k_viewshed); true: the heights (k_viewshed_heights), the same walk with the height
+// e = smax * D - A of each step in place of the test q >= smax, q = (A + target_height) / D.
+template<bool HEIGHTS> __device__ __forceinline__ void hz_vs_walk(const HzViewshed& p)
 {
     const int N = p.N;
     const HzViewshedEye E = p.eye[blockIdx.y];
-    uint32_t* const mask = p.masks + (size_t)blockIdx.y * N * p.w32;
+    uint32_t* const mask = HEIGHTS ? nullptr : p.masks + (size_t)blockIdx.y * N * p.w32;
+    uint32_t* const hts = HEIGHTS ? p.heights + (size_t)blockIdx.y * p.heights_stride : nullptr;
     if(blockIdx.x == 0 && threadIdx.x < 4)
     {
         // the four vertices around the eye
         const int i = (int)floorf(E.vci) + (int)(threadIdx.x & 1), j = (int)floorf(E.vcj) + (int)(threadIdx.x >> 1);
-        atomicOr(mask + (size_t)j * p.w32 + (i >> 5), 1u << (i & 31));
+        if(HEIGHTS) atomicMin(hts + (size_t)j * N + i, 0u);
+        else atomicOr(mask + (size_t)j * p.w32 + (i >> 5), 1u << (i & 31));
     }
 
     const unsigned int lane = threadIdx.x & 31;
@@ -2566,6 +2587,8 @@ k_viewshed(const __grid_constant__ HzViewshed p)
         {
             uint32_t* word = nullptr;
             uint32_t bit = 0;
+            uint32_t cell = HZ_VS_NO_CELL;
+            float e = 0.f;
             if(k0 + u < nsteps)
             {
                 const int a = a0 + (k0 + u) * step;
@@ -2582,8 +2605,16 @@ k_viewshed(const __grid_constant__ HzViewshed p)
                 const float zr = r == b0 ? zlo[u] : zhi[u];
                 const float mr = hz_vs_metres((float)r, vb, dpc, sb);
                 const float d2r = __fadd_rn(__fmul_rn(ma, ma), __fmul_rn(mr, mr));
-                const float q = __fdiv_rn(__fadd_rn(__fsub_rn(__fsub_rn(zr, vz), __fmul_rn(curv, d2r)), th), __fsqrt_rn(d2r));
-                if(q >= smax)
+                if(HEIGHTS)
+                {
+                    // its apparent height A at distance D: e = smax * D - A; -inf (the first step), negatives, -0 and
+                    // NaN all become +0
+                    const float A = __fsub_rn(__fsub_rn(zr, vz), __fmul_rn(curv, d2r));
+                    const float h = __fsub_rn(__fmul_rn(smax, __fsqrt_rn(d2r)), A);
+                    e = h > 0.f ? h : 0.f;
+                    cell = xmaj ? (uint32_t)r * (uint32_t)N + (uint32_t)a : (uint32_t)a * (uint32_t)N + (uint32_t)r;
+                }
+                else if(__fdiv_rn(__fadd_rn(__fsub_rn(__fsub_rn(zr, vz), __fmul_rn(curv, d2r)), th), __fsqrt_rn(d2r)) >= smax)
                 {
                     const int i = xmaj ? a : r, j = xmaj ? r : a;
                     word = mask + (size_t)j * p.w32 + (i >> 5);
@@ -2591,17 +2622,42 @@ k_viewshed(const __grid_constant__ HzViewshed p)
                 }
                 smax = fmaxf(smax, s);
             }
-            hz_vs_collect(pend, pbits, word, bit, false, lane);
+            if(HEIGHTS) hz_vs_height_min(hts, cell, e);
+            else hz_vs_collect(pend, pbits, word, bit, false, lane);
         }
     }
-    hz_vs_collect(pend, pbits, nullptr, 0u, true, lane);
+    if(!HEIGHTS) hz_vs_collect(pend, pbits, nullptr, 0u, true, lane);
+}
+
+__global__ void __launch_bounds__(HZ_VS_WARPS * 32)
+k_viewshed(const __grid_constant__ HzViewshed p)
+{
+    hz_vs_walk<false>(p);
+}
+
+__global__ void __launch_bounds__(HZ_VS_WARPS * 32)
+k_viewshed_heights(const __grid_constant__ HzViewshed p)
+{
+    hz_vs_walk<true>(p);
+}
+
+static dim3 hz_vs_grid(int N, int nviews)
+{
+    const int warps = 2 * ((N + 31) / 32) + 2 * ((N - 2 + 31) / 32);
+    return dim3((unsigned)((warps + HZ_VS_WARPS - 1) / HZ_VS_WARPS), (unsigned)nviews);
 }
 
 cudaError_t hz_launch_viewshed(const HzViewshed& p, int nviews, cudaStream_t stream)
 {
     if(nviews <= 0) return cudaSuccess;
-    const int warps = 2 * ((p.N + 31) / 32) + 2 * ((p.N - 2 + 31) / 32);
-    k_viewshed<<<dim3((unsigned)((warps + HZ_VS_WARPS - 1) / HZ_VS_WARPS), (unsigned)nviews), HZ_VS_WARPS * 32, 0, stream>>>(p);
+    k_viewshed<<<hz_vs_grid(p.N, nviews), HZ_VS_WARPS * 32, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t hz_launch_viewshed_heights(const HzViewshed& p, int nviews, cudaStream_t stream)
+{
+    if(nviews <= 0) return cudaSuccess;
+    k_viewshed_heights<<<hz_vs_grid(p.N, nviews), HZ_VS_WARPS * 32, 0, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -2623,6 +2679,40 @@ cudaError_t hz_launch_viewshed_count(const uint32_t* masks, int nviews, int N, i
 {
     if(nviews <= 0) return cudaSuccess;
     k_viewshed_count<<<dim3((unsigned)((N + 255) / 256), (unsigned)N), 256, 0, stream>>>(masks, nviews, N, w32, counts);
+    return cudaGetLastError();
+}
+
+// least[c] = min(least[c], the nviews heights of cell c): one thread per cell, plain loads, minimum on the patterns
+__global__ void __launch_bounds__(256)
+k_viewshed_least(const uint32_t* __restrict__ heights, int nviews, size_t cells, uint32_t* __restrict__ least)
+{
+    const size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if(c >= cells) return;
+    uint32_t m = least[c];
+    for(int v = 0; v < nviews; v++) m = min(m, __ldg(heights + (size_t)v * cells + c));
+    least[c] = m;
+}
+
+cudaError_t hz_launch_viewshed_least(const uint32_t* heights, int nviews, size_t cells, uint32_t* least,
+                                     cudaStream_t stream)
+{
+    if(nviews <= 0 || cells == 0) return cudaSuccess;
+    k_viewshed_least<<<(unsigned)((cells + 255) / 256), 256, 0, stream>>>(heights, nviews, cells, least);
+    return cudaGetLastError();
+}
+
+// out[0 .. n) = value (a byte memset cannot write +inf)
+__global__ void __launch_bounds__(256) k_fill_u32(uint32_t* __restrict__ out, size_t n, uint32_t value)
+{
+    for(size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (size_t)gridDim.x * blockDim.x)
+        out[k] = value;
+}
+
+cudaError_t hz_launch_fill_u32(uint32_t* out, size_t n, uint32_t value, cudaStream_t stream)
+{
+    if(n == 0) return cudaSuccess;
+    const size_t blocks = (n + 255) / 256;
+    k_fill_u32<<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, stream>>>(out, n, value);
     return cudaGetLastError();
 }
 

@@ -7,7 +7,8 @@ collective on the data path of a render:
 * viewpoint batch -- every viewpoint is an independent render against the same read-only DEM square, which each
   rank loads for itself.  Viewpoints are block-partitioned; outputs stay sharded on the rank that made them.
   Only reduced products (horizon profiles, a few bytes per image column) are gathered.  Viewsheds partition the same
-  way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded).  Labels of
+  way; their per-vertex counts are summed over the ranks with one all_reduce (viewshed_counts_sharded), and their
+  least heights folded with one minimum (viewshed_least_height_sharded).  Labels of
   points of interest too: 16 bytes per (view, POI) are gathered (annotate_sharded), and the scores of an observed
   skyline, 4 bytes per (view, heading column) (skyline_match_sharded), and the ground points of pixels, 32 bytes
   per (view, pixel) (pick_sharded).
@@ -317,6 +318,34 @@ def viewshed_counts_sharded(h, views, group=None, root=None, target_height=0.):
         h.viewshed_device(views[lo:hi], d_counts=counts.data_ptr(), target_height=target_height,
                           stream=torch.cuda.current_stream().cuda_stream)
     return reduce_counts(counts, group, root)
+
+
+def reduce_least(least, group=None, root=None):
+    """The elementwise minimum of every rank's (N, N) least viewshed heights: on every rank with root=None
+    (all_reduce), else only on rank `root` (reduce; the other ranks' tensors then hold partial minima).  In place;
+    returns `least`."""
+    world, _ = _world(group)
+    if world > 1:
+        if root is None:
+            dist.all_reduce(least, op=dist.ReduceOp.MIN, group=group)
+        else:
+            dist.reduce(least, dst=root, op=dist.ReduceOp.MIN, group=group)
+    return least
+
+
+def viewshed_least_height_sharded(h, views, group=None, root=None):
+    """Block-partitions `views` over the ranks, folds this rank's viewshed heights into least on its own GPU
+    (horizonator_viewshed_heights_device) and takes the minimum over the ranks with one collective (see reduce_least).
+    Returns the (N, N) float32 CUDA tensor: for every vertex of the loaded square, the least height above the ground
+    at which any of the views sees it (+inf where none does).  All ranks must hold contexts of the same DEM square."""
+    world, rank = _world(group)
+    lo, hi = block_partition(len(views), world, rank)
+    N = h.size
+    least = torch.full((N, N), float("inf"), dtype=torch.float32,
+                       device=torch.device("cuda", torch.cuda.current_device()))
+    if hi > lo:
+        h.viewshed_heights_device(views[lo:hi], d_least=least.data_ptr(), stream=torch.cuda.current_stream().cuda_stream)
+    return reduce_least(least, group, root)
 
 
 def render_batch_sharded(h, views, group=None, gather_profiles=True):

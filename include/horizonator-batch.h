@@ -193,6 +193,43 @@ bool horizonator_viewshed_device(const horizonator_context_t* ctx, int n, const 
 bool horizonator_viewshed(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
                           float target_height_m, uint32_t* masks, uint32_t* counts);
 
+/* Viewshed heights ("above ground level"): for each of n views and each vertex of the loaded square, how far above the
+ * ground a point at the vertex must rise for the view to see it; and for every vertex the least of that over the views
+ * (how high one may build there and stay hidden from every view).
+ *
+ * Definition: the views, eye, domain, rays, metres and curvature of the viewshed above (az_deg0 / az_deg1 ignored; no
+ * target height).  For a step of a ray that decides vertex v = (i, rint(b)):
+ *   - A = (zr - viewer_z) - curvature * d2r and D = sqrt(d2r): the vertex's apparent height and horizontal distance,
+ *     exactly the terms the mask's test is built from before target_height_m is added (q = (A + t) / D);
+ *   - smax = the largest s of the ray's EARLIER steps (-inf at the first step), as for the mask;
+ *   - the step's height e = smax * D - A in fp32, each operation rounded once in that order, then e > 0 ? e : +0
+ *     (so -inf, negatives and -0 all become +0).
+ *   heights[v] = the least e over all steps of all rays that decide v; the four vertices around the eye are +0; a
+ *   vertex that no step decides is +inf.  Every value is >= +0 or +inf and never NaN, so the minimum is taken exactly
+ *   and in any order on the 32-bit patterns (hz_kernels.cu: k_viewshed_heights, the mask's own walk;
+ *   oracle/viewshed_heights_oracle.c: vs_oracle_r2_heights; the GPU and the oracle agree bit for bit).
+ * Relation to the mask: mathematically heights[v] <= t <=> the viewshed at target_height_m = t sees v.  In fp32 the two
+ * can differ where t is within rounding of the step's terms (e compares smax * D - A with t, the mask (A + t) / D with
+ * smax).  Exactly: isfinite(heights[v]) equals the mask at t = 1e30 (there every decided vertex passes).
+ *
+ * heights: n x N x N float ([view][j][i]), overwritten;
+ * least:   N x N float, least[c] = min(least[c], heights of every view of the call), on the 32-bit patterns (the float
+ *          order for values >= +0 and +inf): the caller fills it with +inf once; several calls and several ranks can
+ *          fold into one buffer;
+ * either may be NULL, not both.  Arguments as for the viewshed: n = 0 does nothing and returns true; n < 0, NULL views,
+ * both outputs NULL, an eye outside [0, N-1)^2 or N * N >= 2^32 - 1 return false and write nothing.
+ * Sizes: one view's heights are 549 MB at N = 11716 (C2, 150 km of SRTM1), 23 MB at N = 2400 (SRTM3, R = 1200):
+ * per-view heights are meant for a few views or small squares; least is the output that scales.  The device call
+ * writes per-view heights in place and needs no scratch; without them the walk folds straight into least. */
+bool horizonator_viewshed_heights_device(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                         float* d_heights, float* d_least, void* stream);
+
+/* Same, into HOST memory, synchronous; least is min-folded into the caller's array.  Uses a device copy of least
+ * (N x N, allocated on first use) and, for per-view heights, a scratch of at most 64 views and at most 2 GiB (3 views
+ * per launch at N = 11716), allocated on first use. */
+bool horizonator_viewshed_heights(const horizonator_context_t* ctx, int n, const horizonator_view_t* views,
+                                  float* heights, float* least);
+
 /* Labels of points of interest (POIs): for each of n views and each of m POIs, whether the view sees the POI and where
  * its marker goes -- the rule of the reference's annotator (annotator.c:280-348), which the command-line tool's
  * --labels output follows (cli/horizonator-standalone.c, write_labels()), evaluated on the GPU for whole batches.

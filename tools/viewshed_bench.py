@@ -1,13 +1,17 @@
 #!/usr/bin/env python
 """viewshed_bench.py -- viewsheds/s of horizonator_viewshed_device() on one B200, one JSON line.
 
-    python tools/viewshed_bench.py [--out profiles/<name>.json] [--min-seconds S]
+    python tools/viewshed_bench.py [--out profiles/<name>.json] [--min-seconds S] [--heights]
 
 Workload: the C2 DEM of bench.py (synthetic SRTM1 4x4 tiles, 150 km radius: N = 11716, 46 860 rays per view) with
 outputs left in HBM:
   bench_b<B>   B = 1, 16, 64, 256 copies of the bench viewpoint per call, masks into device memory (B x 17.2 MB)
   bench_b256_counts  the same 256 views, counts only (the masks go through the chunk scratch)
   c5_grid      BASELINE configs[4]: bench.py's 64x64 grid of distinct viewpoints, 4096 views per call, counts only
+with --heights also (horizonator_viewshed_heights_device), in the same JSON line:
+  heights_bench_b<B>  B = 1, 16 copies of the bench viewpoint, per-view heights into device memory (B x 549 MB)
+  least_bench_b256    256 copies of the bench viewpoint, the least heights only (the walk's atomics go into it)
+  least_c5_grid       the 4096 C5 viewpoints, the least heights only
 Each is timed with CUDA events around whole calls on one stream after one warm-up call, repeated until at least
 --min-seconds have passed.  Ray steps per second come from the steps the definition takes (counted on the host from
 the eyes: per ray |target - first column or row beyond the eye| + 1), not from a profiler.  The device name and power
@@ -82,6 +86,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None, help="also append the JSON line to this file")
     ap.add_argument("--min-seconds", type=float, default=2.0)
+    ap.add_argument("--heights", action="store_true", help="also time the viewshed heights calls")
     args = ap.parse_args()
 
     import torch
@@ -120,6 +125,25 @@ def main():
         grid = [(la, lo) for la, lo in bench.c5_grid(1, 0)]
         ms, reps = timed(lambda: h.viewshed_device(grid, d_counts=counts.data_ptr(), stream=s), stream, args.min_seconds)
         record("c5_grid", grid, ms, reps, "counts in HBM")
+        if args.heights:
+            least = torch.empty((N, N), dtype=torch.float32, device="cuda")
+            heights = torch.empty((16, N, N), dtype=torch.float32, device="cuda")
+            for B in (1, 16):
+                views = one * B
+                ms, reps = timed(lambda: h.viewshed_heights_device(views, d_heights=heights.data_ptr(), stream=s),
+                                 stream, args.min_seconds)
+                record("heights_bench_b%d" % B, views, ms, reps, "per-view heights in HBM")
+            del heights
+            # each call folds into least filled with +inf (the fill, 0.1 ms, is inside the timed window), as a
+            # caller's first call does
+            def fold(views):
+                least.fill_(float("inf"))
+                h.viewshed_heights_device(views, d_least=least.data_ptr(), stream=s)
+            views = one * 256
+            ms, reps = timed(lambda: fold(views), stream, args.min_seconds)
+            record("least_bench_b256", views, ms, reps, "least heights in HBM")
+            ms, reps = timed(lambda: fold(grid), stream, args.min_seconds)
+            record("least_c5_grid", grid, ms, reps, "least heights in HBM")
     torch.cuda.synchronize()
 
     line = {"what": "viewsheds/s of horizonator_viewshed_device(), C2 DEM (synthetic SRTM1, 150 km radius, N=%d, "
